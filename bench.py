@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- grid-cell-days/s of the NESOSIM daily snow-budget hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): 100 km Arctic grid (90x90), one Aug 15 - May 1 season (260 days -> 259
@@ -371,6 +371,8 @@ def run_ours(args):
             pass
 
     stamp("headline timed (%d steps)" % args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, mask, args.dump_outputs)
     # end to end through the host-buffer C-ABI call
     e2e = None
     try:
@@ -492,6 +494,50 @@ def run_ours(args):
     if failures:
         sys.stderr.write("bench.py: FAILED checks: %s\n" % "; ".join(failures))
         sys.exit(3)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 18          # member-day-cells kept per array when the full outputs exceed DUMP_LIMIT_BYTES
+
+
+def dump_outputs(out, mask, directory):
+    """Write the device-resident season of the timed path (rank 0's members) under <directory>.
+
+    NaN and +-inf are outputs of the model (land cells, density below minSnowD, days of NaN forcing), but the files stay
+    finite so that two builds can be compared with a tolerance: <name>.npy (float64) holds 0 where the output is not
+    finite, and <name>_nonfinite.npy (float32, same shape) says what is there: 0 finite, 1 NaN, 2 +inf, 3 -inf.
+    Up to DUMP_LIMIT_BYTES the arrays are written whole.  Above it every array keeps the same DUMP_SAMPLE
+    member-day-cells of the ocean (1 <= mask <= 10, the cells the model computes): sorted flat indices into
+    (members * days, ocean cells in row-major order) drawn by np.random.default_rng(SEED).choice without replacement,
+    so the sample depends only on the shape and the mask; snowDepths keeps both layers, shape (DUMP_SAMPLE, 2)."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    M, T, ny, nx = out["density"].shape
+    plane = ny * nx
+    total = sum(t.numel() for t in out.values()) * (8 + 4)
+    mt = cell = None
+    if total > DUMP_LIMIT_BYTES:
+        ocean = np.flatnonzero((np.asarray(mask) >= 1) & (np.asarray(mask) <= 10))
+        pick = np.sort(np.random.default_rng(SEED).choice(M * T * len(ocean), size=DUMP_SAMPLE, replace=False))
+        dev = out["density"].device
+        mt = torch.from_numpy(pick // len(ocean)).to(dev)
+        cell = torch.from_numpy(ocean[pick % len(ocean)]).to(dev)
+    for name, t in out.items():
+        if mt is None:
+            a = t
+        elif name == "snowDepths":
+            a = t.view(M * T, 2, plane)[mt, :, cell]
+        else:
+            a = t.view(M * T, plane)[mt, cell]
+        a = a.cpu().numpy()
+        code = np.zeros(a.shape, dtype=np.float32)
+        code[np.isnan(a)] = 1
+        code[np.isposinf(a)] = 2
+        code[np.isneginf(a)] = 3
+        np.save(os.path.join(directory, name + ".npy"), np.where(code == 0, a, 0.0))
+        np.save(os.path.join(directory, name + "_nonfinite.npy"), code)
+    stamp("outputs of the last timed step written to %s (%s)" % (directory, "whole" if mt is None else
+                                                                 "%d sampled member-day-cells" % DUMP_SAMPLE))
 
 
 def host_drain_settings(world, cores):
@@ -1062,7 +1108,15 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the host-buffer leg")
     ap.add_argument("--no-other", action="store_true", help="skip the 25 km / 5 km general-path figures")
     ap.add_argument("--no-extra", action="store_true", help="skip the multi-season, 5 km strips and drop-in main legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the arrays of the last one as DIR/<name>.npy, non-finite "
+                         "values as 0 and flagged in DIR/<name>_nonfinite.npy (a fixed sample when they exceed 64 MiB; "
+                         "see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,7 +1,7 @@
-"""The drop-in host module ``nesosim_b200/NESOSIM.py``: forcing reader / season stager against the reference's own
-``loadData`` (CPU, only where /root/reference exists), the stager's self-contained semantics (CPU, anywhere) and
-``main`` / ``calcBudget`` end to end on the GPU with the reference's out-of-scope helpers (grid, mask, NetCDF
-writers, plots) replaced by recording fakes."""
+"""The drop-in host module ``nesosim_b200/NESOSIM.py``: forcing reader / season stager against what the reference's own
+``loadData`` returned on the same files (CPU, stored in ``tests/golden/reference_contracts.npz``), the stager's
+self-contained semantics (CPU) and ``main`` / ``calcBudget`` end to end on the GPU with the reference's out-of-scope
+helpers (grid, mask, NetCDF writers, plots) replaced by recording fakes."""
 import datetime
 import os
 import sys
@@ -11,10 +11,10 @@ import numpy as np
 import numpy.ma as ma
 import pytest
 
+import golden_util
 from nesosim_b200 import NESOSIM as N
 from nesosim_b200 import synthetic as S
 from oracle import nesosim_oracle as O
-from oracle import ref_loader
 
 NY, NX = 12, 10
 DXSTR = "100km"
@@ -121,41 +121,61 @@ def test_stage_season_year_wrap_scaling_and_last_slot(tmp_path, quiet):
     assert same(st["precip"][3], made[(2019, 0)][1] * sf[11])
 
 
-# ------------------------------------------------------------------------------------------ CPU, reference present
+# ------------------------------------------------------------------------------------------ CPU, against the reference
+# The reference's own functions, run verbatim on the inputs below (oracle/ref_loader.py), returned the arrays stored in
+# tests/golden/reference_contracts.npz (tests/golden/make_reference_contracts.py says how they were recorded).
 
-needs_ref = pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
+CONTRACTS = "reference_contracts.npz"
+LOAD_DATA_DAYS = (10, 11, 12, 365)
+LOAD_DATA_NAMES = ("conc", "precip", "drift", "wind", "temp")
+HELPER_YEARS = (2018, 2019, 2020)
+HELPER_DAYS = (0, 1, 30, 31, 58, 59, 60, 243, 334, 364, 365)
 
 
-@needs_ref
-def test_load_data_matches_reference(tmp_path, quiet, capsys):
-    ref = ref_loader.load_reference()
+def load_data_tree(root):
+    """The forcing tree the reader is compared on: masked drift, a temperature file, a missing drift file, and the
+    day-365 snowfall fallback, which the reference looks up under Precip/<var>/sf/<year>/ (NESOSIM.py:395)."""
     days = [(2018, d) for d in (10, 11, 12, 364)]
-    root, _ = write_forcing_tree(str(tmp_path), days, seed=2, with_temp_days=[(2018, 11)], skip_drift_days=[(2018, 12)],
+    root, _ = write_forcing_tree(root, days, seed=2, with_temp_days=[(2018, 11)], skip_drift_days=[(2018, 12)],
                                  masked_drift_days=[(2018, 10)])
-    # the reference's day-365 snowfall fallback looks under Precip/<var>/sf/<year>/ (NESOSIM.py:395)
     src = os.path.join(root, "Precip/ERA5/2018", "ERA5sf%s-2018_d364%s" % (DXSTR, EXTRA))
     os.makedirs(os.path.join(root, "Precip/ERA5/sf/2018"))
     np.load(src, allow_pickle=True).dump(os.path.join(root, "Precip/ERA5/sf/2018", os.path.basename(src)))
-    ref.forcingPath = root
+    return root
+
+
+def load_data_outputs(root):
     N.forcingPath = root
-    for day in (10, 11, 12, 365):
+    out = {}
+    for day in LOAD_DATA_DAYS:
         got = N.loadData(2018, day, "ERA5", "ERA5", "CDR", "OSISAF", DXSTR, EXTRA)
-        exp = ref.loadData(2018, day, "ERA5", "ERA5", "CDR", "OSISAF", DXSTR, EXTRA)
-        for g, e, name in zip(got, exp, ("conc", "precip", "drift", "wind", "temp")):
-            assert same(g, e), "%s day %d" % (name, day)
+        for g, name in zip(got, LOAD_DATA_NAMES):
+            out["load_data__%s__%d" % (name, day)] = np.asarray(g)
+    return out
+
+
+def helper_outputs():
+    out = {"helpers__doyToMonth": np.array([[N.doyToMonth(day, year) for day in HELPER_DAYS] for year in HELPER_YEARS]),
+           "helpers__applyScaling": N.applyScaling(np.arange(6.).reshape(2, 3), 1.5)}
+    for i, a in enumerate(N.genEmptyArrays(4, 3, 2)):
+        out["helpers__genEmptyArrays__%d" % i] = a
+    return out
+
+
+def test_load_data_matches_reference(tmp_path, quiet, capsys):
+    exp = golden_util.load(CONTRACTS)
+    got = load_data_outputs(load_data_tree(str(tmp_path)))
+    assert len(got) == len(LOAD_DATA_DAYS) * len(LOAD_DATA_NAMES)
+    for key, g in got.items():
+        assert same(g, exp[key]), key
     capsys.readouterr()
 
 
-@needs_ref
 def test_helpers_match_reference():
-    ref = ref_loader.load_reference()
-    for year in (2018, 2019, 2020):
-        for day in (0, 1, 30, 31, 58, 59, 60, 243, 334, 364, 365):
-            assert N.doyToMonth(day, year) == ref.doyToMonth(day, year)
-    a = np.arange(6.).reshape(2, 3)
-    assert same(N.applyScaling(a, 1.5), ref.applyScaling(a, 1.5))
-    for g, e in zip(N.genEmptyArrays(4, 3, 2), ref.genEmptyArrays(4, 3, 2)):
-        assert same(g, e)
+    exp = golden_util.load(CONTRACTS)
+    for key, g in helper_outputs().items():
+        assert same(g, exp[key]), key
+        assert np.asarray(g).dtype == exp[key].dtype, key
 
 
 # ------------------------------------------------------------------------------------------ GPU
@@ -277,20 +297,15 @@ def test_calc_budget_shim_has_the_reference_in_place_contract(cuda, quiet):
     assert np.isnan(tempDays[:T - 1]).all()
 
 
-@needs_ref
-def test_drift_regridders_match_reference():
-    """SURVEY 8f N4: `drift_smoothing.int_smooth_drifts_v2/v3` against the reference's own functions run verbatim
-    (utils.py:259-338; astropy's pair replaced by the restatement on both sides): scattered source points with NaN
-    drift, a model grid reaching outside their hull (NaN after interpolation -> the NaN-interpolating branch of the
-    convolution and the final mask), both kernel widths the reference uses."""
-    import sys
+def drift_regridder_outputs():
+    """`drift_smoothing.int_smooth_drifts_v2/v3` (SURVEY 8f N4; utils.py:259-338 in the reference) on scattered source
+    points with NaN drift and a model grid reaching outside their hull (NaN after interpolation -> the NaN-interpolating
+    branch of the convolution and the final mask), both kernel widths the reference uses; astropy's pair is the
+    restatement (oracle/astropy_restated.py), as it was for the reference.  Masked results as (filled with -9, mask)."""
     import numpy.ma as ma
     from scipy.spatial import Delaunay
     from nesosim_b200 import drift_smoothing as D
     from oracle import astropy_restated as ar
-    ref_loader.load_reference()
-    ref_utils = sys.modules["utils"]
-    assert ref_utils.__file__.startswith(ref_loader.REFERENCE_SOURCE)
 
     def cpu_smoother(gx, gy, sigma_factor=1, x_size_val=3):
         k = ar.gaussian2d_kernel(x_stddev=sigma_factor, y_stddev=sigma_factor, theta=0.0, x_size=x_size_val, y_size=x_size_val)
@@ -310,14 +325,25 @@ def test_drift_regridders_match_reference():
     gj, gi = np.meshgrid(np.linspace(-5.0, 118.0, 24), np.linspace(-3.0, 112.0, 20))
     xG, yG = gi, gj
     tri = Delaunay(np.column_stack([xF.ravel(), yF.ravel()]))
+    out = {}
     for sigma in (0.5, 1):
         for name, args in (("int_smooth_drifts_v2", ()), ("int_smooth_drifts_v3", (tri,))):
             got = getattr(D, name)(*args, xG, yG, xF, yF, latsF, drift, sigma_factor=sigma, smoother=cpu_smoother)
-            exp = getattr(ref_utils, name)(*args, xG, yG, xF, yF, latsF, drift, sigma_factor=sigma)
-            assert got.shape == exp.shape == (2, 20, 24)
-            assert np.array_equal(ma.getmaskarray(got), ma.getmaskarray(exp)), (name, sigma)
-            assert ma.getmaskarray(exp).any() and not ma.getmaskarray(exp).all()
-            assert np.array_equal(got.filled(-9.0), exp.filled(-9.0)), (name, sigma)
+            key = "drift__%s__%s" % (name, sigma)
+            out[key + "__filled"] = got.filled(-9.0)
+            out[key + "__mask"] = ma.getmaskarray(got)
+    return out
+
+
+def test_drift_regridders_match_reference():
+    exp = golden_util.load(CONTRACTS)
+    got = drift_regridder_outputs()
+    assert len(got) == 8
+    for key, g in got.items():
+        assert g.shape == exp[key].shape == (2, 20, 24), key
+        assert np.array_equal(g, exp[key]), key
+        if key.endswith("__mask"):
+            assert exp[key].any() and not exp[key].all()
 
 
 class _StandInOps:
@@ -373,21 +399,17 @@ class _StandInOps:
         return ar.convolve_fill0(np.asarray(arr, dtype=np.float64), k, variant=conv_variant)
 
 
-@needs_ref
-def test_per_function_operators_have_the_reference_contracts(monkeypatch):
-    """`calcLeadLoss`, `calcAtmLoss`, `calcWindPacking`, `fillMaskAndNaNWithZero`, `fill_nan_no_negative`, `smooth_snow`,
-    `calcDynamics`, `densityCalc` of the drop-in module against the reference's own functions run verbatim
-    (NESOSIM.py:51-222, 458-473): same arguments, same return values or in-place effect, the module globals as the
-    parameters.  The arithmetic is the stand-in's here; what is tested is everything around it."""
-    import inspect
-    from nesosim_b200 import engine as E
-    for name in ("op_wind_terms", "op_dynamics", "op_fill_zero", "op_fill_nan_no_negative", "op_density", "smooth"):
-        assert inspect.signature(getattr(_StandInOps, name)) == inspect.signature(getattr(E, name)), name
+def use_stand_in_ops(monkeypatch):
+    """The drop-in module on the oracle-backed stand-in operators, its module globals set as ``main`` sets them."""
     monkeypatch.setattr(N, "_ops", lambda: _StandInOps)
-    ref = ref_loader.load_reference()
-    ref_loader.set_globals(ref, 5.8e-7, 5., 2.9e-7, 2.2e-8)
     for k, v in dict(windPackFactor=5.8e-7, windPackThresh=5., leadLossFactor=2.9e-7, atmLossFactor=2.2e-8).items():
         monkeypatch.setattr(N, k, v)
+
+
+def operator_outputs():
+    """`calcLeadLoss`, `calcAtmLoss`, `calcWindPacking`, `calcDynamics`, `densityCalc`, `smooth_snow`,
+    `fill_nan_no_negative`, `fillMaskAndNaNWithZero` of the drop-in module on seeded inputs: return values, or the
+    argument after the in-place call (those return None, as the reference's do)."""
     rng = np.random.default_rng(5)
     ny, nx = 9, 11
     mask = rng.choice(np.array([0, 3, 8, 8, 8, 11, 12]), size=(ny, nx)).astype(float)
@@ -401,33 +423,48 @@ def test_per_function_operators_have_the_reference_contracts(monkeypatch):
     C = np.clip(rng.random((ny, nx)), 0, 1)
     drift = 0.1 * rng.normal(size=(2, ny, nx))
     drift[:, 4:6, 4:7] = np.nan
+    out = {}
     with np.errstate(all="ignore"):
-        assert same(N.calcLeadLoss(h[0], W, C), ref.calcLeadLoss(h[0], W, C))
-        assert same(N.calcAtmLoss(h[0], W), ref.calcAtmLoss(h[0], W))
-        for g, e in zip(N.calcWindPacking(W, h[0]), ref.calcWindPacking(W, h[0])):
-            assert same(g, e)
-        for g, e in zip(N.calcDynamics(drift, h, 100000), ref.calcDynamics(drift, h, 100000)):
-            assert g.shape == (2, ny, nx) and same(g, e)
-        assert same(N.densityCalc(h, C, mask), ref.densityCalc(h, C, mask))
-        clean = np.nan_to_num(h[0], nan=0.0)
-        assert same(N.smooth_snow(clean), ref.smooth_snow(clean))
-        holes = h[0].copy()
-        assert same(N.smooth_snow(holes, stddev_val=0.5), ref.smooth_snow(holes, stddev_val=0.5))
-        with pytest.raises(ValueError):
-            N.smooth_snow(clean, x_size_val=5)
+        out["ops__calcLeadLoss"] = N.calcLeadLoss(h[0], W, C)
+        out["ops__calcAtmLoss"] = N.calcAtmLoss(h[0], W)
+        for i, g in enumerate(N.calcWindPacking(W, h[0])):
+            out["ops__calcWindPacking__%d" % i] = g
+        for i, g in enumerate(N.calcDynamics(drift, h, 100000)):
+            assert g.shape == (2, ny, nx)
+            out["ops__calcDynamics__%d" % i] = g
+        out["ops__densityCalc"] = N.densityCalc(h, C, mask)
+        out["ops__smooth_snow__clean"] = N.smooth_snow(np.nan_to_num(h[0], nan=0.0))
+        out["ops__smooth_snow__holes"] = N.smooth_snow(h[0].copy(), stddev_val=0.5)
         for negz in (True, False):
             a = rng.normal(size=(ny, nx))
             a[3, 3] = np.inf
             a[4, 4] = np.nan
-            b = a.copy()
             assert N.fill_nan_no_negative(a, mask, negative_to_zero=negz) is None
-            ref.fill_nan_no_negative(b, mask, negative_to_zero=negz)
-            assert same(a, b)
+            out["ops__fill_nan_no_negative__%s" % negz] = a
         a = rng.normal(size=(ny, nx))
         a[1, 2], a[2, 1], a[0, 0] = np.nan, np.inf, -np.inf
-        b = a.copy()
         assert N.fillMaskAndNaNWithZero(a) is None
-        ref.fillMaskAndNaNWithZero(b)
-        assert same(a, b) and np.isfinite(a).all()
-        with pytest.raises(TypeError):
-            N.fillMaskAndNaNWithZero(np.ma.masked_invalid(b))
+        out["ops__fillMaskAndNaNWithZero"] = a
+    return out
+
+
+def test_per_function_operators_have_the_reference_contracts(monkeypatch):
+    """The eight functions calcBudget is made of (NESOSIM.py:51-222, 458-473 in the reference) against what the
+    reference's own functions returned on the same arguments: same return values or in-place effect, the module
+    globals as the parameters.  The arithmetic is the stand-in's here; what is tested is everything around it."""
+    import inspect
+    from nesosim_b200 import engine as E
+    for name in ("op_wind_terms", "op_dynamics", "op_fill_zero", "op_fill_nan_no_negative", "op_density", "smooth"):
+        assert inspect.signature(getattr(_StandInOps, name)) == inspect.signature(getattr(E, name)), name
+    use_stand_in_ops(monkeypatch)
+    exp = golden_util.load(CONTRACTS)
+    got = operator_outputs()
+    assert len(got) == 13
+    for key, g in got.items():
+        assert same(g, exp[key]), key
+    assert np.isfinite(got["ops__fillMaskAndNaNWithZero"]).all()
+    clean = np.zeros((9, 11))
+    with pytest.raises(ValueError):
+        N.smooth_snow(clean, x_size_val=5)
+    with pytest.raises(TypeError):
+        N.fillMaskAndNaNWithZero(np.ma.masked_invalid(got["ops__fillMaskAndNaNWithZero"]))
