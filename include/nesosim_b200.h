@@ -180,12 +180,26 @@ int nesosim_final_products(const double *depths_dev, const double *density_dev, 
  * model = (h0+h1)/iceConc at that slot and cell (what main writes as snow depth, NESOSIM.py:654) and
  * misfit_dev[m] = sum over the observations of (model - observed)^2, skipping non-finite differences (land, NaN forcing,
  * zero concentration); count_dev[m] (may be NULL) = the number of observations used.  Sums are formed in a fixed order
- * (bit-reproducible).  Needs the season-resident path (grid up to 96 columns, variable density, one shared forcing);
- * NESOSIM_ERR_ARG otherwise. */
+ * (bit-reproducible).  Needs the season-resident path (grid up to 96 columns, variable density, one shared forcing --
+ * or forcing sets with observations from nesosim_set_observations_sets, below); NESOSIM_ERR_ARG otherwise. */
 int nesosim_set_observations(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_day_host, const int32_t *obs_row_host,
                              const int32_t *obs_col_host, const double *obs_depth_host);
 int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
                               int ic_per_member, double *misfit_dev, int64_t *count_dev, void *stream);
+
+/* Multi-season calibration: observations tagged with the forcing set (season) they belong to; needs
+ * nesosim_set_forcing_sets first (NESOSIM_ERR_STATE otherwise).  obs_day must be < set_days[obs_set]; land/lake
+ * observations are skipped as in nesosim_set_observations; a set index outside [0, n_sets), a day outside its set's
+ * season or a cell outside the grid is NESOSIM_ERR_ARG.  Each set is compiled exactly as nesosim_set_observations
+ * compiles its season, and the next nesosim_run_season_misfit runs every member through its season in one batch and scores
+ * member m against the observations of set member_set[m] only: misfit_dev[m] and count_dev[m] equal, bit for bit, what
+ * that member's season gives on a single-forcing context with the same strips (NESOSIM_ENS_CLUSTER).  The observations
+ * remember the (n_sets, set_days) they were compiled against: once the forcing is registered again with another layout,
+ * or with nesosim_set_forcing, nesosim_run_season_misfit returns NESOSIM_ERR_STATE until observations are registered
+ * again.  Plain observations on a context with forcing sets stay NESOSIM_ERR_ARG at run time. */
+int nesosim_set_observations_sets(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host,
+                                  const int32_t *obs_day_host, const int32_t *obs_row_host,
+                                  const int32_t *obs_col_host, const double *obs_depth_host);
 
 /* Asynchronous mode.  By default nesosim_run_season on the season-resident path synchronises `stream` once to read
  * the kernel's operand-range flag (see above).  With nesosim_set_async(ctx, 1) it never synchronises: the flag is copied

@@ -88,6 +88,8 @@ _SIGNATURES = {
                                            C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
     "nesosim_run_season_misfit": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int, C.c_void_p,
                                             C.c_void_p, C.c_void_p]),
+    "nesosim_set_observations_sets": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                                C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

@@ -210,6 +210,12 @@ struct EnsArgs {
     int dbg;                           // timing experiments only (NESOSIM_ENS_DBG): 1 forcing always from day 0, 2 no L2 prefetch, 4 no bulk stores
     int *status;                       // set to 1 if any operand left the fast divisions' proven range (host reruns)
     long long *timing;                 // debug: [gridDim.x][ENS_NTIMER] phase cycle totals (NULL = off)
+    // misfit mode on forcing sets (nesosim_set_observations_sets): every set has its own obs_first table, obs_first_stride
+    // entries apart; the sets' slots follow one another in obs_day, set s from obs_slot_base[s] on.  A member samples its
+    // own set only, so its row of sample_depth holds that set's slots (from obs_slot_base[set]) and the stride is the
+    // slot count of the largest set, not the sum
+    long long obs_first_stride;
+    const int *obs_slot_base;
 };
 
 __device__ __forceinline__ void cluster_arrive_release() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
@@ -303,7 +309,7 @@ __device__ __forceinline__ void st_cluster(unsigned addr, double v) {
 // threads that push wait on it; (2) "my neighbours' halo cells of day x+1 have landed" -- the barrier counts the
 // bytes they deliver with st.async.  Cluster-wide barriers are used once per member only.
 // SETS: members may use different forcing sets / season lengths (compiled apart so that the plain ensemble keeps its
-// parameter-bank pointers and its uniform trip count)
+// parameter-bank pointers and its uniform trip count); SETS && OBS: misfit mode with per-set observation tables
 template <int NTC, int KR, int KO, bool TIMING, bool SETS, bool OBS = false>
 __global__ void __launch_bounds__(NTC + 32, 1) ensemble_season_kernel(const __grid_constant__ EnsArgs a) {
     constexpr int SXR = ENS_SXR;
@@ -405,7 +411,7 @@ __global__ void __launch_bounds__(NTC + 32, 1) ensemble_season_kernel(const __gr
     // ---- the ocean cells this thread owns for the whole season (entries tid + j*NTC): offset of the cell in an
     // own-cells plane, of its top-left 3x3 tap in the raw tiles, and its mirror in a neighbour's halo
     unsigned b_ci[KO], b_t[KO], b_rem[KO];
-    int o_first[OBS ? KO : 1];         // misfit mode: the cell's first observation
+    int o_first[OBS ? KO : 1];         // misfit mode: the cell's first observation (SETS: loaded per member, by its set)
 #pragma unroll
     for (int j = 0; j < KO; ++j) {
         const int idx = tid + j * NTC;
@@ -414,7 +420,7 @@ __global__ void __launch_bounds__(NTC + 32, 1) ensemble_season_kernel(const __gr
         b_rem[j] = 0;
         if (OBS) o_first[j] = -1;
         if (comp && idx < n_ocean) {
-            if (OBS) o_first[j] = a.obs_first[a.st.ocean_off[k] + idx];
+            if (OBS && !SETS) o_first[j] = a.obs_first[a.st.ocean_off[k] + idx];
             const unsigned code = a.st.codes[a.st.ocean_off[k] + idx];
             const int lr = (int)(code >> 7), c = (int)(code & 127u);
             b_t[j] = L.off_adv + (unsigned)(lr * SXR + c) * 16u;
@@ -573,7 +579,11 @@ __global__ void __launch_bounds__(NTC + 32, 1) ensemble_season_kernel(const __gr
         // goes to the member's sample array and the cursor moves on (the next slot's day is needed tomorrow at the
         // earliest: its load is never waited for)
         int o_idx[OBS ? KO : 1], o_day[OBS ? KO : 1];
-        double *const m_samples = OBS ? a.sample_depth + (long long)m * a.sample_stride : nullptr;
+        // (SETS: the set's tables hold the slots of all sets one after the other, the member's row of sample_depth only
+        // those of its own set: the row is addressed relative to the set's first slot)
+        double *const m_samples = !OBS ? nullptr
+                                  : SETS ? a.sample_depth + ((long long)m * a.sample_stride - a.obs_slot_base[fset])
+                                         : a.sample_depth + (long long)m * a.sample_stride;
         auto obs_take = [&](int j, int slot) {
             if (o_day[j] == slot) {
                 m_samples[o_idx[j]] = add(r_h0[j], r_h1[j]);      // snowDepths[:, 0] + snowDepths[:, 1]   (NESOSIM.py:654)
@@ -584,6 +594,10 @@ __global__ void __launch_bounds__(NTC + 32, 1) ensemble_season_kernel(const __gr
         if (OBS) {
 #pragma unroll
             for (int j = 0; j < KO; ++j) {
+                if (SETS)   // the cell's first slot in its member's set (own cells only: flags bit 8+j)
+                    o_first[j] = ((flags >> (8 + j)) & 1u)
+                                     ? __ldg(a.obs_first + fset * a.obs_first_stride + a.st.ocean_off[k] + tid + j * NTC)
+                                     : -1;
                 o_idx[j] = o_first[j];
                 o_day[j] = o_first[j] >= 0 ? __ldg(a.obs_day + o_idx[j]) : 0x7fffffff;
                 obs_take(j, 0);

@@ -192,6 +192,7 @@ struct nesosim_ctx {
     long long ens_kernel_launches = 0;   // ... and their number (bench.py: roofline of the dominant kernel)
     int n_sets = 1;                 // forcing sets (nesosim_set_forcing_sets); 1 = plain season
     int *member_set_dev = nullptr, *set_steps_dev = nullptr;
+    std::vector<int> set_days;      // days of every forcing set (empty: one shared forcing)
     int ens_status = 0;             // flag read back from the last season-resident launch (1 = rerun needed)
     struct {                        // observations of the calibration driver (nesosim_set_observations)
         bool ready = false;
@@ -201,6 +202,12 @@ struct nesosim_ctx {
         double *val = nullptr;                           // per observation: value, sample slot, day, cell
         int *o_slot = nullptr, *o_day = nullptr, *o_cell = nullptr;
         long long n_used = 0;
+        // nesosim_set_observations_sets: the tables of every set one after the other; set_days = the forcing layout they
+        // were compiled against (empty: plain observations of one shared forcing)
+        std::vector<int> set_days;
+        long long first_stride = 0;                      // entries of one set's `first` table
+        int *slot_base = nullptr;                        // [sets] the set's first slot in `day`
+        int *obs_begin = nullptr;                        // [sets+1] the set's observations
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -503,10 +510,12 @@ struct EnsVariant {
     void (*kernel_timing)(const EnsArgs);
     void (*kernel_sets)(const EnsArgs);    // members on different forcing sets (nesosim_set_forcing_sets)
     void (*kernel_obs)(const EnsArgs);     // misfit mode: observations reduced inside the kernel (nesosim_run_season_misfit)
+    void (*kernel_obs_sets)(const EnsArgs);   // misfit mode on forcing sets (nesosim_set_observations_sets)
 };
 #define ENS_V(ntc, kr, ko) \
     {"t" #ntc "r" #kr "o" #ko, ntc, kr, ko, ensemble_season_kernel<ntc, kr, ko, false, false>, ensemble_season_kernel<ntc, kr, ko, true, false>, \
-     ensemble_season_kernel<ntc, kr, ko, false, true>, ensemble_season_kernel<ntc, kr, ko, false, false, true>}
+     ensemble_season_kernel<ntc, kr, ko, false, true>, ensemble_season_kernel<ntc, kr, ko, false, false, true>, \
+     ensemble_season_kernel<ntc, kr, ko, false, true, true>}
 const EnsVariant *ens_variants(int *n) {
     static const EnsVariant v[] = {
         ENS_V(352, 3, 2), ENS_V(224, 4, 3), ENS_V(480, 2, 2), ENS_V(608, 2, 1), ENS_V(480, 2, 1), ENS_V(736, 2, 1), ENS_V(352, 6, 5),
@@ -758,6 +767,8 @@ struct ObsDevice {                      // misfit mode: device arrays of the sam
     const int *first = nullptr, *day = nullptr;
     double *sample_depth = nullptr;
     long long sample_stride = 0;
+    long long first_stride = 0;         // forcing sets: per-set tables
+    const int *slot_base = nullptr;
 };
 
 int run_ensemble(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, const nesosim_outputs *out, int m0,
@@ -795,7 +806,8 @@ int run_ensemble(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cons
     const EnsVariant *v = &ens_variants(&nv_)[e.variant];
     const int cl = e.tables.cluster;
     const bool dbg_timing = getenv("NESOSIM_ENS_TIMING") != nullptr;   // debug aid: per-phase cycle totals to stderr
-    void (*kernel)(const EnsArgs) = obs ? v->kernel_obs : ctx->member_set_dev ? v->kernel_sets : (dbg_timing ? v->kernel_timing : v->kernel);
+    void (*kernel)(const EnsArgs) = obs ? (ctx->member_set_dev ? v->kernel_obs_sets : v->kernel_obs)
+                                        : ctx->member_set_dev ? v->kernel_sets : (dbg_timing ? v->kernel_timing : v->kernel);
     CU(cudaFuncSetAttribute((const void *)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e.smem_bytes));
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute at[1];
@@ -834,6 +846,8 @@ int run_ensemble(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cons
     a.obs_day = obs ? obs->day : nullptr;
     a.sample_depth = obs ? obs->sample_depth : nullptr;
     a.sample_stride = obs ? obs->sample_stride : 0;
+    a.obs_first_stride = obs ? obs->first_stride : 0;
+    a.obs_slot_base = obs ? obs->slot_base : nullptr;
     a.dbg = getenv("NESOSIM_ENS_DBG") ? atoi(getenv("NESOSIM_ENS_DBG")) : 0;
     a.timing = nullptr;
     if (dbg_timing && !ctx->member_set_dev && !obs) {
@@ -1076,6 +1090,7 @@ int nesosim_destroy(nesosim_ctx *ctx) {
     if (ctx->flag_pool) cudaFreeHost(ctx->flag_pool);
     cudaFree(ctx->obs.first); cudaFree(ctx->obs.day); cudaFree(ctx->obs.val); cudaFree(ctx->obs.samples);
     cudaFree(ctx->obs.o_slot); cudaFree(ctx->obs.o_day); cudaFree(ctx->obs.o_cell);
+    cudaFree(ctx->obs.slot_base); cudaFree(ctx->obs.obs_begin);
     for (int i = 0; i < 2; ++i)
         if (ctx->ens_ev[i]) cudaEventDestroy(ctx->ens_ev[i]);
     strip_release(ctx);
@@ -1118,6 +1133,7 @@ int nesosim_set_forcing(nesosim_ctx *ctx, const double *precip_dev, const double
     }
     ctx->ens.derived_valid = false;
     ctx->n_sets = 1;
+    ctx->set_days.clear();
     cudaFree(ctx->member_set_dev);
     cudaFree(ctx->set_steps_dev);
     ctx->member_set_dev = ctx->set_steps_dev = nullptr;
@@ -1144,6 +1160,7 @@ int nesosim_set_forcing_sets(nesosim_ctx *ctx, int n_sets, const double *precip_
     CU(cudaMemcpy(ctx->member_set_dev, member_set_host, sizeof(int) * M, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(ctx->set_steps_dev, steps.data(), sizeof(int) * n_sets, cudaMemcpyHostToDevice));
     ctx->n_sets = n_sets;
+    ctx->set_days.assign(set_days_host, set_days_host + n_sets);
     return NESOSIM_OK;
 }
 
@@ -1164,27 +1181,40 @@ int nesosim_run_season(nesosim_ctx *ctx, const nesosim_member_params *params_hos
     return run_members(ctx, ic_dev, ic_per_member, out, 0, ctx->cfg.n_members, first_step, num_steps, st);
 }
 
+}  // extern "C"
+
 // Epilogue of the misfit mode: one CTA per member.  model = sampled depth / ice concentration of that day and cell
 // (what main writes as snow depth over ice, NESOSIM.py:654); squared differences to the observations are summed in a
 // fixed order (observation i belongs to thread i % 256, threads are combined by shuffles, warps one after the other).
+// SETS: member m is scored against the observations of its forcing set member_set[m], obs_begin[set] .. obs_begin[set+1]-1,
+// on that set's concentration stack; i counts from the set's first observation, so the member's sum is formed exactly
+// as for its season on its own.
 struct MisfitArgs {
     const double *sample_depth;     // [M][stride]
     long long stride;
     const int *obs_slot, *obs_day, *obs_cell;
     const double *obs_val;
-    const double *conc;             // [T][plane]
+    const double *conc;             // [T][plane] (SETS: [sets][T][plane])
     long long plane, n_obs;
     double *misfit;
     long long *count;
+    const int *member_set, *obs_begin;   // SETS only
+    long long conc_set_stride;           // SETS only: T * plane
 };
+template <bool SETS>
 __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constant__ MisfitArgs a) {
     const int m = blockIdx.x;
     const double *samp = a.sample_depth + (long long)m * a.stride;
+    const int set = SETS ? a.member_set[m] : 0;
+    const long long i0 = SETS ? (long long)a.obs_begin[set] : 0ll;
+    const long long n_obs = SETS ? (long long)a.obs_begin[set + 1] - i0 : a.n_obs;
+    const double *conc = SETS ? a.conc + (long long)set * a.conc_set_stride : a.conc;
     double acc = 0.0;
     long long cnt = 0;
-    for (long long i = threadIdx.x; i < a.n_obs; i += 256) {
-        const double C = __ldg(a.conc + (long long)a.obs_day[i] * a.plane + a.obs_cell[i]);
-        const double diff = sub(div_ieee(samp[a.obs_slot[i]], C), a.obs_val[i]);
+    for (long long i = threadIdx.x; i < n_obs; i += 256) {
+        const long long q = i0 + i;
+        const double C = __ldg(conc + (long long)a.obs_day[q] * a.plane + a.obs_cell[q]);
+        const double diff = sub(div_ieee(samp[a.obs_slot[q]], C), a.obs_val[q]);
         if (nesosim::finite(diff)) {
             acc = add(acc, mul(diff, diff));
             ++cnt;
@@ -1208,6 +1238,91 @@ __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constan
     }
 }
 
+// Observations compiled against the strip tables (host side).  One season's tables: every observation mapped to its
+// owner (strip, index in the strip's ocean list), sorted by owner and day; `first` has list_end+1 entries, sample
+// slots are the distinct (cell, day) pairs per owning cell in day order with one sentinel behind every cell's run.
+// Several seasons (forcing sets) are appended one after the other: a set's `first` entries and o_slot count from the
+// set's first slot, so each set's tables are exactly those its season would get on its own (the caller moves `first`
+// to absolute slots for the season kernel; o_slot stays the slot in the member's row of samples).
+struct ObsPoint { int owner, day, cell; double val; };
+struct ObsTables {
+    std::vector<int> first, slot_day, o_slot, o_day, o_cell;
+    std::vector<double> o_val;
+};
+
+// position of every ocean cell in the concatenated code lists (ocean_off[k] + idx), -1 on land; list_end = the lists' end
+std::vector<int> obs_owners(nesosim_ctx *ctx, int *list_end) {
+    const StripTables &t = ctx->ens.tables;
+    const int nx = ctx->cfg.nx;
+    std::vector<int> owner((size_t)ctx->cfg.ny * nx, -1);
+    *list_end = 0;
+    for (int k = 0; k < t.cluster; ++k) {
+        int idx = 0;
+        for (int r = t.row0[k]; r < t.row0[k + 1]; ++r)
+            for (int col = 0; col < nx; ++col) {
+                const uint8_t m = ctx->mask_host[(size_t)r * nx + col];
+                if (!(m > 10 || m < 1)) owner[(size_t)r * nx + col] = t.ocean_off[k] + idx++;
+            }
+        *list_end = std::max(*list_end, t.ocean_off[k] + idx);
+    }
+    return owner;
+}
+
+// appends one season's observations to `t`; returns the number of sample slots it added (sentinels included)
+size_t compile_obs_set(std::vector<ObsPoint> &obs, int list_end, ObsTables &t) {
+    std::stable_sort(obs.begin(), obs.end(), [](const ObsPoint &x, const ObsPoint &y) { return x.owner != y.owner ? x.owner < y.owner : x.day < y.day; });
+    const size_t f0 = t.first.size(), s0 = t.slot_day.size(), p0 = t.o_slot.size();
+    t.first.resize(f0 + (size_t)list_end + 1, -1);
+    t.o_slot.resize(p0 + obs.size()); t.o_day.resize(p0 + obs.size()); t.o_cell.resize(p0 + obs.size()); t.o_val.resize(p0 + obs.size());
+    t.slot_day.reserve(s0 + obs.size() + list_end + 1);
+    size_t p = 0;
+    for (int o = 0; o < list_end; ++o) {
+        t.first[f0 + o] = (int)(t.slot_day.size() - s0);
+        while (p < obs.size() && obs[p].owner == o) {
+            if (t.slot_day.size() - s0 == (size_t)t.first[f0 + o] || t.slot_day.back() != obs[p].day) t.slot_day.push_back(obs[p].day);
+            t.o_slot[p0 + p] = (int)(t.slot_day.size() - s0) - 1;
+            t.o_day[p0 + p] = obs[p].day;
+            t.o_cell[p0 + p] = obs[p].cell;
+            t.o_val[p0 + p] = obs[p].val;
+            ++p;
+        }
+        t.slot_day.push_back(0x7fffffff);                // sentinel
+    }
+    return t.slot_day.size() - s0;
+}
+
+// replaces the context's observations by `t` (samples: `stride` doubles per member)
+int upload_obs(nesosim_ctx *ctx, const ObsTables &t, long long stride) {
+    auto &ob = ctx->obs;
+    CU(cudaDeviceSynchronize());                         // nothing in flight still reads the previous set
+    cudaFree(ob.first); cudaFree(ob.day); cudaFree(ob.val); cudaFree(ob.samples); cudaFree(ob.o_slot); cudaFree(ob.o_day); cudaFree(ob.o_cell);
+    cudaFree(ob.slot_base); cudaFree(ob.obs_begin);
+    ob = {};
+    const int M = ctx->cfg.n_members;
+    const size_t n = t.o_slot.size();
+    ob.stride = stride;
+    ob.n_used = (long long)n;
+    CU(cudaMalloc(&ob.first, t.first.size() * sizeof(int)));
+    CU(cudaMalloc(&ob.day, t.slot_day.size() * sizeof(int)));
+    CU(cudaMalloc(&ob.samples, (size_t)M * ob.stride * sizeof(double)));
+    CU(cudaMalloc(&ob.val, std::max<size_t>(1, n) * sizeof(double)));
+    CU(cudaMalloc(&ob.o_slot, std::max<size_t>(1, n) * sizeof(int)));
+    CU(cudaMalloc(&ob.o_day, std::max<size_t>(1, n) * sizeof(int)));
+    CU(cudaMalloc(&ob.o_cell, std::max<size_t>(1, n) * sizeof(int)));
+    CU(cudaMemcpy(ob.first, t.first.data(), t.first.size() * sizeof(int), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(ob.day, t.slot_day.data(), t.slot_day.size() * sizeof(int), cudaMemcpyHostToDevice));
+    CU(cudaMemset(ob.samples, 0, (size_t)M * ob.stride * sizeof(double)));
+    if (n) {
+        CU(cudaMemcpy(ob.val, t.o_val.data(), n * sizeof(double), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(ob.o_slot, t.o_slot.data(), n * sizeof(int), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(ob.o_day, t.o_day.data(), n * sizeof(int), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(ob.o_cell, t.o_cell.data(), n * sizeof(int), cudaMemcpyHostToDevice));
+    }
+    return NESOSIM_OK;
+}
+
+extern "C" {
+
 // Observations of the calibration driver, compiled against the strip tables and kept on the device until they are
 // replaced: -> (strip, index in the strip's ocean list), sorted by owner and day, one sentinel per ocean cell.
 int nesosim_set_observations(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_day_host, const int32_t *obs_row_host,
@@ -1223,70 +1338,71 @@ int nesosim_set_observations(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs
     const char *why = "";
     if (!ensemble_eligible(ctx, 0, T - 1, &none, &why))
         return fail(NESOSIM_ERR_ARG, std::string("misfit mode needs the season-resident kernel: ") + why);
-    const StripTables &t = ctx->ens.tables;
-    const int cl = t.cluster;
-    std::vector<int> owner((size_t)ny * nx, -1);        // position in the concatenated code lists (ocean_off[k] + idx)
     int list_end = 0;
-    for (int k = 0; k < cl; ++k) {
-        int idx = 0;
-        for (int r = t.row0[k]; r < t.row0[k + 1]; ++r)
-            for (int col = 0; col < nx; ++col) {
-                const uint8_t m = ctx->mask_host[(size_t)r * nx + col];
-                if (!(m > 10 || m < 1)) owner[(size_t)r * nx + col] = t.ocean_off[k] + idx++;
-            }
-        list_end = std::max(list_end, t.ocean_off[k] + idx);
-    }
-    struct Ob { int owner, day, cell; double val; };
-    std::vector<Ob> obs;
+    const std::vector<int> owner = obs_owners(ctx, &list_end);
+    std::vector<ObsPoint> obs;
     obs.reserve((size_t)n_obs);
     for (int64_t i = 0; i < n_obs; ++i) {
         const int d = obs_day_host[i], r = obs_row_host[i], col = obs_col_host[i];
         if (d < 0 || d >= T || r < 0 || r >= ny || col < 0 || col >= nx) return fail(NESOSIM_ERR_ARG, "observation outside the grid or the season");
         const int o = owner[(size_t)r * nx + col];
         if (o < 0) continue;                             // land / lake: the model value is NaN, the observation is skipped
-        obs.push_back(Ob{o, d, r * nx + col, obs_depth_host[i]});
+        obs.push_back(ObsPoint{o, d, r * nx + col, obs_depth_host[i]});
     }
-    std::stable_sort(obs.begin(), obs.end(), [](const Ob &x, const Ob &y) { return x.owner != y.owner ? x.owner < y.owner : x.day < y.day; });
-    // sample slots: the distinct (cell, day) pairs, per owning cell in day order, one sentinel behind every cell's run
-    std::vector<int> first((size_t)list_end + 1, -1), slot_day, o_slot(obs.size()), o_day(obs.size()), o_cell(obs.size());
-    std::vector<double> o_val(obs.size());
-    slot_day.reserve(obs.size() + list_end + 1);
-    size_t p = 0;
-    for (int o = 0; o < list_end; ++o) {
-        first[o] = (int)slot_day.size();
-        while (p < obs.size() && obs[p].owner == o) {
-            if (slot_day.size() == (size_t)first[o] || slot_day.back() != obs[p].day) slot_day.push_back(obs[p].day);
-            o_slot[p] = (int)slot_day.size() - 1;
-            o_day[p] = obs[p].day;
-            o_cell[p] = obs[p].cell;
-            o_val[p] = obs[p].val;
-            ++p;
-        }
-        slot_day.push_back(0x7fffffff);                  // sentinel
+    ObsTables t;
+    const size_t slots = compile_obs_set(obs, list_end, t);
+    int rc = upload_obs(ctx, t, (long long)((slots + 1) / 2 * 2));
+    if (rc) return rc;
+    ctx->obs.ready = true;
+    return NESOSIM_OK;
+}
+
+int nesosim_set_observations_sets(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
+                                  const int32_t *obs_row_host, const int32_t *obs_col_host, const double *obs_depth_host) {
+    if (!ctx || n_obs < 0) return fail(NESOSIM_ERR_ARG, "bad argument");
+    if (n_obs > 0 && (!obs_set_host || !obs_day_host || !obs_row_host || !obs_col_host || !obs_depth_host))
+        return fail(NESOSIM_ERR_ARG, "NULL observation array");
+    if (!ctx->member_set_dev) return fail(NESOSIM_ERR_STATE, "set observations need nesosim_set_forcing_sets first");
+    CU(cudaSetDevice(ctx->cfg.device));
+    const nesosim_config &c = ctx->cfg;
+    const int T = c.num_days, ny = c.ny, nx = c.nx, S = ctx->n_sets;
+    nesosim_outputs none{};
+    none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
+    none.plane_member_stride = (int64_t)T * ctx->plane;
+    const char *why = "";
+    if (!ensemble_eligible(ctx, 0, T - 1, &none, &why))
+        return fail(NESOSIM_ERR_ARG, std::string("misfit mode needs the season-resident kernel: ") + why);
+    int list_end = 0;
+    const std::vector<int> owner = obs_owners(ctx, &list_end);
+    std::vector<std::vector<ObsPoint>> per_set((size_t)S);
+    for (int64_t i = 0; i < n_obs; ++i) {
+        const int s = obs_set_host[i], d = obs_day_host[i], r = obs_row_host[i], col = obs_col_host[i];
+        if (s < 0 || s >= S) return fail(NESOSIM_ERR_ARG, "observation set index outside [0, n_sets)");
+        if (d < 0 || d >= ctx->set_days[s]) return fail(NESOSIM_ERR_ARG, "observation day outside its set's season [0, set_days)");
+        if (r < 0 || r >= ny || col < 0 || col >= nx) return fail(NESOSIM_ERR_ARG, "observation outside the grid");
+        const int o = owner[(size_t)r * nx + col];
+        if (o < 0) continue;                             // land / lake, as in nesosim_set_observations
+        per_set[s].push_back(ObsPoint{o, d, r * nx + col, obs_depth_host[i]});
     }
+    ObsTables t;
+    std::vector<int> slot_base(S), obs_begin(S + 1, 0);
+    size_t stride = 0;                                   // a member samples one set only: the largest set, not the sum
+    for (int s = 0; s < S; ++s) {
+        slot_base[s] = (int)t.slot_day.size();
+        obs_begin[s] = (int)t.o_slot.size();
+        stride = std::max(stride, compile_obs_set(per_set[s], list_end, t));
+        for (int o = 0; o < list_end; ++o) t.first[(size_t)s * (list_end + 1) + o] += slot_base[s];   // -> index in `day`
+    }
+    obs_begin[S] = (int)t.o_slot.size();
+    int rc = upload_obs(ctx, t, (long long)((stride + 1) / 2 * 2));
+    if (rc) return rc;
     auto &ob = ctx->obs;
-    CU(cudaDeviceSynchronize());                         // nothing in flight still reads the previous set
-    cudaFree(ob.first); cudaFree(ob.day); cudaFree(ob.val); cudaFree(ob.samples); cudaFree(ob.o_slot); cudaFree(ob.o_day); cudaFree(ob.o_cell);
-    ob = {};
-    const int M = c.n_members;
-    ob.stride = (long long)((slot_day.size() + 1) / 2 * 2);
-    ob.n_used = (long long)obs.size();
-    CU(cudaMalloc(&ob.first, first.size() * sizeof(int)));
-    CU(cudaMalloc(&ob.day, slot_day.size() * sizeof(int)));
-    CU(cudaMalloc(&ob.samples, (size_t)M * ob.stride * sizeof(double)));
-    CU(cudaMalloc(&ob.val, std::max<size_t>(1, obs.size()) * sizeof(double)));
-    CU(cudaMalloc(&ob.o_slot, std::max<size_t>(1, obs.size()) * sizeof(int)));
-    CU(cudaMalloc(&ob.o_day, std::max<size_t>(1, obs.size()) * sizeof(int)));
-    CU(cudaMalloc(&ob.o_cell, std::max<size_t>(1, obs.size()) * sizeof(int)));
-    CU(cudaMemcpy(ob.first, first.data(), first.size() * sizeof(int), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ob.day, slot_day.data(), slot_day.size() * sizeof(int), cudaMemcpyHostToDevice));
-    CU(cudaMemset(ob.samples, 0, (size_t)M * ob.stride * sizeof(double)));
-    if (!obs.empty()) {
-        CU(cudaMemcpy(ob.val, o_val.data(), obs.size() * sizeof(double), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(ob.o_slot, o_slot.data(), obs.size() * sizeof(int), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(ob.o_day, o_day.data(), obs.size() * sizeof(int), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(ob.o_cell, o_cell.data(), obs.size() * sizeof(int), cudaMemcpyHostToDevice));
-    }
+    ob.first_stride = (long long)list_end + 1;
+    CU(cudaMalloc(&ob.slot_base, S * sizeof(int)));
+    CU(cudaMalloc(&ob.obs_begin, (S + 1) * sizeof(int)));
+    CU(cudaMemcpy(ob.slot_base, slot_base.data(), S * sizeof(int), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(ob.obs_begin, obs_begin.data(), (S + 1) * sizeof(int), cudaMemcpyHostToDevice));
+    ob.set_days = ctx->set_days;
     ob.ready = true;
     return NESOSIM_OK;
 }
@@ -1296,7 +1412,10 @@ int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *par
     if (!ctx || !params_host || !misfit_dev) return fail(NESOSIM_ERR_ARG, "bad argument");
     if (!ctx->P) return fail(NESOSIM_ERR_STATE, "nesosim_set_forcing has not been called");
     if (!ctx->obs.ready) return fail(NESOSIM_ERR_STATE, "nesosim_set_observations has not been called");
-    if (ctx->member_set_dev) return fail(NESOSIM_ERR_ARG, "misfit mode runs on one shared forcing");
+    const bool sets = !ctx->obs.set_days.empty();
+    if (!sets && ctx->member_set_dev) return fail(NESOSIM_ERR_ARG, "misfit mode runs on one shared forcing");
+    if (sets && ctx->obs.set_days != ctx->set_days)
+        return fail(NESOSIM_ERR_STATE, "the forcing sets changed since nesosim_set_observations_sets; register the observations again");
     CU(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     const nesosim_config &c = ctx->cfg;
@@ -1311,6 +1430,7 @@ int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *par
     if (rc) return rc;
     ObsDevice od;
     od.first = ctx->obs.first; od.day = ctx->obs.day; od.sample_depth = ctx->obs.samples; od.sample_stride = ctx->obs.stride;
+    od.first_stride = ctx->obs.first_stride; od.slot_base = ctx->obs.slot_base;
     ctx->last_path = 2;
     rc = run_ensemble(ctx, ic_dev, ic_per_member, &none, 0, M, st, &od);     // synchronises the stream (operand-range flag)
     if (rc) return rc;
@@ -1319,7 +1439,9 @@ int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *par
     ma.obs_slot = ctx->obs.o_slot; ma.obs_day = ctx->obs.o_day; ma.obs_cell = ctx->obs.o_cell; ma.obs_val = ctx->obs.val;
     ma.conc = ctx->C; ma.plane = ctx->plane; ma.n_obs = ctx->obs.n_used;
     ma.misfit = misfit_dev; ma.count = (long long *)count_dev;
-    misfit_finish_kernel<<<M, 256, 0, st>>>(ma);
+    ma.member_set = ctx->member_set_dev; ma.obs_begin = ctx->obs.obs_begin; ma.conc_set_stride = (long long)T * ctx->plane;
+    if (sets) misfit_finish_kernel<true><<<M, 256, 0, st>>>(ma);
+    else misfit_finish_kernel<false><<<M, 256, 0, st>>>(ma);
     ctx->launches++;
     CU(cudaGetLastError());
     if (ctx->ens_status) return fail(NESOSIM_ERR_ARG, "an operand left the range of the season-resident kernel's fast divisions; misfit mode has no general-path fallback");

@@ -255,6 +255,19 @@ class SnowBudgetEngine:
         _lib.check(self.lib.nesosim_set_observations(self.handle, n, day.ctypes.data_as(i32), row.ctypes.data_as(i32),
                                                      col.ctypes.data_as(i32), depth.ctypes.data_as(C.POINTER(C.c_double))))
 
+    def set_observations_sets(self, obs_set, day, row, col, depth):
+        """Register observations tagged with the forcing set (season) they belong to, for ``run_season_misfit`` on a
+        context with forcing sets (``set_forcing_sets`` first): member m is then scored against the observations of set
+        ``member_set[m]`` only (see nesosim_set_observations_sets)."""
+        s, day, row, col = (np.ascontiguousarray(np.asarray(a), dtype=np.int32) for a in (obs_set, day, row, col))
+        depth = np.ascontiguousarray(np.asarray(depth), dtype=np.float64)
+        n = len(day)
+        assert len(s) == n and len(row) == n and len(col) == n and len(depth) == n
+        i32 = C.POINTER(C.c_int32)
+        _lib.check(self.lib.nesosim_set_observations_sets(self.handle, n, s.ctypes.data_as(i32), day.ctypes.data_as(i32),
+                                                          row.ctypes.data_as(i32), col.ctypes.data_as(i32),
+                                                          depth.ctypes.data_as(C.POINTER(C.c_double))))
+
     def run_season_misfit(self, params, ic, obs=None):
         """The season with the calibration misfit reduced INSIDE the season-resident kernel (nesosim_run_season_misfit)
         against the registered observations (``obs`` given: registered first); returns CUDA tensors (misfit[M] float64,
