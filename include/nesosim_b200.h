@@ -175,7 +175,7 @@ int nesosim_final_products(const double *depths_dev, const double *density_dev, 
  * nesosim_set_observations registers point observations (day slot 0..T-1, row, col, observed snow depth over ice [m];
  * host arrays, copied): they are compiled against the kernel's cell ownership once (distinct (cell, day) pairs =
  * "sample slots", sorted per owning thread) and stay on the device until replaced.  During nesosim_run_season_misfit the
- * thread that owns an observed cell stores the total depth h0+h1 of the observed days -- 8 bytes per observed cell-day
+ * thread that owns an observed cell stores the two layers h0, h1 of the observed days -- 16 bytes per observed cell-day
  * instead of 96 per cell-day, nothing on the day's critical path waits for it -- and a one-CTA-per-member epilogue forms
  * model = (h0+h1)/iceConc at that slot and cell (what main writes as snow depth, NESOSIM.py:654) and
  * misfit_dev[m] = sum over the observations of (model - observed)^2, skipping non-finite differences (land, NaN forcing,
@@ -200,6 +200,40 @@ int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *par
 int nesosim_set_observations_sets(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host,
                                   const int32_t *obs_day_host, const int32_t *obs_row_host,
                                   const int32_t *obs_col_host, const double *obs_depth_host);
+
+/* Calibration scores: observation errors, several observed quantities and the model value at every observation.
+ * nesosim_set_observations_ex registers observations of any kind with an error sigma each (obs_set NULL: one shared
+ * forcing, as nesosim_set_observations; else tagged with their forcing set, as nesosim_set_observations_sets; obs_kind
+ * NULL: all depth; obs_sigma NULL: all 1) and replaces the registered ones.  Every kind is a function of the two snow
+ * layers (h0, h1) of the observed day, which the season kernel stores per observed (cell, day): observations of several
+ * kinds at one cell and day share that sample.  nesosim_run_season_scores runs the season as nesosim_run_season_misfit and
+ * writes, per member m and kind k, chi2_dev[m][k] = sum over the member's observations of that kind of
+ * ((model - observed)/sigma)^2 and count_dev[m][k] (may be NULL) = the number of terms; a term is used only if it is
+ * finite (land, NaN forcing, zero concentration, density below minSnowD and NaN observed values are skipped).  Each kind
+ * is summed in a fixed order, exactly as if it had been registered alone: with sigma 1, chi2_dev[m][NESOSIM_OBS_DEPTH]
+ * of depth observations is bit-identical to nesosim_run_season_misfit's misfit.  model_dev (may be NULL) receives the
+ * fp64 model value of every observation at its index among its set's input observations (its input index with one
+ * forcing): model_dev[m*model_stride + i]; observations on land or lake hold NaN.  A density observation on day 0 has no
+ * model counterpart (the reference never computes density[0], NESOSIM.py:350-376) and is rejected.
+ * NESOSIM_ERR_ARG: a kind outside [0, NESOSIM_OBS_KINDS), a density observation on day 0, a sigma that is not finite and
+ * > 0, model_stride < the row length, and whatever nesosim_set_observations / _sets reject; a rejected registration
+ * leaves the previous observations in force.  NESOSIM_ERR_STATE as for nesosim_run_season_misfit; and
+ * nesosim_run_season_misfit itself returns it when the registered observations hold a kind other than depth or a
+ * sigma other than 1, which its one number per member cannot report. */
+#define NESOSIM_OBS_DEPTH   0   /* snow depth over ice (h0+h1)/iceConc [m] (NESOSIM.py:654)        */
+#define NESOSIM_OBS_VOLUME  1   /* snow volume per grid-cell area h0+h1 [m]                         */
+#define NESOSIM_OBS_DENSITY 2   /* bulk snow density, densityCalc (NESOSIM.py:458-473) [kg m^-3]    */
+#define NESOSIM_OBS_KINDS   3
+
+int nesosim_set_observations_ex(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host,
+                                const int32_t *obs_day_host, const int32_t *obs_row_host, const int32_t *obs_col_host,
+                                const int32_t *obs_kind_host, const double *obs_value_host, const double *obs_sigma_host);
+/* length of a member's model row: the largest number of input observations of one set (n_obs with one forcing) */
+int nesosim_observation_row_length(const nesosim_ctx *ctx, int64_t *row_len);
+/* chi2_dev [M][NESOSIM_OBS_KINDS]; count_dev same shape or NULL; model_dev [M][model_stride] or NULL */
+int nesosim_run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                              int ic_per_member, double *chi2_dev, int64_t *count_dev,
+                              double *model_dev, int64_t model_stride, void *stream);
 
 /* Asynchronous mode.  By default nesosim_run_season on the season-resident path synchronises `stream` once to read
  * the kernel's operand-range flag (see above).  With nesosim_set_async(ctx, 1) it never synchronises: the flag is copied

@@ -15,6 +15,9 @@ LIB_PATH = os.environ.get("NESOSIM_B200_LIB") or os.path.join(_HERE, "libnesosim
 OK = 0
 ERR_ARG, ERR_CUDA, ERR_STATE, ERR_NOMEM = -1, -2, -3, -4
 
+# observed quantities of nesosim_set_observations_ex (NESOSIM_OBS_*): snow depth over ice, snow volume, bulk density
+OBS_DEPTH, OBS_VOLUME, OBS_DENSITY, OBS_KINDS = 0, 1, 2, 3
+
 
 class NesosimError(RuntimeError):
     def __init__(self, code, msg):
@@ -90,6 +93,12 @@ _SIGNATURES = {
                                             C.c_void_p, C.c_void_p]),
     "nesosim_set_observations_sets": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                                 C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
+    "nesosim_set_observations_ex": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    "nesosim_observation_row_length": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "nesosim_run_season_scores": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

@@ -201,18 +201,19 @@ struct EnsArgs {
     // misfit mode (calibration driver, SURVEY.md 8f N3): the (cell, day) pairs at which snow depth is observed, sorted by
     // owning cell and day ("sample slots"); obs_first is indexed like `codes` (ocean list of every strip) and points at
     // the cell's first slot, every cell's run ends with a sentinel day (INT_MAX).  The thread that owns a cell stores the
-    // total depth h0+h1 of the observed days into sample_depth[member][slot] -- 8 bytes per observed cell-day instead of
-    // 96 per cell-day -- fire and forget: nothing on the day's critical path waits for memory.  The observation operator
-    // proper (division by the ice concentration) and the sum of squares run in a small epilogue kernel.
+    // two layers {h0, h1} of the observed days into sample_hh[member][slot] -- 16 bytes per observed cell-day instead of
+    // 96 per cell-day -- fire and forget: nothing on the day's critical path waits for memory.  The observation operators
+    // proper (depth over ice, volume, density: all functions of the two layers and the day's ice concentration) and the
+    // sums of squares run in a small epilogue kernel.
     const int *obs_first, *obs_day;
-    double *sample_depth;
+    double2 *sample_hh;
     long long sample_stride;
     int dbg;                           // timing experiments only (NESOSIM_ENS_DBG): 1 forcing always from day 0, 2 no L2 prefetch, 4 no bulk stores
     int *status;                       // set to 1 if any operand left the fast divisions' proven range (host reruns)
     long long *timing;                 // debug: [gridDim.x][ENS_NTIMER] phase cycle totals (NULL = off)
     // misfit mode on forcing sets (nesosim_set_observations_sets): every set has its own obs_first table, obs_first_stride
     // entries apart; the sets' slots follow one another in obs_day, set s from obs_slot_base[s] on.  A member samples its
-    // own set only, so its row of sample_depth holds that set's slots (from obs_slot_base[set]) and the stride is the
+    // own set only, so its row of sample_hh holds that set's slots (from obs_slot_base[set]) and the stride is the
     // slot count of the largest set, not the sum
     long long obs_first_stride;
     const int *obs_slot_base;
@@ -575,18 +576,18 @@ __global__ void __launch_bounds__(NTC + 32, 1) ensemble_season_kernel(const __gr
             r_h1[j] = LD(HOWN + PEXB + b_ci[j]);
             r_dn[j] = r_adv[j] = r_div[j] = r_lead[j] = r_atm[j] = r_wpl[j] = r_wpg[j] = r_wp[j] = 0.0;
         }
-        // misfit mode: every owned cell walks its own (day-sorted) sample slots; on an observed day the total depth
-        // goes to the member's sample array and the cursor moves on (the next slot's day is needed tomorrow at the
+        // misfit mode: every owned cell walks its own (day-sorted) sample slots; on an observed day the two layers
+        // go to the member's sample array and the cursor moves on (the next slot's day is needed tomorrow at the
         // earliest: its load is never waited for)
         int o_idx[OBS ? KO : 1], o_day[OBS ? KO : 1];
-        // (SETS: the set's tables hold the slots of all sets one after the other, the member's row of sample_depth only
+        // (SETS: the set's tables hold the slots of all sets one after the other, the member's row of sample_hh only
         // those of its own set: the row is addressed relative to the set's first slot)
-        double *const m_samples = !OBS ? nullptr
-                                  : SETS ? a.sample_depth + ((long long)m * a.sample_stride - a.obs_slot_base[fset])
-                                         : a.sample_depth + (long long)m * a.sample_stride;
+        double2 *const m_samples = !OBS ? nullptr
+                                   : SETS ? a.sample_hh + ((long long)m * a.sample_stride - a.obs_slot_base[fset])
+                                          : a.sample_hh + (long long)m * a.sample_stride;
         auto obs_take = [&](int j, int slot) {
             if (o_day[j] == slot) {
-                m_samples[o_idx[j]] = add(r_h0[j], r_h1[j]);      // snowDepths[:, 0] + snowDepths[:, 1]   (NESOSIM.py:654)
+                m_samples[o_idx[j]] = make_double2(r_h0[j], r_h1[j]);   // snowDepths[slot, 0], snowDepths[slot, 1]
                 ++o_idx[j];
                 o_day[j] = __ldg(a.obs_day + o_idx[j]);
             }

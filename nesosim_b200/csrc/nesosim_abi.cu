@@ -197,17 +197,18 @@ struct nesosim_ctx {
     struct {                        // observations of the calibration driver (nesosim_set_observations)
         bool ready = false;
         int *first = nullptr, *day = nullptr;            // sample slots: first slot of every owned cell, day of every slot
-        double *samples = nullptr;                       // [M][stride] total depth at every slot (written by the season kernel)
+        double2 *samples = nullptr;                      // [M][stride] {h0, h1} at every slot (written by the season kernel)
         long long stride = 0;
-        double *val = nullptr;                           // per observation: value, sample slot, day, cell
-        int *o_slot = nullptr, *o_day = nullptr, *o_cell = nullptr;
-        long long n_used = 0;
+        double *val = nullptr, *sigma = nullptr;         // per observation: value, error, sample slot, day, cell, index
+        int *o_slot = nullptr, *o_day = nullptr, *o_cell = nullptr, *src = nullptr;   // among its set's input observations
+        int *kind_begin = nullptr;                       // [sets][NESOSIM_OBS_KINDS+1] every set's observations, by kind
+        long long row_len = 0;                           // the largest number of input observations of one set
+        bool depth_only = true;                          // every observation is depth with sigma 1 (misfit can report it)
         // nesosim_set_observations_sets: the tables of every set one after the other; set_days = the forcing layout they
         // were compiled against (empty: plain observations of one shared forcing)
         std::vector<int> set_days;
         long long first_stride = 0;                      // entries of one set's `first` table
         int *slot_base = nullptr;                        // [sets] the set's first slot in `day`
-        int *obs_begin = nullptr;                        // [sets+1] the set's observations
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -348,6 +349,14 @@ cudaError_t launch_day_kernel(void (*kern)(KArgs...), dim3 grid, int threads, cu
     cfg.attrs = attr;
     cfg.numAttrs = pdl ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kern, args...);
+}
+
+void obs_release(nesosim_ctx *ctx) {
+    auto &ob = ctx->obs;
+    cudaFree(ob.first); cudaFree(ob.day); cudaFree(ob.val); cudaFree(ob.sigma); cudaFree(ob.samples);
+    cudaFree(ob.o_slot); cudaFree(ob.o_day); cudaFree(ob.o_cell); cudaFree(ob.src);
+    cudaFree(ob.kind_begin); cudaFree(ob.slot_base);
+    ob = {};
 }
 
 void strip_release(nesosim_ctx *ctx) {
@@ -765,7 +774,7 @@ bool ensemble_eligible(nesosim_ctx *ctx, int first_step, int num_steps, const ne
 
 struct ObsDevice {                      // misfit mode: device arrays of the sample slots (see EnsArgs)
     const int *first = nullptr, *day = nullptr;
-    double *sample_depth = nullptr;
+    double2 *sample_hh = nullptr;
     long long sample_stride = 0;
     long long first_stride = 0;         // forcing sets: per-set tables
     const int *slot_base = nullptr;
@@ -844,7 +853,7 @@ int run_ensemble(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cons
     a.status = ctx->flags_dev;
     a.obs_first = obs ? obs->first : nullptr;
     a.obs_day = obs ? obs->day : nullptr;
-    a.sample_depth = obs ? obs->sample_depth : nullptr;
+    a.sample_hh = obs ? obs->sample_hh : nullptr;
     a.sample_stride = obs ? obs->sample_stride : 0;
     a.obs_first_stride = obs ? obs->first_stride : 0;
     a.obs_slot_base = obs ? obs->slot_base : nullptr;
@@ -1088,9 +1097,7 @@ int nesosim_destroy(nesosim_ctx *ctx) {
     }
     ctx->pending.clear();
     if (ctx->flag_pool) cudaFreeHost(ctx->flag_pool);
-    cudaFree(ctx->obs.first); cudaFree(ctx->obs.day); cudaFree(ctx->obs.val); cudaFree(ctx->obs.samples);
-    cudaFree(ctx->obs.o_slot); cudaFree(ctx->obs.o_day); cudaFree(ctx->obs.o_cell);
-    cudaFree(ctx->obs.slot_base); cudaFree(ctx->obs.obs_begin);
+    obs_release(ctx);
     for (int i = 0; i < 2; ++i)
         if (ctx->ens_ev[i]) cudaEventDestroy(ctx->ens_ev[i]);
     strip_release(ctx);
@@ -1183,71 +1190,88 @@ int nesosim_run_season(nesosim_ctx *ctx, const nesosim_member_params *params_hos
 
 }  // extern "C"
 
-// Epilogue of the misfit mode: one CTA per member.  model = sampled depth / ice concentration of that day and cell
-// (what main writes as snow depth over ice, NESOSIM.py:654); squared differences to the observations are summed in a
-// fixed order (observation i belongs to thread i % 256, threads are combined by shuffles, warps one after the other).
-// SETS: member m is scored against the observations of its forcing set member_set[m], obs_begin[set] .. obs_begin[set+1]-1,
-// on that set's concentration stack; i counts from the set's first observation, so the member's sum is formed exactly
-// as for its season on its own.
+// Epilogue of the misfit mode: one CTA per member.  The sample {h0, h1} of an observation's slot gives the model value of
+// its kind: depth over ice (h0+h1)/iceConc of that day and cell (what main writes as snow depth, NESOSIM.py:654), volume
+// h0+h1, or the bulk density densityCalc(h0, h1) (NESOSIM.py:458-473).  The terms ((model - observed)/sigma)^2 of a kind
+// are summed in a fixed order over that kind's contiguous range of observations (observation i of the range belongs to
+// thread i % 256, threads are combined by shuffles, warps one after the other): each kind's sum is formed exactly as if
+// it had been registered alone.  SETS: member m is scored against the observations of its forcing set member_set[m], on
+// that set's concentration stack, exactly as for its season on its own.
 struct MisfitArgs {
-    const double *sample_depth;     // [M][stride]
+    const double2 *samples;         // [M][stride]
     long long stride;
-    const int *obs_slot, *obs_day, *obs_cell;
-    const double *obs_val;
+    const int *obs_slot, *obs_day, *obs_cell, *src;
+    const double *obs_val, *sigma;
+    const int *kind_begin;          // [sets][NESOSIM_OBS_KINDS+1]
     const double *conc;             // [T][plane] (SETS: [sets][T][plane])
-    long long plane, n_obs;
-    double *misfit;
-    long long *count;
-    const int *member_set, *obs_begin;   // SETS only
-    long long conc_set_stride;           // SETS only: T * plane
+    long long plane;
+    ModelConsts k;
+    double *chi2;                   // [M][n_kinds]
+    long long *count;               // same shape, or NULL
+    int n_kinds;                    // kinds reported: NESOSIM_OBS_KINDS, or 1 (depth only, nesosim_run_season_misfit)
+    double *model;                  // [M][model_stride]: the model value at every observation's input index, or NULL
+    long long model_stride;
+    const int *member_set;          // SETS only
+    long long conc_set_stride;      // SETS only: T * plane
 };
 template <bool SETS>
 __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constant__ MisfitArgs a) {
     const int m = blockIdx.x;
-    const double *samp = a.sample_depth + (long long)m * a.stride;
+    const double2 *samp = a.samples + (long long)m * a.stride;
     const int set = SETS ? a.member_set[m] : 0;
-    const long long i0 = SETS ? (long long)a.obs_begin[set] : 0ll;
-    const long long n_obs = SETS ? (long long)a.obs_begin[set + 1] - i0 : a.n_obs;
+    const int *kb = a.kind_begin + set * (NESOSIM_OBS_KINDS + 1);
     const double *conc = SETS ? a.conc + (long long)set * a.conc_set_stride : a.conc;
-    double acc = 0.0;
-    long long cnt = 0;
-    for (long long i = threadIdx.x; i < n_obs; i += 256) {
-        const long long q = i0 + i;
-        const double C = __ldg(conc + (long long)a.obs_day[q] * a.plane + a.obs_cell[q]);
-        const double diff = sub(div_ieee(samp[a.obs_slot[q]], C), a.obs_val[q]);
-        if (nesosim::finite(diff)) {
-            acc = add(acc, mul(diff, diff));
-            ++cnt;
-        }
-    }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        acc = add(acc, __shfl_down_sync(0xffffffffu, acc, off));
-        cnt += __shfl_down_sync(0xffffffffu, cnt, off);
-    }
+    double *model = a.model ? a.model + (long long)m * a.model_stride : nullptr;
     __shared__ double red[8];
     __shared__ long long redc[8];
-    if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = acc; redc[threadIdx.x >> 5] = cnt; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-        long long n = 0;
-        for (int w = 0; w < 8; ++w) { t = add(t, red[w]); n += redc[w]; }
-        a.misfit[m] = t;
-        if (a.count) a.count[m] = n;
+    for (int kind = 0; kind < a.n_kinds; ++kind) {
+        const long long i0 = kb[kind], n_obs = (long long)kb[kind + 1] - i0;
+        double acc = 0.0;
+        long long cnt = 0;
+        for (long long i = threadIdx.x; i < n_obs; i += 256) {
+            const long long q = i0 + i;
+            const double2 h = samp[a.obs_slot[q]];
+            double v;
+            if (kind == NESOSIM_OBS_DEPTH) v = div_ieee(add(h.x, h.y), __ldg(conc + (long long)a.obs_day[q] * a.plane + a.obs_cell[q]));
+            else if (kind == NESOSIM_OBS_VOLUME) v = add(h.x, h.y);
+            else v = density_variable(h.x, h.y, false, a.k);
+            if (model) model[a.src[q]] = v;
+            const double r = div_ieee(sub(v, a.obs_val[q]), a.sigma[q]);   // sigma 1: exact, r = model - observed
+            if (nesosim::finite(r)) {
+                acc = add(acc, mul(r, r));
+                ++cnt;
+            }
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            acc = add(acc, __shfl_down_sync(0xffffffffu, acc, off));
+            cnt += __shfl_down_sync(0xffffffffu, cnt, off);
+        }
+        if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = acc; redc[threadIdx.x >> 5] = cnt; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double t = 0.0;
+            long long n = 0;
+            for (int w = 0; w < 8; ++w) { t = add(t, red[w]); n += redc[w]; }
+            a.chi2[(long long)m * a.n_kinds + kind] = t;
+            if (a.count) a.count[(long long)m * a.n_kinds + kind] = n;
+        }
+        __syncthreads();                                 // red / redc are reused by the next kind
     }
 }
 
 // Observations compiled against the strip tables (host side).  One season's tables: every observation mapped to its
 // owner (strip, index in the strip's ocean list), sorted by owner and day; `first` has list_end+1 entries, sample
-// slots are the distinct (cell, day) pairs per owning cell in day order with one sentinel behind every cell's run.
-// Several seasons (forcing sets) are appended one after the other: a set's `first` entries and o_slot count from the
-// set's first slot, so each set's tables are exactly those its season would get on its own (the caller moves `first`
-// to absolute slots for the season kernel; o_slot stays the slot in the member's row of samples).
-struct ObsPoint { int owner, day, cell; double val; };
+// slots are the distinct (cell, day) pairs per owning cell in day order with one sentinel behind every cell's run --
+// observations of different kinds at one cell and day share a slot.  The observations are then stable-partitioned by
+// kind (kind_begin: NESOSIM_OBS_KINDS+1 entries per set), so each kind's sub-sequence is the one a registration of that
+// kind alone gets.  Several seasons (forcing sets) are appended one after the other: a set's `first` entries and o_slot
+// count from the set's first slot, so each set's tables are exactly those its season would get on its own (the caller
+// moves `first` to absolute slots for the season kernel; o_slot stays the slot in the member's row of samples).
+struct ObsPoint { int owner, day, cell, kind, src; double val, sigma; };
 struct ObsTables {
-    std::vector<int> first, slot_day, o_slot, o_day, o_cell;
-    std::vector<double> o_val;
+    std::vector<int> first, slot_day, o_slot, o_day, o_cell, o_src, kind_begin;
+    std::vector<double> o_val, o_sigma;
 };
 
 // position of every ocean cell in the concatenated code lists (ocean_off[k] + idx), -1 on land; list_end = the lists' end
@@ -1271,101 +1295,81 @@ std::vector<int> obs_owners(nesosim_ctx *ctx, int *list_end) {
 // appends one season's observations to `t`; returns the number of sample slots it added (sentinels included)
 size_t compile_obs_set(std::vector<ObsPoint> &obs, int list_end, ObsTables &t) {
     std::stable_sort(obs.begin(), obs.end(), [](const ObsPoint &x, const ObsPoint &y) { return x.owner != y.owner ? x.owner < y.owner : x.day < y.day; });
-    const size_t f0 = t.first.size(), s0 = t.slot_day.size(), p0 = t.o_slot.size();
+    const size_t f0 = t.first.size(), s0 = t.slot_day.size();
     t.first.resize(f0 + (size_t)list_end + 1, -1);
-    t.o_slot.resize(p0 + obs.size()); t.o_day.resize(p0 + obs.size()); t.o_cell.resize(p0 + obs.size()); t.o_val.resize(p0 + obs.size());
     t.slot_day.reserve(s0 + obs.size() + list_end + 1);
+    std::vector<int> slot(obs.size());
     size_t p = 0;
     for (int o = 0; o < list_end; ++o) {
         t.first[f0 + o] = (int)(t.slot_day.size() - s0);
         while (p < obs.size() && obs[p].owner == o) {
             if (t.slot_day.size() - s0 == (size_t)t.first[f0 + o] || t.slot_day.back() != obs[p].day) t.slot_day.push_back(obs[p].day);
-            t.o_slot[p0 + p] = (int)(t.slot_day.size() - s0) - 1;
-            t.o_day[p0 + p] = obs[p].day;
-            t.o_cell[p0 + p] = obs[p].cell;
-            t.o_val[p0 + p] = obs[p].val;
+            slot[p] = (int)(t.slot_day.size() - s0) - 1;
             ++p;
         }
         t.slot_day.push_back(0x7fffffff);                // sentinel
     }
+    for (int k = 0; k < NESOSIM_OBS_KINDS; ++k) {
+        t.kind_begin.push_back((int)t.o_slot.size());
+        for (size_t q = 0; q < obs.size(); ++q) {
+            if (obs[q].kind != k) continue;
+            t.o_slot.push_back(slot[q]);
+            t.o_day.push_back(obs[q].day);
+            t.o_cell.push_back(obs[q].cell);
+            t.o_src.push_back(obs[q].src);
+            t.o_val.push_back(obs[q].val);
+            t.o_sigma.push_back(obs[q].sigma);
+        }
+    }
+    t.kind_begin.push_back((int)t.o_slot.size());
     return t.slot_day.size() - s0;
 }
 
-// replaces the context's observations by `t` (samples: `stride` doubles per member)
+// replaces the context's observations by `t` (samples: `stride` slots per member)
 int upload_obs(nesosim_ctx *ctx, const ObsTables &t, long long stride) {
-    auto &ob = ctx->obs;
     CU(cudaDeviceSynchronize());                         // nothing in flight still reads the previous set
-    cudaFree(ob.first); cudaFree(ob.day); cudaFree(ob.val); cudaFree(ob.samples); cudaFree(ob.o_slot); cudaFree(ob.o_day); cudaFree(ob.o_cell);
-    cudaFree(ob.slot_base); cudaFree(ob.obs_begin);
-    ob = {};
+    obs_release(ctx);
+    auto &ob = ctx->obs;
     const int M = ctx->cfg.n_members;
-    const size_t n = t.o_slot.size();
+    const size_t n = t.o_slot.size(), nb = std::max<size_t>(1, n);
     ob.stride = stride;
-    ob.n_used = (long long)n;
     CU(cudaMalloc(&ob.first, t.first.size() * sizeof(int)));
     CU(cudaMalloc(&ob.day, t.slot_day.size() * sizeof(int)));
-    CU(cudaMalloc(&ob.samples, (size_t)M * ob.stride * sizeof(double)));
-    CU(cudaMalloc(&ob.val, std::max<size_t>(1, n) * sizeof(double)));
-    CU(cudaMalloc(&ob.o_slot, std::max<size_t>(1, n) * sizeof(int)));
-    CU(cudaMalloc(&ob.o_day, std::max<size_t>(1, n) * sizeof(int)));
-    CU(cudaMalloc(&ob.o_cell, std::max<size_t>(1, n) * sizeof(int)));
+    CU(cudaMalloc(&ob.samples, (size_t)M * ob.stride * sizeof(double2)));
+    CU(cudaMalloc(&ob.val, nb * sizeof(double)));
+    CU(cudaMalloc(&ob.sigma, nb * sizeof(double)));
+    CU(cudaMalloc(&ob.o_slot, nb * sizeof(int)));
+    CU(cudaMalloc(&ob.o_day, nb * sizeof(int)));
+    CU(cudaMalloc(&ob.o_cell, nb * sizeof(int)));
+    CU(cudaMalloc(&ob.src, nb * sizeof(int)));
+    CU(cudaMalloc(&ob.kind_begin, t.kind_begin.size() * sizeof(int)));
     CU(cudaMemcpy(ob.first, t.first.data(), t.first.size() * sizeof(int), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(ob.day, t.slot_day.data(), t.slot_day.size() * sizeof(int), cudaMemcpyHostToDevice));
-    CU(cudaMemset(ob.samples, 0, (size_t)M * ob.stride * sizeof(double)));
+    CU(cudaMemset(ob.samples, 0, (size_t)M * ob.stride * sizeof(double2)));
+    CU(cudaMemcpy(ob.kind_begin, t.kind_begin.data(), t.kind_begin.size() * sizeof(int), cudaMemcpyHostToDevice));
     if (n) {
         CU(cudaMemcpy(ob.val, t.o_val.data(), n * sizeof(double), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(ob.sigma, t.o_sigma.data(), n * sizeof(double), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(ob.o_slot, t.o_slot.data(), n * sizeof(int), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(ob.o_day, t.o_day.data(), n * sizeof(int), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(ob.o_cell, t.o_cell.data(), n * sizeof(int), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(ob.src, t.o_src.data(), n * sizeof(int), cudaMemcpyHostToDevice));
     }
     return NESOSIM_OK;
 }
 
-extern "C" {
-
-// Observations of the calibration driver, compiled against the strip tables and kept on the device until they are
-// replaced: -> (strip, index in the strip's ocean list), sorted by owner and day, one sentinel per ocean cell.
-int nesosim_set_observations(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_day_host, const int32_t *obs_row_host,
-                             const int32_t *obs_col_host, const double *obs_depth_host) {
+// Validates every observation, then compiles them against the strip tables and replaces the context's observations.
+// sets: tagged with their forcing set (obs_set_host); else one shared forcing.  Nothing is freed before the last check.
+int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
+                          const int32_t *obs_row_host, const int32_t *obs_col_host, const int32_t *obs_kind_host,
+                          const double *obs_value_host, const double *obs_sigma_host) {
     if (!ctx || n_obs < 0) return fail(NESOSIM_ERR_ARG, "bad argument");
-    if (n_obs > 0 && (!obs_day_host || !obs_row_host || !obs_col_host || !obs_depth_host)) return fail(NESOSIM_ERR_ARG, "NULL observation array");
-    CU(cudaSetDevice(ctx->cfg.device));
-    const nesosim_config &c = ctx->cfg;
-    const int T = c.num_days, ny = c.ny, nx = c.nx;
-    nesosim_outputs none{};
-    none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
-    none.plane_member_stride = (int64_t)T * ctx->plane;
-    const char *why = "";
-    if (!ensemble_eligible(ctx, 0, T - 1, &none, &why))
-        return fail(NESOSIM_ERR_ARG, std::string("misfit mode needs the season-resident kernel: ") + why);
-    int list_end = 0;
-    const std::vector<int> owner = obs_owners(ctx, &list_end);
-    std::vector<ObsPoint> obs;
-    obs.reserve((size_t)n_obs);
-    for (int64_t i = 0; i < n_obs; ++i) {
-        const int d = obs_day_host[i], r = obs_row_host[i], col = obs_col_host[i];
-        if (d < 0 || d >= T || r < 0 || r >= ny || col < 0 || col >= nx) return fail(NESOSIM_ERR_ARG, "observation outside the grid or the season");
-        const int o = owner[(size_t)r * nx + col];
-        if (o < 0) continue;                             // land / lake: the model value is NaN, the observation is skipped
-        obs.push_back(ObsPoint{o, d, r * nx + col, obs_depth_host[i]});
-    }
-    ObsTables t;
-    const size_t slots = compile_obs_set(obs, list_end, t);
-    int rc = upload_obs(ctx, t, (long long)((slots + 1) / 2 * 2));
-    if (rc) return rc;
-    ctx->obs.ready = true;
-    return NESOSIM_OK;
-}
-
-int nesosim_set_observations_sets(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
-                                  const int32_t *obs_row_host, const int32_t *obs_col_host, const double *obs_depth_host) {
-    if (!ctx || n_obs < 0) return fail(NESOSIM_ERR_ARG, "bad argument");
-    if (n_obs > 0 && (!obs_set_host || !obs_day_host || !obs_row_host || !obs_col_host || !obs_depth_host))
+    if (n_obs > 0 && ((sets && !obs_set_host) || !obs_day_host || !obs_row_host || !obs_col_host || !obs_value_host))
         return fail(NESOSIM_ERR_ARG, "NULL observation array");
-    if (!ctx->member_set_dev) return fail(NESOSIM_ERR_STATE, "set observations need nesosim_set_forcing_sets first");
+    if (sets && !ctx->member_set_dev) return fail(NESOSIM_ERR_STATE, "set observations need nesosim_set_forcing_sets first");
     CU(cudaSetDevice(ctx->cfg.device));
     const nesosim_config &c = ctx->cfg;
-    const int T = c.num_days, ny = c.ny, nx = c.nx, S = ctx->n_sets;
+    const int T = c.num_days, ny = c.ny, nx = c.nx, S = sets ? ctx->n_sets : 1;
     nesosim_outputs none{};
     none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
     none.plane_member_stride = (int64_t)T * ctx->plane;
@@ -1375,43 +1379,59 @@ int nesosim_set_observations_sets(nesosim_ctx *ctx, int64_t n_obs, const int32_t
     int list_end = 0;
     const std::vector<int> owner = obs_owners(ctx, &list_end);
     std::vector<std::vector<ObsPoint>> per_set((size_t)S);
+    std::vector<int> n_in((size_t)S, 0);                 // input observations of every set so far (-> src)
+    bool depth_only = true;
     for (int64_t i = 0; i < n_obs; ++i) {
-        const int s = obs_set_host[i], d = obs_day_host[i], r = obs_row_host[i], col = obs_col_host[i];
+        const int s = sets ? obs_set_host[i] : 0, d = obs_day_host[i], r = obs_row_host[i], col = obs_col_host[i];
+        const int kind = obs_kind_host ? obs_kind_host[i] : NESOSIM_OBS_DEPTH;
+        const double sigma = obs_sigma_host ? obs_sigma_host[i] : 1.0;
         if (s < 0 || s >= S) return fail(NESOSIM_ERR_ARG, "observation set index outside [0, n_sets)");
-        if (d < 0 || d >= ctx->set_days[s]) return fail(NESOSIM_ERR_ARG, "observation day outside its set's season [0, set_days)");
+        if (d < 0 || d >= (sets ? ctx->set_days[s] : T)) return fail(NESOSIM_ERR_ARG, "observation day outside its season");
         if (r < 0 || r >= ny || col < 0 || col >= nx) return fail(NESOSIM_ERR_ARG, "observation outside the grid");
+        if (kind < 0 || kind >= NESOSIM_OBS_KINDS) return fail(NESOSIM_ERR_ARG, "observation kind outside [0, NESOSIM_OBS_KINDS)");
+        if (kind == NESOSIM_OBS_DENSITY && d == 0)
+            return fail(NESOSIM_ERR_ARG, "density observation on day 0: the model has no density there (NESOSIM.py:350-376)");
+        if (!(std::isfinite(sigma) && sigma > 0.0)) return fail(NESOSIM_ERR_ARG, "observation error sigma must be finite and > 0");
+        depth_only = depth_only && kind == NESOSIM_OBS_DEPTH && sigma == 1.0;
+        const int src = n_in[s]++;
         const int o = owner[(size_t)r * nx + col];
-        if (o < 0) continue;                             // land / lake, as in nesosim_set_observations
-        per_set[s].push_back(ObsPoint{o, d, r * nx + col, obs_depth_host[i]});
+        if (o < 0) continue;                             // land / lake: the model value is NaN, the observation is skipped
+        per_set[s].push_back(ObsPoint{o, d, r * nx + col, kind, src, obs_value_host[i], sigma});
     }
     ObsTables t;
-    std::vector<int> slot_base(S), obs_begin(S + 1, 0);
+    std::vector<int> slot_base(S);
     size_t stride = 0;                                   // a member samples one set only: the largest set, not the sum
     for (int s = 0; s < S; ++s) {
         slot_base[s] = (int)t.slot_day.size();
-        obs_begin[s] = (int)t.o_slot.size();
         stride = std::max(stride, compile_obs_set(per_set[s], list_end, t));
         for (int o = 0; o < list_end; ++o) t.first[(size_t)s * (list_end + 1) + o] += slot_base[s];   // -> index in `day`
     }
-    obs_begin[S] = (int)t.o_slot.size();
-    int rc = upload_obs(ctx, t, (long long)((stride + 1) / 2 * 2));
+    int rc = upload_obs(ctx, t, (long long)stride);
     if (rc) return rc;
     auto &ob = ctx->obs;
-    ob.first_stride = (long long)list_end + 1;
-    CU(cudaMalloc(&ob.slot_base, S * sizeof(int)));
-    CU(cudaMalloc(&ob.obs_begin, (S + 1) * sizeof(int)));
-    CU(cudaMemcpy(ob.slot_base, slot_base.data(), S * sizeof(int), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ob.obs_begin, obs_begin.data(), (S + 1) * sizeof(int), cudaMemcpyHostToDevice));
-    ob.set_days = ctx->set_days;
+    ob.row_len = *std::max_element(n_in.begin(), n_in.end());
+    ob.depth_only = depth_only;
+    if (sets) {
+        ob.first_stride = (long long)list_end + 1;
+        CU(cudaMalloc(&ob.slot_base, S * sizeof(int)));
+        CU(cudaMemcpy(ob.slot_base, slot_base.data(), S * sizeof(int), cudaMemcpyHostToDevice));
+        ob.set_days = ctx->set_days;
+    }
     ob.ready = true;
     return NESOSIM_OK;
 }
 
-int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
-                              int ic_per_member, double *misfit_dev, int64_t *count_dev, void *stream) {
-    if (!ctx || !params_host || !misfit_dev) return fail(NESOSIM_ERR_ARG, "bad argument");
+// The season with fused sampling, then the scores epilogue: n_kinds = NESOSIM_OBS_KINDS (nesosim_run_season_scores) or
+// 1 (nesosim_run_season_misfit: the depth sum only, which needs observations that are all depth with sigma 1).
+int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev, int ic_per_member,
+                      double *chi2_dev, int64_t *count_dev, int n_kinds, double *model_dev, int64_t model_stride,
+                      void *stream) {
+    if (!ctx || !params_host || !chi2_dev) return fail(NESOSIM_ERR_ARG, "bad argument");
     if (!ctx->P) return fail(NESOSIM_ERR_STATE, "nesosim_set_forcing has not been called");
     if (!ctx->obs.ready) return fail(NESOSIM_ERR_STATE, "nesosim_set_observations has not been called");
+    if (n_kinds == 1 && !ctx->obs.depth_only)
+        return fail(NESOSIM_ERR_STATE, "the registered observations are not all depth with sigma 1; use nesosim_run_season_scores");
+    if (model_dev && model_stride < ctx->obs.row_len) return fail(NESOSIM_ERR_ARG, "model_stride is shorter than the observation row");
     const bool sets = !ctx->obs.set_days.empty();
     if (!sets && ctx->member_set_dev) return fail(NESOSIM_ERR_ARG, "misfit mode runs on one shared forcing");
     if (sets && ctx->obs.set_days != ctx->set_days)
@@ -1429,23 +1449,70 @@ int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *par
     int rc = upload_coef(ctx, params_host, st);
     if (rc) return rc;
     ObsDevice od;
-    od.first = ctx->obs.first; od.day = ctx->obs.day; od.sample_depth = ctx->obs.samples; od.sample_stride = ctx->obs.stride;
+    od.first = ctx->obs.first; od.day = ctx->obs.day; od.sample_hh = ctx->obs.samples; od.sample_stride = ctx->obs.stride;
     od.first_stride = ctx->obs.first_stride; od.slot_base = ctx->obs.slot_base;
     ctx->last_path = 2;
     rc = run_ensemble(ctx, ic_dev, ic_per_member, &none, 0, M, st, &od);     // synchronises the stream (operand-range flag)
     if (rc) return rc;
+    // observations dropped at registration (land, lake) have no model value: their entries stay NaN (all bits set)
+    if (model_dev && ctx->obs.row_len)
+        CU(cudaMemset2DAsync(model_dev, (size_t)model_stride * sizeof(double), 0xff, (size_t)ctx->obs.row_len * sizeof(double), M, st));
     MisfitArgs ma;
-    ma.sample_depth = ctx->obs.samples; ma.stride = ctx->obs.stride;
-    ma.obs_slot = ctx->obs.o_slot; ma.obs_day = ctx->obs.o_day; ma.obs_cell = ctx->obs.o_cell; ma.obs_val = ctx->obs.val;
-    ma.conc = ctx->C; ma.plane = ctx->plane; ma.n_obs = ctx->obs.n_used;
-    ma.misfit = misfit_dev; ma.count = (long long *)count_dev;
-    ma.member_set = ctx->member_set_dev; ma.obs_begin = ctx->obs.obs_begin; ma.conc_set_stride = (long long)T * ctx->plane;
+    ma.samples = ctx->obs.samples; ma.stride = ctx->obs.stride;
+    ma.obs_slot = ctx->obs.o_slot; ma.obs_day = ctx->obs.o_day; ma.obs_cell = ctx->obs.o_cell; ma.src = ctx->obs.src;
+    ma.obs_val = ctx->obs.val; ma.sigma = ctx->obs.sigma; ma.kind_begin = ctx->obs.kind_begin;
+    ma.conc = ctx->C; ma.plane = ctx->plane; ma.k = ctx->k;
+    ma.chi2 = chi2_dev; ma.count = (long long *)count_dev; ma.n_kinds = n_kinds;
+    ma.model = model_dev; ma.model_stride = model_stride;
+    ma.member_set = ctx->member_set_dev; ma.conc_set_stride = (long long)T * ctx->plane;
     if (sets) misfit_finish_kernel<true><<<M, 256, 0, st>>>(ma);
     else misfit_finish_kernel<false><<<M, 256, 0, st>>>(ma);
     ctx->launches++;
     CU(cudaGetLastError());
     if (ctx->ens_status) return fail(NESOSIM_ERR_ARG, "an operand left the range of the season-resident kernel's fast divisions; misfit mode has no general-path fallback");
     return NESOSIM_OK;
+}
+
+extern "C" {
+
+// Observations of the calibration driver, compiled against the strip tables and kept on the device until they are
+// replaced: -> (strip, index in the strip's ocean list), sorted by owner and day, one sentinel per ocean cell.
+int nesosim_set_observations(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_day_host, const int32_t *obs_row_host,
+                             const int32_t *obs_col_host, const double *obs_depth_host) {
+    return register_observations(ctx, false, n_obs, nullptr, obs_day_host, obs_row_host, obs_col_host, nullptr,
+                                 obs_depth_host, nullptr);
+}
+
+int nesosim_set_observations_sets(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
+                                  const int32_t *obs_row_host, const int32_t *obs_col_host, const double *obs_depth_host) {
+    return register_observations(ctx, true, n_obs, obs_set_host, obs_day_host, obs_row_host, obs_col_host, nullptr,
+                                 obs_depth_host, nullptr);
+}
+
+int nesosim_set_observations_ex(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
+                                const int32_t *obs_row_host, const int32_t *obs_col_host, const int32_t *obs_kind_host,
+                                const double *obs_value_host, const double *obs_sigma_host) {
+    return register_observations(ctx, obs_set_host != nullptr, n_obs, obs_set_host, obs_day_host, obs_row_host,
+                                 obs_col_host, obs_kind_host, obs_value_host, obs_sigma_host);
+}
+
+int nesosim_observation_row_length(const nesosim_ctx *ctx, int64_t *row_len) {
+    if (!ctx || !row_len) return fail(NESOSIM_ERR_ARG, "bad argument");
+    if (!ctx->obs.ready) return fail(NESOSIM_ERR_STATE, "no observations are registered");
+    *row_len = ctx->obs.row_len;
+    return NESOSIM_OK;
+}
+
+int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                              int ic_per_member, double *misfit_dev, int64_t *count_dev, void *stream) {
+    return run_season_scores(ctx, params_host, ic_dev, ic_per_member, misfit_dev, count_dev, 1, nullptr, 0, stream);
+}
+
+int nesosim_run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                              int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
+                              int64_t model_stride, void *stream) {
+    return run_season_scores(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, NESOSIM_OBS_KINDS, model_dev,
+                             model_stride, stream);
 }
 
 int nesosim_set_async(nesosim_ctx *ctx, int on) {

@@ -268,6 +268,51 @@ class SnowBudgetEngine:
                                                           row.ctypes.data_as(i32), col.ctypes.data_as(i32),
                                                           depth.ctypes.data_as(C.POINTER(C.c_double))))
 
+    def set_observations_ex(self, day, row, col, value, kind=None, sigma=None, obs_set=None):
+        """Register observations of any kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``; None: all depth) with
+        an error each (``sigma``; None: all 1), on one shared forcing or (``obs_set`` given) tagged with their forcing set,
+        for ``run_season_scores`` (see nesosim_set_observations_ex)."""
+        day, row, col = (np.ascontiguousarray(np.asarray(a), dtype=np.int32) for a in (day, row, col))
+        value = np.ascontiguousarray(np.asarray(value), dtype=np.float64)
+        n = len(day)
+        opt = []
+        for a, dt in ((obs_set, np.int32), (kind, np.int32), (sigma, np.float64)):
+            a = None if a is None else np.ascontiguousarray(np.asarray(a), dtype=dt)
+            assert a is None or len(a) == n
+            opt.append(a)
+        assert len(row) == n and len(col) == n and len(value) == n
+        i32, f64 = C.POINTER(C.c_int32), C.POINTER(C.c_double)
+        s, k, sg = (None if a is None else a.ctypes.data_as(t) for a, t in zip(opt, (i32, i32, f64)))
+        _lib.check(self.lib.nesosim_set_observations_ex(self.handle, n, s, day.ctypes.data_as(i32), row.ctypes.data_as(i32),
+                                                        col.ctypes.data_as(i32), k, value.ctypes.data_as(f64), sg))
+
+    def observation_row_length(self):
+        """Entries of a member's model row: the largest number of input observations of one set."""
+        n = C.c_int64(0)
+        _lib.check(self.lib.nesosim_observation_row_length(self.handle, C.byref(n)))
+        return int(n.value)
+
+    def run_season_scores(self, params, ic, model=False):
+        """The season with the registered observations scored inside the fused path (nesosim_run_season_scores); returns
+        CUDA tensors (chi2[M, OBS_KINDS] float64, used[M, OBS_KINDS] int64, model[M, row_len] float64 or None): per kind
+        the sum of ((model - observed)/sigma)^2 and its number of finite terms, and the model value at every input
+        observation (NaN on land)."""
+        torch = _torch()
+        p = _lib.member_params_array(params)
+        assert len(p) == self.M
+        ic_t = None if ic is None else self._dev(ic)
+        per_member = 1 if (ic_t is not None and ic_t.dim() == 3 and self.M > 1) else 0
+        dev = "cuda:%d" % self.device
+        chi2 = torch.empty(self.M, _lib.OBS_KINDS, dtype=torch.float64, device=dev)
+        used = torch.empty(self.M, _lib.OBS_KINDS, dtype=torch.int64, device=dev)
+        mod = torch.empty(self.M, self.observation_row_length(), dtype=torch.float64, device=dev) if model else None
+        _lib.check(self.lib.nesosim_run_season_scores(self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member,
+                                                      chi2.data_ptr(), used.data_ptr(),
+                                                      None if mod is None else mod.data_ptr(),
+                                                      0 if mod is None else mod.shape[1], self._stream()))
+        self._keep = (ic_t, chi2, used, mod)
+        return chi2, used, mod
+
     def run_season_misfit(self, params, ic, obs=None):
         """The season with the calibration misfit reduced INSIDE the season-resident kernel (nesosim_run_season_misfit)
         against the registered observations (``obs`` given: registered first); returns CUDA tensors (misfit[M] float64,

@@ -14,6 +14,11 @@ all-gathered into member order (the only communication).
 
 scores every parameter set on several observed seasons at once: the (parameter set, season) pairs are the members of one
 batch of forcing sets, and the misfit of each pair is reduced against that season's observations.
+
+    res = run_calibration_scores(mask, seasons, params, dx, model=True)   # chi2/used [P, S, 3], model rows per season
+
+does the same with observation errors and three observed quantities (snow depth over ice, snow volume, bulk density):
+per kind the sum of ((model - observed)/sigma)^2, and optionally the model value at every observation.
 """
 import numpy as np
 
@@ -32,6 +37,66 @@ def depth_misfit(snowDepths, conc, obs):
     diff = model - depth.to(torch.float64).unsqueeze(0)
     ok = torch.isfinite(diff)
     return torch.where(ok, diff * diff, torch.zeros_like(diff)).sum(dim=1), ok.sum(dim=1)
+
+
+def normalize_observations(obs):
+    """A season's observations as a dict of numpy arrays day, row, col (int32), value, sigma (float64), kind (int32).
+    ``obs``: a dict with day, row, col, value and optionally kind (default depth) and sigma (default 1), or the 4-tuple
+    (day, row, col, depth), which means depth observations with sigma 1."""
+    from . import _lib
+    if not isinstance(obs, dict):
+        day, row, col, value = obs
+        obs = {"day": day, "row": row, "col": col, "value": value}
+    out = {k: np.asarray(obs[k], dtype=np.int32).ravel() for k in ("day", "row", "col")}
+    out["value"] = np.asarray(obs["value"], dtype=np.float64).ravel()
+    n = len(out["day"])
+    kind, sigma = obs.get("kind"), obs.get("sigma")
+    out["kind"] = np.full(n, _lib.OBS_DEPTH, np.int32) if kind is None else np.asarray(kind, dtype=np.int32).ravel()
+    out["sigma"] = np.ones(n) if sigma is None else np.asarray(sigma, dtype=np.float64).ravel()
+    if any(len(v) != n for v in out.values()):
+        raise ValueError("observation arrays of different lengths")
+    return out
+
+
+def check_observations(obs):
+    """Rejects what nesosim_set_observations_ex rejects beyond the grid and day range: a kind outside [0, OBS_KINDS), a
+    density observation on day 0 (the model has no density there) and a sigma that is not finite and > 0."""
+    from . import _lib
+    kind, sigma = obs["kind"], obs["sigma"]
+    if ((kind < 0) | (kind >= _lib.OBS_KINDS)).any():
+        raise ValueError("observation kind outside [0, %d)" % _lib.OBS_KINDS)
+    if ((kind == _lib.OBS_DENSITY) & (obs["day"] == 0)).any():
+        raise ValueError("density observation on day 0: the model has no density there")
+    if not (np.isfinite(sigma) & (sigma > 0)).all():
+        raise ValueError("observation error sigma must be finite and > 0")
+
+
+def observation_scores(snowDepths, density, conc, obs, mask=None):
+    """Per-member scores of ``obs`` (see ``normalize_observations``) on grids the season kernel does not take, from the
+    arrays ``run_season`` writes: ``snowDepths`` (M,T,2,ny,nx), ``density`` (M,T,ny,nx), ``conc`` (T,ny,nx), all on
+    one device.  Returns (chi2[M, OBS_KINDS], used[M, OBS_KINDS], model[M, n_obs]): the model value of every observation
+    (depth over ice (h0+h1)/conc, volume h0+h1, or density), and per kind the sum of the finite ((model - value)/sigma)^2
+    and their number -- what nesosim_run_season_scores reduces on the fused path.  ``mask`` (ny,nx) given: observations on
+    land or lake cells (outside 1..10) have the model value NaN and are skipped, as on the fused path."""
+    import torch
+    from . import _lib
+    obs = normalize_observations(obs)
+    check_observations(obs)
+    dev = snowDepths.device
+    day, row, col, kind = (torch.as_tensor(obs[k], device=dev).long() for k in ("day", "row", "col", "kind"))
+    value, sigma = (torch.as_tensor(obs[k], device=dev) for k in ("value", "sigma"))
+    vol = snowDepths[:, day, 0, row, col] + snowDepths[:, day, 1, row, col]          # (M, n_obs)
+    model = torch.where(kind == _lib.OBS_VOLUME, vol, density[:, day, row, col])
+    model = torch.where(kind == _lib.OBS_DEPTH, vol / conc[day, row, col], model)
+    if mask is not None:
+        m = np.asarray(mask)[obs["row"], obs["col"]]
+        model = torch.where(torch.as_tensor((m >= 1) & (m <= 10), device=dev), model, torch.full_like(model, float("nan")))
+    r = (model - value) / sigma
+    ok = torch.isfinite(r)
+    sq = torch.where(ok, r * r, torch.zeros_like(r))
+    chi2 = torch.stack([torch.where(kind == k, sq, torch.zeros_like(sq)).sum(dim=1) for k in range(_lib.OBS_KINDS)], 1)
+    used = torch.stack([(ok & (kind == k)).sum(dim=1) for k in range(_lib.OBS_KINDS)], 1)
+    return chi2, used, model
 
 
 def run_ensemble(mask, forcing, ic, params, dx, obs, rank=0, world=1, device=0, group=None, fused=None, **flags):
@@ -96,25 +161,36 @@ def gather_calibration(mis, used, P, S, rank=0, world=1, group=None):
     return assemble_calibration(mis.cpu().numpy(), P, S), assemble_calibration(used.cpu().numpy(), P, S)
 
 
-def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, **flags):
-    """Multi-season calibration: every parameter set scored on every observed season in one native call per rank.
-    ``seasons``: list of {"forcing": dict of (T_s,ny,nx) / drift (T_s,2,ny,nx) arrays, "ic": (ny,nx),
-    "obs": (day, row, col, depth)}, each with its own length T_s.  Returns (misfit[P,S], used[P,S]) as numpy arrays,
-    identical on every rank.  A rank stages only the seasons its (parameter set, season) pairs use, stacked as forcing
-    sets of the longest of them, with each member's season IC as a per-member IC.  ``fused`` as in ``run_ensemble``:
-    None = observations reduced inside the season kernel where it applies, True = insist on it, False = depths to HBM
-    and a per-season reduction there."""
-    import torch
+def assemble_scores(chi2, used, model, P, S, n_obs):
+    """Scores of all P*S members in member order -> {"chi2": [P, S, OBS_KINDS], "used": [P, S, OBS_KINDS], "model": per
+    season s the array [P, n_obs[s]] (rows padded to the largest season: the padding is dropped), or None}."""
     from . import _lib
+    out = {"chi2": np.asarray(chi2).reshape(P, S, _lib.OBS_KINDS), "used": np.asarray(used).reshape(P, S, _lib.OBS_KINDS),
+           "model": None}
+    if model is not None:
+        m = np.asarray(model).reshape(P, S, -1)
+        out["model"] = [m[:, s, :n_obs[s]] for s in range(S)]
+    return out
+
+
+def gather_scores(chi2, used, model, P, S, n_obs, rank=0, world=1, group=None):
+    """All-gather the ranks' per-member scores (model rows padded to the largest season) and reassemble them as numpy
+    arrays (``assemble_scores``), identical on every rank."""
+    if world > 1:
+        chi2 = sharding.gather_member_results(chi2, P * S, rank, world, group)
+        used = sharding.gather_member_results(used, P * S, rank, world, group)
+        if model is not None:
+            model = sharding.gather_member_results(model, P * S, rank, world, group)
+    return assemble_scores(chi2.cpu().numpy(), used.cpu().numpy(), None if model is None else model.cpu().numpy(),
+                           P, S, n_obs)
+
+
+def stage_calibration(mask, seasons, params, dx, plan, device=0, **flags):
+    """The native call of a calibration rank: the seasons its pairs use (``plan`` = ``calibration_plan``) stacked as
+    forcing sets of the longest of them, on a context of one member per pair, season by season, with each member's season
+    IC as a per-member IC.  Returns (engine, parameters [M, 4], IC) of those members."""
     from .engine import SnowBudgetEngine
-    params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
-    P, S = len(params), len(seasons)
-    plan = calibration_plan(P, S, rank, world)
-    pairs, staged, order, member_set = plan["pairs"], plan["seasons"], plan["order"], plan["member_set"]
-    dev = "cuda:%d" % device
-    if not pairs:   # more ranks than members: nothing to run, but the gather still needs this rank
-        mis, used = torch.zeros(0, dtype=torch.float64, device=dev), torch.zeros(0, dtype=torch.int64, device=dev)
-        return gather_calibration(mis, used, P, S, rank, world, group)
+    staged, member_set = plan["seasons"], plan["member_set"]
     days = [int(seasons[s]["forcing"]["precip"].shape[0]) for s in staged]
     T = max(days)
 
@@ -126,15 +202,37 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
         return out
 
     forcing = {k: stack(k) for k in ("precip", "conc", "wind", "drift")}
-    run = [pairs[i] for i in order]                 # the native call's members, season by season
+    run = [plan["pairs"][i] for i in plan["order"]]   # the native call's members, season by season
     ic = np.stack([np.asarray(seasons[s]["ic"], dtype=np.float64) for _, s in run])
-    mine = params[[p for p, _ in run]]
     M = len(run)
     eng = SnowBudgetEngine(mask, T, dx, n_members=M, device=device, **flags)
     eng.set_forcing_sets(forcing["precip"], forcing["conc"], forcing["wind"], forcing["drift"], member_set, days)
+    return eng, params[[p for p, _ in run]], (ic if M > 1 else ic[0])
+
+
+def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, **flags):
+    """Multi-season calibration: every parameter set scored on every observed season in one native call per rank.
+    ``seasons``: list of {"forcing": dict of (T_s,ny,nx) / drift (T_s,2,ny,nx) arrays, "ic": (ny,nx),
+    "obs": (day, row, col, depth)}, each with its own length T_s.  Returns (misfit[P,S], used[P,S]) as numpy arrays,
+    identical on every rank.  A rank stages only the seasons its (parameter set, season) pairs use, stacked as forcing
+    sets of the longest of them, with each member's season IC as a per-member IC.  ``fused`` as in ``run_ensemble``:
+    None = observations reduced inside the season kernel where it applies, True = insist on it, False = depths to HBM
+    and a per-season reduction there."""
+    import torch
+    from . import _lib
+    params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
+    P, S = len(params), len(seasons)
+    plan = calibration_plan(P, S, rank, world)
+    pairs, staged, order, member_set = plan["pairs"], plan["seasons"], plan["order"], plan["member_set"]
+    dev = "cuda:%d" % device
+    if not pairs:   # more ranks than members: nothing to run, but the gather still needs this rank
+        mis, used = torch.zeros(0, dtype=torch.float64, device=dev), torch.zeros(0, dtype=torch.int64, device=dev)
+        return gather_calibration(mis, used, P, S, rank, world, group)
+    eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
+    M = len(mine)
 
     def hbm_round_trip():
-        out = eng.run_season(mine, ic if M > 1 else ic[0], eng.alloc_outputs(names=("snowDepths",)))["snowDepths"]
+        out = eng.run_season(mine, ic, eng.alloc_outputs(names=("snowDepths",)))["snowDepths"]
         mis = torch.zeros(M, dtype=torch.float64, device=out.device)
         used = torch.zeros(M, dtype=torch.int64, device=out.device)
         for i, s in enumerate(staged):
@@ -151,7 +249,7 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
                 cols = [np.concatenate([np.asarray(seasons[s]["obs"][j]).ravel() for s in staged]) for j in range(4)]
                 tag = np.concatenate([np.full(len(seasons[s]["obs"][0]), i, dtype=np.int32) for i, s in enumerate(staged)])
                 eng.set_observations_sets(tag, *cols)
-                mis, used = eng.run_season_misfit(mine, ic if M > 1 else ic[0])
+                mis, used = eng.run_season_misfit(mine, ic)
             except _lib.NesosimError as e:
                 if fused is True or e.code != _lib.ERR_ARG:
                     raise
@@ -161,3 +259,68 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
         eng.close()
     back = torch.as_tensor(np.argsort(order), device=mis.device)     # native member order -> this rank's pair order
     return gather_calibration(mis[back], used[back], P, S, rank, world, group)
+
+
+def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, model=False,
+                           **flags):
+    """``run_calibration`` with observation errors and three observed quantities.  A season's ``"obs"`` is a dict with
+    day, row, col, value and optionally kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``, default depth) and
+    sigma (default 1), or the 4-tuple (day, row, col, depth).  Returns {"chi2": [P, S, OBS_KINDS], "used": [P, S,
+    OBS_KINDS], "model": per season the array [P, n_obs] of model values (NaN on land), or None unless ``model``}, numpy,
+    identical on every rank.  ``fused`` as in ``run_calibration``: None = scored inside the fused path where it applies
+    (falling back on grids wider than the season kernel takes), True = insist on it, False = snowDepths and density to
+    HBM and ``observation_scores`` there.  Bad kinds, sigmas and density observations on day 0 raise ValueError before
+    any device work, on either path."""
+    import torch
+    from . import _lib
+    params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
+    P, S = len(params), len(seasons)
+    obs = [normalize_observations(s["obs"]) for s in seasons]
+    for o in obs:
+        check_observations(o)
+    n_obs = [len(o["day"]) for o in obs]
+    width = max(n_obs, default=0)
+    plan = calibration_plan(P, S, rank, world)
+    pairs, staged, order, member_set = plan["pairs"], plan["seasons"], plan["order"], plan["member_set"]
+    dev = "cuda:%d" % device
+    K = _lib.OBS_KINDS
+    if not pairs:   # more ranks than members: nothing to run, but the gather still needs this rank
+        chi2, used = torch.zeros(0, K, dtype=torch.float64, device=dev), torch.zeros(0, K, dtype=torch.int64, device=dev)
+        mod = torch.zeros(0, width, dtype=torch.float64, device=dev) if model else None
+        return gather_scores(chi2, used, mod, P, S, n_obs, rank, world, group)
+    eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
+    M = len(mine)
+
+    def hbm_round_trip():
+        out = eng.run_season(mine, ic, eng.alloc_outputs(names=("snowDepths", "density")))
+        chi2 = torch.zeros(M, K, dtype=torch.float64, device=dev)
+        used = torch.zeros(M, K, dtype=torch.int64, device=dev)
+        mod = torch.full((M, width), float("nan"), dtype=torch.float64, device=dev)
+        for i, s in enumerate(staged):
+            sel = torch.as_tensor(np.flatnonzero(member_set == i), device=dev)
+            c, u, m = observation_scores(out["snowDepths"][sel], out["density"][sel], eng._forcing[1][i], obs[s], mask)
+            chi2[sel], used[sel], mod[sel, :n_obs[s]] = c, u.to(torch.int64), m
+        return chi2, used, mod
+
+    try:
+        if fused is False:
+            chi2, used, mod = hbm_round_trip()
+        else:
+            try:
+                cols = {k: np.concatenate([obs[s][k] for s in staged]) for k in obs[0]}
+                tag = np.concatenate([np.full(n_obs[s], i, dtype=np.int32) for i, s in enumerate(staged)])
+                eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"],
+                                        cols["sigma"], obs_set=tag)
+                chi2, used, m = eng.run_season_scores(mine, ic, model=model)
+                if model:   # rows of the staged seasons' length -> the largest season's (NaN past a row's end)
+                    mod = torch.full((M, width), float("nan"), dtype=torch.float64, device=dev)
+                    mod[:, :m.shape[1]] = m
+            except _lib.NesosimError as e:
+                if fused is True or e.code != _lib.ERR_ARG:
+                    raise
+                # grids the season-resident kernel does not take: snowDepths and density to HBM, scored there per season
+                chi2, used, mod = hbm_round_trip()
+    finally:
+        eng.close()
+    back = torch.as_tensor(np.argsort(order), device=chi2.device)    # native member order -> this rank's pair order
+    return gather_scores(chi2[back], used[back], mod[back] if model else None, P, S, n_obs, rank, world, group)
