@@ -58,10 +58,18 @@ def normalize_observations(obs):
     return out
 
 
-def check_observations(obs):
-    """Rejects what nesosim_set_observations_ex rejects beyond the grid and day range: a kind outside [0, OBS_KINDS), a
-    density observation on day 0 (the model has no density there) and a sigma that is not finite and > 0."""
+def check_observations(obs, shape=None, days=None):
+    """Rejects what nesosim_set_observations_ex rejects: a kind outside [0, OBS_KINDS), a density observation on day 0
+    (the model has no density there) and a sigma that is not finite and > 0; with ``shape`` = (ny, nx) a row or column
+    outside the grid, with ``days`` a day outside [0, days) of the observations' own season.  (Indexing the model's
+    arrays with such an observation would wrap around, read a slot past the season, or fault on the device.)"""
     from . import _lib
+    if shape is not None:
+        ny, nx = shape
+        if ((obs["row"] < 0) | (obs["row"] >= ny) | (obs["col"] < 0) | (obs["col"] >= nx)).any():
+            raise ValueError("observation outside the %d x %d grid" % (ny, nx))
+    if days is not None and ((obs["day"] < 0) | (obs["day"] >= days)).any():
+        raise ValueError("observation day outside its season [0, %d)" % days)
     kind, sigma = obs["kind"], obs["sigma"]
     if ((kind < 0) | (kind >= _lib.OBS_KINDS)).any():
         raise ValueError("observation kind outside [0, %d)" % _lib.OBS_KINDS)
@@ -69,6 +77,17 @@ def check_observations(obs):
         raise ValueError("density observation on day 0: the model has no density there")
     if not (np.isfinite(sigma) & (sigma > 0)).all():
         raise ValueError("observation error sigma must be finite and > 0")
+
+
+def season_observations(mask, seasons):
+    """Every season's observations, normalized and checked against the grid and that season's own length -- all seasons
+    on every rank, so that the ranks raise alike and before any device work."""
+    out = []
+    for s in seasons:
+        o = normalize_observations(s["obs"])
+        check_observations(o, np.shape(mask), np.shape(s["forcing"]["precip"])[0])
+        out.append(o)
+    return out
 
 
 def observation_scores(snowDepths, density, conc, obs, mask=None):
@@ -81,7 +100,7 @@ def observation_scores(snowDepths, density, conc, obs, mask=None):
     import torch
     from . import _lib
     obs = normalize_observations(obs)
-    check_observations(obs)
+    check_observations(obs, tuple(snowDepths.shape[-2:]), snowDepths.shape[1])
     dev = snowDepths.device
     day, row, col, kind = (torch.as_tensor(obs[k], device=dev).long() for k in ("day", "row", "col", "kind"))
     value, sigma = (torch.as_tensor(obs[k], device=dev) for k in ("value", "sigma"))
@@ -102,13 +121,15 @@ def observation_scores(snowDepths, density, conc, obs, mask=None):
 def run_ensemble(mask, forcing, ic, params, dx, obs, rank=0, world=1, device=0, group=None, fused=None, **flags):
     """Returns (misfit[M], n_used[M]) as numpy arrays in member order (identical on every rank).  ``fused``: None =
     inside the season kernel where it applies, True = insist on it, False = depths to HBM + reduction there (the
-    round-1 path, kept as the cross-check)."""
+    round-1 path, kept as the cross-check).  Observations outside the grid or the season's days raise ValueError
+    before any device work, on either path."""
     import torch
     from .engine import SnowBudgetEngine
     params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
     M = len(params)
     lo, hi = sharding.member_range(M, rank, world)
     T = forcing["precip"].shape[0]
+    check_observations(normalize_observations(obs), np.shape(mask), T)
     eng = SnowBudgetEngine(mask, T, dx, n_members=hi - lo, device=device, **flags)
     eng.set_forcing(forcing["precip"], forcing["conc"], forcing["wind"], forcing["drift"])
     from . import _lib
@@ -217,11 +238,13 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
     identical on every rank.  A rank stages only the seasons its (parameter set, season) pairs use, stacked as forcing
     sets of the longest of them, with each member's season IC as a per-member IC.  ``fused`` as in ``run_ensemble``:
     None = observations reduced inside the season kernel where it applies, True = insist on it, False = depths to HBM
-    and a per-season reduction there."""
+    and a per-season reduction there.  Observations outside the grid or outside their season's days raise ValueError
+    before any device work, on either path."""
     import torch
     from . import _lib
     params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
     P, S = len(params), len(seasons)
+    season_observations(mask, seasons)
     plan = calibration_plan(P, S, rank, world)
     pairs, staged, order, member_set = plan["pairs"], plan["seasons"], plan["order"], plan["member_set"]
     dev = "cuda:%d" % device
@@ -269,15 +292,13 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     OBS_KINDS], "model": per season the array [P, n_obs] of model values (NaN on land), or None unless ``model``}, numpy,
     identical on every rank.  ``fused`` as in ``run_calibration``: None = scored inside the fused path where it applies
     (falling back on grids wider than the season kernel takes), True = insist on it, False = snowDepths and density to
-    HBM and ``observation_scores`` there.  Bad kinds, sigmas and density observations on day 0 raise ValueError before
-    any device work, on either path."""
+    HBM and ``observation_scores`` there.  Observations outside the grid or outside their season's days, bad kinds,
+    sigmas and density observations on day 0 raise ValueError before any device work, on either path."""
     import torch
     from . import _lib
     params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
     P, S = len(params), len(seasons)
-    obs = [normalize_observations(s["obs"]) for s in seasons]
-    for o in obs:
-        check_observations(o)
+    obs = season_observations(mask, seasons)
     n_obs = [len(o["day"]) for o in obs]
     width = max(n_obs, default=0)
     plan = calibration_plan(P, S, rank, world)
