@@ -235,6 +235,45 @@ int nesosim_run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *par
                               int ic_per_member, double *chi2_dev, int64_t *count_dev,
                               double *model_dev, int64_t model_stride, void *stream);
 
+/* Footprint observations: means over many cells and/or days (drifting-station climatologies, monthly gridded products,
+ * basin means).  A footprint belongs to one forcing set (fp_set NULL: one shared forcing), has a kind (fp_kind NULL: all
+ * depth), an observed value, a sigma (fp_sigma NULL: all 1) and the points [fp_begin[g], fp_begin[g+1]) of the
+ * pt_* arrays, each (day, row, col, weight) (pt_weight NULL: all 1).  nesosim_set_observations_fp registers point
+ * observations (exactly as nesosim_set_observations_ex) and footprints together and replaces what was registered.
+ * Footprint points on land or lake cells are dropped, as point observations are.  The points share the sample slots of
+ * the observed (cell, day) pairs with the point observations but never enter the point tables: the point results are
+ * bit-identical with and without footprints.
+ * nesosim_run_season_scores_fp writes the point outputs of nesosim_run_season_scores, and per member m: the model value
+ * of footprint g, fp_model_dev[m*fp_model_stride + g] (g = its index among its set's input footprints; padding past
+ * the set's count up to the row length is NaN), and per kind fp_chi2_dev[m][k] = the sum of the finite
+ * ((model - value)/sigma)^2 over the set's footprints of kind k, fp_count_dev[m][k] their number (may be NULL).
+ * The model value of a footprint is the weighted mean of its points' model values (the operators of the point
+ * observations), over the points whose value is finite, in a fixed order: the footprint's j-th kept point (input order)
+ * goes to lane j % 32 of one warp, which adds w*v and w in order from 0.0; lane 0 collects both with the shuffle-down
+ * tree 16, 8, 4, 2, 1; the mean is their quotient, NaN when no point was finite.  The footprint terms are summed as the
+ * point terms (one kind's range, in input order within the set, thread i % 256 of one block).  Five launches: the
+ * pre-pass (2), the season kernel, the footprint means, the epilogue.  While footprints are registered,
+ * nesosim_run_season_misfit and nesosim_run_season_scores return NESOSIM_ERR_STATE (they would drop them).
+ * NESOSIM_ERR_ARG: whatever nesosim_set_observations_ex rejects; fp_begin not starting at 0 or not increasing (an
+ * empty footprint); a weight that is not finite and > 0; a kind, sigma or set tag as for point observations; a point
+ * outside the grid or outside its set's season; a density point on day 0; a set's slots or points that do not fit
+ * int indices; fp_model_stride < the footprint row length.  A rejected registration leaves the previous one in force;
+ * the stale-layout rule of nesosim_set_observations_sets applies unchanged. */
+int nesosim_set_observations_fp(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host,
+                                const int32_t *obs_day_host, const int32_t *obs_row_host, const int32_t *obs_col_host,
+                                const int32_t *obs_kind_host, const double *obs_value_host, const double *obs_sigma_host,
+                                int64_t n_fp, const int32_t *fp_set_host, const int32_t *fp_kind_host,
+                                const double *fp_value_host, const double *fp_sigma_host, const int64_t *fp_begin_host,
+                                const int32_t *pt_day_host, const int32_t *pt_row_host, const int32_t *pt_col_host,
+                                const double *pt_weight_host);
+/* length of a member's footprint model row: the largest number of input footprints of one set (0: none) */
+int nesosim_footprint_row_length(const nesosim_ctx *ctx, int64_t *row_len);
+/* fp_chi2_dev [M][NESOSIM_OBS_KINDS]; fp_count_dev same shape or NULL; fp_model_dev [M][fp_model_stride] or NULL */
+int nesosim_run_season_scores_fp(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                                 int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
+                                 int64_t model_stride, double *fp_chi2_dev, int64_t *fp_count_dev,
+                                 double *fp_model_dev, int64_t fp_model_stride, void *stream);
+
 /* Asynchronous mode.  By default nesosim_run_season on the season-resident path synchronises `stream` once to read
  * the kernel's operand-range flag (see above).  With nesosim_set_async(ctx, 1) it never synchronises: the flag is copied
  * to pinned host memory behind the kernel and examined by nesosim_sync (which waits for every season enqueued so far on

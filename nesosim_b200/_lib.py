@@ -99,6 +99,16 @@ _SIGNATURES = {
     "nesosim_observation_row_length": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "nesosim_run_season_scores": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "nesosim_set_observations_fp": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_int64,
+                                              C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double),
+                                              C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
+    "nesosim_footprint_row_length": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "nesosim_run_season_scores_fp": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_int64, C.c_void_p]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

@@ -3,6 +3,7 @@
 
 #include <chrono>
 #include <cmath>
+#include <climits>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -209,6 +210,17 @@ struct nesosim_ctx {
         std::vector<int> set_days;
         long long first_stride = 0;                      // entries of one set's `first` table
         int *slot_base = nullptr;                        // [sets] the set's first slot in `day`
+        // footprints (nesosim_set_observations_fp): every set's footprints one set after the other, each set's
+        // stable-partitioned by kind; the points of footprint q are [fp_begin[q], fp_begin[q+1]) of the pt_* tables
+        long long n_fp = 0;                              // footprints registered (0: point observations only)
+        long long fp_row_len = 0;                        // the largest number of input footprints of one set
+        long long *fp_begin = nullptr;                   // [n_fp+1]
+        int *fp_kind = nullptr, *fp_src = nullptr;       // per footprint: kind, index among its set's input footprints
+        double *fp_val = nullptr, *fp_sigma = nullptr;   // per footprint: observed value, error
+        int *fp_kind_begin = nullptr;                    // [sets][NESOSIM_OBS_KINDS+1] every set's footprints, by kind
+        int *pt_slot = nullptr, *pt_day = nullptr, *pt_cell = nullptr;   // per footprint point: sample slot, day, cell,
+        double *pt_w = nullptr;                          // weight
+        double *fp_mean = nullptr;                       // [M][max(1, fp_row_len)] footprint means in table order
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -356,6 +368,9 @@ void obs_release(nesosim_ctx *ctx) {
     cudaFree(ob.first); cudaFree(ob.day); cudaFree(ob.val); cudaFree(ob.sigma); cudaFree(ob.samples);
     cudaFree(ob.o_slot); cudaFree(ob.o_day); cudaFree(ob.o_cell); cudaFree(ob.src);
     cudaFree(ob.kind_begin); cudaFree(ob.slot_base);
+    cudaFree(ob.fp_begin); cudaFree(ob.fp_kind); cudaFree(ob.fp_src); cudaFree(ob.fp_val); cudaFree(ob.fp_sigma);
+    cudaFree(ob.fp_kind_begin); cudaFree(ob.pt_slot); cudaFree(ob.pt_day); cudaFree(ob.pt_cell); cudaFree(ob.pt_w);
+    cudaFree(ob.fp_mean);
     ob = {};
 }
 
@@ -1213,7 +1228,37 @@ struct MisfitArgs {
     long long model_stride;
     const int *member_set;          // SETS only
     long long conc_set_stride;      // SETS only: T * plane
+    // footprint stage (nesosim_run_season_scores_fp), skipped when fp_chi2 is NULL: the footprint means of
+    // footprint_mean_kernel scored per kind exactly as the point observations
+    const double *fp_mean;          // [M][fp_stride] in table order within the member's set
+    long long fp_stride;
+    const double *fp_val, *fp_sigma;
+    const int *fp_kind_begin;       // [sets][NESOSIM_OBS_KINDS+1]
+    double *fp_chi2;                // [M][NESOSIM_OBS_KINDS] or NULL
+    long long *fp_count;            // same shape, or NULL
 };
+
+// The fixed-order block total of the thread partial sums (acc, cnt): shuffle-down tree per warp, then the 8 warps one
+// after the other; thread 0 gets the result.  Ends with a barrier, so red / redc can be reused at once.
+__device__ __forceinline__ void block_total(double acc, long long cnt, double *red, long long *redc, double *total,
+                                            long long *total_count) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        acc = add(acc, __shfl_down_sync(0xffffffffu, acc, off));
+        cnt += __shfl_down_sync(0xffffffffu, cnt, off);
+    }
+    if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = acc; redc[threadIdx.x >> 5] = cnt; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        long long n = 0;
+        for (int w = 0; w < 8; ++w) { t = add(t, red[w]); n += redc[w]; }
+        *total = t;
+        if (total_count) *total_count = n;
+    }
+    __syncthreads();
+}
+
 template <bool SETS>
 __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constant__ MisfitArgs a) {
     const int m = blockIdx.x;
@@ -1242,21 +1287,114 @@ __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constan
                 ++cnt;
             }
         }
+        block_total(acc, cnt, red, redc, a.chi2 + (long long)m * a.n_kinds + kind,
+                    a.count ? a.count + (long long)m * a.n_kinds + kind : nullptr);
+    }
+    if (!a.fp_chi2) return;
+    // footprints: the same fixed order over each kind's range of the set's footprint table
+    const int *fkb = a.fp_kind_begin + set * (NESOSIM_OBS_KINDS + 1);
+    const double *mean = a.fp_mean + (long long)m * a.fp_stride - fkb[0];   // indexed by table position
+    for (int kind = 0; kind < NESOSIM_OBS_KINDS; ++kind) {
+        const long long i0 = fkb[kind], n_fp = (long long)fkb[kind + 1] - i0;
+        double acc = 0.0;
+        long long cnt = 0;
+        for (long long i = threadIdx.x; i < n_fp; i += 256) {
+            const long long q = i0 + i;
+            const double r = div_ieee(sub(mean[q], a.fp_val[q]), a.fp_sigma[q]);
+            if (nesosim::finite(r)) {
+                acc = add(acc, mul(r, r));
+                ++cnt;
+            }
+        }
+        block_total(acc, cnt, red, redc, a.fp_chi2 + (long long)m * NESOSIM_OBS_KINDS + kind,
+                    a.fp_count ? a.fp_count + (long long)m * NESOSIM_OBS_KINDS + kind : nullptr);
+    }
+}
+
+// Footprint means: one warp per (member, footprint).  The model value of every point is formed with exactly the
+// operator of misfit_finish_kernel (depth (h0+h1)/iceConc, volume h0+h1, density densityCalc).  Point j of the
+// footprint (in input order, land points dropped at registration) belongs to lane j % 32, which adds w*v to sw and w to
+// s in order, skipping non-finite v; lane 0 collects both with the shuffle-down tree 16, 8, 4, 2, 1, and the mean is
+// sw / s (NaN when no point was finite: 0/0).  Each lane keeps FP_UNROLL points' loads in flight: a monthly regional
+// mean has tens of thousands of points.  A block is one warp: footprints differ in size by orders of magnitude, and a
+// finished warp's slot is refilled at once instead of waiting for the longest warp of its block.  The point tables do
+// not depend on the member, so the warps of every member on the same footprint (adjacent blocks: block = footprint *
+// M + member) read them from L2.  Warps past the set's footprint count write the NaN padding of the caller's model row.
+struct FootprintArgs {
+    const double2 *samples;         // [M][stride]
+    long long stride;
+    const long long *begin;         // [n_fp+1]
+    const int *kind, *src;
+    const int *pt_slot, *pt_day, *pt_cell;
+    const double *pt_w;
+    const int *kind_begin;          // [sets][NESOSIM_OBS_KINDS+1]
+    const double *conc;             // [T][plane] (SETS: [sets][T][plane])
+    long long plane;
+    ModelConsts k;
+    int n_members;
+    long long row_len;              // footprints per member row (the largest set's)
+    double *mean;                   // [M][mean_stride] in table order within the set
+    long long mean_stride;
+    double *model;                  // [M][model_stride] at the input index within the set, or NULL
+    long long model_stride;
+    const int *member_set;          // SETS only
+    long long conc_set_stride;      // SETS only
+};
+constexpr int FP_UNROLL = 8;
+template <bool SETS>
+__global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constant__ FootprintArgs a) {
+    const int m = (int)(blockIdx.x % (unsigned)a.n_members);
+    const long long g = blockIdx.x / (unsigned)a.n_members;
+    const int lane = threadIdx.x;
+    if (g >= a.row_len) return;
+    const int set = SETS ? a.member_set[m] : 0;
+    const int *kb = a.kind_begin + set * (NESOSIM_OBS_KINDS + 1);
+    double *model = a.model ? a.model + (long long)m * a.model_stride : nullptr;
+    if (g >= (long long)kb[NESOSIM_OBS_KINDS] - kb[0]) {          // padding of a set with fewer footprints
+        if (model && lane == 0) model[g] = nesosim::qnan();
+        return;
+    }
+    const long long q = kb[0] + g;
+    const int kind = a.kind[q];
+    const double2 *samp = a.samples + (long long)m * a.stride;
+    const double *conc = SETS ? a.conc + (long long)set * a.conc_set_stride : a.conc;
+    const long long p1 = a.begin[q + 1];
+    double sw = 0.0, s = 0.0;
+    for (long long p = a.begin[q] + lane; p < p1; p += 32 * FP_UNROLL) {
+        double2 h[FP_UNROLL];
+        double w[FP_UNROLL], c[FP_UNROLL];
 #pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            acc = add(acc, __shfl_down_sync(0xffffffffu, acc, off));
-            cnt += __shfl_down_sync(0xffffffffu, cnt, off);
+        for (int u = 0; u < FP_UNROLL; ++u) {
+            const long long pp = p + 32 * u;
+            if (pp < p1) {
+                h[u] = samp[__ldg(a.pt_slot + pp)];
+                w[u] = __ldg(a.pt_w + pp);
+                c[u] = kind == NESOSIM_OBS_DEPTH ? __ldg(conc + (long long)__ldg(a.pt_day + pp) * a.plane + __ldg(a.pt_cell + pp)) : 1.0;
+            }
         }
-        if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = acc; redc[threadIdx.x >> 5] = cnt; }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            double t = 0.0;
-            long long n = 0;
-            for (int w = 0; w < 8; ++w) { t = add(t, red[w]); n += redc[w]; }
-            a.chi2[(long long)m * a.n_kinds + kind] = t;
-            if (a.count) a.count[(long long)m * a.n_kinds + kind] = n;
+#pragma unroll
+        for (int u = 0; u < FP_UNROLL; ++u) {
+            if (p + 32 * u < p1) {
+                double v;
+                if (kind == NESOSIM_OBS_DEPTH) v = div_ieee(add(h[u].x, h[u].y), c[u]);
+                else if (kind == NESOSIM_OBS_VOLUME) v = add(h[u].x, h[u].y);
+                else v = density_variable(h[u].x, h[u].y, false, a.k);
+                if (nesosim::finite(v)) {
+                    sw = add(sw, mul(w[u], v));
+                    s = add(s, w[u]);
+                }
+            }
         }
-        __syncthreads();                                 // red / redc are reused by the next kind
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        sw = add(sw, __shfl_down_sync(0xffffffffu, sw, off));
+        s = add(s, __shfl_down_sync(0xffffffffu, s, off));
+    }
+    if (lane == 0) {
+        const double v = div_ieee(sw, s);
+        a.mean[(long long)m * a.mean_stride + g] = v;
+        if (model) model[a.src[q]] = v;
     }
 }
 
@@ -1292,8 +1430,10 @@ std::vector<int> obs_owners(nesosim_ctx *ctx, int *list_end) {
     return owner;
 }
 
-// appends one season's observations to `t`; returns the number of sample slots it added (sentinels included)
-size_t compile_obs_set(std::vector<ObsPoint> &obs, int list_end, ObsTables &t) {
+// appends one season's observations to `t`; returns the number of sample slots it added (sentinels included).
+// Footprint points (kind -1, src = their index in the set's point table) take part in the slot assignment only:
+// pt_slot[src] receives their slot, and they never enter the observation tables.
+size_t compile_obs_set(std::vector<ObsPoint> &obs, int list_end, ObsTables &t, std::vector<int> &pt_slot) {
     std::stable_sort(obs.begin(), obs.end(), [](const ObsPoint &x, const ObsPoint &y) { return x.owner != y.owner ? x.owner < y.owner : x.day < y.day; });
     const size_t f0 = t.first.size(), s0 = t.slot_day.size();
     t.first.resize(f0 + (size_t)list_end + 1, -1);
@@ -1305,6 +1445,7 @@ size_t compile_obs_set(std::vector<ObsPoint> &obs, int list_end, ObsTables &t) {
         while (p < obs.size() && obs[p].owner == o) {
             if (t.slot_day.size() - s0 == (size_t)t.first[f0 + o] || t.slot_day.back() != obs[p].day) t.slot_day.push_back(obs[p].day);
             slot[p] = (int)(t.slot_day.size() - s0) - 1;
+            if (obs[p].kind < 0) pt_slot[obs[p].src] = slot[p];
             ++p;
         }
         t.slot_day.push_back(0x7fffffff);                // sentinel
@@ -1358,14 +1499,83 @@ int upload_obs(nesosim_ctx *ctx, const ObsTables &t, long long stride) {
     return NESOSIM_OK;
 }
 
-// Validates every observation, then compiles them against the strip tables and replaces the context's observations.
-// sets: tagged with their forcing set (obs_set_host); else one shared forcing.  Nothing is freed before the last check.
+// Footprints of one set as the registration collects them: per footprint (input order within the set) its kind,
+// value, sigma and range of kept points in the set's point arrays.
+struct FpSet {
+    std::vector<int> kind;
+    std::vector<double> val, sigma;
+    std::vector<long long> begin{0};                     // [footprints+1] into the point arrays
+    std::vector<int> pt_slot, pt_day, pt_cell;
+    std::vector<double> pt_w;
+};
+struct FpTables {
+    std::vector<long long> begin;
+    std::vector<int> kind, src, kind_begin, pt_slot, pt_day, pt_cell;
+    std::vector<double> val, sigma, pt_w;
+};
+
+// appends one set's footprints to `t`, stable-partitioned by kind (each kind's footprints in input order)
+void append_fp_set(const FpSet &f, FpTables &t) {
+    for (int k = 0; k < NESOSIM_OBS_KINDS; ++k) {
+        t.kind_begin.push_back((int)t.kind.size());
+        for (size_t g = 0; g < f.kind.size(); ++g) {
+            if (f.kind[g] != k) continue;
+            t.begin.push_back((long long)t.pt_slot.size());
+            t.kind.push_back(k);
+            t.src.push_back((int)g);
+            t.val.push_back(f.val[g]);
+            t.sigma.push_back(f.sigma[g]);
+            const long long b = f.begin[g], e = f.begin[g + 1];
+            t.pt_slot.insert(t.pt_slot.end(), f.pt_slot.begin() + b, f.pt_slot.begin() + e);
+            t.pt_day.insert(t.pt_day.end(), f.pt_day.begin() + b, f.pt_day.begin() + e);
+            t.pt_cell.insert(t.pt_cell.end(), f.pt_cell.begin() + b, f.pt_cell.begin() + e);
+            t.pt_w.insert(t.pt_w.end(), f.pt_w.begin() + b, f.pt_w.begin() + e);
+        }
+    }
+    t.kind_begin.push_back((int)t.kind.size());
+}
+
+template <typename T>
+int upload_vec(T **dst, const std::vector<T> &v) {
+    CU(cudaMalloc(dst, std::max<size_t>(1, v.size()) * sizeof(T)));
+    if (!v.empty()) CU(cudaMemcpy(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+    return NESOSIM_OK;
+}
+
+// adds the footprint tables `t` to the context's freshly uploaded observations
+int upload_fp(nesosim_ctx *ctx, FpTables &t, long long row_len) {
+    auto &ob = ctx->obs;
+    t.begin.push_back((long long)t.pt_slot.size());
+    ob.n_fp = (long long)t.kind.size();
+    ob.fp_row_len = row_len;
+    int rc;
+    if ((rc = upload_vec(&ob.fp_begin, t.begin)) || (rc = upload_vec(&ob.fp_kind, t.kind)) ||
+        (rc = upload_vec(&ob.fp_src, t.src)) || (rc = upload_vec(&ob.fp_val, t.val)) ||
+        (rc = upload_vec(&ob.fp_sigma, t.sigma)) || (rc = upload_vec(&ob.fp_kind_begin, t.kind_begin)) ||
+        (rc = upload_vec(&ob.pt_slot, t.pt_slot)) || (rc = upload_vec(&ob.pt_day, t.pt_day)) ||
+        (rc = upload_vec(&ob.pt_cell, t.pt_cell)) || (rc = upload_vec(&ob.pt_w, t.pt_w)))
+        return rc;
+    CU(cudaMalloc(&ob.fp_mean, (size_t)ctx->cfg.n_members * std::max(1LL, row_len) * sizeof(double)));
+    return NESOSIM_OK;
+}
+
+// Validates every observation and footprint, then compiles them against the strip tables and replaces the context's
+// observations.  sets: tagged with their forcing set (obs_set_host / fp_set_host); else one shared forcing.  Footprint
+// points get sample slots with the point observations (one slot per distinct (cell, day)) but never enter the point
+// tables, so the point results do not depend on the footprints.  Nothing is freed before the last check.
 int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
                           const int32_t *obs_row_host, const int32_t *obs_col_host, const int32_t *obs_kind_host,
-                          const double *obs_value_host, const double *obs_sigma_host) {
-    if (!ctx || n_obs < 0) return fail(NESOSIM_ERR_ARG, "bad argument");
+                          const double *obs_value_host, const double *obs_sigma_host,
+                          int64_t n_fp = 0, const int32_t *fp_set_host = nullptr, const int32_t *fp_kind_host = nullptr,
+                          const double *fp_value_host = nullptr, const double *fp_sigma_host = nullptr,
+                          const int64_t *fp_begin_host = nullptr, const int32_t *pt_day_host = nullptr,
+                          const int32_t *pt_row_host = nullptr, const int32_t *pt_col_host = nullptr,
+                          const double *pt_weight_host = nullptr) {
+    if (!ctx || n_obs < 0 || n_fp < 0) return fail(NESOSIM_ERR_ARG, "bad argument");
     if (n_obs > 0 && ((sets && !obs_set_host) || !obs_day_host || !obs_row_host || !obs_col_host || !obs_value_host))
         return fail(NESOSIM_ERR_ARG, "NULL observation array");
+    if (n_fp > 0 && ((sets && !fp_set_host) || !fp_value_host || !fp_begin_host || !pt_day_host || !pt_row_host || !pt_col_host))
+        return fail(NESOSIM_ERR_ARG, "NULL footprint array");
     if (sets && !ctx->member_set_dev) return fail(NESOSIM_ERR_STATE, "set observations need nesosim_set_forcing_sets first");
     CU(cudaSetDevice(ctx->cfg.device));
     const nesosim_config &c = ctx->cfg;
@@ -1393,21 +1603,67 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
             return fail(NESOSIM_ERR_ARG, "density observation on day 0: the model has no density there (NESOSIM.py:350-376)");
         if (!(std::isfinite(sigma) && sigma > 0.0)) return fail(NESOSIM_ERR_ARG, "observation error sigma must be finite and > 0");
         depth_only = depth_only && kind == NESOSIM_OBS_DEPTH && sigma == 1.0;
+        if (n_in[s] == INT_MAX) return fail(NESOSIM_ERR_ARG, "a set's observations do not fit the tables' int indices");
         const int src = n_in[s]++;
         const int o = owner[(size_t)r * nx + col];
         if (o < 0) continue;                             // land / lake: the model value is NaN, the observation is skipped
         per_set[s].push_back(ObsPoint{o, d, r * nx + col, kind, src, obs_value_host[i], sigma});
     }
+    std::vector<FpSet> fps((size_t)S);
+    if (n_fp > 0 && fp_begin_host[0] != 0) return fail(NESOSIM_ERR_ARG, "fp_begin[0] must be 0");
+    for (int64_t g = 0; g < n_fp; ++g) {
+        const int s = sets ? fp_set_host[g] : 0;
+        const int kind = fp_kind_host ? fp_kind_host[g] : NESOSIM_OBS_DEPTH;
+        const double sigma = fp_sigma_host ? fp_sigma_host[g] : 1.0;
+        if (s < 0 || s >= S) return fail(NESOSIM_ERR_ARG, "footprint set index outside [0, n_sets)");
+        if (kind < 0 || kind >= NESOSIM_OBS_KINDS) return fail(NESOSIM_ERR_ARG, "footprint kind outside [0, NESOSIM_OBS_KINDS)");
+        if (!(std::isfinite(sigma) && sigma > 0.0)) return fail(NESOSIM_ERR_ARG, "footprint error sigma must be finite and > 0");
+        if (fp_begin_host[g + 1] <= fp_begin_host[g]) return fail(NESOSIM_ERR_ARG, "fp_begin must increase: a footprint needs a point");
+        FpSet &f = fps[s];
+        if (f.kind.size() == (size_t)INT_MAX) return fail(NESOSIM_ERR_ARG, "a set's footprints do not fit the tables' int indices");
+        const int days = sets ? ctx->set_days[s] : T;
+        for (int64_t j = fp_begin_host[g]; j < fp_begin_host[g + 1]; ++j) {
+            const int d = pt_day_host[j], r = pt_row_host[j], col = pt_col_host[j];
+            const double w = pt_weight_host ? pt_weight_host[j] : 1.0;
+            if (d < 0 || d >= days) return fail(NESOSIM_ERR_ARG, "footprint point day outside its season");
+            if (r < 0 || r >= ny || col < 0 || col >= nx) return fail(NESOSIM_ERR_ARG, "footprint point outside the grid");
+            if (kind == NESOSIM_OBS_DENSITY && d == 0)
+                return fail(NESOSIM_ERR_ARG, "density footprint point on day 0: the model has no density there (NESOSIM.py:350-376)");
+            if (!(std::isfinite(w) && w > 0.0)) return fail(NESOSIM_ERR_ARG, "footprint point weight must be finite and > 0");
+            const int o = owner[(size_t)r * nx + col];
+            if (o < 0) continue;                         // land / lake: dropped, as point observations are
+            if (f.pt_day.size() + per_set[s].size() >= (size_t)INT_MAX)
+                return fail(NESOSIM_ERR_ARG, "a set's points do not fit the tables' int indices");
+            per_set[s].push_back(ObsPoint{o, d, r * nx + col, -1, (int)f.pt_day.size(), 0.0, 0.0});
+            f.pt_day.push_back(d);
+            f.pt_cell.push_back(r * nx + col);
+            f.pt_w.push_back(w);
+        }
+        f.kind.push_back(kind);
+        f.val.push_back(fp_value_host[g]);
+        f.sigma.push_back(sigma);
+        f.begin.push_back((long long)f.pt_day.size());
+    }
     ObsTables t;
+    FpTables ft;
     std::vector<int> slot_base(S);
     size_t stride = 0;                                   // a member samples one set only: the largest set, not the sum
+    size_t fp_row_len = 0;
     for (int s = 0; s < S; ++s) {
+        if (t.slot_day.size() + per_set[s].size() + list_end + 1 > (size_t)INT_MAX)
+            return fail(NESOSIM_ERR_ARG, "the sample slots do not fit the tables' int indices");
         slot_base[s] = (int)t.slot_day.size();
-        stride = std::max(stride, compile_obs_set(per_set[s], list_end, t));
+        fps[s].pt_slot.assign(fps[s].pt_day.size(), 0);
+        stride = std::max(stride, compile_obs_set(per_set[s], list_end, t, fps[s].pt_slot));
         for (int o = 0; o < list_end; ++o) t.first[(size_t)s * (list_end + 1) + o] += slot_base[s];   // -> index in `day`
+        fp_row_len = std::max(fp_row_len, fps[s].kind.size());
     }
+    if (t.o_slot.size() > (size_t)INT_MAX || (size_t)n_fp > (size_t)INT_MAX)
+        return fail(NESOSIM_ERR_ARG, "the observations do not fit the tables' int indices");
+    for (int s = 0; s < S; ++s) append_fp_set(fps[s], ft);
     int rc = upload_obs(ctx, t, (long long)stride);
     if (rc) return rc;
+    if ((rc = upload_fp(ctx, ft, (long long)fp_row_len))) return rc;
     auto &ob = ctx->obs;
     ob.row_len = *std::max_element(n_in.begin(), n_in.end());
     ob.depth_only = depth_only;
@@ -1423,15 +1679,22 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
 
 // The season with fused sampling, then the scores epilogue: n_kinds = NESOSIM_OBS_KINDS (nesosim_run_season_scores) or
 // 1 (nesosim_run_season_misfit: the depth sum only, which needs observations that are all depth with sigma 1).
+// fp: nesosim_run_season_scores_fp -- the footprint means (footprint_mean_kernel) between the season and the epilogue,
+// which then also scores them; without it, registered footprints are NESOSIM_ERR_STATE (their data would be dropped).
 int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev, int ic_per_member,
                       double *chi2_dev, int64_t *count_dev, int n_kinds, double *model_dev, int64_t model_stride,
-                      void *stream) {
-    if (!ctx || !params_host || !chi2_dev) return fail(NESOSIM_ERR_ARG, "bad argument");
+                      void *stream, bool fp = false, double *fp_chi2_dev = nullptr, int64_t *fp_count_dev = nullptr,
+                      double *fp_model_dev = nullptr, int64_t fp_model_stride = 0) {
+    if (!ctx || !params_host || !chi2_dev || (fp && !fp_chi2_dev)) return fail(NESOSIM_ERR_ARG, "bad argument");
     if (!ctx->P) return fail(NESOSIM_ERR_STATE, "nesosim_set_forcing has not been called");
     if (!ctx->obs.ready) return fail(NESOSIM_ERR_STATE, "nesosim_set_observations has not been called");
+    if (!fp && ctx->obs.n_fp)
+        return fail(NESOSIM_ERR_STATE, "footprints are registered; use nesosim_run_season_scores_fp");
     if (n_kinds == 1 && !ctx->obs.depth_only)
         return fail(NESOSIM_ERR_STATE, "the registered observations are not all depth with sigma 1; use nesosim_run_season_scores");
     if (model_dev && model_stride < ctx->obs.row_len) return fail(NESOSIM_ERR_ARG, "model_stride is shorter than the observation row");
+    if (fp_model_dev && fp_model_stride < ctx->obs.fp_row_len)
+        return fail(NESOSIM_ERR_ARG, "fp_model_stride is shorter than the footprint row");
     const bool sets = !ctx->obs.set_days.empty();
     if (!sets && ctx->member_set_dev) return fail(NESOSIM_ERR_ARG, "misfit mode runs on one shared forcing");
     if (sets && ctx->obs.set_days != ctx->set_days)
@@ -1465,6 +1728,29 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     ma.chi2 = chi2_dev; ma.count = (long long *)count_dev; ma.n_kinds = n_kinds;
     ma.model = model_dev; ma.model_stride = model_stride;
     ma.member_set = ctx->member_set_dev; ma.conc_set_stride = (long long)T * ctx->plane;
+    ma.fp_chi2 = nullptr; ma.fp_count = nullptr;
+    if (fp) {
+        const auto &ob = ctx->obs;
+        if (ob.fp_row_len) {
+            FootprintArgs fa;
+            fa.samples = ob.samples; fa.stride = ob.stride;
+            fa.begin = ob.fp_begin; fa.kind = ob.fp_kind; fa.src = ob.fp_src;
+            fa.pt_slot = ob.pt_slot; fa.pt_day = ob.pt_day; fa.pt_cell = ob.pt_cell; fa.pt_w = ob.pt_w;
+            fa.kind_begin = ob.fp_kind_begin; fa.conc = ctx->C; fa.plane = ctx->plane; fa.k = ctx->k;
+            fa.n_members = M; fa.row_len = ob.fp_row_len; fa.mean = ob.fp_mean; fa.mean_stride = ob.fp_row_len;
+            fa.model = fp_model_dev; fa.model_stride = fp_model_stride;
+            fa.member_set = ctx->member_set_dev; fa.conc_set_stride = (long long)T * ctx->plane;
+            const long long blocks = ob.fp_row_len * M;
+            if (blocks > INT_MAX) return fail(NESOSIM_ERR_ARG, "too many footprints x members for one launch");
+            if (sets) footprint_mean_kernel<true><<<(unsigned)blocks, 32, 0, st>>>(fa);
+            else footprint_mean_kernel<false><<<(unsigned)blocks, 32, 0, st>>>(fa);
+            ctx->launches++;
+            CU(cudaGetLastError());
+        }
+        ma.fp_mean = ob.fp_mean; ma.fp_stride = std::max(1LL, ob.fp_row_len);
+        ma.fp_val = ob.fp_val; ma.fp_sigma = ob.fp_sigma; ma.fp_kind_begin = ob.fp_kind_begin;
+        ma.fp_chi2 = fp_chi2_dev; ma.fp_count = (long long *)fp_count_dev;
+    }
     if (sets) misfit_finish_kernel<true><<<M, 256, 0, st>>>(ma);
     else misfit_finish_kernel<false><<<M, 256, 0, st>>>(ma);
     ctx->launches++;
@@ -1513,6 +1799,33 @@ int nesosim_run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *par
                               int64_t model_stride, void *stream) {
     return run_season_scores(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, NESOSIM_OBS_KINDS, model_dev,
                              model_stride, stream);
+}
+
+int nesosim_set_observations_fp(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_set_host, const int32_t *obs_day_host,
+                                const int32_t *obs_row_host, const int32_t *obs_col_host, const int32_t *obs_kind_host,
+                                const double *obs_value_host, const double *obs_sigma_host, int64_t n_fp,
+                                const int32_t *fp_set_host, const int32_t *fp_kind_host, const double *fp_value_host,
+                                const double *fp_sigma_host, const int64_t *fp_begin_host, const int32_t *pt_day_host,
+                                const int32_t *pt_row_host, const int32_t *pt_col_host, const double *pt_weight_host) {
+    return register_observations(ctx, obs_set_host != nullptr || fp_set_host != nullptr, n_obs, obs_set_host,
+                                 obs_day_host, obs_row_host, obs_col_host, obs_kind_host, obs_value_host, obs_sigma_host,
+                                 n_fp, fp_set_host, fp_kind_host, fp_value_host, fp_sigma_host, fp_begin_host,
+                                 pt_day_host, pt_row_host, pt_col_host, pt_weight_host);
+}
+
+int nesosim_footprint_row_length(const nesosim_ctx *ctx, int64_t *row_len) {
+    if (!ctx || !row_len) return fail(NESOSIM_ERR_ARG, "bad argument");
+    if (!ctx->obs.ready) return fail(NESOSIM_ERR_STATE, "no observations are registered");
+    *row_len = ctx->obs.fp_row_len;
+    return NESOSIM_OK;
+}
+
+int nesosim_run_season_scores_fp(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                                 int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
+                                 int64_t model_stride, double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
+                                 int64_t fp_model_stride, void *stream) {
+    return run_season_scores(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, NESOSIM_OBS_KINDS, model_dev,
+                             model_stride, stream, true, fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride);
 }
 
 int nesosim_set_async(nesosim_ctx *ctx, int on) {

@@ -313,6 +313,69 @@ class SnowBudgetEngine:
         self._keep = (ic_t, chi2, used, mod)
         return chi2, used, mod
 
+    def set_observations_fp(self, obs, footprints, obs_set=None, fp_set=None):
+        """Register point observations and footprint observations together, for ``run_season_scores_fp`` (see
+        nesosim_set_observations_fp).  ``obs``: dict of day, row, col, value, kind, sigma arrays (``ensemble.
+        normalize_observations``), or None for no points; ``footprints``: dict of kind, value, sigma (per footprint),
+        begin (int64, [n_fp+1]) and day, row, col, weight (per point) arrays (``ensemble.normalize_footprints``);
+        ``obs_set`` / ``fp_set``: forcing-set tags of the points / footprints on a context with forcing sets."""
+        i32, i64, f64 = C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_double)
+
+        def arr(a, dt, t):
+            if a is None:
+                return None, None
+            a = np.ascontiguousarray(np.asarray(a), dtype=dt)
+            return a, a.ctypes.data_as(t)
+
+        n = 0 if obs is None else len(obs["day"])
+        po = [arr(None if obs is None else obs[k], dt, t) for k, dt, t in
+              (("day", np.int32, i32), ("row", np.int32, i32), ("col", np.int32, i32), ("kind", np.int32, i32),
+               ("value", np.float64, f64), ("sigma", np.float64, f64))]
+        fp = footprints
+        n_fp = len(fp["value"])
+        fo = [arr(fp[k], dt, t) for k, dt, t in
+              (("kind", np.int32, i32), ("value", np.float64, f64), ("sigma", np.float64, f64), ("begin", np.int64, i64),
+               ("day", np.int32, i32), ("row", np.int32, i32), ("col", np.int32, i32), ("weight", np.float64, f64))]
+        os_, fs = arr(obs_set, np.int32, i32), arr(fp_set, np.int32, i32)
+        assert len(fo[3][0]) == n_fp + 1
+        (_, day), (_, row), (_, col), (_, kind), (_, value), (_, sigma) = po
+        (_, fkind), (_, fval), (_, fsig), (_, begin), (_, pday), (_, prow), (_, pcol), (_, pw) = fo
+        _lib.check(self.lib.nesosim_set_observations_fp(self.handle, n, os_[1], day, row, col, kind, value, sigma,
+                                                        n_fp, fs[1], fkind, fval, fsig, begin, pday, prow, pcol, pw))
+
+    def footprint_row_length(self):
+        """Entries of a member's footprint model row: the largest number of input footprints of one set."""
+        n = C.c_int64(0)
+        _lib.check(self.lib.nesosim_footprint_row_length(self.handle, C.byref(n)))
+        return int(n.value)
+
+    def run_season_scores_fp(self, params, ic, model=False):
+        """``run_season_scores`` with the registered footprints scored too (nesosim_run_season_scores_fp); returns CUDA
+        tensors (chi2, used, model) of the point observations as ``run_season_scores`` and (fp_chi2[M, OBS_KINDS]
+        float64, fp_used[M, OBS_KINDS] int64, fp_model[M, fp_row_len] float64 or None): per kind the sum of
+        ((mean - observed)/sigma)^2 over the footprints and its number of finite terms, and every footprint's model
+        value (the weighted mean of its points' model values, NaN when none is finite)."""
+        torch = _torch()
+        p = _lib.member_params_array(params)
+        assert len(p) == self.M
+        ic_t = None if ic is None else self._dev(ic)
+        per_member = 1 if (ic_t is not None and ic_t.dim() == 3 and self.M > 1) else 0
+        dev = "cuda:%d" % self.device
+        K = _lib.OBS_KINDS
+        chi2 = torch.empty(self.M, K, dtype=torch.float64, device=dev)
+        used = torch.empty(self.M, K, dtype=torch.int64, device=dev)
+        fp_chi2 = torch.empty(self.M, K, dtype=torch.float64, device=dev)
+        fp_used = torch.empty(self.M, K, dtype=torch.int64, device=dev)
+        mod = torch.empty(self.M, self.observation_row_length(), dtype=torch.float64, device=dev) if model else None
+        fmod = torch.empty(self.M, self.footprint_row_length(), dtype=torch.float64, device=dev) if model else None
+        _lib.check(self.lib.nesosim_run_season_scores_fp(
+            self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member, chi2.data_ptr(), used.data_ptr(),
+            None if mod is None else mod.data_ptr(), 0 if mod is None else mod.shape[1], fp_chi2.data_ptr(),
+            fp_used.data_ptr(), None if fmod is None else fmod.data_ptr(), 0 if fmod is None else fmod.shape[1],
+            self._stream()))
+        self._keep = (ic_t, chi2, used, mod, fp_chi2, fp_used, fmod)
+        return chi2, used, mod, fp_chi2, fp_used, fmod
+
     def run_season_misfit(self, params, ic, obs=None):
         """The season with the calibration misfit reduced INSIDE the season-resident kernel (nesosim_run_season_misfit)
         against the registered observations (``obs`` given: registered first); returns CUDA tensors (misfit[M] float64,

@@ -18,7 +18,8 @@ batch of forcing sets, and the misfit of each pair is reduced against that seaso
     res = run_calibration_scores(mask, seasons, params, dx, model=True)   # chi2/used [P, S, 3], model rows per season
 
 does the same with observation errors and three observed quantities (snow depth over ice, snow volume, bulk density):
-per kind the sum of ((model - observed)/sigma)^2, and optionally the model value at every observation.
+per kind the sum of ((model - observed)/sigma)^2, and optionally the model value at every observation.  A season's
+``"footprints"`` (``region_footprints``) add observed means over many cells and/or days, scored in the same call.
 """
 import numpy as np
 
@@ -118,6 +119,114 @@ def observation_scores(snowDepths, density, conc, obs, mask=None):
     return chi2, used, model
 
 
+def normalize_footprints(fps):
+    """A season's footprint observations as a dict of numpy arrays: per footprint kind (int32), value and sigma
+    (float64); ``begin`` (int64, [n_fp+1]): footprint g's points are [begin[g], begin[g+1]) of the per-point arrays day,
+    row, col (int32) and weight (float64).  ``fps``: a dict with value, begin, day, row, col and optionally kind (default
+    depth), sigma and weight (default 1)."""
+    from . import _lib
+    out = {"value": np.asarray(fps["value"], dtype=np.float64).ravel()}
+    n = len(out["value"])
+    kind, sigma, weight = fps.get("kind"), fps.get("sigma"), fps.get("weight")
+    out["kind"] = np.full(n, _lib.OBS_DEPTH, np.int32) if kind is None else np.asarray(kind, dtype=np.int32).ravel()
+    out["sigma"] = np.ones(n) if sigma is None else np.asarray(sigma, dtype=np.float64).ravel()
+    out["begin"] = np.asarray(fps["begin"], dtype=np.int64).ravel()
+    for k in ("day", "row", "col"):
+        out[k] = np.asarray(fps[k], dtype=np.int32).ravel()
+    npt = len(out["day"])
+    out["weight"] = np.ones(npt) if weight is None else np.asarray(weight, dtype=np.float64).ravel()
+    if len(out["kind"]) != n or len(out["sigma"]) != n or len(out["begin"]) != n + 1:
+        raise ValueError("footprint arrays of different lengths (begin needs n_fp + 1 entries)")
+    if any(len(out[k]) != npt for k in ("row", "col", "weight")):
+        raise ValueError("footprint point arrays of different lengths")
+    return out
+
+
+def check_footprints(fps, shape=None, days=None):
+    """Rejects what nesosim_set_observations_fp rejects (``fps`` normalized): ``begin`` not starting at 0, not
+    increasing (an empty footprint) or not ending at the number of points; a kind outside [0, OBS_KINDS); a sigma or a
+    weight that is not finite and > 0; a density point on day 0; more points than int indices hold; with ``shape`` a
+    point outside the grid, with ``days`` a point outside [0, days) of its season."""
+    from . import _lib
+    b = fps["begin"]
+    if b[0] != 0 or (np.diff(b) <= 0).any() or b[-1] != len(fps["day"]):
+        raise ValueError("footprint begin must start at 0, increase (no empty footprint) and end at the point count")
+    if len(fps["day"]) >= 2 ** 31 - 1:
+        raise ValueError("more footprint points than int indices hold")
+    kind = fps["kind"]
+    if ((kind < 0) | (kind >= _lib.OBS_KINDS)).any():
+        raise ValueError("footprint kind outside [0, %d)" % _lib.OBS_KINDS)
+    if not (np.isfinite(fps["sigma"]) & (fps["sigma"] > 0)).all():
+        raise ValueError("footprint error sigma must be finite and > 0")
+    if not (np.isfinite(fps["weight"]) & (fps["weight"] > 0)).all():
+        raise ValueError("footprint point weight must be finite and > 0")
+    pkind = np.repeat(kind, np.diff(b))
+    if ((pkind == _lib.OBS_DENSITY) & (fps["day"] == 0)).any():
+        raise ValueError("density footprint point on day 0: the model has no density there")
+    if shape is not None:
+        ny, nx = shape
+        if ((fps["row"] < 0) | (fps["row"] >= ny) | (fps["col"] < 0) | (fps["col"] >= nx)).any():
+            raise ValueError("footprint point outside the %d x %d grid" % (ny, nx))
+    if days is not None and ((fps["day"] < 0) | (fps["day"] >= days)).any():
+        raise ValueError("footprint point day outside its season [0, %d)" % days)
+
+
+def empty_footprints():
+    return normalize_footprints({"value": [], "begin": [0], "day": [], "row": [], "col": []})
+
+
+def region_footprints(mask, codes, windows, kind, value, sigma=1.0):
+    """One footprint per day window [d0, d1) over every ocean cell (mask 1..10) whose mask code is in ``codes``, all
+    weights 1, points day by day in row-major cell order -- the shape of a drifting-station climatology or a monthly
+    gridded product.  ``value`` and ``sigma``: one number or one per window.  Returns ``normalize_footprints``' dict."""
+    mask = np.asarray(mask)
+    cells = np.flatnonzero(np.isin(mask, list(codes)) & (mask >= 1) & (mask <= 10))
+    if not len(cells) or any(d1 <= d0 for d0, d1 in windows):
+        raise ValueError("a footprint needs a point: no ocean cell has one of the codes, or a window is empty")
+    n = len(windows)
+    day = [np.repeat(np.arange(d0, d1, dtype=np.int64), len(cells)) for d0, d1 in windows]
+    cell = [np.tile(cells, d1 - d0) for d0, d1 in windows]
+    npt = np.array([len(d) for d in day], dtype=np.int64)
+    cell = np.concatenate(cell) if n else np.zeros(0, np.int64)
+    return normalize_footprints({
+        "kind": np.full(n, kind), "value": np.broadcast_to(np.asarray(value, dtype=np.float64), (n,)).copy(),
+        "sigma": np.broadcast_to(np.asarray(sigma, dtype=np.float64), (n,)).copy(),
+        "begin": np.concatenate([[0], np.cumsum(npt)]),
+        "day": np.concatenate(day) if n else [], "row": cell // mask.shape[1], "col": cell % mask.shape[1]})
+
+
+def footprint_scores(snowDepths, density, conc, fps, mask):
+    """Per-member scores of the footprints ``fps`` (see ``normalize_footprints``) from the arrays ``run_season`` writes:
+    ``snowDepths`` (M,T,2,ny,nx), ``density`` (M,T,ny,nx), ``conc`` (T,ny,nx), all on one device; ``mask`` (ny,nx):
+    points on land or lake cells are dropped.  Returns (fp_chi2[M, OBS_KINDS], fp_used[M, OBS_KINDS], fp_model[M, n_fp]):
+    every footprint's weighted mean of its points' finite model values (NaN when none is finite), and per kind the sum of
+    the finite ((mean - value)/sigma)^2 and their number -- what nesosim_run_season_scores_fp computes on the fused path
+    (in another summation order)."""
+    import torch
+    from . import _lib
+    fps = normalize_footprints(fps)
+    check_footprints(fps, tuple(snowDepths.shape[-2:]), snowDepths.shape[1])
+    dev = snowDepths.device
+    M, G = snowDepths.shape[0], len(fps["value"])
+    seg = torch.as_tensor(np.repeat(np.arange(G), np.diff(fps["begin"])), device=dev)
+    kind = torch.as_tensor(fps["kind"], device=dev).long()
+    pts = {"day": fps["day"], "row": fps["row"], "col": fps["col"], "value": np.zeros(len(fps["day"])),
+           "kind": np.repeat(fps["kind"], np.diff(fps["begin"]))}
+    _, _, v = observation_scores(snowDepths, density, conc, pts, mask)                 # (M, points), NaN on land
+    w = torch.as_tensor(fps["weight"], device=dev).unsqueeze(0).expand_as(v)
+    ok = torch.isfinite(v)
+    zero = torch.zeros_like(v)
+    sw = torch.zeros(M, G, dtype=torch.float64, device=dev).index_add_(1, seg, torch.where(ok, w * v, zero))
+    s = torch.zeros(M, G, dtype=torch.float64, device=dev).index_add_(1, seg, torch.where(ok, w, zero))
+    model = sw / s
+    r = (model - torch.as_tensor(fps["value"], device=dev)) / torch.as_tensor(fps["sigma"], device=dev)
+    good = torch.isfinite(r)
+    sq = torch.where(good, r * r, torch.zeros_like(r))
+    chi2 = torch.stack([torch.where(kind == k, sq, torch.zeros_like(sq)).sum(dim=1) for k in range(_lib.OBS_KINDS)], 1)
+    used = torch.stack([(good & (kind == k)).sum(dim=1) for k in range(_lib.OBS_KINDS)], 1)
+    return chi2, used, model
+
+
 def run_ensemble(mask, forcing, ic, params, dx, obs, rank=0, world=1, device=0, group=None, fused=None, **flags):
     """Returns (misfit[M], n_used[M]) as numpy arrays in member order (identical on every rank).  ``fused``: None =
     inside the season kernel where it applies, True = insist on it, False = depths to HBM + reduction there (the
@@ -204,6 +313,48 @@ def gather_scores(chi2, used, model, P, S, n_obs, rank=0, world=1, group=None):
             model = sharding.gather_member_results(model, P * S, rank, world, group)
     return assemble_scores(chi2.cpu().numpy(), used.cpu().numpy(), None if model is None else model.cpu().numpy(),
                            P, S, n_obs)
+
+
+def assemble_footprint_scores(fp_chi2, fp_used, fp_model, P, S, n_fp):
+    """Footprint scores of all P*S members in member order -> {"fp_chi2": [P, S, OBS_KINDS], "fp_used": [P, S,
+    OBS_KINDS], "fp_model": per season s the array [P, n_fp[s]] (rows padded to the largest season: the padding is
+    dropped)}."""
+    from . import _lib
+    m = np.asarray(fp_model).reshape(P, S, -1)
+    return {"fp_chi2": np.asarray(fp_chi2).reshape(P, S, _lib.OBS_KINDS),
+            "fp_used": np.asarray(fp_used).reshape(P, S, _lib.OBS_KINDS),
+            "fp_model": [m[:, s, :n_fp[s]] for s in range(S)]}
+
+
+def gather_footprint_scores(fp_chi2, fp_used, fp_model, P, S, n_fp, rank=0, world=1, group=None):
+    """All-gather the ranks' per-member footprint scores (model rows padded to the largest season) and reassemble them
+    (``assemble_footprint_scores``), identical on every rank."""
+    if world > 1:
+        fp_chi2 = sharding.gather_member_results(fp_chi2, P * S, rank, world, group)
+        fp_used = sharding.gather_member_results(fp_used, P * S, rank, world, group)
+        fp_model = sharding.gather_member_results(fp_model, P * S, rank, world, group)
+    return assemble_footprint_scores(fp_chi2.cpu().numpy(), fp_used.cpu().numpy(), fp_model.cpu().numpy(), P, S, n_fp)
+
+
+def season_footprints(mask, seasons):
+    """Every season's footprints (``"footprints"`` entry; none: no footprints), normalized and checked against the grid
+    and that season's own length, on every rank before any device work."""
+    out = []
+    for s in seasons:
+        f = s.get("footprints")
+        f = empty_footprints() if f is None else normalize_footprints(f)
+        check_footprints(f, np.shape(mask), np.shape(s["forcing"]["precip"])[0])
+        out.append(f)
+    return out
+
+
+def concat_footprints(fps):
+    """Several seasons' footprints as one registration: (footprints, set tag per footprint)."""
+    out = {k: np.concatenate([f[k] for f in fps]) for k in ("kind", "value", "sigma", "day", "row", "col", "weight")}
+    npt = np.concatenate([np.diff(f["begin"]) for f in fps])
+    out["begin"] = np.concatenate([[0], np.cumsum(npt)]).astype(np.int64)
+    tag = np.concatenate([np.full(len(f["value"]), i, dtype=np.int32) for i, f in enumerate(fps)])
+    return out, tag
 
 
 def stage_calibration(mask, seasons, params, dx, plan, device=0, **flags):
@@ -293,46 +444,77 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     identical on every rank.  ``fused`` as in ``run_calibration``: None = scored inside the fused path where it applies
     (falling back on grids wider than the season kernel takes), True = insist on it, False = snowDepths and density to
     HBM and ``observation_scores`` there.  Observations outside the grid or outside their season's days, bad kinds,
-    sigmas and density observations on day 0 raise ValueError before any device work, on either path."""
+    sigmas and density observations on day 0 raise ValueError before any device work, on either path.
+
+    A season may also have ``"footprints"`` (``normalize_footprints``; e.g. ``region_footprints``): observed means over
+    many cells and/or days.  When some season has any, the result also holds "fp_chi2" / "fp_used" [P, S, OBS_KINDS]
+    and "fp_model" (per season the array [P, n_fp] of footprint model values); the fused path scores them in the same
+    call (nesosim_run_season_scores_fp), the HBM path with ``footprint_scores``.  Without footprints the result is
+    unchanged."""
     import torch
     from . import _lib
     params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
     P, S = len(params), len(seasons)
     obs = season_observations(mask, seasons)
+    fps = season_footprints(mask, seasons)
     n_obs = [len(o["day"]) for o in obs]
-    width = max(n_obs, default=0)
+    n_fp = [len(f["value"]) for f in fps]
+    width, fp_width = max(n_obs, default=0), max(n_fp, default=0)
+    with_fp = fp_width > 0
     plan = calibration_plan(P, S, rank, world)
     pairs, staged, order, member_set = plan["pairs"], plan["seasons"], plan["order"], plan["member_set"]
     dev = "cuda:%d" % device
     K = _lib.OBS_KINDS
+
+    def gather(chi2, used, mod, fp):
+        res = gather_scores(chi2, used, mod, P, S, n_obs, rank, world, group)
+        if with_fp:
+            res.update(gather_footprint_scores(*fp, P, S, n_fp, rank, world, group))
+        return res
+
     if not pairs:   # more ranks than members: nothing to run, but the gather still needs this rank
         chi2, used = torch.zeros(0, K, dtype=torch.float64, device=dev), torch.zeros(0, K, dtype=torch.int64, device=dev)
         mod = torch.zeros(0, width, dtype=torch.float64, device=dev) if model else None
-        return gather_scores(chi2, used, mod, P, S, n_obs, rank, world, group)
+        fp = (chi2, used, torch.zeros(0, fp_width, dtype=torch.float64, device=dev))
+        return gather(chi2, used, mod, fp)
     eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
     M = len(mine)
 
     def hbm_round_trip():
         out = eng.run_season(mine, ic, eng.alloc_outputs(names=("snowDepths", "density")))
-        chi2 = torch.zeros(M, K, dtype=torch.float64, device=dev)
-        used = torch.zeros(M, K, dtype=torch.int64, device=dev)
+        chi2, fchi2 = (torch.zeros(M, K, dtype=torch.float64, device=dev) for _ in range(2))
+        used, fused_ = (torch.zeros(M, K, dtype=torch.int64, device=dev) for _ in range(2))
         mod = torch.full((M, width), float("nan"), dtype=torch.float64, device=dev)
+        fmod = torch.full((M, fp_width), float("nan"), dtype=torch.float64, device=dev)
         for i, s in enumerate(staged):
             sel = torch.as_tensor(np.flatnonzero(member_set == i), device=dev)
-            c, u, m = observation_scores(out["snowDepths"][sel], out["density"][sel], eng._forcing[1][i], obs[s], mask)
+            arrays = (out["snowDepths"][sel], out["density"][sel], eng._forcing[1][i])
+            c, u, m = observation_scores(*arrays, obs[s], mask)
             chi2[sel], used[sel], mod[sel, :n_obs[s]] = c, u.to(torch.int64), m
-        return chi2, used, mod
+            if with_fp:
+                c, u, m = footprint_scores(*arrays, fps[s], mask)
+                fchi2[sel], fused_[sel], fmod[sel, :n_fp[s]] = c, u.to(torch.int64), m
+        return chi2, used, mod, (fchi2, fused_, fmod)
 
     try:
         if fused is False:
-            chi2, used, mod = hbm_round_trip()
+            chi2, used, mod, fp = hbm_round_trip()
         else:
             try:
                 cols = {k: np.concatenate([obs[s][k] for s in staged]) for k in obs[0]}
                 tag = np.concatenate([np.full(n_obs[s], i, dtype=np.int32) for i, s in enumerate(staged)])
-                eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"],
-                                        cols["sigma"], obs_set=tag)
-                chi2, used, m = eng.run_season_scores(mine, ic, model=model)
+                if with_fp:
+                    fcols, ftag = concat_footprints([fps[s] for s in staged])
+                    eng.set_observations_fp(cols, fcols, obs_set=tag, fp_set=ftag)
+                    chi2, used, m, fchi2, fused_, fm = eng.run_season_scores_fp(mine, ic, model=True)
+                    fmod = torch.full((M, fp_width), float("nan"), dtype=torch.float64, device=dev)
+                    fmod[:, :fm.shape[1]] = fm
+                    fp = (fchi2, fused_, fmod)
+                else:
+                    eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"],
+                                            cols["sigma"], obs_set=tag)
+                    chi2, used, m = eng.run_season_scores(mine, ic, model=model)
+                    fp = None
                 if model:   # rows of the staged seasons' length -> the largest season's (NaN past a row's end)
                     mod = torch.full((M, width), float("nan"), dtype=torch.float64, device=dev)
                     mod[:, :m.shape[1]] = m
@@ -340,8 +522,10 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
                 if fused is True or e.code != _lib.ERR_ARG:
                     raise
                 # grids the season-resident kernel does not take: snowDepths and density to HBM, scored there per season
-                chi2, used, mod = hbm_round_trip()
+                chi2, used, mod, fp = hbm_round_trip()
     finally:
         eng.close()
     back = torch.as_tensor(np.argsort(order), device=chi2.device)    # native member order -> this rank's pair order
-    return gather_scores(chi2[back], used[back], mod[back] if model else None, P, S, n_obs, rank, world, group)
+    if with_fp:
+        fp = tuple(t[back] for t in fp)
+    return gather(chi2[back], used[back], mod[back] if model else None, fp)
