@@ -181,7 +181,9 @@ int nesosim_final_products(const double *depths_dev, const double *density_dev, 
  * misfit_dev[m] = sum over the observations of (model - observed)^2, skipping non-finite differences (land, NaN forcing,
  * zero concentration); count_dev[m] (may be NULL) = the number of observations used.  Sums are formed in a fixed order
  * (bit-reproducible).  Needs the season-resident path (grid up to 96 columns, variable density, one shared forcing --
- * or forcing sets with observations from nesosim_set_observations_sets, below); NESOSIM_ERR_ARG otherwise. */
+ * or forcing sets with observations from nesosim_set_observations_sets, below); NESOSIM_ERR_ARG otherwise -- unless
+ * the observations are registered after nesosim_set_path(ctx, 1): then the general day kernel produces the same
+ * samples on any grid (see nesosim_set_path). */
 int nesosim_set_observations(nesosim_ctx *ctx, int64_t n_obs, const int32_t *obs_day_host, const int32_t *obs_row_host,
                              const int32_t *obs_col_host, const double *obs_depth_host);
 int nesosim_run_season_misfit(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
@@ -286,7 +288,19 @@ int nesosim_sync(nesosim_ctx *ctx, int *seasons_redone);
 
 /* Kernel path of nesosim_run_season: 0 = automatic (default), 1 = general per-day kernel (any grid),
  * 2 = season-resident cluster kernel (grids up to 96x96, variable density, whole season; error otherwise).
- * Both paths produce identical values.  nesosim_last_path reports which one the last season used. */
+ * Both paths produce identical values.  nesosim_last_path reports which one the last season used.
+ * The path also chooses the producer of the calibration samples.  Observations registered (nesosim_set_observations,
+ * _sets, _ex, _fp) under path 1 are compiled for the general path and scored (nesosim_run_season_misfit, _scores,
+ * _scores_fp) on any grid by the scoring build of the day kernel: it advances only the two depth layers, in a two-slot
+ * ring (32 bytes per member-cell; no accumulator or density is loaded or stored, nothing is written to caller arrays),
+ * and copies the observed cells of each day into the samples; then the same epilogues run.  The scores, counts and
+ * model rows are bit-identical to the season kernel's where it applies (the fixed order depends only on the (cell,
+ * day) order of the observations).  The call takes T+2 launches (T+3 with footprints: init, T-1 day kernels, the
+ * last-day samples, [footprint means,] epilogue) and never synchronises the stream (there is no operand-range flag).
+ * Registration under path 1 also returns NESOSIM_ERR_ARG on a strip context (nesosim_strip_setup) and with
+ * densityType='clim' (the density observation operator is densityCalc).  Under paths 0 and 2 registration needs the
+ * season-resident kernel, as before.  Observations remember the path they were compiled for: after a change between
+ * path 1 and paths 0/2 the scoring calls return NESOSIM_ERR_STATE until the observations are registered again. */
 int nesosim_set_path(nesosim_ctx *ctx, int path);
 int nesosim_last_path(const nesosim_ctx *ctx);
 

@@ -48,6 +48,24 @@ struct DayArgs {
 constexpr int TX = 32;
 constexpr int TY = 16;
 
+// Scoring instantiation (SCORE, nesosim_run_season_scores* on the general path): the day kernel as the producer of the
+// calibration samples on any grid.  Only the two depth layers are advanced, in a two-slot ring (the nine accumulators
+// and density are neither loaded nor stored: h0/h1 of slot x+1 never depend on them), and after pdl_wait every CTA
+// copies the observed cells of its tile on day x -- slot x, complete at that point -- into the members' sample rows.
+// The entries of one (set, day, tile) are a contiguous run of a CSR table (cell, slot in the member's row); entry i of
+// the run belongs to thread i % threads.  sample_last_day_kernel samples each member's last day from its ring slot.
+struct SampleArgs {
+    const int *begin;          // [sets][T][tiles] + 1 run starts of the (set, day, tile) entry lists
+    const int2 *entry;         // (cell, slot)
+    double2 *samples;          // [M][stride] {h0, h1}
+    long long stride;
+    int T, tiles;
+    // sample_last_day_kernel only: the depth ring [parity][layer][M][plane] and the members' seasons
+    const double *ring;
+    long long plane, layer_stride;
+    const int *member_set, *set_steps;   // NULL: one shared season of T days
+};
+
 // Row-strip domain decomposition over peer memory (SURVEY.md §8e "Space"; host side: nesosim_strip_* in the ABI).
 // This context's grid is one strip of a larger grid, extended by STRIP_GHOST ghost rows towards each neighbouring
 // strip.  Only the two depth layers of the ghost rows are ever needed from a neighbour (fused stencil radius 2 of
@@ -132,8 +150,9 @@ __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, c
     }
 }
 
-// 3x3 smoothing of the four raw planes, the point-wise budget terms and the twelve stores of this thread's cells.
-template <bool INTERIOR, bool STRIP, int DAY_THREADS>
+// 3x3 smoothing of the four raw planes, the point-wise budget terms and the twelve stores of this thread's cells
+// (SCORE: the two depth stores only).
+template <bool INTERIOR, bool STRIP, int DAY_THREADS, bool SCORE = false>
 __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0, const int y0, const int m,
                                                  double (&s_h)[2][TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
                                                  const double *h0p, const double *h1p, const MemberCoef &mc,
@@ -184,6 +203,7 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
         auto prev = [&](int v) { return pf_prev[rr][v - V_ACC]; };
         const long long ip = (long long)m * a.plane_mstride + o, id = (long long)m * a.depth_mstride + o;
         auto store = [&](int v, double val) {       // only the density output is optional
+            if (SCORE && v != V_H0 && v != V_H1) return;
             if (v != V_DENS || a.next[v]) a.next[v][(v == V_H0 || v == V_H1) ? id : ip] = val;
         };
         store(V_ACC, add(prev(V_ACC), acc));
@@ -225,10 +245,11 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
 // INTERIOR: the tile with its two-cell halo lies inside the grid and none of its raw-dynamics cells is a grid-edge
 // cell, so there are no bounds tests, every difference is centred and the divisor is a launch constant (the
 // overwhelming majority of the CTAs on the 25 km and 5 km grids).
-template <bool INTERIOR, bool STRIP = false, int DAY_THREADS = 256>
+template <bool INTERIOR, bool STRIP = false, int DAY_THREADS = 256, bool SCORE = false>
 __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2][TY + 4][TX + 4], double (&s_ut)[TY + 4][TX + 4],
                                               double (&s_vt)[TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
-                                              const int bx, const int by, const StripLink *sl = nullptr) {
+                                              const int bx, const int by, const StripLink *sl = nullptr,
+                                              const SampleArgs *sa = nullptr) {
     const int m = blockIdx.z;
     const int x0 = bx * TX, y0 = by * TY;     // (bx, by): the tile (blockIdx, or what a strip / season CTA picked)
     const int tid = threadIdx.x;
@@ -279,12 +300,21 @@ __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2]
 
     pdl_wait();      // ---- from here on yesterday's slot may be read
 
+    if (SCORE) {     // the observed cells of this tile on day x, before any thread of the CTA may leave
+        const int *b = sa->begin + ((long long)fset * sa->T + a.x) * sa->tiles + (long long)by * gridDim.x + bx;
+        double2 *row = sa->samples + (long long)m * sa->stride;
+        for (int i = b[0] + tid; i < b[1]; i += DAY_THREADS) {
+            const int2 e = sa->entry[i];
+            row[e.y] = make_double2(h0p[e.x], h1p[e.x]);
+        }
+    }
+
 #pragma unroll
     for (int rr = 0; rr < CPT; ++rr) {
         const int gy = y0 + (tid / TX) + rr * (DAY_THREADS / TX);
 #pragma unroll
         for (int v = 0; v < 9; ++v) pf_prev[rr][v] = 0.0;
-        if (INTERIOR || (pgx < nx && gy < ny)) {
+        if (!SCORE && (INTERIOR || (pgx < nx && gy < ny))) {
             const long long ip = (long long)m * a.plane_mstride + (long long)gy * nx + pgx;
 #pragma unroll
             for (int v = 0; v < 9; ++v) pf_prev[rr][v] = a.prev[V_ACC + v][ip];
@@ -318,7 +348,8 @@ __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2]
         __syncthreads();
     }
 
-    tile_point_phase<INTERIOR, STRIP, DAY_THREADS>(a, x0, y0, m, s_h, s_raw, h0p, h1p, mc, pf_P, pf_C, pf_W, pf_prev, pf_land, sl);
+    tile_point_phase<INTERIOR, STRIP, DAY_THREADS, SCORE>(a, x0, y0, m, s_h, s_raw, h0p, h1p, mc, pf_P, pf_C, pf_W, pf_prev,
+                                                          pf_land, sl);
 }
 
 // A tile without a single ocean cell (more than half of the polar grid is land, and it comes in large blocks).  From
@@ -380,6 +411,28 @@ __device__ __forceinline__ void day_step_land_tile(const DayArgs &a, const int b
     }
 }
 
+// The land tile of the scoring build: only its NaN depths are stored (a land tile has no observed cell to sample).
+template <int DAY_THREADS>
+__device__ __forceinline__ void day_step_land_depths(const DayArgs &a, const int bx, const int by) {
+    const int m = blockIdx.z;
+    const int fset = a.member_set ? a.member_set[m] : 0;
+    if (a.set_steps && a.x >= a.set_steps[fset]) {
+        pdl_wait();
+        return;
+    }
+    const int gx = bx * TX + (threadIdx.x & (TX - 1));
+    if (gx >= a.nx) return;
+    pdl_wait();
+#pragma unroll
+    for (int rr = 0; rr < TY / (DAY_THREADS / TX); ++rr) {
+        const int gy = by * TY + (threadIdx.x / TX) + rr * (DAY_THREADS / TX);
+        if (gy >= a.ny) break;
+        const long long id = (long long)m * a.depth_mstride + (long long)gy * a.nx + gx;
+        a.next[V_H0][id] = qnan();
+        a.next[V_H1][id] = qnan();
+    }
+}
+
 struct TileSmem {
     double h[2][TY + 4][TX + 4];
     double ut[TY + 4][TX + 4];       // raw drift components (multiplied by deltaT where they are read)
@@ -387,11 +440,13 @@ struct TileSmem {
     double raw[4][TY + 2][TX + 2];   // adv0, adv1, div0, div1 after the NaN->0 fill
 };
 
-template <int DAY_THREADS>
-__device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, const int bx, const int by) {
+template <int DAY_THREADS, bool SCORE = false>
+__device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, const int bx, const int by,
+                                              const SampleArgs *sa = nullptr) {
     pdl_launch_dependents();
     if (a.tile_land && a.tile_land[by * ((a.nx + TX - 1) / TX) + bx]) {
-        day_step_land_tile<DAY_THREADS>(a, bx, by);
+        if (SCORE) day_step_land_depths<DAY_THREADS>(a, bx, by);
+        else day_step_land_tile<DAY_THREADS>(a, bx, by);
         return;
     }
     auto &s_h = sm.h;
@@ -400,8 +455,8 @@ __device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, co
     auto &s_raw = sm.raw;
     const int x0 = bx * TX, y0 = by * TY;
     const bool interior = x0 >= 2 && y0 >= 2 && x0 + TX + 2 <= a.nx && y0 + TY + 2 <= a.ny;
-    if (interior) day_step_body<true, false, DAY_THREADS>(a, s_h, s_ut, s_vt, s_raw, bx, by);
-    else day_step_body<false, false, DAY_THREADS>(a, s_h, s_ut, s_vt, s_raw, bx, by);
+    if (interior) day_step_body<true, false, DAY_THREADS, SCORE>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa);
+    else day_step_body<false, false, DAY_THREADS, SCORE>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa);
 }
 
 // Two builds of the same tile code: 256 threads x 2 cells (large grids: fewer, fatter threads) and 512 threads x 1
@@ -413,6 +468,35 @@ __global__ void __launch_bounds__(256) day_step_kernel(const __grid_constant__ D
 __global__ void __launch_bounds__(512, 2) day_step_kernel_512(const __grid_constant__ DayArgs a) {
     __shared__ TileSmem sm;
     day_step_tile<512>(a, sm, blockIdx.x, blockIdx.y);
+}
+
+// The scoring builds of the same two shapes (SampleArgs above).
+__global__ void __launch_bounds__(256) day_step_score_kernel(const __grid_constant__ DayArgs a,
+                                                             const __grid_constant__ SampleArgs s) {
+    __shared__ TileSmem sm;
+    day_step_tile<256, true>(a, sm, blockIdx.x, blockIdx.y, &s);
+}
+__global__ void __launch_bounds__(512, 2) day_step_score_kernel_512(const __grid_constant__ DayArgs a,
+                                                                    const __grid_constant__ SampleArgs s) {
+    __shared__ TileSmem sm;
+    day_step_tile<512, true>(a, sm, blockIdx.x, blockIdx.y, &s);
+}
+
+// The last day of every member's season (set_steps[set], or T-1), which no day kernel reads: one CTA per member copies
+// its set's entries of that day from the member's ring slot.  A member whose season ended early has not touched its
+// ring since (its CTAs leave the later day kernels at once).
+__global__ void __launch_bounds__(256) sample_last_day_kernel(const __grid_constant__ SampleArgs s) {
+    const int m = blockIdx.x;
+    const int set = s.member_set ? s.member_set[m] : 0;
+    const int day = s.set_steps ? s.set_steps[set] : s.T - 1;
+    const double *h0 = s.ring + (long long)(day & 1) * 2 * s.layer_stride + (long long)m * s.plane;
+    const double *h1 = h0 + s.layer_stride;
+    const long long b = ((long long)set * s.T + day) * s.tiles;
+    double2 *row = s.samples + (long long)m * s.stride;
+    for (int i = s.begin[b] + threadIdx.x; i < s.begin[b + s.tiles]; i += blockDim.x) {
+        const int2 e = s.entry[i];
+        row[e.y] = make_double2(h0[e.x], h1[e.x]);
+    }
 }
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {

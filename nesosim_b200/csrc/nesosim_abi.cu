@@ -221,6 +221,13 @@ struct nesosim_ctx {
         int *pt_slot = nullptr, *pt_day = nullptr, *pt_cell = nullptr;   // per footprint point: sample slot, day, cell,
         double *pt_w = nullptr;                          // weight
         double *fp_mean = nullptr;                       // [M][max(1, fp_row_len)] footprint means in table order
+        // compiled for the general path (nesosim_set_path(ctx, 1)): owners are the row-major ocean-cell indices, the
+        // samples are filled by day_step_score_kernel (SampleArgs in day_kernels.cuh) from a two-slot depth ring
+        bool general = false;
+        int *smp_begin = nullptr;                        // [sets][T][tiles] + 1 run starts of the sampling entries
+        int2 *smp_entry = nullptr;                       // (cell, slot in the member's row)
+        int smp_tiles = 0;                               // day-kernel tiles of the grid
+        double *ring = nullptr;                          // [parity 2][layer 2][M][plane]
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -371,6 +378,7 @@ void obs_release(nesosim_ctx *ctx) {
     cudaFree(ob.fp_begin); cudaFree(ob.fp_kind); cudaFree(ob.fp_src); cudaFree(ob.fp_val); cudaFree(ob.fp_sigma);
     cudaFree(ob.fp_kind_begin); cudaFree(ob.pt_slot); cudaFree(ob.pt_day); cudaFree(ob.pt_cell); cudaFree(ob.pt_w);
     cudaFree(ob.fp_mean);
+    cudaFree(ob.smp_begin); cudaFree(ob.smp_entry); cudaFree(ob.ring);
     ob = {};
 }
 
@@ -1430,6 +1438,49 @@ std::vector<int> obs_owners(nesosim_ctx *ctx, int *list_end) {
     return owner;
 }
 
+// General path: the owner of an ocean cell is its index among the ocean cells in row-major order -- monotone in
+// row*nx + col as the strip owner is, so compile_obs_set orders the observations exactly as for the season kernel.
+// cells[o] = the cell of owner o.
+std::vector<int> ocean_owners(const nesosim_ctx *ctx, int *list_end, std::vector<int> &cells) {
+    std::vector<int> owner(ctx->mask_host.size(), -1);
+    cells.clear();
+    for (size_t i = 0; i < owner.size(); ++i) {
+        const uint8_t m = ctx->mask_host[i];
+        if (!(m > 10 || m < 1)) {
+            owner[i] = (int)cells.size();
+            cells.push_back((int)i);
+        }
+    }
+    *list_end = (int)cells.size();
+    return owner;
+}
+
+// The sampling entries of the general path: every sample slot of every set (sentinels excluded) as (cell, slot relative
+// to the set's row), grouped by (set, day, day-kernel tile); begin[(s*T + day)*tiles + tile] starts a group.
+void sample_lists(const nesosim_ctx *ctx, const ObsTables &t, const std::vector<int> &slot_base, const std::vector<int> &cells,
+                  std::vector<int> &begin, std::vector<int2> &entry) {
+    const int T = ctx->cfg.num_days, nx = ctx->cfg.nx, tgx = (nx + TX - 1) / TX;
+    const long long tiles = (long long)tgx * ((ctx->cfg.ny + TY - 1) / TY), L = (long long)cells.size();
+    const size_t S = slot_base.size();
+    std::vector<long long> key;
+    std::vector<int2> ent;
+    for (size_t s = 0; s < S; ++s)
+        for (long long o = 0; o < L; ++o) {
+            const int cell = cells[o];
+            const long long tile = (long long)(cell / nx / TY) * tgx + (cell % nx) / TX;
+            for (int j = t.first[s * (L + 1) + o]; t.slot_day[j] != 0x7fffffff; ++j) {
+                key.push_back(((long long)s * T + t.slot_day[j]) * tiles + tile);
+                ent.push_back(make_int2(cell, j - slot_base[s]));
+            }
+        }
+    begin.assign((size_t)(S * T * tiles) + 1, 0);
+    for (long long k : key) ++begin[k + 1];
+    for (size_t i = 1; i < begin.size(); ++i) begin[i] += begin[i - 1];
+    entry.resize(ent.size());
+    std::vector<int> fill(begin.begin(), begin.end() - 1);
+    for (size_t i = 0; i < ent.size(); ++i) entry[fill[key[i]]++] = ent[i];
+}
+
 // appends one season's observations to `t`; returns the number of sample slots it added (sentinels included).
 // Footprint points (kind -1, src = their index in the set's point table) take part in the slot assignment only:
 // pt_slot[src] receives their slot, and they never enter the observation tables.
@@ -1584,10 +1635,17 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
     none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
     none.plane_member_stride = (int64_t)T * ctx->plane;
     const char *why = "";
-    if (!ensemble_eligible(ctx, 0, T - 1, &none, &why))
+    const bool general = ctx->path == 1;
+    if (general) {
+        if (ctx->strip.on) return fail(NESOSIM_ERR_ARG, "the general scoring path does not take a strip of a decomposed grid");
+        if (c.density_clim)
+            return fail(NESOSIM_ERR_ARG, "the general scoring path does not take densityType='clim' (its density operator is densityCalc)");
+    } else if (!ensemble_eligible(ctx, 0, T - 1, &none, &why)) {
         return fail(NESOSIM_ERR_ARG, std::string("misfit mode needs the season-resident kernel: ") + why);
+    }
     int list_end = 0;
-    const std::vector<int> owner = obs_owners(ctx, &list_end);
+    std::vector<int> cells;
+    const std::vector<int> owner = general ? ocean_owners(ctx, &list_end, cells) : obs_owners(ctx, &list_end);
     std::vector<std::vector<ObsPoint>> per_set((size_t)S);
     std::vector<int> n_in((size_t)S, 0);                 // input observations of every set so far (-> src)
     bool depth_only = true;
@@ -1661,10 +1719,19 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
     if (t.o_slot.size() > (size_t)INT_MAX || (size_t)n_fp > (size_t)INT_MAX)
         return fail(NESOSIM_ERR_ARG, "the observations do not fit the tables' int indices");
     for (int s = 0; s < S; ++s) append_fp_set(fps[s], ft);
+    std::vector<int> smp_begin;
+    std::vector<int2> smp_entry;
+    if (general) sample_lists(ctx, t, slot_base, cells, smp_begin, smp_entry);
     int rc = upload_obs(ctx, t, (long long)stride);
     if (rc) return rc;
     if ((rc = upload_fp(ctx, ft, (long long)fp_row_len))) return rc;
     auto &ob = ctx->obs;
+    if (general) {
+        if ((rc = upload_vec(&ob.smp_begin, smp_begin)) || (rc = upload_vec(&ob.smp_entry, smp_entry))) return rc;
+        ob.smp_tiles = (int)(((nx + TX - 1) / TX) * ((ny + TY - 1) / TY));
+        CU(cudaMalloc(&ob.ring, (size_t)4 * c.n_members * ctx->plane * sizeof(double)));
+        ob.general = true;
+    }
     ob.row_len = *std::max_element(n_in.begin(), n_in.end());
     ob.depth_only = depth_only;
     if (sets) {
@@ -1674,6 +1741,57 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
         ob.set_days = ctx->set_days;
     }
     ob.ready = true;
+    return NESOSIM_OK;
+}
+
+// The sample producer of the general path: slot 0 of the depth ring (init_slot0_kernel), the T-1 scoring day kernels
+// (day x samples day x, then advances the depths to slot x+1) and sample_last_day_kernel: T+1 launches, no pre-pass,
+// nothing written outside the context, no synchronisation.
+int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cudaStream_t st) {
+    const auto &ob = ctx->obs;
+    const nesosim_config &c = ctx->cfg;
+    const int T = c.num_days, M = c.n_members;
+    const long long plane = ctx->plane, layer = (long long)M * plane;
+    auto ring = [&](int t, int l) { return ob.ring + ((long long)(t & 1) * 2 + l) * layer; };
+    InitArgs ia{};
+    ia.plane = plane;
+    ia.ic = ic_dev;
+    ia.ic_stride = ic_per_member ? plane : 0;
+    ia.conc0 = ctx->C;
+    ia.member_set = ctx->member_set_dev;
+    ia.set_stride = (long long)T * plane;
+    ia.minConc = c.minConc;
+    ia.slot0[V_H0] = ring(0, 0);
+    ia.slot0[V_H1] = ring(0, 1);
+    ia.stride[V_H0] = ia.stride[V_H1] = plane;
+    init_slot0_kernel<<<dim3((unsigned)((plane + 255) / 256), M), 256, 0, st>>>(ia);
+    ctx->launches++;
+    CU(cudaGetLastError());
+    SampleArgs sa;
+    sa.begin = ob.smp_begin; sa.entry = ob.smp_entry; sa.samples = ob.samples; sa.stride = ob.stride;
+    sa.T = T; sa.tiles = ob.smp_tiles;
+    sa.ring = ob.ring; sa.plane = plane; sa.layer_stride = layer;
+    sa.member_set = ctx->member_set_dev; sa.set_steps = ctx->set_steps_dev;
+    const dim3 grid((c.nx + TX - 1) / TX, (c.ny + TY - 1) / TY, M);
+    nesosim_outputs none{};
+    for (int x = 0; x < T - 1; ++x) {
+        DayArgs a;
+        fill_day_args(ctx, x, ctx->P + x * plane, ctx->C + x * plane, ctx->W + x * plane, ctx->UV + (long long)x * 2 * plane,
+                      ctx->UV + ((long long)x * 2 + 1) * plane, c.snowDensityFresh, &none, 0, x > 0, a);
+        for (int v = 0; v < NVAR; ++v) a.prev[v] = a.next[v] = nullptr;
+        for (int l = 0; l < 2; ++l) {
+            a.prev[V_H0 + l] = ring(x, l);
+            a.next[V_H0 + l] = ring(x + 1, l);
+        }
+        a.depth_mstride = a.plane_mstride = plane;
+        const bool pdl = ctx->pdl && x > 0;       // behind this call's own previous day kernel only (see launch_day)
+        if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_score_kernel_512, grid, 512, st, pdl, a, sa));
+        else CU(launch_day_kernel(day_step_score_kernel, grid, 256, st, pdl, a, sa));
+        ctx->launches++;
+    }
+    sample_last_day_kernel<<<M, 256, 0, st>>>(sa);
+    ctx->launches++;
+    CU(cudaGetLastError());
     return NESOSIM_OK;
 }
 
@@ -1699,24 +1817,33 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     if (!sets && ctx->member_set_dev) return fail(NESOSIM_ERR_ARG, "misfit mode runs on one shared forcing");
     if (sets && ctx->obs.set_days != ctx->set_days)
         return fail(NESOSIM_ERR_STATE, "the forcing sets changed since nesosim_set_observations_sets; register the observations again");
+    const bool general = ctx->obs.general;
+    if (general != (ctx->path == 1))
+        return fail(NESOSIM_ERR_STATE, "the kernel path changed since the observations were registered; register them again");
     CU(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     const nesosim_config &c = ctx->cfg;
     const int T = c.num_days, M = c.n_members;
-    nesosim_outputs none{};
-    none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
-    none.plane_member_stride = (int64_t)T * ctx->plane;
-    const char *why = "";
-    if (!ensemble_eligible(ctx, 0, T - 1, &none, &why))
-        return fail(NESOSIM_ERR_ARG, std::string("misfit mode needs the season-resident kernel: ") + why);
-    int rc = upload_coef(ctx, params_host, st);
-    if (rc) return rc;
-    ObsDevice od;
-    od.first = ctx->obs.first; od.day = ctx->obs.day; od.sample_hh = ctx->obs.samples; od.sample_stride = ctx->obs.stride;
-    od.first_stride = ctx->obs.first_stride; od.slot_base = ctx->obs.slot_base;
-    ctx->last_path = 2;
-    rc = run_ensemble(ctx, ic_dev, ic_per_member, &none, 0, M, st, &od);     // synchronises the stream (operand-range flag)
-    if (rc) return rc;
+    int rc;
+    if (general) {
+        if ((rc = upload_coef(ctx, params_host, st))) return rc;
+        ctx->last_path = 1;
+        if ((rc = run_score_days(ctx, ic_dev, ic_per_member, st))) return rc;
+    } else {
+        nesosim_outputs none{};
+        none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
+        none.plane_member_stride = (int64_t)T * ctx->plane;
+        const char *why = "";
+        if (!ensemble_eligible(ctx, 0, T - 1, &none, &why))
+            return fail(NESOSIM_ERR_ARG, std::string("misfit mode needs the season-resident kernel: ") + why);
+        if ((rc = upload_coef(ctx, params_host, st))) return rc;
+        ObsDevice od;
+        od.first = ctx->obs.first; od.day = ctx->obs.day; od.sample_hh = ctx->obs.samples; od.sample_stride = ctx->obs.stride;
+        od.first_stride = ctx->obs.first_stride; od.slot_base = ctx->obs.slot_base;
+        ctx->last_path = 2;
+        rc = run_ensemble(ctx, ic_dev, ic_per_member, &none, 0, M, st, &od);     // synchronises the stream (operand-range flag)
+        if (rc) return rc;
+    }
     // observations dropped at registration (land, lake) have no model value: their entries stay NaN (all bits set)
     if (model_dev && ctx->obs.row_len)
         CU(cudaMemset2DAsync(model_dev, (size_t)model_stride * sizeof(double), 0xff, (size_t)ctx->obs.row_len * sizeof(double), M, st));
@@ -1755,7 +1882,7 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     else misfit_finish_kernel<false><<<M, 256, 0, st>>>(ma);
     ctx->launches++;
     CU(cudaGetLastError());
-    if (ctx->ens_status) return fail(NESOSIM_ERR_ARG, "an operand left the range of the season-resident kernel's fast divisions; misfit mode has no general-path fallback");
+    if (!general && ctx->ens_status) return fail(NESOSIM_ERR_ARG, "an operand left the range of the season-resident kernel's fast divisions; misfit mode has no general-path fallback");
     return NESOSIM_OK;
 }
 

@@ -377,9 +377,10 @@ class SnowBudgetEngine:
         return chi2, used, mod, fp_chi2, fp_used, fmod
 
     def run_season_misfit(self, params, ic, obs=None):
-        """The season with the calibration misfit reduced INSIDE the season-resident kernel (nesosim_run_season_misfit)
-        against the registered observations (``obs`` given: registered first); returns CUDA tensors (misfit[M] float64,
-        used[M] int64).  No output array is written."""
+        """The season with the calibration misfit reduced INSIDE the season-resident kernel (nesosim_run_season_misfit;
+        after ``set_path('general')``: sampled by the general day kernel, on any grid) against the registered
+        observations (``obs`` given: registered first); returns CUDA tensors (misfit[M] float64, used[M] int64).  No
+        output array is written."""
         torch = _torch()
         if obs is not None:
             self.set_observations(obs)
@@ -410,7 +411,10 @@ class SnowBudgetEngine:
     PATHS = {"auto": 0, "general": 1, "ensemble": 2}
 
     def set_path(self, path):
-        """'auto' | 'general' (per-day kernel) | 'ensemble' (season-resident cluster kernel)."""
+        """'auto' | 'general' (per-day kernel) | 'ensemble' (season-resident cluster kernel).  Observations registered
+        after ``set_path('general')`` are scored by the general day kernel on any grid (``run_season_misfit``,
+        ``run_season_scores``, ``run_season_scores_fp``: the same fixed order as the season kernel, bit for bit);
+        changing the path afterwards makes those calls fail until the observations are registered again."""
         _lib.check(self.lib.nesosim_set_path(self.handle, self.PATHS[path]))
 
     def last_path(self):

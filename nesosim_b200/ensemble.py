@@ -227,11 +227,26 @@ def footprint_scores(snowDepths, density, conc, fps, mask):
     return chi2, used, model
 
 
+def fused_on_general_path(eng, fused_call, hbm_round_trip):
+    """The fused call again on the general day-kernel path, for grids the season-resident kernel does not take: the
+    engine is switched to ``set_path("general")`` and ``fused_call`` registers the observations and runs the scoring
+    call (bit-identical to the season kernel's fixed order).  Where that path does not apply either (densityType='clim'
+    or a strip context), ``hbm_round_trip`` instead."""
+    from . import _lib
+    eng.set_path("general")
+    try:
+        return fused_call()
+    except _lib.NesosimError as e:
+        if e.code != _lib.ERR_ARG:
+            raise
+        return hbm_round_trip()
+
+
 def run_ensemble(mask, forcing, ic, params, dx, obs, rank=0, world=1, device=0, group=None, fused=None, **flags):
     """Returns (misfit[M], n_used[M]) as numpy arrays in member order (identical on every rank).  ``fused``: None =
-    inside the season kernel where it applies, True = insist on it, False = depths to HBM + reduction there (the
-    round-1 path, kept as the cross-check).  Observations outside the grid or the season's days raise ValueError
-    before any device work, on either path."""
+    inside the season kernel where it applies, else fused on the general day-kernel path; True = insist on the season
+    kernel; False = depths to HBM + reduction there (the round-1 path, kept as the cross-check).  Observations outside
+    the grid or the season's days raise ValueError before any device work, on either path."""
     import torch
     from .engine import SnowBudgetEngine
     params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
@@ -242,18 +257,21 @@ def run_ensemble(mask, forcing, ic, params, dx, obs, rank=0, world=1, device=0, 
     eng = SnowBudgetEngine(mask, T, dx, n_members=hi - lo, device=device, **flags)
     eng.set_forcing(forcing["precip"], forcing["conc"], forcing["wind"], forcing["drift"])
     from . import _lib
+
+    def hbm_round_trip():   # depths to HBM, reduced there (still nothing crosses PCIe)
+        out = eng.run_season(params[lo:hi], ic, eng.alloc_outputs(names=("snowDepths",)))
+        return depth_misfit(out["snowDepths"], eng._forcing[1], obs)
+
     try:
         # fused: the observation operator and the reduction run inside the season-resident kernel, nothing is stored
         mis, used = eng.run_season_misfit(params[lo:hi], ic, obs)
     except _lib.NesosimError as e:
         if fused is True or e.code != _lib.ERR_ARG:
             raise
-        # grids the season-resident kernel does not take: depths to HBM, reduced there (still nothing crosses PCIe)
-        out = eng.run_season(params[lo:hi], ic, eng.alloc_outputs(names=("snowDepths",)))
-        mis, used = depth_misfit(out["snowDepths"], eng._forcing[1], obs)
+        if fused is None:   # grids the season-resident kernel does not take: sampled by the general day kernel
+            mis, used = fused_on_general_path(eng, lambda: eng.run_season_misfit(params[lo:hi], ic, obs), hbm_round_trip)
     if fused is False:
-        out = eng.run_season(params[lo:hi], ic, eng.alloc_outputs(names=("snowDepths",)))
-        mis, used = depth_misfit(out["snowDepths"], eng._forcing[1], obs)
+        mis, used = hbm_round_trip()
     eng.close()
     if world > 1:
         mis = sharding.gather_member_results(mis, M, rank, world, group)
@@ -388,8 +406,9 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
     "obs": (day, row, col, depth)}, each with its own length T_s.  Returns (misfit[P,S], used[P,S]) as numpy arrays,
     identical on every rank.  A rank stages only the seasons its (parameter set, season) pairs use, stacked as forcing
     sets of the longest of them, with each member's season IC as a per-member IC.  ``fused`` as in ``run_ensemble``:
-    None = observations reduced inside the season kernel where it applies, True = insist on it, False = depths to HBM
-    and a per-season reduction there.  Observations outside the grid or outside their season's days raise ValueError
+    None = observations reduced inside the season kernel where it applies, else fused on the general day-kernel path
+    (``fused_on_general_path``), True = insist on the season kernel, False = depths to HBM and a per-season reduction
+    there.  Observations outside the grid or outside their season's days raise ValueError
     before any device work, on either path."""
     import torch
     from . import _lib
@@ -415,20 +434,23 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
             mis[sel], used[sel] = m_i, u_i.to(torch.int64)
         return mis, used
 
+    def fused_call():
+        cols = [np.concatenate([np.asarray(seasons[s]["obs"][j]).ravel() for s in staged]) for j in range(4)]
+        tag = np.concatenate([np.full(len(seasons[s]["obs"][0]), i, dtype=np.int32) for i, s in enumerate(staged)])
+        eng.set_observations_sets(tag, *cols)
+        return eng.run_season_misfit(mine, ic)
+
     try:
         if fused is False:
             mis, used = hbm_round_trip()
         else:
             try:
-                cols = [np.concatenate([np.asarray(seasons[s]["obs"][j]).ravel() for s in staged]) for j in range(4)]
-                tag = np.concatenate([np.full(len(seasons[s]["obs"][0]), i, dtype=np.int32) for i, s in enumerate(staged)])
-                eng.set_observations_sets(tag, *cols)
-                mis, used = eng.run_season_misfit(mine, ic)
+                mis, used = fused_call()
             except _lib.NesosimError as e:
                 if fused is True or e.code != _lib.ERR_ARG:
                     raise
-                # grids the season-resident kernel does not take: depths to HBM, reduced there per season
-                mis, used = hbm_round_trip()
+                # grids the season-resident kernel does not take: sampled by the general day kernel
+                mis, used = fused_on_general_path(eng, fused_call, hbm_round_trip)
     finally:
         eng.close()
     back = torch.as_tensor(np.argsort(order), device=mis.device)     # native member order -> this rank's pair order
@@ -441,8 +463,9 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     day, row, col, value and optionally kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``, default depth) and
     sigma (default 1), or the 4-tuple (day, row, col, depth).  Returns {"chi2": [P, S, OBS_KINDS], "used": [P, S,
     OBS_KINDS], "model": per season the array [P, n_obs] of model values (NaN on land), or None unless ``model``}, numpy,
-    identical on every rank.  ``fused`` as in ``run_calibration``: None = scored inside the fused path where it applies
-    (falling back on grids wider than the season kernel takes), True = insist on it, False = snowDepths and density to
+    identical on every rank.  ``fused`` as in ``run_calibration``: None = scored inside the season kernel where it applies
+    and on the general day-kernel path on grids wider than it takes (the same fixed order, bit for bit), True = insist
+    on the season kernel, False = snowDepths and density to
     HBM and ``observation_scores`` there.  Observations outside the grid or outside their season's days, bad kinds,
     sigmas and density observations on day 0 raise ValueError before any device work, on either path.
 
@@ -496,33 +519,38 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
                 fchi2[sel], fused_[sel], fmod[sel, :n_fp[s]] = c, u.to(torch.int64), m
         return chi2, used, mod, (fchi2, fused_, fmod)
 
+    def fused_call():
+        cols = {k: np.concatenate([obs[s][k] for s in staged]) for k in obs[0]}
+        tag = np.concatenate([np.full(n_obs[s], i, dtype=np.int32) for i, s in enumerate(staged)])
+        if with_fp:
+            fcols, ftag = concat_footprints([fps[s] for s in staged])
+            eng.set_observations_fp(cols, fcols, obs_set=tag, fp_set=ftag)
+            chi2, used, m, fchi2, fused_, fm = eng.run_season_scores_fp(mine, ic, model=True)
+            fmod = torch.full((M, fp_width), float("nan"), dtype=torch.float64, device=dev)
+            fmod[:, :fm.shape[1]] = fm
+            fp = (fchi2, fused_, fmod)
+        else:
+            eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"],
+                                    cols["sigma"], obs_set=tag)
+            chi2, used, m = eng.run_season_scores(mine, ic, model=model)
+            fp = None
+        mod = None
+        if model:   # rows of the staged seasons' length -> the largest season's (NaN past a row's end)
+            mod = torch.full((M, width), float("nan"), dtype=torch.float64, device=dev)
+            mod[:, :m.shape[1]] = m
+        return chi2, used, mod, fp
+
     try:
         if fused is False:
             chi2, used, mod, fp = hbm_round_trip()
         else:
             try:
-                cols = {k: np.concatenate([obs[s][k] for s in staged]) for k in obs[0]}
-                tag = np.concatenate([np.full(n_obs[s], i, dtype=np.int32) for i, s in enumerate(staged)])
-                if with_fp:
-                    fcols, ftag = concat_footprints([fps[s] for s in staged])
-                    eng.set_observations_fp(cols, fcols, obs_set=tag, fp_set=ftag)
-                    chi2, used, m, fchi2, fused_, fm = eng.run_season_scores_fp(mine, ic, model=True)
-                    fmod = torch.full((M, fp_width), float("nan"), dtype=torch.float64, device=dev)
-                    fmod[:, :fm.shape[1]] = fm
-                    fp = (fchi2, fused_, fmod)
-                else:
-                    eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"],
-                                            cols["sigma"], obs_set=tag)
-                    chi2, used, m = eng.run_season_scores(mine, ic, model=model)
-                    fp = None
-                if model:   # rows of the staged seasons' length -> the largest season's (NaN past a row's end)
-                    mod = torch.full((M, width), float("nan"), dtype=torch.float64, device=dev)
-                    mod[:, :m.shape[1]] = m
+                chi2, used, mod, fp = fused_call()
             except _lib.NesosimError as e:
                 if fused is True or e.code != _lib.ERR_ARG:
                     raise
-                # grids the season-resident kernel does not take: snowDepths and density to HBM, scored there per season
-                chi2, used, mod, fp = hbm_round_trip()
+                # grids the season-resident kernel does not take: sampled by the general day kernel
+                chi2, used, mod, fp = fused_on_general_path(eng, fused_call, hbm_round_trip)
     finally:
         eng.close()
     back = torch.as_tensor(np.argsort(order), device=chi2.device)    # native member order -> this rank's pair order
