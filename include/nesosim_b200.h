@@ -304,6 +304,31 @@ int nesosim_sync(nesosim_ctx *ctx, int *seasons_redone);
 int nesosim_set_path(nesosim_ctx *ctx, int path);
 int nesosim_last_path(const nesosim_ctx *ctx);
 
+/* Calibration gradients (general path only): exact tangent-linear derivatives of the scores of
+ * nesosim_run_season_scores(_fp) with respect to three parameters of every member.  The model is piecewise linear in
+ * them for fixed forcing, so a tangent build of the scoring day kernel carries d(h0, h1)/dtheta through the season in the
+ * same fixed orders as the primal (DESIGN.md §4.1): the pathwise derivative, with the kinks (clamps, NaN masks, the
+ * density clamps) taken on the side the primal took.  windPackThresh enters only through the step W > thresh: its
+ * derivative is 0 almost everywhere and undefined at the step, and it is not reported.
+ * Outputs besides those of nesosim_run_season_scores_fp, which are bit-identical to that call's:
+ *   grad_dev [M][NESOSIM_OBS_KINDS][NESOSIM_GRAD_DIRS]: per kind d chi2 / d theta_j = sum of 2 r (dv_j / sigma) over the
+ *     terms chi2 counts, in chi2's order;
+ *   jac_dev [M][NESOSIM_GRAD_DIRS][jac_stride] or NULL: dv_j at every input observation (NaN where v is not finite and
+ *     for observations dropped at registration);
+ *   fp_grad_dev, fp_jac_dev: the same for the footprints (d mean = sum w dv over the points with finite v / sum w).
+ * Needs observations registered under path 1 (else NESOSIM_ERR_STATE); with footprints registered fp_chi2_dev and
+ * fp_grad_dev are required (NESOSIM_ERR_STATE), without them the fp_* arguments are ignored.  NESOSIM_ERR_ARG: a NULL
+ * grad_dev, a stride shorter than its row, more members or tile rows than a launch grid holds.  The tangent state
+ * (96 bytes per member-cell) is allocated by the first call and freed with the observations.  T+2 launches (T+3 with
+ * footprints), no stream synchronisation, as nesosim_run_season_scores_fp. */
+#define NESOSIM_GRAD_DIRS 3   /* windPackFactor, leadLossFactor, atmLossFactor */
+int nesosim_run_season_score_grads(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                                   int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
+                                   int64_t model_stride, double *grad_dev, double *jac_dev, int64_t jac_stride,
+                                   double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
+                                   int64_t fp_model_stride, double *fp_grad_dev, double *fp_jac_dev, int64_t fp_jac_stride,
+                                   void *stream);
+
 /* ---- Row-strip domain decomposition over peer memory (grids too large for one GPU: the 5 km case; the reference
  * has no counterpart -- its grid is one numpy array -- so the contract is that of calcBudget on the whole grid).
  * A context created on rows [lo-2, hi+2) of the full grid (mask and forcing sliced the same way; 2 = radius of

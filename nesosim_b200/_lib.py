@@ -17,6 +17,10 @@ ERR_ARG, ERR_CUDA, ERR_STATE, ERR_NOMEM = -1, -2, -3, -4
 
 # observed quantities of nesosim_set_observations_ex (NESOSIM_OBS_*): snow depth over ice, snow volume, bulk density
 OBS_DEPTH, OBS_VOLUME, OBS_DENSITY, OBS_KINDS = 0, 1, 2, 3
+# parameter directions of nesosim_run_season_score_grads (NESOSIM_GRAD_DIRS): windPackFactor, leadLossFactor,
+# atmLossFactor -- the columns GRAD_PARAMS of a parameter row [WPF, WPT, LLF, ALF] (windPackThresh has no derivative)
+GRAD_DIRS = 3
+GRAD_PARAMS = (0, 2, 3)
 
 
 class NesosimError(RuntimeError):
@@ -109,6 +113,10 @@ _SIGNATURES = {
     "nesosim_run_season_scores_fp": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int, C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                                C.c_int64, C.c_void_p]),
+    "nesosim_run_season_score_grads": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                                 C.c_int64, C.c_void_p]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

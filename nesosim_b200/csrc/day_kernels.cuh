@@ -66,6 +66,20 @@ struct SampleArgs {
     const int *member_set, *set_steps;   // NULL: one shared season of T days
 };
 
+// Gradient instantiation (GRAD, nesosim_run_season_score_grads): the scoring build plus the tangent-linear step of the
+// two depth layers in GRAD_DIRS parameter directions (windPackFactor, leadLossFactor, atmLossFactor), DESIGN.md §4.1.
+// The tangents live in a ring [parity][dir][layer][M][plane] beside the depth ring; slot 0 is zero (the IC does not
+// depend on the parameters), so day 0 reads no ring at all.  The tangent samples are [M][dir][stride] {t0, t1}, written
+// where the depth samples are.
+constexpr int GRAD_DIRS = 3;         // NESOSIM_GRAD_DIRS
+struct TangentArgs {
+    const double *prev;        // slot x   of direction 0, layer 0, member 0 (dir_stride, layer_stride further: the rest)
+    double *next;              // slot x+1
+    long long layer_stride, dir_stride;
+    double2 *samples;          // [M][GRAD_DIRS][stride] {t0, t1} (stride of SampleArgs)
+    const double *ring;        // sample_last_day_grad_kernel only: the ring's parity 0
+};
+
 // Row-strip domain decomposition over peer memory (SURVEY.md §8e "Space"; host side: nesosim_strip_* in the ABI).
 // This context's grid is one strip of a larger grid, extended by STRIP_GHOST ghost rows towards each neighbouring
 // strip.  Only the two depth layers of the ghost rows are ever needed from a neighbour (fused stencil radius 2 of
@@ -113,10 +127,15 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 
 // Raw advection / divergence of both layers (calcDynamics, NESOSIM.py:189-222, then fillMaskAndNaNWithZero) on the tile
 // grown by one cell, from the staged depth and raw-drift tiles; zero outside the grid (convolve's boundary='fill').
-template <bool INTERIOR, int DAY_THREADS>
+// The gradient build (GRAD below) runs it twice more per direction: RAW_RECORD is the primal pass that also keeps, in
+// `fin`, one bit per raw term of this thread (4 per raw cell it owns: adv0, adv1, div0, div1) telling whether the term
+// was finite; RAW_TANGENT runs the same linear stencils on a staged tangent tile and zeroes each term whose primal was
+// not finite (zero_if_nonfinite made the primal a constant there).  Same cell-to-thread assignment in every mode.
+enum RawMode { RAW_PRIMAL = 0, RAW_RECORD, RAW_TANGENT };
+template <bool INTERIOR, int DAY_THREADS, int MODE = RAW_PRIMAL>
 __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, const int y0, double (&s_h)[2][TY + 4][TX + 4],
                                                double (&s_ut)[TY + 4][TX + 4], double (&s_vt)[TY + 4][TX + 4],
-                                               double (&s_raw)[4][TY + 2][TX + 2]) {
+                                               double (&s_raw)[4][TY + 2][TX + 2], unsigned *fin = nullptr) {
     const int tid = threadIdx.x;
     const int ny = a.ny, nx = a.nx;
     const double dT = a.k.deltaT;
@@ -138,8 +157,18 @@ __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, c
                 const double h = s_h[l][sr][sc];
                 const double gxh = grad(s_h[l][sr][sc - 1], h, s_h[l][sr][sc + 1], gx, nx);
                 const double gyh = grad(s_h[l][sr - 1][sc], h, s_h[l][sr + 1][sc], gy, ny);
-                const double dv = zero_if_nonfinite(div_term(h, gxu, gyv));
-                const double ad = zero_if_nonfinite(adv_term(ut, vt, gxh, gyh));
+                double dv, ad;
+                const int k = (i - tid) / DAY_THREADS;     // this thread's k-th raw cell
+                if (MODE == RAW_TANGENT) {
+                    dv = ((*fin >> (4 * k + 2 + l)) & 1u) ? div_term(h, gxu, gyv) : 0.0;
+                    ad = ((*fin >> (4 * k + l)) & 1u) ? adv_term(ut, vt, gxh, gyh) : 0.0;
+                } else {
+                    dv = zero_if_nonfinite(div_term(h, gxu, gyv));
+                    ad = zero_if_nonfinite(adv_term(ut, vt, gxh, gyh));
+                    if (MODE == RAW_RECORD)
+                        *fin |= ((unsigned)nesosim::finite(adv_term(ut, vt, gxh, gyh)) << (4 * k + l)) |
+                                ((unsigned)nesosim::finite(div_term(h, gxu, gyv)) << (4 * k + 2 + l));
+                }
                 if (l == 0) { adv0 = ad; div0 = dv; } else { adv1 = ad; div1 = dv; }
             }
         }
@@ -150,9 +179,16 @@ __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, c
     }
 }
 
+// What the tangent passes of the gradient build need of a cell's primal step, kept in registers: yesterday's h0 and
+// whether fill_nan_no_negative replaced the new h0 / h1 (NaN: non-finite or land; 0: the clamp fired).
+struct GradCell {
+    double h0;
+    bool kill0, kill1;
+};
+
 // 3x3 smoothing of the four raw planes, the point-wise budget terms and the twelve stores of this thread's cells
-// (SCORE: the two depth stores only).
-template <bool INTERIOR, bool STRIP, int DAY_THREADS, bool SCORE = false>
+// (SCORE: the two depth stores only; GRAD: also fills `gc`).
+template <bool INTERIOR, bool STRIP, int DAY_THREADS, bool SCORE = false, bool GRAD = false>
 __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0, const int y0, const int m,
                                                  double (&s_h)[2][TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
                                                  const double *h0p, const double *h1p, const MemberCoef &mc,
@@ -160,7 +196,8 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
                                                  const double (&pf_C)[TY / (DAY_THREADS / TX)],
                                                  const double (&pf_W)[TY / (DAY_THREADS / TX)],
                                                  const double (&pf_prev)[TY / (DAY_THREADS / TX)][9],
-                                                 const bool (&pf_land)[TY / (DAY_THREADS / TX)], const StripLink *sl) {
+                                                 const bool (&pf_land)[TY / (DAY_THREADS / TX)], const StripLink *sl,
+                                                 GradCell *gc = nullptr) {
     const int tid = threadIdx.x;
     const int ny = a.ny, nx = a.nx;
     const int tx = tid & (TX - 1);
@@ -219,6 +256,11 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
         // NESOSIM.py:327,329 (left to right), then fill_nan_no_negative (332-333)
         double h0n = add(add(add(add(add(add(h0, acc), wpl), lead), atm), adv0), div0);
         double h1n = add(add(add(h1, wpg), adv1), div1);
+        if (GRAD) {
+            gc[rr].h0 = h0;
+            gc[rr].kill0 = !nesosim::finite(h0n) || land || h0n < 0.0;
+            gc[rr].kill1 = !nesosim::finite(h1n) || land || h1n < 0.0;
+        }
         h0n = mask_nan(h0n, land, true);
         h1n = mask_nan(h1n, land, true);
         store(V_H0, h0n);
@@ -242,14 +284,85 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
     }
 }
 
+// The tangent of tile_point_phase in direction j (0 windPackFactor, 1 leadLossFactor, 2 atmLossFactor) for this thread's
+// cells: the smoothed raw tangents (0 on land), then every point term applied to the tangent, plus -- in the parameter's
+// own direction -- the same term of the primal depth with that parameter set to 1; the new tangents are summed in the
+// primal's order (acc has no tangent) and zeroed where fill_nan_no_negative replaced the primal value.  `t0p`/`t1p`:
+// slot x of this member's tangents (read only without dynamics: with them the staged tile is used).
+template <bool INTERIOR, int DAY_THREADS>
+__device__ __forceinline__ void tile_tangent_phase(const DayArgs &a, const int x0, const int y0, const int j,
+                                                   double (&s_h)[2][TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
+                                                   const double *t0p, const double *t1p, double *t0n, double *t1n,
+                                                   const MemberCoef &mc, const double (&pf_C)[TY / (DAY_THREADS / TX)],
+                                                   const double (&pf_W)[TY / (DAY_THREADS / TX)],
+                                                   const bool (&pf_land)[TY / (DAY_THREADS / TX)], const GradCell *gc) {
+    const int tid = threadIdx.x;
+    const int ny = a.ny, nx = a.nx;
+    const int tx = tid & (TX - 1);
+    const int gx = x0 + tx;
+    if (!INTERIOR && gx >= nx) return;
+#pragma unroll
+    for (int rr = 0; rr < TY / (DAY_THREADS / TX); ++rr) {
+        const int ty = (tid / TX) + rr * (DAY_THREADS / TX);
+        const int gy = y0 + ty;
+        if (!INTERIOR && gy >= ny) break;
+        const long long o = (long long)gy * nx + gx;
+        const bool land = pf_land[rr];
+        double adv0 = 0.0, adv1 = 0.0, div0 = 0.0, div1 = 0.0, t0, t1;
+        if (a.sw.dynamics) {
+            double sm[4];
+#pragma unroll
+            for (int p = 0; p < 4; ++p) {
+                const double top = conv3x3(a.w, [&](int ii, int jj) { return s_raw[p][ty + ii][tx + jj]; });
+                sm[p] = land ? 0.0 : div_const(top, a.conv_div);
+            }
+            adv0 = sm[0]; adv1 = sm[1]; div0 = sm[2]; div1 = sm[3];
+            t0 = s_h[0][ty + 2][tx + 2];
+            t1 = s_h[1][ty + 2][tx + 2];
+        } else {
+            t0 = a.x > 0 ? t0p[o] : 0.0;
+            t1 = a.x > 0 ? t1p[o] : 0.0;
+        }
+        const double W = pf_W[rr], C = pf_C[rr], h0 = gc[rr].h0, dT = a.k.deltaT;
+        const double wt = wind_flag(W, mc.wpt);
+        MemberCoef one = mc;                 // the coefficients of the parameter's own direction set to 1
+        one.neg_wpf_dt = -dT;
+        one.wpf_dt = dT;
+        one.llf = 1.0;
+        one.alf = 1.0;
+        double lead = 0.0, atm = 0.0, wpl = 0.0, wpg = 0.0, net;
+        if (a.sw.leadloss) {
+            lead = lead_loss(wt, t0, W, C, mc, a.k);
+            if (j == 1) lead = add(lead, lead_loss(wt, h0, W, C, one, a.k));
+        }
+        if (a.sw.atmloss) {
+            atm = atm_loss(wt, t0, W, mc, a.k);
+            if (j == 2) atm = add(atm, atm_loss(wt, h0, W, one, a.k));
+        }
+        if (a.sw.windpack) {
+            wind_packing(wt, t0, mc, a.k, wpl, wpg, net);
+            if (j == 0) {
+                double l, g;
+                wind_packing(wt, h0, one, a.k, l, g, net);
+                wpl = add(wpl, l);
+                wpg = add(wpg, g);
+            }
+        }
+        const double d0 = add(add(add(add(add(t0, wpl), lead), atm), adv0), div0);
+        const double d1 = add(add(add(t1, wpg), adv1), div1);
+        t0n[o] = gc[rr].kill0 ? 0.0 : d0;
+        t1n[o] = gc[rr].kill1 ? 0.0 : d1;
+    }
+}
+
 // INTERIOR: the tile with its two-cell halo lies inside the grid and none of its raw-dynamics cells is a grid-edge
 // cell, so there are no bounds tests, every difference is centred and the divisor is a launch constant (the
 // overwhelming majority of the CTAs on the 25 km and 5 km grids).
-template <bool INTERIOR, bool STRIP = false, int DAY_THREADS = 256, bool SCORE = false>
+template <bool INTERIOR, bool STRIP = false, int DAY_THREADS = 256, bool SCORE = false, bool GRAD = false>
 __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2][TY + 4][TX + 4], double (&s_ut)[TY + 4][TX + 4],
                                               double (&s_vt)[TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
                                               const int bx, const int by, const StripLink *sl = nullptr,
-                                              const SampleArgs *sa = nullptr) {
+                                              const SampleArgs *sa = nullptr, const TangentArgs *ta = nullptr) {
     const int m = blockIdx.z;
     const int x0 = bx * TX, y0 = by * TY;     // (bx, by): the tile (blockIdx, or what a strip / season CTA picked)
     const int tid = threadIdx.x;
@@ -271,6 +384,8 @@ __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2]
     const int ptx = tid & (TX - 1), pgx = x0 + ptx;
     double pf_P[CPT], pf_C[CPT], pf_W[CPT], pf_prev[CPT][9];
     bool pf_land[CPT];
+    GradCell gc[CPT];          // GRAD only: the primal state the tangent passes need
+    unsigned fin = 0;          // GRAD only: finite bits of this thread's primal raw terms (tile_raw_phase)
 #pragma unroll
     for (int rr = 0; rr < CPT; ++rr) {
         const int gy = y0 + (tid / TX) + rr * (DAY_THREADS / TX);
@@ -306,6 +421,14 @@ __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2]
         for (int i = b[0] + tid; i < b[1]; i += DAY_THREADS) {
             const int2 e = sa->entry[i];
             row[e.y] = make_double2(h0p[e.x], h1p[e.x]);
+            if (GRAD) {
+#pragma unroll
+                for (int j = 0; j < GRAD_DIRS; ++j) {
+                    const double *t0 = ta->prev + j * ta->dir_stride + (long long)m * a.depth_mstride;
+                    ta->samples[((long long)m * GRAD_DIRS + j) * sa->stride + e.y] =
+                        a.x > 0 ? make_double2(t0[e.x], t0[ta->layer_stride + e.x]) : make_double2(0.0, 0.0);
+                }
+            }
         }
     }
 
@@ -344,12 +467,37 @@ __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2]
         }
         cp_async_wait_all();
         __syncthreads();
-        tile_raw_phase<INTERIOR, DAY_THREADS>(a, x0, y0, s_h, s_ut, s_vt, s_raw);
+        tile_raw_phase<INTERIOR, DAY_THREADS, GRAD ? RAW_RECORD : RAW_PRIMAL>(a, x0, y0, s_h, s_ut, s_vt, s_raw, &fin);
         __syncthreads();
     }
 
-    tile_point_phase<INTERIOR, STRIP, DAY_THREADS, SCORE>(a, x0, y0, m, s_h, s_raw, h0p, h1p, mc, pf_P, pf_C, pf_W, pf_prev,
-                                                          pf_land, sl);
+    tile_point_phase<INTERIOR, STRIP, DAY_THREADS, SCORE, GRAD>(a, x0, y0, m, s_h, s_raw, h0p, h1p, mc, pf_P, pf_C, pf_W,
+                                                                pf_prev, pf_land, sl, gc);
+    if (GRAD) {
+        // The three tangent passes reuse the tile's shared buffers: the tangent tile of direction j replaces the depth tile,
+        // its raw terms the raw terms (the drift tiles stay), so the gradient build needs no more shared memory.
+#pragma unroll 1
+        for (int j = 0; j < GRAD_DIRS; ++j) {
+            const double *t0p = ta->prev + j * ta->dir_stride + (long long)m * a.depth_mstride, *t1p = t0p + ta->layer_stride;
+            double *t0n = ta->next + j * ta->dir_stride + (long long)m * a.depth_mstride, *t1n = t0n + ta->layer_stride;
+            if (a.sw.dynamics) {
+                __syncthreads();      // every thread is done with the previous pass's tiles
+                for (int i = tid; i < (TY + 4) * (TX + 4); i += DAY_THREADS) {
+                    const int r = i / (TX + 4), c = i - r * (TX + 4);
+                    const int gy = y0 + r - 2, gx = x0 + c - 2;
+                    const bool in = INTERIOR || (gy >= 0 && gy < ny && gx >= 0 && gx < nx);
+                    const long long o = in ? (long long)gy * nx + gx : 0;
+                    cp_async8(&s_h[0][r][c], t0p + o, in && a.x > 0);
+                    cp_async8(&s_h[1][r][c], t1p + o, in && a.x > 0);
+                }
+                cp_async_wait_all();
+                __syncthreads();
+                tile_raw_phase<INTERIOR, DAY_THREADS, RAW_TANGENT>(a, x0, y0, s_h, s_ut, s_vt, s_raw, &fin);
+                __syncthreads();
+            }
+            tile_tangent_phase<INTERIOR, DAY_THREADS>(a, x0, y0, j, s_h, s_raw, t0p, t1p, t0n, t1n, mc, pf_C, pf_W, pf_land, gc);
+        }
+    }
 }
 
 // A tile without a single ocean cell (more than half of the polar grid is land, and it comes in large blocks).  From
@@ -411,9 +559,11 @@ __device__ __forceinline__ void day_step_land_tile(const DayArgs &a, const int b
     }
 }
 
-// The land tile of the scoring build: only its NaN depths are stored (a land tile has no observed cell to sample).
-template <int DAY_THREADS>
-__device__ __forceinline__ void day_step_land_depths(const DayArgs &a, const int bx, const int by) {
+// The land tile of the scoring build: only its NaN depths are stored (a land tile has no observed cell to sample);
+// GRAD: and zero tangents.
+template <int DAY_THREADS, bool GRAD = false>
+__device__ __forceinline__ void day_step_land_depths(const DayArgs &a, const int bx, const int by,
+                                                     const TangentArgs *ta = nullptr) {
     const int m = blockIdx.z;
     const int fset = a.member_set ? a.member_set[m] : 0;
     if (a.set_steps && a.x >= a.set_steps[fset]) {
@@ -430,6 +580,13 @@ __device__ __forceinline__ void day_step_land_depths(const DayArgs &a, const int
         const long long id = (long long)m * a.depth_mstride + (long long)gy * a.nx + gx;
         a.next[V_H0][id] = qnan();
         a.next[V_H1][id] = qnan();
+        if (GRAD) {
+#pragma unroll
+            for (int j = 0; j < GRAD_DIRS; ++j) {
+                ta->next[j * ta->dir_stride + id] = 0.0;
+                ta->next[j * ta->dir_stride + ta->layer_stride + id] = 0.0;
+            }
+        }
     }
 }
 
@@ -440,12 +597,12 @@ struct TileSmem {
     double raw[4][TY + 2][TX + 2];   // adv0, adv1, div0, div1 after the NaN->0 fill
 };
 
-template <int DAY_THREADS, bool SCORE = false>
+template <int DAY_THREADS, bool SCORE = false, bool GRAD = false>
 __device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, const int bx, const int by,
-                                              const SampleArgs *sa = nullptr) {
+                                              const SampleArgs *sa = nullptr, const TangentArgs *ta = nullptr) {
     pdl_launch_dependents();
     if (a.tile_land && a.tile_land[by * ((a.nx + TX - 1) / TX) + bx]) {
-        if (SCORE) day_step_land_depths<DAY_THREADS>(a, bx, by);
+        if (SCORE) day_step_land_depths<DAY_THREADS, GRAD>(a, bx, by, ta);
         else day_step_land_tile<DAY_THREADS>(a, bx, by);
         return;
     }
@@ -455,8 +612,8 @@ __device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, co
     auto &s_raw = sm.raw;
     const int x0 = bx * TX, y0 = by * TY;
     const bool interior = x0 >= 2 && y0 >= 2 && x0 + TX + 2 <= a.nx && y0 + TY + 2 <= a.ny;
-    if (interior) day_step_body<true, false, DAY_THREADS, SCORE>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa);
-    else day_step_body<false, false, DAY_THREADS, SCORE>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa);
+    if (interior) day_step_body<true, false, DAY_THREADS, SCORE, GRAD>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa, ta);
+    else day_step_body<false, false, DAY_THREADS, SCORE, GRAD>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa, ta);
 }
 
 // Two builds of the same tile code: 256 threads x 2 cells (large grids: fewer, fatter threads) and 512 threads x 1
@@ -482,10 +639,25 @@ __global__ void __launch_bounds__(512, 2) day_step_score_kernel_512(const __grid
     day_step_tile<512, true>(a, sm, blockIdx.x, blockIdx.y, &s);
 }
 
+// The gradient builds of the same two shapes (TangentArgs above).
+__global__ void __launch_bounds__(256) day_step_grad_kernel(const __grid_constant__ DayArgs a,
+                                                            const __grid_constant__ SampleArgs s,
+                                                            const __grid_constant__ TangentArgs t) {
+    __shared__ TileSmem sm;
+    day_step_tile<256, true, true>(a, sm, blockIdx.x, blockIdx.y, &s, &t);
+}
+__global__ void __launch_bounds__(512, 2) day_step_grad_kernel_512(const __grid_constant__ DayArgs a,
+                                                                   const __grid_constant__ SampleArgs s,
+                                                                   const __grid_constant__ TangentArgs t) {
+    __shared__ TileSmem sm;
+    day_step_tile<512, true, true>(a, sm, blockIdx.x, blockIdx.y, &s, &t);
+}
+
 // The last day of every member's season (set_steps[set], or T-1), which no day kernel reads: one CTA per member copies
 // its set's entries of that day from the member's ring slot.  A member whose season ended early has not touched its
-// ring since (its CTAs leave the later day kernels at once).
-__global__ void __launch_bounds__(256) sample_last_day_kernel(const __grid_constant__ SampleArgs s) {
+// ring since (its CTAs leave the later day kernels at once).  GRAD: the tangent samples of that day too.
+template <bool GRAD>
+__device__ __forceinline__ void sample_last_day(const SampleArgs &s, const TangentArgs *t) {
     const int m = blockIdx.x;
     const int set = s.member_set ? s.member_set[m] : 0;
     const int day = s.set_steps ? s.set_steps[set] : s.T - 1;
@@ -496,7 +668,23 @@ __global__ void __launch_bounds__(256) sample_last_day_kernel(const __grid_const
     for (int i = s.begin[b] + threadIdx.x; i < s.begin[b + s.tiles]; i += blockDim.x) {
         const int2 e = s.entry[i];
         row[e.y] = make_double2(h0[e.x], h1[e.x]);
+        if (GRAD) {
+#pragma unroll
+            for (int j = 0; j < GRAD_DIRS; ++j) {
+                const double *t0 = t->ring + (long long)(day & 1) * GRAD_DIRS * t->dir_stride + j * t->dir_stride +
+                                   (long long)m * s.plane;
+                t->samples[((long long)m * GRAD_DIRS + j) * s.stride + e.y] =
+                    day > 0 ? make_double2(t0[e.x], t0[t->layer_stride + e.x]) : make_double2(0.0, 0.0);
+            }
+        }
     }
+}
+__global__ void __launch_bounds__(256) sample_last_day_kernel(const __grid_constant__ SampleArgs s) {
+    sample_last_day<false>(s, nullptr);
+}
+__global__ void __launch_bounds__(256) sample_last_day_grad_kernel(const __grid_constant__ SampleArgs s,
+                                                                   const __grid_constant__ TangentArgs t) {
+    sample_last_day<true>(s, &t);
 }
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {

@@ -228,6 +228,12 @@ struct nesosim_ctx {
         int2 *smp_entry = nullptr;                       // (cell, slot in the member's row)
         int smp_tiles = 0;                               // day-kernel tiles of the grid
         double *ring = nullptr;                          // [parity 2][layer 2][M][plane]
+        // nesosim_run_season_score_grads (allocated by its first call, freed with the observations): the tangent ring
+        // [parity 2][GRAD_DIRS][layer 2][M][plane], the tangent samples [M][GRAD_DIRS][stride] and the footprint mean
+        // derivatives [M][GRAD_DIRS][max(1, fp_row_len)]
+        double *tring = nullptr;
+        double2 *tsamples = nullptr;
+        double *fp_dmean = nullptr;
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -379,6 +385,7 @@ void obs_release(nesosim_ctx *ctx) {
     cudaFree(ob.fp_kind_begin); cudaFree(ob.pt_slot); cudaFree(ob.pt_day); cudaFree(ob.pt_cell); cudaFree(ob.pt_w);
     cudaFree(ob.fp_mean);
     cudaFree(ob.smp_begin); cudaFree(ob.smp_entry); cudaFree(ob.ring);
+    cudaFree(ob.tring); cudaFree(ob.tsamples); cudaFree(ob.fp_dmean);
     ob = {};
 }
 
@@ -1267,8 +1274,34 @@ __device__ __forceinline__ void block_total(double acc, long long cnt, double *r
     __syncthreads();
 }
 
-template <bool SETS>
-__global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constant__ MisfitArgs a) {
+// Gradient stage of the epilogue (misfit_finish_grad_kernel, nesosim_run_season_score_grads): the tangent samples give
+// each observation's derivative dv in GRAD_DIRS directions (density_tangent for density), NaN where v is not finite;
+// per kind and direction the terms 2 r (dv / sigma) of the observations chi2 counts are summed in chi2's order.
+struct MisfitGrad {
+    const double2 *tsamples;        // [M][GRAD_DIRS][stride] {t0, t1}
+    double *grad;                   // [M][NESOSIM_OBS_KINDS][GRAD_DIRS]
+    double *jac;                    // [M][GRAD_DIRS][jac_stride] at the input index, or NULL
+    long long jac_stride;
+    const double *fp_dmean;         // [M][GRAD_DIRS][fp_stride] footprint mean derivatives (footprint_mean_grad_kernel)
+    double *fp_grad;                // [M][NESOSIM_OBS_KINDS][GRAD_DIRS] (read only with the footprint stage)
+};
+
+// d(densityCalc)/dtheta at a sample from the primal quotient q and den = h0 + h1 (quotient rule), 0 where a clamp set q
+__device__ __forceinline__ double density_tangent(double h0, double h1, double t0, double t1, const ModelConsts &k) {
+    const double den = add(h0, h1);
+    const double q = div_ieee(add(mul(h0, k.rhoFresh), mul(h1, k.rhoOld)), den);
+    if (q > k.rhoOld || q < k.rhoFresh) return 0.0;
+    return div_ieee(sub(add(mul(t0, k.rhoFresh), mul(t1, k.rhoOld)), mul(q, add(t0, t1))), den);
+}
+
+__device__ __forceinline__ double obs_tangent(int kind, double2 h, double2 t, double C, const ModelConsts &k) {
+    if (kind == NESOSIM_OBS_DEPTH) return div_ieee(add(t.x, t.y), C);
+    if (kind == NESOSIM_OBS_VOLUME) return add(t.x, t.y);
+    return density_tangent(h.x, h.y, t.x, t.y, k);
+}
+
+template <bool SETS, bool GRAD>
+__device__ __forceinline__ void misfit_finish(const MisfitArgs &a, const MisfitGrad *g) {
     const int m = blockIdx.x;
     const double2 *samp = a.samples + (long long)m * a.stride;
     const int set = SETS ? a.member_set[m] : 0;
@@ -1279,7 +1312,7 @@ __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constan
     __shared__ long long redc[8];
     for (int kind = 0; kind < a.n_kinds; ++kind) {
         const long long i0 = kb[kind], n_obs = (long long)kb[kind + 1] - i0;
-        double acc = 0.0;
+        double acc = 0.0, gacc[GRAD_DIRS] = {0.0, 0.0, 0.0};
         long long cnt = 0;
         for (long long i = threadIdx.x; i < n_obs; i += 256) {
             const long long q = i0 + i;
@@ -1289,14 +1322,33 @@ __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constan
             else if (kind == NESOSIM_OBS_VOLUME) v = add(h.x, h.y);
             else v = density_variable(h.x, h.y, false, a.k);
             if (model) model[a.src[q]] = v;
+            double dv[GRAD_DIRS];
+            if (GRAD) {
+                const double C = kind == NESOSIM_OBS_DEPTH ? __ldg(conc + (long long)a.obs_day[q] * a.plane + a.obs_cell[q]) : 1.0;
+#pragma unroll
+                for (int j = 0; j < GRAD_DIRS; ++j) {
+                    const double2 t = g->tsamples[((long long)m * GRAD_DIRS + j) * a.stride + a.obs_slot[q]];
+                    dv[j] = nesosim::finite(v) ? obs_tangent(kind, h, t, C, a.k) : nesosim::qnan();
+                    if (g->jac) g->jac[((long long)m * GRAD_DIRS + j) * g->jac_stride + a.src[q]] = dv[j];
+                }
+            }
             const double r = div_ieee(sub(v, a.obs_val[q]), a.sigma[q]);   // sigma 1: exact, r = model - observed
             if (nesosim::finite(r)) {
                 acc = add(acc, mul(r, r));
                 ++cnt;
+                if (GRAD) {
+#pragma unroll
+                    for (int j = 0; j < GRAD_DIRS; ++j) gacc[j] = add(gacc[j], mul(mul(2.0, r), div_ieee(dv[j], a.sigma[q])));
+                }
             }
         }
         block_total(acc, cnt, red, redc, a.chi2 + (long long)m * a.n_kinds + kind,
                     a.count ? a.count + (long long)m * a.n_kinds + kind : nullptr);
+        if (GRAD) {
+#pragma unroll
+            for (int j = 0; j < GRAD_DIRS; ++j)
+                block_total(gacc[j], 0, red, redc, g->grad + ((long long)m * NESOSIM_OBS_KINDS + kind) * GRAD_DIRS + j, nullptr);
+        }
     }
     if (!a.fp_chi2) return;
     // footprints: the same fixed order over each kind's range of the set's footprint table
@@ -1304,7 +1356,7 @@ __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constan
     const double *mean = a.fp_mean + (long long)m * a.fp_stride - fkb[0];   // indexed by table position
     for (int kind = 0; kind < NESOSIM_OBS_KINDS; ++kind) {
         const long long i0 = fkb[kind], n_fp = (long long)fkb[kind + 1] - i0;
-        double acc = 0.0;
+        double acc = 0.0, gacc[GRAD_DIRS] = {0.0, 0.0, 0.0};
         long long cnt = 0;
         for (long long i = threadIdx.x; i < n_fp; i += 256) {
             const long long q = i0 + i;
@@ -1312,11 +1364,33 @@ __global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constan
             if (nesosim::finite(r)) {
                 acc = add(acc, mul(r, r));
                 ++cnt;
+                if (GRAD) {
+#pragma unroll
+                    for (int j = 0; j < GRAD_DIRS; ++j) {
+                        const double dm = g->fp_dmean[((long long)m * GRAD_DIRS + j) * a.fp_stride - fkb[0] + q];
+                        gacc[j] = add(gacc[j], mul(mul(2.0, r), div_ieee(dm, a.fp_sigma[q])));
+                    }
+                }
             }
         }
         block_total(acc, cnt, red, redc, a.fp_chi2 + (long long)m * NESOSIM_OBS_KINDS + kind,
                     a.fp_count ? a.fp_count + (long long)m * NESOSIM_OBS_KINDS + kind : nullptr);
+        if (GRAD) {
+#pragma unroll
+            for (int j = 0; j < GRAD_DIRS; ++j)
+                block_total(gacc[j], 0, red, redc, g->fp_grad + ((long long)m * NESOSIM_OBS_KINDS + kind) * GRAD_DIRS + j, nullptr);
+        }
     }
+}
+
+template <bool SETS>
+__global__ void __launch_bounds__(256) misfit_finish_kernel(const __grid_constant__ MisfitArgs a) {
+    misfit_finish<SETS, false>(a, nullptr);
+}
+template <bool SETS>
+__global__ void __launch_bounds__(256) misfit_finish_grad_kernel(const __grid_constant__ MisfitArgs a,
+                                                                 const __grid_constant__ MisfitGrad g) {
+    misfit_finish<SETS, true>(a, &g);
 }
 
 // Footprint means: one warp per (member, footprint).  The model value of every point is formed with exactly the
@@ -1349,8 +1423,16 @@ struct FootprintArgs {
     long long conc_set_stride;      // SETS only
 };
 constexpr int FP_UNROLL = 8;
-template <bool SETS>
-__global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constant__ FootprintArgs a) {
+// GRAD (footprint_mean_grad_kernel): lane l also adds w*dv of the same points, in the same order, for every direction,
+// and the same tree gives the derivative of the mean, sdw / s (NaN where the mean is not finite).
+struct FootprintGrad {
+    const double2 *tsamples;        // [M][GRAD_DIRS][stride]
+    double *dmean;                  // [M][GRAD_DIRS][mean_stride] in table order within the set
+    double *jac;                    // [M][GRAD_DIRS][jac_stride] at the input index within the set, or NULL
+    long long jac_stride;
+};
+template <bool SETS, bool GRAD>
+__device__ __forceinline__ void footprint_mean(const FootprintArgs &a, const FootprintGrad *fg) {
     const int m = (int)(blockIdx.x % (unsigned)a.n_members);
     const long long g = blockIdx.x / (unsigned)a.n_members;
     const int lane = threadIdx.x;
@@ -1360,6 +1442,8 @@ __global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constan
     double *model = a.model ? a.model + (long long)m * a.model_stride : nullptr;
     if (g >= (long long)kb[NESOSIM_OBS_KINDS] - kb[0]) {          // padding of a set with fewer footprints
         if (model && lane == 0) model[g] = nesosim::qnan();
+        if (GRAD && fg->jac && lane == 0)
+            for (int j = 0; j < GRAD_DIRS; ++j) fg->jac[((long long)m * GRAD_DIRS + j) * fg->jac_stride + g] = nesosim::qnan();
         return;
     }
     const long long q = kb[0] + g;
@@ -1367,7 +1451,7 @@ __global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constan
     const double2 *samp = a.samples + (long long)m * a.stride;
     const double *conc = SETS ? a.conc + (long long)set * a.conc_set_stride : a.conc;
     const long long p1 = a.begin[q + 1];
-    double sw = 0.0, s = 0.0;
+    double sw = 0.0, s = 0.0, sdw[GRAD_DIRS] = {0.0, 0.0, 0.0};
     for (long long p = a.begin[q] + lane; p < p1; p += 32 * FP_UNROLL) {
         double2 h[FP_UNROLL];
         double w[FP_UNROLL], c[FP_UNROLL];
@@ -1390,6 +1474,14 @@ __global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constan
                 if (nesosim::finite(v)) {
                     sw = add(sw, mul(w[u], v));
                     s = add(s, w[u]);
+                    if (GRAD) {
+                        const int slot = __ldg(a.pt_slot + p + 32 * u);
+#pragma unroll
+                        for (int j = 0; j < GRAD_DIRS; ++j) {
+                            const double2 t = fg->tsamples[((long long)m * GRAD_DIRS + j) * a.stride + slot];
+                            sdw[j] = add(sdw[j], mul(w[u], obs_tangent(kind, h[u], t, c[u], a.k)));
+                        }
+                    }
                 }
             }
         }
@@ -1398,12 +1490,32 @@ __global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constan
     for (int off = 16; off > 0; off >>= 1) {
         sw = add(sw, __shfl_down_sync(0xffffffffu, sw, off));
         s = add(s, __shfl_down_sync(0xffffffffu, s, off));
+        if (GRAD) {
+#pragma unroll
+            for (int j = 0; j < GRAD_DIRS; ++j) sdw[j] = add(sdw[j], __shfl_down_sync(0xffffffffu, sdw[j], off));
+        }
     }
     if (lane == 0) {
         const double v = div_ieee(sw, s);
         a.mean[(long long)m * a.mean_stride + g] = v;
         if (model) model[a.src[q]] = v;
+        if (GRAD) {
+            for (int j = 0; j < GRAD_DIRS; ++j) {
+                const double dm = nesosim::finite(v) ? div_ieee(sdw[j], s) : nesosim::qnan();
+                fg->dmean[((long long)m * GRAD_DIRS + j) * a.mean_stride + g] = dm;
+                if (fg->jac) fg->jac[((long long)m * GRAD_DIRS + j) * fg->jac_stride + a.src[q]] = dm;
+            }
+        }
     }
+}
+template <bool SETS>
+__global__ void __launch_bounds__(32) footprint_mean_kernel(const __grid_constant__ FootprintArgs a) {
+    footprint_mean<SETS, false>(a, nullptr);
+}
+template <bool SETS>
+__global__ void __launch_bounds__(32) footprint_mean_grad_kernel(const __grid_constant__ FootprintArgs a,
+                                                                 const __grid_constant__ FootprintGrad fg) {
+    footprint_mean<SETS, true>(a, &fg);
 }
 
 // Observations compiled against the strip tables (host side).  One season's tables: every observation mapped to its
@@ -1747,7 +1859,9 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
 // The sample producer of the general path: slot 0 of the depth ring (init_slot0_kernel), the T-1 scoring day kernels
 // (day x samples day x, then advances the depths to slot x+1) and sample_last_day_kernel: T+1 launches, no pre-pass,
 // nothing written outside the context, no synchronisation.
-int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cudaStream_t st) {
+// grad: the gradient builds (day_step_grad_kernel, sample_last_day_grad_kernel), which also advance and sample the
+// tangents; still T+1 launches.
+int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cudaStream_t st, bool grad = false) {
     const auto &ob = ctx->obs;
     const nesosim_config &c = ctx->cfg;
     const int T = c.num_days, M = c.n_members;
@@ -1773,6 +1887,12 @@ int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cu
     sa.ring = ob.ring; sa.plane = plane; sa.layer_stride = layer;
     sa.member_set = ctx->member_set_dev; sa.set_steps = ctx->set_steps_dev;
     const dim3 grid((c.nx + TX - 1) / TX, (c.ny + TY - 1) / TY, M);
+    TangentArgs ta{};
+    ta.layer_stride = layer;
+    ta.dir_stride = 2 * layer;
+    ta.samples = ob.tsamples;
+    ta.ring = ob.tring;
+    auto tring = [&](int t) { return ob.tring + (long long)(t & 1) * GRAD_DIRS * 2 * layer; };
     nesosim_outputs none{};
     for (int x = 0; x < T - 1; ++x) {
         DayArgs a;
@@ -1785,11 +1905,20 @@ int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cu
         }
         a.depth_mstride = a.plane_mstride = plane;
         const bool pdl = ctx->pdl && x > 0;       // behind this call's own previous day kernel only (see launch_day)
-        if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_score_kernel_512, grid, 512, st, pdl, a, sa));
-        else CU(launch_day_kernel(day_step_score_kernel, grid, 256, st, pdl, a, sa));
+        if (grad) {
+            ta.prev = tring(x);
+            ta.next = tring(x + 1);
+            if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_grad_kernel_512, grid, 512, st, pdl, a, sa, ta));
+            else CU(launch_day_kernel(day_step_grad_kernel, grid, 256, st, pdl, a, sa, ta));
+        } else if (ctx->day_variant == 512) {
+            CU(launch_day_kernel(day_step_score_kernel_512, grid, 512, st, pdl, a, sa));
+        } else {
+            CU(launch_day_kernel(day_step_score_kernel, grid, 256, st, pdl, a, sa));
+        }
         ctx->launches++;
     }
-    sample_last_day_kernel<<<M, 256, 0, st>>>(sa);
+    if (grad) sample_last_day_grad_kernel<<<M, 256, 0, st>>>(sa, ta);
+    else sample_last_day_kernel<<<M, 256, 0, st>>>(sa);
     ctx->launches++;
     CU(cudaGetLastError());
     return NESOSIM_OK;
@@ -1799,10 +1928,30 @@ int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cu
 // 1 (nesosim_run_season_misfit: the depth sum only, which needs observations that are all depth with sigma 1).
 // fp: nesosim_run_season_scores_fp -- the footprint means (footprint_mean_kernel) between the season and the epilogue,
 // which then also scores them; without it, registered footprints are NESOSIM_ERR_STATE (their data would be dropped).
+// g: nesosim_run_season_score_grads -- the gradient builds of the day kernel and of both epilogues (general path only).
+struct GradOutputs {
+    double *grad, *jac;
+    int64_t jac_stride;
+    double *fp_grad, *fp_jac;
+    int64_t fp_jac_stride;
+};
 int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev, int ic_per_member,
                       double *chi2_dev, int64_t *count_dev, int n_kinds, double *model_dev, int64_t model_stride,
                       void *stream, bool fp = false, double *fp_chi2_dev = nullptr, int64_t *fp_count_dev = nullptr,
-                      double *fp_model_dev = nullptr, int64_t fp_model_stride = 0) {
+                      double *fp_model_dev = nullptr, int64_t fp_model_stride = 0, const GradOutputs *g = nullptr) {
+    if (g) {
+        if (!ctx || !params_host || !chi2_dev || !g->grad) return fail(NESOSIM_ERR_ARG, "bad argument");
+        if (!ctx->obs.ready || !ctx->obs.general)
+            return fail(NESOSIM_ERR_STATE, "gradients need observations registered on the general path (nesosim_set_path(ctx, 1) first)");
+        if (ctx->obs.n_fp && (!fp_chi2_dev || !g->fp_grad))
+            return fail(NESOSIM_ERR_STATE, "footprints are registered: fp_chi2_dev and fp_grad_dev are required");
+        if (g->jac && g->jac_stride < ctx->obs.row_len) return fail(NESOSIM_ERR_ARG, "jac_stride is shorter than the observation row");
+        if (ctx->obs.n_fp && g->fp_jac && g->fp_jac_stride < ctx->obs.fp_row_len)
+            return fail(NESOSIM_ERR_ARG, "fp_jac_stride is shorter than the footprint row");
+        if (ctx->cfg.n_members > 65535 || (ctx->cfg.ny + TY - 1) / TY > 65535)
+            return fail(NESOSIM_ERR_ARG, "members or tile rows exceed the day kernel's grid dimensions");
+        fp = ctx->obs.n_fp > 0;
+    }
     if (!ctx || !params_host || !chi2_dev || (fp && !fp_chi2_dev)) return fail(NESOSIM_ERR_ARG, "bad argument");
     if (!ctx->P) return fail(NESOSIM_ERR_STATE, "nesosim_set_forcing has not been called");
     if (!ctx->obs.ready) return fail(NESOSIM_ERR_STATE, "nesosim_set_observations has not been called");
@@ -1825,10 +1974,20 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     const nesosim_config &c = ctx->cfg;
     const int T = c.num_days, M = c.n_members;
     int rc;
+    auto &ob = ctx->obs;
+    if (g) {
+        const size_t tr = (size_t)2 * GRAD_DIRS * 2 * M * ctx->plane, ts = (size_t)M * GRAD_DIRS * ob.stride;
+        if (!ob.tring) CU(cudaMalloc(&ob.tring, tr * sizeof(double)));
+        if (!ob.tsamples) {
+            CU(cudaMalloc(&ob.tsamples, ts * sizeof(double2)));
+            CU(cudaMemset(ob.tsamples, 0, ts * sizeof(double2)));
+        }
+        if (!ob.fp_dmean) CU(cudaMalloc(&ob.fp_dmean, (size_t)M * GRAD_DIRS * std::max(1LL, ob.fp_row_len) * sizeof(double)));
+    }
     if (general) {
         if ((rc = upload_coef(ctx, params_host, st))) return rc;
         ctx->last_path = 1;
-        if ((rc = run_score_days(ctx, ic_dev, ic_per_member, st))) return rc;
+        if ((rc = run_score_days(ctx, ic_dev, ic_per_member, st, g != nullptr))) return rc;
     } else {
         nesosim_outputs none{};
         none.depth_member_stride = (int64_t)T * 2 * ctx->plane;
@@ -1847,6 +2006,14 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     // observations dropped at registration (land, lake) have no model value: their entries stay NaN (all bits set)
     if (model_dev && ctx->obs.row_len)
         CU(cudaMemset2DAsync(model_dev, (size_t)model_stride * sizeof(double), 0xff, (size_t)ctx->obs.row_len * sizeof(double), M, st));
+    if (g && g->jac && ob.row_len)
+        CU(cudaMemset2DAsync(g->jac, (size_t)g->jac_stride * sizeof(double), 0xff, (size_t)ob.row_len * sizeof(double),
+                             (size_t)M * GRAD_DIRS, st));
+    MisfitGrad mg{};
+    if (g) {
+        mg.tsamples = ob.tsamples; mg.grad = g->grad; mg.jac = g->jac; mg.jac_stride = g->jac_stride;
+        mg.fp_dmean = ob.fp_dmean; mg.fp_grad = g->fp_grad;
+    }
     MisfitArgs ma;
     ma.samples = ctx->obs.samples; ma.stride = ctx->obs.stride;
     ma.obs_slot = ctx->obs.o_slot; ma.obs_day = ctx->obs.o_day; ma.obs_cell = ctx->obs.o_cell; ma.src = ctx->obs.src;
@@ -1857,7 +2024,6 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     ma.member_set = ctx->member_set_dev; ma.conc_set_stride = (long long)T * ctx->plane;
     ma.fp_chi2 = nullptr; ma.fp_count = nullptr;
     if (fp) {
-        const auto &ob = ctx->obs;
         if (ob.fp_row_len) {
             FootprintArgs fa;
             fa.samples = ob.samples; fa.stride = ob.stride;
@@ -1869,7 +2035,10 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
             fa.member_set = ctx->member_set_dev; fa.conc_set_stride = (long long)T * ctx->plane;
             const long long blocks = ob.fp_row_len * M;
             if (blocks > INT_MAX) return fail(NESOSIM_ERR_ARG, "too many footprints x members for one launch");
-            if (sets) footprint_mean_kernel<true><<<(unsigned)blocks, 32, 0, st>>>(fa);
+            FootprintGrad fg{ob.tsamples, ob.fp_dmean, g ? g->fp_jac : nullptr, g ? g->fp_jac_stride : 0};
+            if (g && sets) footprint_mean_grad_kernel<true><<<(unsigned)blocks, 32, 0, st>>>(fa, fg);
+            else if (g) footprint_mean_grad_kernel<false><<<(unsigned)blocks, 32, 0, st>>>(fa, fg);
+            else if (sets) footprint_mean_kernel<true><<<(unsigned)blocks, 32, 0, st>>>(fa);
             else footprint_mean_kernel<false><<<(unsigned)blocks, 32, 0, st>>>(fa);
             ctx->launches++;
             CU(cudaGetLastError());
@@ -1878,7 +2047,9 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
         ma.fp_val = ob.fp_val; ma.fp_sigma = ob.fp_sigma; ma.fp_kind_begin = ob.fp_kind_begin;
         ma.fp_chi2 = fp_chi2_dev; ma.fp_count = (long long *)fp_count_dev;
     }
-    if (sets) misfit_finish_kernel<true><<<M, 256, 0, st>>>(ma);
+    if (g && sets) misfit_finish_grad_kernel<true><<<M, 256, 0, st>>>(ma, mg);
+    else if (g) misfit_finish_grad_kernel<false><<<M, 256, 0, st>>>(ma, mg);
+    else if (sets) misfit_finish_kernel<true><<<M, 256, 0, st>>>(ma);
     else misfit_finish_kernel<false><<<M, 256, 0, st>>>(ma);
     ctx->launches++;
     CU(cudaGetLastError());
@@ -1953,6 +2124,17 @@ int nesosim_run_season_scores_fp(nesosim_ctx *ctx, const nesosim_member_params *
                                  int64_t fp_model_stride, void *stream) {
     return run_season_scores(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, NESOSIM_OBS_KINDS, model_dev,
                              model_stride, stream, true, fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride);
+}
+
+int nesosim_run_season_score_grads(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                                   int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
+                                   int64_t model_stride, double *grad_dev, double *jac_dev, int64_t jac_stride,
+                                   double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
+                                   int64_t fp_model_stride, double *fp_grad_dev, double *fp_jac_dev, int64_t fp_jac_stride,
+                                   void *stream) {
+    const GradOutputs g{grad_dev, jac_dev, jac_stride, fp_grad_dev, fp_jac_dev, fp_jac_stride};
+    return run_season_scores(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, NESOSIM_OBS_KINDS, model_dev,
+                             model_stride, stream, false, fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, &g);
 }
 
 int nesosim_set_async(nesosim_ctx *ctx, int on) {

@@ -376,6 +376,48 @@ class SnowBudgetEngine:
         self._keep = (ic_t, chi2, used, mod, fp_chi2, fp_used, fmod)
         return chi2, used, mod, fp_chi2, fp_used, fmod
 
+    def run_season_score_grads(self, params, ic, model=False, jac=False):
+        """``run_season_scores_fp`` with the exact derivatives of the scores with respect to windPackFactor,
+        leadLossFactor and atmLossFactor (``_lib.GRAD_PARAMS``) of every member (nesosim_run_season_score_grads; needs
+        observations registered after ``set_path('general')``).  Returns a dict of CUDA tensors: "chi2", "used",
+        "model" (or None) as ``run_season_scores`` and bit-identical to it; "grad" [M, OBS_KINDS, GRAD_DIRS] (d chi2 /
+        d theta per kind); with ``jac`` "jac" [M, GRAD_DIRS, row_len] (d model / d theta per observation, NaN where the
+        model value is not finite).  With footprints registered also "fp_chi2", "fp_used", "fp_model" (or None),
+        "fp_grad" and, with ``jac``, "fp_jac" [M, GRAD_DIRS, fp_row_len].  windPackThresh enters through a step
+        function only and has no derivative here."""
+        torch = _torch()
+        p = _lib.member_params_array(params)
+        assert len(p) == self.M
+        ic_t = None if ic is None else self._dev(ic)
+        per_member = 1 if (ic_t is not None and ic_t.dim() == 3 and self.M > 1) else 0
+        dev = "cuda:%d" % self.device
+        K, D = _lib.OBS_KINDS, _lib.GRAD_DIRS
+        n_row, n_fp = self.observation_row_length(), self.footprint_row_length()
+        f64 = dict(dtype=torch.float64, device=dev)
+        r = {"chi2": torch.empty(self.M, K, **f64), "used": torch.empty(self.M, K, dtype=torch.int64, device=dev),
+             "model": torch.empty(self.M, n_row, **f64) if model else None, "grad": torch.empty(self.M, K, D, **f64),
+             "jac": torch.empty(self.M, D, n_row, **f64) if jac else None}
+        if n_fp:
+            r.update({"fp_chi2": torch.empty(self.M, K, **f64), "fp_used": torch.empty(self.M, K, dtype=torch.int64, device=dev),
+                      "fp_model": torch.empty(self.M, n_fp, **f64) if model else None,
+                      "fp_grad": torch.empty(self.M, K, D, **f64),
+                      "fp_jac": torch.empty(self.M, D, n_fp, **f64) if jac else None})
+
+        def ptr(name):
+            t = r.get(name)
+            return None if t is None else t.data_ptr()
+
+        def width(name):
+            t = r.get(name)
+            return 0 if t is None else t.shape[-1]
+
+        _lib.check(self.lib.nesosim_run_season_score_grads(
+            self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member, ptr("chi2"), ptr("used"), ptr("model"),
+            width("model"), ptr("grad"), ptr("jac"), width("jac"), ptr("fp_chi2"), ptr("fp_used"), ptr("fp_model"),
+            width("fp_model"), ptr("fp_grad"), ptr("fp_jac"), width("fp_jac"), self._stream()))
+        self._keep = (ic_t, r)
+        return r
+
     def run_season_misfit(self, params, ic, obs=None):
         """The season with the calibration misfit reduced INSIDE the season-resident kernel (nesosim_run_season_misfit;
         after ``set_path('general')``: sampled by the general day kernel, on any grid) against the registered

@@ -20,6 +20,11 @@ batch of forcing sets, and the misfit of each pair is reduced against that seaso
 does the same with observation errors and three observed quantities (snow depth over ice, snow volume, bulk density):
 per kind the sum of ((model - observed)/sigma)^2, and optionally the model value at every observation.  A season's
 ``"footprints"`` (``region_footprints``) add observed means over many cells and/or days, scored in the same call.
+
+    res = run_calibration_scores(mask, seasons, params, dx, grad=True, jac=True)  # + grad [P, S, 3, 3], jac per season
+
+adds the exact derivatives of chi2 (and of every model value) with respect to windPackFactor, leadLossFactor and
+atmLossFactor, from the tangent-linear build of the scoring day kernel.
 """
 import numpy as np
 
@@ -354,6 +359,28 @@ def gather_footprint_scores(fp_chi2, fp_used, fp_model, P, S, n_fp, rank=0, worl
     return assemble_footprint_scores(fp_chi2.cpu().numpy(), fp_used.cpu().numpy(), fp_model.cpu().numpy(), P, S, n_fp)
 
 
+def assemble_gradients(grad, jac, P, S, n_obs, prefix=""):
+    """Gradients of all P*S members in member order -> {prefix + "grad": [P, S, OBS_KINDS, GRAD_DIRS], prefix + "jac":
+    per season s the array [P, GRAD_DIRS, n_obs[s]] (rows padded to the largest season: the padding is dropped), or
+    None}; prefix "fp_" for the footprints."""
+    from . import _lib
+    out = {prefix + "grad": np.asarray(grad).reshape(P, S, _lib.OBS_KINDS, _lib.GRAD_DIRS), prefix + "jac": None}
+    if jac is not None:
+        j = np.asarray(jac).reshape(P, S, _lib.GRAD_DIRS, -1)
+        out[prefix + "jac"] = [j[:, s, :, :n_obs[s]] for s in range(S)]
+    return out
+
+
+def gather_gradients(grad, jac, P, S, n_obs, rank=0, world=1, group=None, prefix=""):
+    """All-gather the ranks' per-member gradients (Jacobian rows padded to the largest season) and reassemble them
+    (``assemble_gradients``), identical on every rank."""
+    if world > 1:
+        grad = sharding.gather_member_results(grad, P * S, rank, world, group)
+        if jac is not None:
+            jac = sharding.gather_member_results(jac, P * S, rank, world, group)
+    return assemble_gradients(grad.cpu().numpy(), None if jac is None else jac.cpu().numpy(), P, S, n_obs, prefix)
+
+
 def season_footprints(mask, seasons):
     """Every season's footprints (``"footprints"`` entry; none: no footprints), normalized and checked against the grid
     and that season's own length, on every rank before any device work."""
@@ -458,7 +485,7 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
 
 
 def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, model=False,
-                           **flags):
+                           grad=False, jac=False, **flags):
     """``run_calibration`` with observation errors and three observed quantities.  A season's ``"obs"`` is a dict with
     day, row, col, value and optionally kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``, default depth) and
     sigma (default 1), or the 4-tuple (day, row, col, depth).  Returns {"chi2": [P, S, OBS_KINDS], "used": [P, S,
@@ -473,9 +500,22 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     many cells and/or days.  When some season has any, the result also holds "fp_chi2" / "fp_used" [P, S, OBS_KINDS]
     and "fp_model" (per season the array [P, n_fp] of footprint model values); the fused path scores them in the same
     call (nesosim_run_season_scores_fp), the HBM path with ``footprint_scores``.  Without footprints the result is
-    unchanged."""
+    unchanged.
+
+    ``grad=True`` adds "grad" [P, S, OBS_KINDS, GRAD_DIRS]: the exact derivative of every chi2 with respect to
+    windPackFactor, leadLossFactor and atmLossFactor (parameter columns ``_lib.GRAD_PARAMS``; windPackThresh enters
+    through a step function and has none), from the tangent-linear build of the scoring day kernel
+    (nesosim_run_season_score_grads).  It always scores on the general day-kernel path, whose chi2, used and model are
+    bit-identical to the season kernel's; ``fused`` must stay None (neither the HBM round trip nor the season kernel has
+    tangents: ValueError before any device work).  ``jac=True`` (with ``grad``) adds "jac": per season the array [P,
+    GRAD_DIRS, n_obs] of d model / d theta (NaN where the model value is not finite).  With footprints also "fp_grad"
+    and, with ``jac``, "fp_jac" (per season [P, GRAD_DIRS, n_fp])."""
     import torch
     from . import _lib
+    if grad and fused is not None:
+        raise ValueError("grad=True needs fused=None: only the general day-kernel path has tangents")
+    if jac and not grad:
+        raise ValueError("jac=True needs grad=True")
     params = np.asarray(params, dtype=np.float64).reshape(-1, 4)
     P, S = len(params), len(seasons)
     obs = season_observations(mask, seasons)
@@ -489,17 +529,26 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     dev = "cuda:%d" % device
     K = _lib.OBS_KINDS
 
-    def gather(chi2, used, mod, fp):
+    D = _lib.GRAD_DIRS
+
+    def gather(chi2, used, mod, fp, g=None):
         res = gather_scores(chi2, used, mod, P, S, n_obs, rank, world, group)
         if with_fp:
             res.update(gather_footprint_scores(*fp, P, S, n_fp, rank, world, group))
+        if grad:
+            res.update(gather_gradients(g[0], g[1], P, S, n_obs, rank, world, group))
+            if with_fp:
+                res.update(gather_gradients(g[2], g[3], P, S, n_fp, rank, world, group, prefix="fp_"))
         return res
 
     if not pairs:   # more ranks than members: nothing to run, but the gather still needs this rank
         chi2, used = torch.zeros(0, K, dtype=torch.float64, device=dev), torch.zeros(0, K, dtype=torch.int64, device=dev)
         mod = torch.zeros(0, width, dtype=torch.float64, device=dev) if model else None
         fp = (chi2, used, torch.zeros(0, fp_width, dtype=torch.float64, device=dev))
-        return gather(chi2, used, mod, fp)
+        g0 = torch.zeros(0, K, D, dtype=torch.float64, device=dev)
+        g = (g0, torch.zeros(0, D, width, dtype=torch.float64, device=dev) if jac else None,
+             g0, torch.zeros(0, D, fp_width, dtype=torch.float64, device=dev) if jac else None)
+        return gather(chi2, used, mod, fp, g)
     eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
     M = len(mine)
 
@@ -540,8 +589,39 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
             mod[:, :m.shape[1]] = m
         return chi2, used, mod, fp
 
+    def padded(t, n, rows):   # [M, ..., n_staged] -> [M, ..., n] with NaN past a row's end (or all NaN: no such rows)
+        out = torch.full(rows + (n,), float("nan"), dtype=torch.float64, device=dev)
+        if t is not None:
+            out[..., :t.shape[-1]] = t
+        return out
+
+    def grad_call():   # the general path's tangent build: registered after set_path("general")
+        eng.set_path("general")
+        cols = {k: np.concatenate([obs[s][k] for s in staged]) for k in obs[0]}
+        tag = np.concatenate([np.full(n_obs[s], i, dtype=np.int32) for i, s in enumerate(staged)])
+        if with_fp:
+            fcols, ftag = concat_footprints([fps[s] for s in staged])
+            eng.set_observations_fp(cols, fcols, obs_set=tag, fp_set=ftag)
+        else:
+            eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"], cols["sigma"],
+                                    obs_set=tag)
+        r = eng.run_season_score_grads(mine, ic, model=model or with_fp, jac=jac)
+        mod = padded(r["model"], width, (M,)) if model else None
+        fp, fg, fj = None, None, None
+        if with_fp:   # the staged seasons may have no footprint at all: zero sums, NaN rows
+            zk = lambda dt: torch.zeros(M, K, dtype=dt, device=dev)
+            fp = (r.get("fp_chi2", zk(torch.float64)), r.get("fp_used", zk(torch.int64)),
+                  padded(r.get("fp_model"), fp_width, (M,)))
+            fg = r.get("fp_grad", torch.zeros(M, K, D, dtype=torch.float64, device=dev))
+            fj = padded(r.get("fp_jac"), fp_width, (M, D)) if jac else None
+        g = (r["grad"], padded(r["jac"], width, (M, D)) if jac else None, fg, fj)
+        return r["chi2"], r["used"], mod, fp, g
+
+    g = None
     try:
-        if fused is False:
+        if grad:
+            chi2, used, mod, fp, g = grad_call()
+        elif fused is False:
             chi2, used, mod, fp = hbm_round_trip()
         else:
             try:
@@ -556,4 +636,6 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     back = torch.as_tensor(np.argsort(order), device=chi2.device)    # native member order -> this rank's pair order
     if with_fp:
         fp = tuple(t[back] for t in fp)
-    return gather(chi2[back], used[back], mod[back] if model else None, fp)
+    if grad:
+        g = tuple(None if t is None else t[back] for t in g)
+    return gather(chi2[back], used[back], mod[back] if model else None, fp, g)
