@@ -329,6 +329,32 @@ int nesosim_run_season_score_grads(nesosim_ctx *ctx, const nesosim_member_params
                                    int64_t fp_model_stride, double *fp_grad_dev, double *fp_jac_dev, int64_t fp_jac_stride,
                                    void *stream);
 
+/* Calibration adjoint (general path only): reverse-mode derivatives of the objective
+ *   J_m = sum_k weights_host[k] chi2[m][k] + sum_k fp_weights_host[k] fp_chi2[m][k]
+ * of every member m with respect to its initial snow-depth field and to the three parameters of
+ * nesosim_run_season_score_grads, by one backward sweep through the season (DESIGN.md §4.1): the same pathwise
+ * derivative as the tangent build, with every kink on the side the primal took.  Outputs besides those of
+ * nesosim_run_season_scores_fp, which are bit-identical to that call's:
+ *   theta_grad_dev [M][NESOSIM_GRAD_DIRS]: dJ_m / d(windPackFactor, leadLossFactor, atmLossFactor);
+ *   ic_grad_dev [M][ny][nx]: dJ_m / d ic, per member even when the IC is shared (sum over members for the total);
+ *     exactly 0 where conc[0] < minConc (the IC is zeroed there), and possibly non-zero on land, whose finite IC the
+ *     first day's dynamics read.
+ * The weights are host arrays [NESOSIM_OBS_KINDS] and must be finite and >= 0 (NESOSIM_ERR_ARG).  Needs observations
+ * registered under path 1 (else NESOSIM_ERR_STATE); with footprints registered fp_chi2_dev is required
+ * (NESOSIM_ERR_STATE).  NESOSIM_ERR_ARG also for a NULL theta_grad_dev or ic_grad_dev, a stride shorter than its row and
+ * more members or tile rows than a launch grid holds.  The adjoint state, allocated by the first call and freed with the
+ * observations, is 17 T + 56 bytes per member-cell (the depth trajectory, one record byte per day, a two-slot ring of
+ * the adjoint depths and the three parameter accumulators) plus 16 bytes per member and sample slot; when it does not
+ * fit the call frees what it allocated, returns NESOSIM_ERR_NOMEM and the context stays usable.  The first call also
+ * uploads the per-slot seed tables with synchronous copies (and cudaMalloc may synchronise the device); later calls
+ * issue 2T+4 kernel launches (2T+5 with footprints; one fewer on a grid without ocean, which has no sample slot), one
+ * memset (two with model_dev) and no stream synchronisation. */
+int nesosim_run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                                     int ic_per_member, const double *weights_host, const double *fp_weights_host,
+                                     double *chi2_dev, int64_t *count_dev, double *model_dev, int64_t model_stride,
+                                     double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
+                                     int64_t fp_model_stride, double *theta_grad_dev, double *ic_grad_dev, void *stream);
+
 /* ---- Row-strip domain decomposition over peer memory (grids too large for one GPU: the 5 km case; the reference
  * has no counterpart -- its grid is one numpy array -- so the contract is that of calcBudget on the whole grid).
  * A context created on rows [lo-2, hi+2) of the full grid (mask and forcing sliced the same way; 2 = radius of

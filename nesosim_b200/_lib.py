@@ -117,6 +117,10 @@ _SIGNATURES = {
                                                  C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
                                                  C.c_int64, C.c_void_p]),
+    "nesosim_run_season_score_adjoint": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int,
+                                                   C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

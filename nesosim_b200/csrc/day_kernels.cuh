@@ -131,11 +131,14 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 // `fin`, one bit per raw term of this thread (4 per raw cell it owns: adv0, adv1, div0, div1) telling whether the term
 // was finite; RAW_TANGENT runs the same linear stencils on a staged tangent tile and zeroes each term whose primal was
 // not finite (zero_if_nonfinite made the primal a constant there).  Same cell-to-thread assignment in every mode.
-enum RawMode { RAW_PRIMAL = 0, RAW_RECORD, RAW_TANGENT };
+// RAW_FLAGS (the adjoint's record build) is the primal pass that also writes, for every cell of the tile, the finite bits
+// of its four raw terms into s_fin (bits 2..5 of the cell's record byte: adv0, adv1, div0, div1).
+enum RawMode { RAW_PRIMAL = 0, RAW_RECORD, RAW_TANGENT, RAW_FLAGS };
 template <bool INTERIOR, int DAY_THREADS, int MODE = RAW_PRIMAL>
 __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, const int y0, double (&s_h)[2][TY + 4][TX + 4],
                                                double (&s_ut)[TY + 4][TX + 4], double (&s_vt)[TY + 4][TX + 4],
-                                               double (&s_raw)[4][TY + 2][TX + 2], unsigned *fin = nullptr) {
+                                               double (&s_raw)[4][TY + 2][TX + 2], unsigned *fin = nullptr,
+                                               uint8_t *s_fin = nullptr) {
     const int tid = threadIdx.x;
     const int ny = a.ny, nx = a.nx;
     const double dT = a.k.deltaT;
@@ -143,6 +146,7 @@ __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, c
         const int r = i / (TX + 2), c = i - r * (TX + 2);
         const int gy = y0 + r - 1, gx = x0 + c - 1;
         double adv0 = 0.0, adv1 = 0.0, div0 = 0.0, div1 = 0.0;   // zero padding of convolve(boundary='fill')
+        unsigned fbits = 0;
         if (INTERIOR || (gy >= 0 && gy < ny && gx >= 0 && gx < nx)) {
             const int sr = r + 1, sc = c + 1;
             const double ut = mul(s_ut[sr][sc], dT), vt = mul(s_vt[sr][sc], dT);   // driftGday*deltaT
@@ -168,10 +172,14 @@ __device__ __forceinline__ void tile_raw_phase(const DayArgs &a, const int x0, c
                     if (MODE == RAW_RECORD)
                         *fin |= ((unsigned)nesosim::finite(adv_term(ut, vt, gxh, gyh)) << (4 * k + l)) |
                                 ((unsigned)nesosim::finite(div_term(h, gxu, gyv)) << (4 * k + 2 + l));
+                    if (MODE == RAW_FLAGS)
+                        fbits |= ((unsigned)nesosim::finite(adv_term(ut, vt, gxh, gyh)) << (2 + l)) |
+                                 ((unsigned)nesosim::finite(div_term(h, gxu, gyv)) << (4 + l));
                 }
                 if (l == 0) { adv0 = ad; div0 = dv; } else { adv1 = ad; div1 = dv; }
             }
         }
+        if (MODE == RAW_FLAGS && r >= 1 && r <= TY && c >= 1 && c <= TX) s_fin[(r - 1) * TX + (c - 1)] = (uint8_t)fbits;
         s_raw[0][r][c] = adv0;
         s_raw[1][r][c] = adv1;
         s_raw[2][r][c] = div0;
@@ -186,9 +194,17 @@ struct GradCell {
     bool kill0, kill1;
 };
 
+// Record instantiation (REC, nesosim_run_season_score_adjoint): the scoring build writing the depths into a trajectory
+// [T][layer][M][plane] (the host points prev/next at slots x and x+1) and one record byte per member-cell-day
+// ([T-1][M][plane]): bit 0 kill0, bit 1 kill1 (fill_nan_no_negative replaced the new h0 / h1), bits 2..5 the finite bits
+// of the cell's raw terms adv0, adv1, div0, div1 (0 without dynamics) -- what the backward step cannot re-derive.
+struct RecArgs {
+    uint8_t *flags;            // day x's record bytes [M][plane] (member stride depth_mstride)
+};
+
 // 3x3 smoothing of the four raw planes, the point-wise budget terms and the twelve stores of this thread's cells
-// (SCORE: the two depth stores only; GRAD: also fills `gc`).
-template <bool INTERIOR, bool STRIP, int DAY_THREADS, bool SCORE = false, bool GRAD = false>
+// (SCORE: the two depth stores only; GRAD: also fills `gc`; REC: also writes the record byte from `s_fin`).
+template <bool INTERIOR, bool STRIP, int DAY_THREADS, bool SCORE = false, bool GRAD = false, bool REC = false>
 __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0, const int y0, const int m,
                                                  double (&s_h)[2][TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
                                                  const double *h0p, const double *h1p, const MemberCoef &mc,
@@ -197,7 +213,8 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
                                                  const double (&pf_W)[TY / (DAY_THREADS / TX)],
                                                  const double (&pf_prev)[TY / (DAY_THREADS / TX)][9],
                                                  const bool (&pf_land)[TY / (DAY_THREADS / TX)], const StripLink *sl,
-                                                 GradCell *gc = nullptr) {
+                                                 GradCell *gc = nullptr, const RecArgs *rec = nullptr,
+                                                 const uint8_t *s_fin = nullptr) {
     const int tid = threadIdx.x;
     const int ny = a.ny, nx = a.nx;
     const int tx = tid & (TX - 1);
@@ -260,6 +277,11 @@ __device__ __forceinline__ void tile_point_phase(const DayArgs &a, const int x0,
             gc[rr].h0 = h0;
             gc[rr].kill0 = !nesosim::finite(h0n) || land || h0n < 0.0;
             gc[rr].kill1 = !nesosim::finite(h1n) || land || h1n < 0.0;
+        }
+        if (REC) {
+            const unsigned k0 = !nesosim::finite(h0n) || land || h0n < 0.0, k1 = !nesosim::finite(h1n) || land || h1n < 0.0;
+            const unsigned fb = a.sw.dynamics ? s_fin[ty * TX + tx] : 0u;
+            rec->flags[id] = (uint8_t)(fb | k0 | (k1 << 1));
         }
         h0n = mask_nan(h0n, land, true);
         h1n = mask_nan(h1n, land, true);
@@ -358,11 +380,12 @@ __device__ __forceinline__ void tile_tangent_phase(const DayArgs &a, const int x
 // INTERIOR: the tile with its two-cell halo lies inside the grid and none of its raw-dynamics cells is a grid-edge
 // cell, so there are no bounds tests, every difference is centred and the divisor is a launch constant (the
 // overwhelming majority of the CTAs on the 25 km and 5 km grids).
-template <bool INTERIOR, bool STRIP = false, int DAY_THREADS = 256, bool SCORE = false, bool GRAD = false>
+template <bool INTERIOR, bool STRIP = false, int DAY_THREADS = 256, bool SCORE = false, bool GRAD = false, bool REC = false>
 __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2][TY + 4][TX + 4], double (&s_ut)[TY + 4][TX + 4],
                                               double (&s_vt)[TY + 4][TX + 4], double (&s_raw)[4][TY + 2][TX + 2],
                                               const int bx, const int by, const StripLink *sl = nullptr,
-                                              const SampleArgs *sa = nullptr, const TangentArgs *ta = nullptr) {
+                                              const SampleArgs *sa = nullptr, const TangentArgs *ta = nullptr,
+                                              const RecArgs *rec = nullptr, uint8_t *s_fin = nullptr) {
     const int m = blockIdx.z;
     const int x0 = bx * TX, y0 = by * TY;     // (bx, by): the tile (blockIdx, or what a strip / season CTA picked)
     const int tid = threadIdx.x;
@@ -467,12 +490,13 @@ __device__ __forceinline__ void day_step_body(const DayArgs &a, double (&s_h)[2]
         }
         cp_async_wait_all();
         __syncthreads();
-        tile_raw_phase<INTERIOR, DAY_THREADS, GRAD ? RAW_RECORD : RAW_PRIMAL>(a, x0, y0, s_h, s_ut, s_vt, s_raw, &fin);
+        tile_raw_phase<INTERIOR, DAY_THREADS, GRAD ? RAW_RECORD : (REC ? RAW_FLAGS : RAW_PRIMAL)>(a, x0, y0, s_h, s_ut, s_vt,
+                                                                                                  s_raw, &fin, s_fin);
         __syncthreads();
     }
 
-    tile_point_phase<INTERIOR, STRIP, DAY_THREADS, SCORE, GRAD>(a, x0, y0, m, s_h, s_raw, h0p, h1p, mc, pf_P, pf_C, pf_W,
-                                                                pf_prev, pf_land, sl, gc);
+    tile_point_phase<INTERIOR, STRIP, DAY_THREADS, SCORE, GRAD, REC>(a, x0, y0, m, s_h, s_raw, h0p, h1p, mc, pf_P, pf_C,
+                                                                     pf_W, pf_prev, pf_land, sl, gc, rec, s_fin);
     if (GRAD) {
         // The three tangent passes reuse the tile's shared buffers: the tangent tile of direction j replaces the depth tile,
         // its raw terms the raw terms (the drift tiles stay), so the gradient build needs no more shared memory.
@@ -560,10 +584,10 @@ __device__ __forceinline__ void day_step_land_tile(const DayArgs &a, const int b
 }
 
 // The land tile of the scoring build: only its NaN depths are stored (a land tile has no observed cell to sample);
-// GRAD: and zero tangents.
-template <int DAY_THREADS, bool GRAD = false>
+// GRAD: and zero tangents; REC: and the record byte of a land cell (both kills, no finite raw term).
+template <int DAY_THREADS, bool GRAD = false, bool REC = false>
 __device__ __forceinline__ void day_step_land_depths(const DayArgs &a, const int bx, const int by,
-                                                     const TangentArgs *ta = nullptr) {
+                                                     const TangentArgs *ta = nullptr, const RecArgs *rec = nullptr) {
     const int m = blockIdx.z;
     const int fset = a.member_set ? a.member_set[m] : 0;
     if (a.set_steps && a.x >= a.set_steps[fset]) {
@@ -580,6 +604,7 @@ __device__ __forceinline__ void day_step_land_depths(const DayArgs &a, const int
         const long long id = (long long)m * a.depth_mstride + (long long)gy * a.nx + gx;
         a.next[V_H0][id] = qnan();
         a.next[V_H1][id] = qnan();
+        if (REC) rec->flags[id] = 3;
         if (GRAD) {
 #pragma unroll
             for (int j = 0; j < GRAD_DIRS; ++j) {
@@ -597,12 +622,13 @@ struct TileSmem {
     double raw[4][TY + 2][TX + 2];   // adv0, adv1, div0, div1 after the NaN->0 fill
 };
 
-template <int DAY_THREADS, bool SCORE = false, bool GRAD = false>
+template <int DAY_THREADS, bool SCORE = false, bool GRAD = false, bool REC = false>
 __device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, const int bx, const int by,
-                                              const SampleArgs *sa = nullptr, const TangentArgs *ta = nullptr) {
+                                              const SampleArgs *sa = nullptr, const TangentArgs *ta = nullptr,
+                                              const RecArgs *rec = nullptr, uint8_t *s_fin = nullptr) {
     pdl_launch_dependents();
     if (a.tile_land && a.tile_land[by * ((a.nx + TX - 1) / TX) + bx]) {
-        if (SCORE) day_step_land_depths<DAY_THREADS, GRAD>(a, bx, by, ta);
+        if (SCORE) day_step_land_depths<DAY_THREADS, GRAD, REC>(a, bx, by, ta, rec);
         else day_step_land_tile<DAY_THREADS>(a, bx, by);
         return;
     }
@@ -612,8 +638,8 @@ __device__ __forceinline__ void day_step_tile(const DayArgs &a, TileSmem &sm, co
     auto &s_raw = sm.raw;
     const int x0 = bx * TX, y0 = by * TY;
     const bool interior = x0 >= 2 && y0 >= 2 && x0 + TX + 2 <= a.nx && y0 + TY + 2 <= a.ny;
-    if (interior) day_step_body<true, false, DAY_THREADS, SCORE, GRAD>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa, ta);
-    else day_step_body<false, false, DAY_THREADS, SCORE, GRAD>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa, ta);
+    if (interior) day_step_body<true, false, DAY_THREADS, SCORE, GRAD, REC>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa, ta, rec, s_fin);
+    else day_step_body<false, false, DAY_THREADS, SCORE, GRAD, REC>(a, s_h, s_ut, s_vt, s_raw, bx, by, nullptr, sa, ta, rec, s_fin);
 }
 
 // Two builds of the same tile code: 256 threads x 2 cells (large grids: fewer, fatter threads) and 512 threads x 1
@@ -653,15 +679,32 @@ __global__ void __launch_bounds__(512, 2) day_step_grad_kernel_512(const __grid_
     day_step_tile<512, true, true>(a, sm, blockIdx.x, blockIdx.y, &s, &t);
 }
 
+// The record builds of the same two shapes (RecArgs above).
+__global__ void __launch_bounds__(256) day_step_record_kernel(const __grid_constant__ DayArgs a,
+                                                              const __grid_constant__ SampleArgs s,
+                                                              const __grid_constant__ RecArgs r) {
+    __shared__ TileSmem sm;
+    __shared__ uint8_t s_fin[TY * TX];
+    day_step_tile<256, true, false, true>(a, sm, blockIdx.x, blockIdx.y, &s, nullptr, &r, s_fin);
+}
+__global__ void __launch_bounds__(512, 2) day_step_record_kernel_512(const __grid_constant__ DayArgs a,
+                                                                     const __grid_constant__ SampleArgs s,
+                                                                     const __grid_constant__ RecArgs r) {
+    __shared__ TileSmem sm;
+    __shared__ uint8_t s_fin[TY * TX];
+    day_step_tile<512, true, false, true>(a, sm, blockIdx.x, blockIdx.y, &s, nullptr, &r, s_fin);
+}
+
 // The last day of every member's season (set_steps[set], or T-1), which no day kernel reads: one CTA per member copies
 // its set's entries of that day from the member's ring slot.  A member whose season ended early has not touched its
-// ring since (its CTAs leave the later day kernels at once).  GRAD: the tangent samples of that day too.
-template <bool GRAD>
+// ring since (its CTAs leave the later day kernels at once).  GRAD: the tangent samples of that day too.  TRAJ: `ring`
+// is the record build's trajectory [T][layer][M][plane].
+template <bool GRAD, bool TRAJ = false>
 __device__ __forceinline__ void sample_last_day(const SampleArgs &s, const TangentArgs *t) {
     const int m = blockIdx.x;
     const int set = s.member_set ? s.member_set[m] : 0;
     const int day = s.set_steps ? s.set_steps[set] : s.T - 1;
-    const double *h0 = s.ring + (long long)(day & 1) * 2 * s.layer_stride + (long long)m * s.plane;
+    const double *h0 = s.ring + (long long)(TRAJ ? day : (day & 1)) * 2 * s.layer_stride + (long long)m * s.plane;
     const double *h1 = h0 + s.layer_stride;
     const long long b = ((long long)set * s.T + day) * s.tiles;
     double2 *row = s.samples + (long long)m * s.stride;
@@ -685,6 +728,250 @@ __global__ void __launch_bounds__(256) sample_last_day_kernel(const __grid_const
 __global__ void __launch_bounds__(256) sample_last_day_grad_kernel(const __grid_constant__ SampleArgs s,
                                                                    const __grid_constant__ TangentArgs t) {
     sample_last_day<true>(s, &t);
+}
+__global__ void __launch_bounds__(256) sample_last_day_traj_kernel(const __grid_constant__ SampleArgs s) {
+    sample_last_day<false, true>(s, nullptr);
+}
+
+
+// Backward day step of the calibration adjoint (nesosim_run_season_score_adjoint, DESIGN.md §4.1): lambda(x) from
+// lambda(x+1), day x's record bytes, h0(x) and the day's forcing, as the transpose of the tangent step
+// (tile_tangent_phase), then the day's seeds at its sample slots; and each cell's parameter terms mu * term(h0, param = 1)
+// into the per-member-cell accumulators.  Order (restated by oracle/score_adjoint.py):
+//   mu = kill ? 0 : lambda(x+1);  staged m = mu / divisor on the tile grown by 2 (0 outside the grid);
+//   per raw cell r of the tile grown by 1 and layer l, where adv_l(r) was finite: nu = transposed 3x3 sum of m around r,
+//   px = (nu * ut) / d_x, py = (nu * vt) / d_y (d = dx on that axis's grid edge, else 2 dx), else 0;
+//   per own cell c: lam0 = ((((mu0 + wpl(mu0)) + lead(mu0)) + atm(mu0)) + wpg(mu1)) + dyn0 (terms of a killed layer
+//   skipped), lam1 = mu1 + dyn1, dyn = dd - ((px[c-1] - px[c+1] + Ex) + (py[c-1] - py[c+1] + Ey)), E = (last ? p[c] : 0)
+//   - (first ? p[c] : 0), dd = -((nud gxu) + (nud gyv)) where div_l(c) was finite.
+// Every gate is a select: a killed cell's coefficients may be NaN.
+struct AdjArgs {
+    const double *lam_in;      // lambda(x+1): layer 0 of member 0 (layer_stride further: layer 1)
+    double *lam_out;           // lambda(x)
+    long long layer_stride;
+    const double *h0;          // trajectory slot x, layer 0 (member stride depth_mstride)
+    const uint8_t *flags;      // day x's record bytes [M][plane]
+    double *theta;             // [M][GRAD_DIRS][plane] accumulators
+    const double2 *seeds;      // [M][stride] dJ/d(h0, h1) at every sample slot
+    const int *begin;          // sampling CSR of SampleArgs
+    const int2 *entry;
+    long long stride;
+    int T, tiles;
+};
+
+// transposed 3x3 sum of the staged plane around (sr, sc)
+__device__ __forceinline__ double conv3x3_t(const DayArgs &a, const double (&p)[TY + 4][TX + 4], int sr, int sc) {
+    double acc = 0.0;
+#pragma unroll
+    for (int ii = 0; ii < 3; ++ii)
+#pragma unroll
+        for (int jj = 0; jj < 3; ++jj) acc = add(acc, mul(p[sr + 1 - ii][sc + 1 - jj], a.w[(2 - ii) * 3 + (2 - jj)]));
+    return acc;
+}
+
+template <int DAY_THREADS>
+__device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs &j, TileSmem &sm,
+                                                 uint8_t (&s_flag)[TY + 4][TX + 4]) {
+    pdl_launch_dependents();
+    const int m = blockIdx.z, bx = blockIdx.x, by = blockIdx.y;
+    const int fset = a.member_set ? a.member_set[m] : 0;
+    if (a.set_steps && a.x >= a.set_steps[fset]) {
+        pdl_wait();
+        return;
+    }
+    const int tid = threadIdx.x, ny = a.ny, nx = a.nx;
+    const int x0 = bx * TX, y0 = by * TY;
+    const int tx = tid & (TX - 1), gx = x0 + tx;
+    constexpr int CPT = TY / (DAY_THREADS / TX);
+    const long long ms = (long long)m * a.depth_mstride;
+    const double *l0p = j.lam_in + ms, *l1p = j.lam_in + j.layer_stride + ms;
+    double *o0p = j.lam_out + ms, *o1p = j.lam_out + j.layer_stride + ms;
+    if (a.tile_land && a.tile_land[by * ((nx + TX - 1) / TX) + bx]) {
+        // x > 0: every raw term that reads a land depth is NaN, so lambda is 0 on the whole tile and no term is added
+        pdl_wait();
+        if (gx >= nx) return;
+#pragma unroll
+        for (int rr = 0; rr < CPT; ++rr) {
+            const int gy = y0 + (tid / TX) + rr * (DAY_THREADS / TX);
+            if (gy >= ny) break;
+            const long long o = (long long)gy * nx + gx;
+            o0p[o] = 0.0;
+            o1p[o] = 0.0;
+        }
+        return;
+    }
+    const long long fo = (long long)fset * a.set_stride;
+    const double *aC = a.C + fo, *aW = a.W + fo, *aU = a.U + 2 * fo, *aV = a.V + 2 * fo;
+    const uint8_t *fl = j.flags + ms;
+    auto &s_m = sm.h;
+    auto &s_ut = sm.ut;
+    auto &s_vt = sm.vt;
+    auto &s_p = sm.raw;       // px0, py0, px1, py1
+    // day-x inputs (written before the backward sweep began): record bytes, drift tile, own cells' forcing and h0
+    for (int i = tid; i < (TY + 4) * (TX + 4); i += DAY_THREADS) {
+        const int r = i / (TX + 4), c = i - r * (TX + 4);
+        const int gy = y0 + r - 2, gxx = x0 + c - 2;
+        const bool in = gy >= 0 && gy < ny && gxx >= 0 && gxx < nx;
+        const long long o = in ? (long long)gy * nx + gxx : 0;
+        s_flag[r][c] = in ? fl[o] : (uint8_t)0;
+        if (a.sw.dynamics) {
+            cp_async8(&s_ut[r][c], aU + o, in);
+            cp_async8(&s_vt[r][c], aV + o, in);
+        }
+    }
+    double pf_C[CPT], pf_W[CPT], pf_h0[CPT];
+#pragma unroll
+    for (int rr = 0; rr < CPT; ++rr) {
+        const int gy = y0 + (tid / TX) + rr * (DAY_THREADS / TX);
+        pf_C[rr] = pf_W[rr] = pf_h0[rr] = 0.0;
+        if (gx < nx && gy < ny) {
+            const long long o = (long long)gy * nx + gx;
+            pf_C[rr] = __ldg(aC + o);
+            pf_W[rr] = __ldg(aW + o);
+            pf_h0[rr] = j.h0[ms + o];
+        }
+    }
+    const MemberCoef mc = a.coef[m];
+    __syncthreads();      // s_flag is read by other threads than the one that loaded it
+
+    pdl_wait();      // ---- lambda(x+1) and the accumulators may be read from here on
+
+    const double dT = a.k.deltaT;
+    if (a.sw.dynamics) {
+        for (int i = tid; i < (TY + 4) * (TX + 4); i += DAY_THREADS) {
+            const int r = i / (TX + 4), c = i - r * (TX + 4);
+            const int gy = y0 + r - 2, gxx = x0 + c - 2;
+            double m0 = 0.0, m1 = 0.0;
+            if (gy >= 0 && gy < ny && gxx >= 0 && gxx < nx) {
+                const long long o = (long long)gy * nx + gxx;
+                const unsigned f = s_flag[r][c];
+                m0 = (f & 1u) ? 0.0 : div_const(l0p[o], a.conv_div);
+                m1 = (f & 2u) ? 0.0 : div_const(l1p[o], a.conv_div);
+            }
+            s_m[0][r][c] = m0;
+            s_m[1][r][c] = m1;
+        }
+        cp_async_wait_all();
+        __syncthreads();
+        for (int i = tid; i < (TY + 2) * (TX + 2); i += DAY_THREADS) {
+            const int r = i / (TX + 2), c = i - r * (TX + 2);
+            const int gy = y0 + r - 1, gxx = x0 + c - 1;
+            double p[4] = {0.0, 0.0, 0.0, 0.0};
+            if (gy >= 0 && gy < ny && gxx >= 0 && gxx < nx) {
+                const int sr = r + 1, sc = c + 1;
+                const unsigned f = s_flag[sr][sc];
+                const double ut = mul(s_ut[sr][sc], dT), vt = mul(s_vt[sr][sc], dT);
+                const bool ex = gxx == 0 || gxx == nx - 1, ey = gy == 0 || gy == ny - 1;
+                ConstDiv dxd, dyd;
+                dxd.c = ex ? a.g.dx.c : a.g.two_dx.c;
+                dxd.rc = ex ? a.g.dx.rc : a.g.two_dx.rc;
+                dyd.c = ey ? a.g.dx.c : a.g.two_dx.c;
+                dyd.rc = ey ? a.g.dx.rc : a.g.two_dx.rc;
+                dxd.fast = dyd.fast = a.g.dx.fast & a.g.two_dx.fast;
+#pragma unroll
+                for (int l = 0; l < 2; ++l) {
+                    if ((f >> (2 + l)) & 1u) {
+                        const double nu = conv3x3_t(a, s_m[l], sr, sc);
+                        p[2 * l] = div_const(mul(nu, ut), dxd);
+                        p[2 * l + 1] = div_const(mul(nu, vt), dyd);
+                    }
+                }
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) s_p[q][r][c] = p[q];
+        }
+        __syncthreads();
+    }
+
+    if (gx < nx) {
+        MemberCoef one = mc;
+        one.neg_wpf_dt = -dT;
+        one.wpf_dt = dT;
+        one.llf = 1.0;
+        one.alf = 1.0;
+#pragma unroll
+        for (int rr = 0; rr < CPT; ++rr) {
+            const int ty = (tid / TX) + rr * (DAY_THREADS / TX);
+            const int gy = y0 + ty;
+            if (gy >= ny) break;
+            const long long o = (long long)gy * nx + gx;
+            const unsigned f = s_flag[ty + 2][tx + 2];
+            const bool k0 = f & 1u, k1 = (f >> 1) & 1u;
+            const double mu0 = k0 ? 0.0 : l0p[o], mu1 = k1 ? 0.0 : l1p[o];
+            const double W = pf_W[rr], C = pf_C[rr], h0 = pf_h0[rr];
+            const double wt = wind_flag(W, mc.wpt);
+            double a0 = mu0, wl, wg, wn;
+            if (!k0) {
+                if (a.sw.windpack) { wind_packing(wt, mu0, mc, a.k, wl, wg, wn); a0 = add(a0, wl); }
+                if (a.sw.leadloss) a0 = add(a0, lead_loss(wt, mu0, W, C, mc, a.k));
+                if (a.sw.atmloss) a0 = add(a0, atm_loss(wt, mu0, W, mc, a.k));
+            }
+            if (!k1 && a.sw.windpack) { wind_packing(wt, mu1, mc, a.k, wl, wg, wn); a0 = add(a0, wg); }
+            double lam0 = a0, lam1 = mu1;
+            if (a.sw.dynamics) {
+                const int sr = ty + 2, sc = tx + 2, pr = ty + 1, pc = tx + 1;
+                const double gxu = gradient1d(mul(s_ut[sr][sc - 1], dT), mul(s_ut[sr][sc], dT), mul(s_ut[sr][sc + 1], dT), gx, nx, a.g);
+                const double gyv = gradient1d(mul(s_vt[sr - 1][sc], dT), mul(s_vt[sr][sc], dT), mul(s_vt[sr + 1][sc], dT), gy, ny, a.g);
+                const bool fx = gx == 0, lx = gx == nx - 1, fy = gy == 0, ly = gy == ny - 1;
+                double dyn[2];
+#pragma unroll
+                for (int l = 0; l < 2; ++l) {
+                    double dd = 0.0;
+                    if ((f >> (4 + l)) & 1u) dd = div_term(conv3x3_t(a, s_m[l], sr, sc), gxu, gyv);
+                    const double (&px)[TY + 2][TX + 2] = s_p[2 * l];
+                    const double (&py)[TY + 2][TX + 2] = s_p[2 * l + 1];
+                    const double ex = sub(lx ? px[pr][pc] : 0.0, fx ? px[pr][pc] : 0.0);
+                    const double ey = sub(ly ? py[pr][pc] : 0.0, fy ? py[pr][pc] : 0.0);
+                    const double sx = add(sub(px[pr][pc - 1], px[pr][pc + 1]), ex);
+                    const double sy = add(sub(py[pr - 1][pc], py[pr + 1][pc]), ey);
+                    dyn[l] = sub(dd, add(sx, sy));
+                }
+                lam0 = add(lam0, dyn[0]);
+                lam1 = add(lam1, dyn[1]);
+            }
+            o0p[o] = lam0;
+            o1p[o] = lam1;
+            // parameter terms (windPackFactor: both layers' terms first), in day order per cell
+            double s0 = 0.0, s1 = 0.0;
+            if (a.sw.windpack) {
+                wind_packing(wt, h0, one, a.k, wl, wg, wn);
+                s0 = k0 ? 0.0 : mul(mu0, wl);
+                s1 = k1 ? 0.0 : mul(mu1, wg);
+            }
+            const double th[GRAD_DIRS] = {
+                add(s0, s1),
+                (a.sw.leadloss && !k0) ? mul(mu0, lead_loss(wt, h0, W, C, one, a.k)) : 0.0,
+                (a.sw.atmloss && !k0) ? mul(mu0, atm_loss(wt, h0, W, one, a.k)) : 0.0};
+#pragma unroll
+            for (int d = 0; d < GRAD_DIRS; ++d) {
+                double *t = j.theta + ((long long)m * GRAD_DIRS + d) * a.depth_mstride + o;
+                *t = add(*t, th[d]);
+            }
+        }
+    }
+    __syncthreads();       // the tile's lambda(x) is stored: add the day's seeds at its sample slots
+    const int *b = j.begin + ((long long)fset * j.T + a.x) * j.tiles + (long long)by * gridDim.x + bx;
+    const double2 *sd = j.seeds + (long long)m * j.stride;
+    for (int i = b[0] + tid; i < b[1]; i += DAY_THREADS) {
+        const int2 e = j.entry[i];
+        const double2 v = sd[e.y];
+        o0p[e.x] = add(o0p[e.x], v.x);
+        o1p[e.x] = add(o1p[e.x], v.y);
+    }
+}
+
+// The two CTA shapes of the general path.
+__global__ void __launch_bounds__(256) day_step_adjoint_kernel(const __grid_constant__ DayArgs a,
+                                                               const __grid_constant__ AdjArgs j) {
+    __shared__ TileSmem sm;
+    __shared__ uint8_t s_flag[TY + 4][TX + 4];
+    day_step_adjoint<256>(a, j, sm, s_flag);
+}
+__global__ void __launch_bounds__(512, 2) day_step_adjoint_kernel_512(const __grid_constant__ DayArgs a,
+                                                                      const __grid_constant__ AdjArgs j) {
+    __shared__ TileSmem sm;
+    __shared__ uint8_t s_flag[TY + 4][TX + 4];
+    day_step_adjoint<512>(a, j, sm, s_flag);
 }
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {

@@ -234,6 +234,18 @@ struct nesosim_ctx {
         double *tring = nullptr;
         double2 *tsamples = nullptr;
         double *fp_dmean = nullptr;
+        // nesosim_run_season_score_adjoint: the seed contributions of every sample slot, slot-major ([sets][stride] + 1
+        // run starts; item (q, p): point observation q of kind -1-p when p < 0, else point p of footprint q), built at
+        // registration and uploaded by the first adjoint call, which also allocates the adjoint state: the trajectory
+        // [T][layer][M][plane], the record bytes [T-1][M][plane], the lambda ring [parity][layer][M][plane], the theta
+        // accumulators [M][GRAD_DIRS][plane], the seeds [M][stride] and the footprint coefficients [M][fp_row_len]
+        std::vector<int> adj_begin_h;
+        std::vector<int2> adj_item_h;
+        int *adj_begin = nullptr;
+        int2 *adj_item = nullptr;
+        double *traj = nullptr, *lam = nullptr, *theta_acc = nullptr, *fp_coef = nullptr;
+        uint8_t *rec_flags = nullptr;
+        double2 *seeds = nullptr;
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -386,6 +398,8 @@ void obs_release(nesosim_ctx *ctx) {
     cudaFree(ob.fp_mean);
     cudaFree(ob.smp_begin); cudaFree(ob.smp_entry); cudaFree(ob.ring);
     cudaFree(ob.tring); cudaFree(ob.tsamples); cudaFree(ob.fp_dmean);
+    cudaFree(ob.adj_begin); cudaFree(ob.adj_item); cudaFree(ob.traj); cudaFree(ob.lam); cudaFree(ob.theta_acc);
+    cudaFree(ob.fp_coef); cudaFree(ob.rec_flags); cudaFree(ob.seeds);
     ob = {};
 }
 
@@ -1431,8 +1445,15 @@ struct FootprintGrad {
     double *jac;                    // [M][GRAD_DIRS][jac_stride] at the input index within the set, or NULL
     long long jac_stride;
 };
-template <bool SETS, bool GRAD>
-__device__ __forceinline__ void footprint_mean(const FootprintArgs &a, const FootprintGrad *fg) {
+// ADJ (footprint_mean_adj_kernel, nesosim_run_season_score_adjoint): lane 0 also writes the footprint's seed
+// coefficient b = (((2 r) fw[kind]) / sigma) / s, NaN where r is not finite (the footprint is not counted).
+struct FootprintAdj {
+    double *coef;                   // [M][mean_stride] in table order within the set
+    const double *val, *sigma;      // the footprint table's values and errors
+    double fw[NESOSIM_OBS_KINDS];
+};
+template <bool SETS, bool GRAD, bool ADJ = false>
+__device__ __forceinline__ void footprint_mean(const FootprintArgs &a, const FootprintGrad *fg, const FootprintAdj *fa = nullptr) {
     const int m = (int)(blockIdx.x % (unsigned)a.n_members);
     const long long g = blockIdx.x / (unsigned)a.n_members;
     const int lane = threadIdx.x;
@@ -1499,6 +1520,11 @@ __device__ __forceinline__ void footprint_mean(const FootprintArgs &a, const Foo
         const double v = div_ieee(sw, s);
         a.mean[(long long)m * a.mean_stride + g] = v;
         if (model) model[a.src[q]] = v;
+        if (ADJ) {
+            const double r = div_ieee(sub(v, fa->val[q]), fa->sigma[q]);
+            fa->coef[(long long)m * a.mean_stride + g] =
+                nesosim::finite(r) ? div_ieee(div_ieee(mul(mul(2.0, r), fa->fw[kind]), fa->sigma[q]), s) : nesosim::qnan();
+        }
         if (GRAD) {
             for (int j = 0; j < GRAD_DIRS; ++j) {
                 const double dm = nesosim::finite(v) ? div_ieee(sdw[j], s) : nesosim::qnan();
@@ -1516,6 +1542,153 @@ template <bool SETS>
 __global__ void __launch_bounds__(32) footprint_mean_grad_kernel(const __grid_constant__ FootprintArgs a,
                                                                  const __grid_constant__ FootprintGrad fg) {
     footprint_mean<SETS, true>(a, &fg);
+}
+template <bool SETS>
+__global__ void __launch_bounds__(32) footprint_mean_adj_kernel(const __grid_constant__ FootprintArgs a,
+                                                                const __grid_constant__ FootprintAdj fa) {
+    footprint_mean<SETS, false, true>(a, nullptr, &fa);
+}
+
+// Seeds of the adjoint: one thread per (member, sample slot) sums dJ/d(h0, h1) from 0.0 over the slot's items in table
+// order -- the point observations chi2 counts, in chi2's order, then the kept footprint points with finite v, in
+// footprint input order -- each adding a * dv/d(h0, h1): a = ((2 r) w[kind]) / sigma for a point, b * w_p for a
+// footprint point; depth (a/C, a/C), volume (a, a), density ((a (rhoF - q)) / den, (a (rhoO - q)) / den), 0 at a clamp.
+struct SeedArgs {
+    const double2 *samples;
+    double2 *seeds;                 // [M][stride]
+    long long stride;
+    const int *begin;               // [sets][stride] + 1
+    const int2 *item;
+    const int *obs_day, *obs_cell;
+    const double *obs_val, *sigma;
+    const double *fp_coef;          // [M][fp_stride]
+    long long fp_stride;
+    const int *fp_kind, *fp_kind_begin, *pt_day, *pt_cell;
+    const double *pt_w;
+    const double *conc;             // [sets][T][plane]
+    long long plane, conc_set_stride;
+    const int *member_set;
+    ModelConsts k;
+    double w[NESOSIM_OBS_KINDS];
+};
+__device__ __forceinline__ void seed_partials(int kind, double2 h, double C, double a, const ModelConsts &k, double &g0,
+                                              double &g1) {
+    if (kind == NESOSIM_OBS_DEPTH) {
+        g0 = g1 = div_ieee(a, C);
+    } else if (kind == NESOSIM_OBS_VOLUME) {
+        g0 = g1 = a;
+    } else {
+        const double den = add(h.x, h.y);
+        const double q = div_ieee(add(mul(h.x, k.rhoFresh), mul(h.y, k.rhoOld)), den);
+        if (q > k.rhoOld || q < k.rhoFresh) {
+            g0 = g1 = 0.0;
+        } else {
+            g0 = div_ieee(mul(a, sub(k.rhoFresh, q)), den);
+            g1 = div_ieee(mul(a, sub(k.rhoOld, q)), den);
+        }
+    }
+}
+__global__ void __launch_bounds__(256) adjoint_seed_kernel(const __grid_constant__ SeedArgs a) {
+    const long long sl = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int m = blockIdx.y;
+    if (sl >= a.stride) return;
+    const int set = a.member_set ? a.member_set[m] : 0;
+    const double *conc = a.conc + (long long)set * a.conc_set_stride;
+    const double2 h = a.samples[(long long)m * a.stride + sl];
+    const long long b = (long long)set * a.stride + sl;
+    double s0 = 0.0, s1 = 0.0;
+    for (int i = a.begin[b]; i < a.begin[b + 1]; ++i) {
+        const int2 it = a.item[i];
+        int kind;
+        double av, C = 1.0;
+        if (it.y < 0) {
+            const int q = it.x;
+            kind = -1 - it.y;
+            double v;
+            if (kind == NESOSIM_OBS_DEPTH) {
+                C = __ldg(conc + (long long)a.obs_day[q] * a.plane + a.obs_cell[q]);
+                v = div_ieee(add(h.x, h.y), C);
+            } else if (kind == NESOSIM_OBS_VOLUME) v = add(h.x, h.y);
+            else v = density_variable(h.x, h.y, false, a.k);
+            const double r = div_ieee(sub(v, a.obs_val[q]), a.sigma[q]);
+            if (!nesosim::finite(r)) continue;
+            av = div_ieee(mul(mul(2.0, r), a.w[kind]), a.sigma[q]);
+        } else {
+            const int q = it.x, p = it.y;
+            kind = a.fp_kind[q];
+            const double bc = a.fp_coef[(long long)m * a.fp_stride + q - a.fp_kind_begin[set * (NESOSIM_OBS_KINDS + 1)]];
+            if (!nesosim::finite(bc)) continue;
+            double v;
+            if (kind == NESOSIM_OBS_DEPTH) {
+                C = __ldg(conc + (long long)a.pt_day[p] * a.plane + a.pt_cell[p]);
+                v = div_ieee(add(h.x, h.y), C);
+            } else if (kind == NESOSIM_OBS_VOLUME) v = add(h.x, h.y);
+            else v = density_variable(h.x, h.y, false, a.k);
+            if (!nesosim::finite(v)) continue;
+            av = mul(bc, a.pt_w[p]);
+        }
+        double g0, g1;
+        seed_partials(kind, h, C, av, a.k, g0, g1);
+        s0 = add(s0, g0);
+        s1 = add(s1, g1);
+    }
+    a.seeds[(long long)m * a.stride + sl] = make_double2(s0, s1);
+}
+
+// lambda at each member's last slot L (set_steps, or T-1): 0, plus the seeds of day L at its sample slots.
+struct AdjInitArgs {
+    double *lam;                    // ring [parity][layer][M][plane]
+    long long plane, layer_stride;
+    const double2 *seeds;
+    long long stride;
+    const int *begin;
+    const int2 *entry;
+    int T, tiles;
+    const int *member_set, *set_steps;
+};
+__global__ void __launch_bounds__(256) adjoint_init_kernel(const __grid_constant__ AdjInitArgs a) {
+    const int m = blockIdx.x;
+    const int set = a.member_set ? a.member_set[m] : 0;
+    const int L = a.set_steps ? a.set_steps[set] : a.T - 1;
+    double *l0 = a.lam + (long long)(L & 1) * 2 * a.layer_stride + (long long)m * a.plane, *l1 = l0 + a.layer_stride;
+    for (long long i = threadIdx.x; i < a.plane; i += blockDim.x) l0[i] = l1[i] = 0.0;
+    __syncthreads();
+    const long long b = ((long long)set * a.T + L) * a.tiles;
+    const double2 *sd = a.seeds + (long long)m * a.stride;
+    for (int i = a.begin[b] + threadIdx.x; i < a.begin[b + a.tiles]; i += blockDim.x) {
+        const int2 e = a.entry[i];
+        l0[e.x] = add(l0[e.x], sd[e.y].x);
+        l1[e.x] = add(l1[e.x], sd[e.y].y);
+    }
+}
+
+// One CTA per member: theta_grad[m][j] = the fixed-order sum of the accumulators over the cells (cell i to thread
+// i % 256, block_total), and ic_grad = (lambda0(0) + lambda1(0)) * 0.5, 0 where conc[0] < minConc.
+struct AdjFinishArgs {
+    const double *theta_acc;        // [M][GRAD_DIRS][plane]
+    const double *lam0;             // ring slot 0, layer 0 (layer_stride further: layer 1)
+    long long plane, layer_stride;
+    const double *conc0;            // first day's concentration of set 0 (set_stride further: the next set)
+    long long set_stride;
+    const int *member_set;
+    double minConc;
+    double *theta_grad;             // [M][GRAD_DIRS]
+    double *ic_grad;                // [M][plane]
+};
+__global__ void __launch_bounds__(256) adjoint_finish_kernel(const __grid_constant__ AdjFinishArgs a) {
+    const int m = blockIdx.x;
+    __shared__ double red[8];
+    __shared__ long long redc[8];
+    for (int j = 0; j < GRAD_DIRS; ++j) {
+        const double *t = a.theta_acc + ((long long)m * GRAD_DIRS + j) * a.plane;
+        double acc = 0.0;
+        for (long long i = threadIdx.x; i < a.plane; i += 256) acc = add(acc, t[i]);
+        block_total(acc, 0, red, redc, a.theta_grad + (long long)m * GRAD_DIRS + j, nullptr);
+    }
+    const double *c0 = a.conc0 + (a.member_set ? a.member_set[m] * a.set_stride : 0);
+    const double *l0 = a.lam0 + (long long)m * a.plane, *l1 = l0 + a.layer_stride;
+    for (long long i = threadIdx.x; i < a.plane; i += 256)
+        a.ic_grad[(long long)m * a.plane + i] = __ldg(c0 + i) < a.minConc ? 0.0 : mul(add(l0[i], l1[i]), 0.5);
 }
 
 // Observations compiled against the strip tables (host side).  One season's tables: every observation mapped to its
@@ -1722,6 +1895,38 @@ int upload_fp(nesosim_ctx *ctx, FpTables &t, long long row_len) {
     return NESOSIM_OK;
 }
 
+// The seed items of every sample slot of the general path, slot-major ([sets][stride] + 1 run starts), each slot's items
+// in the order adjoint_seed_kernel sums them: the set's point observations in chi2's order (kinds in turn, table order),
+// then its footprints in input order with their points in order.  `ft.begin` has its closing entry (upload_fp).
+void adjoint_items(const ObsTables &t, const FpTables &ft, int S, long long stride, std::vector<int> &begin,
+                   std::vector<int2> &item) {
+    std::vector<long long> key;
+    std::vector<int2> it;
+    for (int s = 0; s < S; ++s) {
+        const int *kb = t.kind_begin.data() + (size_t)s * (NESOSIM_OBS_KINDS + 1);
+        for (int k = 0; k < NESOSIM_OBS_KINDS; ++k)
+            for (int q = kb[k]; q < kb[k + 1]; ++q) {
+                key.push_back((long long)s * stride + t.o_slot[q]);
+                it.push_back(make_int2(q, -1 - k));
+            }
+        const int *fb = ft.kind_begin.data() + (size_t)s * (NESOSIM_OBS_KINDS + 1);
+        std::vector<int> fq;
+        for (int q = fb[0]; q < fb[NESOSIM_OBS_KINDS]; ++q) fq.push_back(q);
+        std::stable_sort(fq.begin(), fq.end(), [&](int x, int y) { return ft.src[x] < ft.src[y]; });
+        for (int q : fq)
+            for (long long p = ft.begin[q]; p < ft.begin[q + 1]; ++p) {
+                key.push_back((long long)s * stride + ft.pt_slot[p]);
+                it.push_back(make_int2(q, (int)p));
+            }
+    }
+    begin.assign((size_t)S * stride + 1, 0);
+    for (long long k : key) ++begin[k + 1];
+    for (size_t i = 1; i < begin.size(); ++i) begin[i] += begin[i - 1];
+    item.resize(it.size());
+    std::vector<int> fill(begin.begin(), begin.end() - 1);
+    for (size_t i = 0; i < it.size(); ++i) item[fill[key[i]]++] = it[i];
+}
+
 // Validates every observation and footprint, then compiles them against the strip tables and replaces the context's
 // observations.  sets: tagged with their forcing set (obs_set_host / fp_set_host); else one shared forcing.  Footprint
 // points get sample slots with the point observations (one slot per distinct (cell, day)) but never enter the point
@@ -1838,6 +2043,7 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
     if (rc) return rc;
     if ((rc = upload_fp(ctx, ft, (long long)fp_row_len))) return rc;
     auto &ob = ctx->obs;
+    if (general) adjoint_items(t, ft, S, (long long)stride, ob.adj_begin_h, ob.adj_item_h);
     if (general) {
         if ((rc = upload_vec(&ob.smp_begin, smp_begin)) || (rc = upload_vec(&ob.smp_entry, smp_entry))) return rc;
         ob.smp_tiles = (int)(((nx + TX - 1) / TX) * ((ny + TY - 1) / TY));
@@ -1861,12 +2067,16 @@ int register_observations(nesosim_ctx *ctx, bool sets, int64_t n_obs, const int3
 // nothing written outside the context, no synchronisation.
 // grad: the gradient builds (day_step_grad_kernel, sample_last_day_grad_kernel), which also advance and sample the
 // tangents; still T+1 launches.
-int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cudaStream_t st, bool grad = false) {
+// rec: the record builds (day_step_record_kernel, sample_last_day_traj_kernel) into the adjoint's trajectory; T+1 launches.
+int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cudaStream_t st, bool grad = false,
+                   bool rec = false) {
     const auto &ob = ctx->obs;
     const nesosim_config &c = ctx->cfg;
     const int T = c.num_days, M = c.n_members;
     const long long plane = ctx->plane, layer = (long long)M * plane;
-    auto ring = [&](int t, int l) { return ob.ring + ((long long)(t & 1) * 2 + l) * layer; };
+    auto ring = [&](int t, int l) {
+        return rec ? ob.traj + ((long long)t * 2 + l) * layer : ob.ring + ((long long)(t & 1) * 2 + l) * layer;
+    };
     InitArgs ia{};
     ia.plane = plane;
     ia.ic = ic_dev;
@@ -1884,7 +2094,7 @@ int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cu
     SampleArgs sa;
     sa.begin = ob.smp_begin; sa.entry = ob.smp_entry; sa.samples = ob.samples; sa.stride = ob.stride;
     sa.T = T; sa.tiles = ob.smp_tiles;
-    sa.ring = ob.ring; sa.plane = plane; sa.layer_stride = layer;
+    sa.ring = rec ? ob.traj : ob.ring; sa.plane = plane; sa.layer_stride = layer;
     sa.member_set = ctx->member_set_dev; sa.set_steps = ctx->set_steps_dev;
     const dim3 grid((c.nx + TX - 1) / TX, (c.ny + TY - 1) / TY, M);
     TangentArgs ta{};
@@ -1905,7 +2115,11 @@ int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cu
         }
         a.depth_mstride = a.plane_mstride = plane;
         const bool pdl = ctx->pdl && x > 0;       // behind this call's own previous day kernel only (see launch_day)
-        if (grad) {
+        if (rec) {
+            const RecArgs ra{ob.rec_flags + (long long)x * layer};
+            if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_record_kernel_512, grid, 512, st, pdl, a, sa, ra));
+            else CU(launch_day_kernel(day_step_record_kernel, grid, 256, st, pdl, a, sa, ra));
+        } else if (grad) {
             ta.prev = tring(x);
             ta.next = tring(x + 1);
             if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_grad_kernel_512, grid, 512, st, pdl, a, sa, ta));
@@ -1917,7 +2131,8 @@ int run_score_days(nesosim_ctx *ctx, const double *ic_dev, int ic_per_member, cu
         }
         ctx->launches++;
     }
-    if (grad) sample_last_day_grad_kernel<<<M, 256, 0, st>>>(sa, ta);
+    if (rec) sample_last_day_traj_kernel<<<M, 256, 0, st>>>(sa);
+    else if (grad) sample_last_day_grad_kernel<<<M, 256, 0, st>>>(sa, ta);
     else sample_last_day_kernel<<<M, 256, 0, st>>>(sa);
     ctx->launches++;
     CU(cudaGetLastError());
@@ -2057,6 +2272,181 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
     return NESOSIM_OK;
 }
 
+// nesosim_run_season_score_adjoint: the record build of the season (T+1 launches), the footprint means with their seed
+// coefficients (one launch, with footprints), the scores epilogue (one), the seeds (one), lambda at the last slots (one),
+// the T-1 backward day kernels and the finish (one): 2T+4 launches, 2T+5 with footprints (the seeds are skipped on a
+// grid without ocean), and one memset (two with model rows).
+struct AdjOutputs {
+    const double *w, *fw;           // host [NESOSIM_OBS_KINDS]
+    double *theta_grad, *ic_grad;
+};
+// frees the per-call adjoint state (the seed item tables stay: they belong to the registration)
+template <typename Obs>
+void adj_release(Obs &ob) {
+    cudaFree(ob.traj); cudaFree(ob.rec_flags); cudaFree(ob.lam); cudaFree(ob.theta_acc); cudaFree(ob.seeds);
+    cudaFree(ob.fp_coef);
+    ob.traj = ob.lam = ob.theta_acc = ob.fp_coef = nullptr;
+    ob.rec_flags = nullptr;
+    ob.seeds = nullptr;
+}
+template <typename T>
+int adj_alloc(T **p, size_t n) {
+    if (*p) return NESOSIM_OK;
+    if (cudaMalloc(p, std::max<size_t>(1, n) * sizeof(T)) != cudaSuccess) {
+        cudaGetLastError();
+        *p = nullptr;
+        return fail(NESOSIM_ERR_NOMEM, "the adjoint state does not fit the device");
+    }
+    return NESOSIM_OK;
+}
+int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                             int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
+                             int64_t model_stride, double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
+                             int64_t fp_model_stride, const AdjOutputs &ad, void *stream) {
+    if (!ctx || !params_host || !chi2_dev || !ad.theta_grad || !ad.ic_grad || !ad.w || !ad.fw)
+        return fail(NESOSIM_ERR_ARG, "bad argument");
+    for (int k = 0; k < NESOSIM_OBS_KINDS; ++k)
+        if (!(std::isfinite(ad.w[k]) && ad.w[k] >= 0.0 && std::isfinite(ad.fw[k]) && ad.fw[k] >= 0.0))
+            return fail(NESOSIM_ERR_ARG, "the objective's weights must be finite and >= 0");
+    if (!ctx->obs.ready || !ctx->obs.general)
+        return fail(NESOSIM_ERR_STATE, "the adjoint needs observations registered on the general path (nesosim_set_path(ctx, 1) first)");
+    auto &ob = ctx->obs;
+    if (ob.n_fp && !fp_chi2_dev) return fail(NESOSIM_ERR_STATE, "footprints are registered: fp_chi2_dev is required");
+    if (model_dev && model_stride < ob.row_len) return fail(NESOSIM_ERR_ARG, "model_stride is shorter than the observation row");
+    if (ob.n_fp && fp_model_dev && fp_model_stride < ob.fp_row_len)
+        return fail(NESOSIM_ERR_ARG, "fp_model_stride is shorter than the footprint row");
+    if (ctx->cfg.n_members > 65535 || (ctx->cfg.ny + TY - 1) / TY > 65535)
+        return fail(NESOSIM_ERR_ARG, "members or tile rows exceed the day kernel's grid dimensions");
+    if (!ctx->P) return fail(NESOSIM_ERR_STATE, "nesosim_set_forcing has not been called");
+    const bool sets = !ob.set_days.empty();
+    if (!sets && ctx->member_set_dev) return fail(NESOSIM_ERR_ARG, "misfit mode runs on one shared forcing");
+    if (sets && ob.set_days != ctx->set_days)
+        return fail(NESOSIM_ERR_STATE, "the forcing sets changed since nesosim_set_observations_sets; register the observations again");
+    if (ctx->path != 1)
+        return fail(NESOSIM_ERR_STATE, "the kernel path changed since the observations were registered; register them again");
+    CU(cudaSetDevice(ctx->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const nesosim_config &c = ctx->cfg;
+    const int T = c.num_days, M = c.n_members;
+    const long long plane = ctx->plane, layer = (long long)M * plane;
+    int rc;
+    if (!ob.adj_begin) {          // both tables or neither: a failed upload leaves nothing behind
+        int *b = nullptr;
+        int2 *it = nullptr;
+        if ((rc = upload_vec(&b, ob.adj_begin_h)) || (rc = upload_vec(&it, ob.adj_item_h))) {
+            cudaFree(b);
+            cudaFree(it);
+            cudaGetLastError();
+            return rc;
+        }
+        ob.adj_begin = b;
+        ob.adj_item = it;
+    }
+    if ((rc = adj_alloc(&ob.traj, (size_t)T * 2 * layer)) || (rc = adj_alloc(&ob.rec_flags, (size_t)std::max(1, T - 1) * layer)) ||
+        (rc = adj_alloc(&ob.lam, (size_t)4 * layer)) || (rc = adj_alloc(&ob.theta_acc, (size_t)GRAD_DIRS * layer)) ||
+        (rc = adj_alloc(&ob.seeds, (size_t)M * ob.stride)) ||
+        (rc = adj_alloc(&ob.fp_coef, (size_t)M * std::max(1LL, ob.fp_row_len)))) {
+        adj_release(ob);          // what did fit is not kept for a call that cannot run
+        return rc;
+    }
+    if ((rc = upload_coef(ctx, params_host, st))) return rc;
+    ctx->last_path = 1;
+    CU(cudaMemsetAsync(ob.theta_acc, 0, (size_t)GRAD_DIRS * layer * sizeof(double), st));
+    if ((rc = run_score_days(ctx, ic_dev, ic_per_member, st, false, true))) return rc;
+    if (model_dev && ob.row_len)
+        CU(cudaMemset2DAsync(model_dev, (size_t)model_stride * sizeof(double), 0xff, (size_t)ob.row_len * sizeof(double), M, st));
+    MisfitArgs ma;
+    ma.samples = ob.samples; ma.stride = ob.stride;
+    ma.obs_slot = ob.o_slot; ma.obs_day = ob.o_day; ma.obs_cell = ob.o_cell; ma.src = ob.src;
+    ma.obs_val = ob.val; ma.sigma = ob.sigma; ma.kind_begin = ob.kind_begin;
+    ma.conc = ctx->C; ma.plane = plane; ma.k = ctx->k;
+    ma.chi2 = chi2_dev; ma.count = (long long *)count_dev; ma.n_kinds = NESOSIM_OBS_KINDS;
+    ma.model = model_dev; ma.model_stride = model_stride;
+    ma.member_set = ctx->member_set_dev; ma.conc_set_stride = (long long)T * plane;
+    ma.fp_chi2 = nullptr; ma.fp_count = nullptr;
+    if (ob.n_fp) {
+        if (ob.fp_row_len) {
+            FootprintArgs fa;
+            fa.samples = ob.samples; fa.stride = ob.stride;
+            fa.begin = ob.fp_begin; fa.kind = ob.fp_kind; fa.src = ob.fp_src;
+            fa.pt_slot = ob.pt_slot; fa.pt_day = ob.pt_day; fa.pt_cell = ob.pt_cell; fa.pt_w = ob.pt_w;
+            fa.kind_begin = ob.fp_kind_begin; fa.conc = ctx->C; fa.plane = plane; fa.k = ctx->k;
+            fa.n_members = M; fa.row_len = ob.fp_row_len; fa.mean = ob.fp_mean; fa.mean_stride = ob.fp_row_len;
+            fa.model = fp_model_dev; fa.model_stride = fp_model_stride;
+            fa.member_set = ctx->member_set_dev; fa.conc_set_stride = (long long)T * plane;
+            const long long blocks = ob.fp_row_len * M;
+            if (blocks > INT_MAX) return fail(NESOSIM_ERR_ARG, "too many footprints x members for one launch");
+            FootprintAdj fj;
+            fj.coef = ob.fp_coef; fj.val = ob.fp_val; fj.sigma = ob.fp_sigma;
+            for (int k = 0; k < NESOSIM_OBS_KINDS; ++k) fj.fw[k] = ad.fw[k];
+            if (sets) footprint_mean_adj_kernel<true><<<(unsigned)blocks, 32, 0, st>>>(fa, fj);
+            else footprint_mean_adj_kernel<false><<<(unsigned)blocks, 32, 0, st>>>(fa, fj);
+            ctx->launches++;
+            CU(cudaGetLastError());
+        }
+        ma.fp_mean = ob.fp_mean; ma.fp_stride = std::max(1LL, ob.fp_row_len);
+        ma.fp_val = ob.fp_val; ma.fp_sigma = ob.fp_sigma; ma.fp_kind_begin = ob.fp_kind_begin;
+        ma.fp_chi2 = fp_chi2_dev; ma.fp_count = (long long *)fp_count_dev;
+    }
+    if (sets) misfit_finish_kernel<true><<<M, 256, 0, st>>>(ma);
+    else misfit_finish_kernel<false><<<M, 256, 0, st>>>(ma);
+    ctx->launches++;
+    CU(cudaGetLastError());
+
+    SeedArgs sd;
+    sd.samples = ob.samples; sd.seeds = ob.seeds; sd.stride = ob.stride;
+    sd.begin = ob.adj_begin; sd.item = ob.adj_item;
+    sd.obs_day = ob.o_day; sd.obs_cell = ob.o_cell; sd.obs_val = ob.val; sd.sigma = ob.sigma;
+    sd.fp_coef = ob.fp_coef; sd.fp_stride = std::max(1LL, ob.fp_row_len);
+    sd.fp_kind = ob.fp_kind; sd.fp_kind_begin = ob.fp_kind_begin; sd.pt_day = ob.pt_day; sd.pt_cell = ob.pt_cell;
+    sd.pt_w = ob.pt_w; sd.conc = ctx->C; sd.plane = plane; sd.conc_set_stride = (long long)T * plane;
+    sd.member_set = ctx->member_set_dev; sd.k = ctx->k;
+    for (int k = 0; k < NESOSIM_OBS_KINDS; ++k) sd.w[k] = ad.w[k];
+    if (ob.stride) {              // a grid without an ocean cell has no sample slot and nothing to seed
+        adjoint_seed_kernel<<<dim3((unsigned)((ob.stride + 255) / 256), M), 256, 0, st>>>(sd);
+        ctx->launches++;
+        CU(cudaGetLastError());
+    }
+
+    AdjInitArgs ai;
+    ai.lam = ob.lam; ai.plane = plane; ai.layer_stride = layer; ai.seeds = ob.seeds; ai.stride = ob.stride;
+    ai.begin = ob.smp_begin; ai.entry = ob.smp_entry; ai.T = T; ai.tiles = ob.smp_tiles;
+    ai.member_set = ctx->member_set_dev; ai.set_steps = ctx->set_steps_dev;
+    adjoint_init_kernel<<<M, 256, 0, st>>>(ai);
+    ctx->launches++;
+    CU(cudaGetLastError());
+
+    auto lam = [&](int t) { return ob.lam + (long long)(t & 1) * 2 * layer; };
+    AdjArgs aj;
+    aj.layer_stride = layer; aj.theta = ob.theta_acc; aj.seeds = ob.seeds;
+    aj.begin = ob.smp_begin; aj.entry = ob.smp_entry; aj.stride = ob.stride; aj.T = T; aj.tiles = ob.smp_tiles;
+    const dim3 grid((c.nx + TX - 1) / TX, (c.ny + TY - 1) / TY, M);
+    nesosim_outputs none{};
+    for (int x = T - 2; x >= 0; --x) {
+        DayArgs a;
+        fill_day_args(ctx, x, ctx->P + x * plane, ctx->C + x * plane, ctx->W + x * plane, ctx->UV + (long long)x * 2 * plane,
+                      ctx->UV + ((long long)x * 2 + 1) * plane, c.snowDensityFresh, &none, 0, x > 0, a);
+        for (int v = 0; v < NVAR; ++v) a.prev[v] = a.next[v] = nullptr;
+        a.depth_mstride = a.plane_mstride = plane;
+        aj.lam_in = lam(x + 1);
+        aj.lam_out = lam(x);
+        aj.h0 = ob.traj + (long long)x * 2 * layer;
+        aj.flags = ob.rec_flags + (long long)x * layer;
+        const bool pdl = ctx->pdl && x < T - 2;   // behind this call's own previous backward kernel only
+        if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_adjoint_kernel_512, grid, 512, st, pdl, a, aj));
+        else CU(launch_day_kernel(day_step_adjoint_kernel, grid, 256, st, pdl, a, aj));
+        ctx->launches++;
+    }
+    AdjFinishArgs af;
+    af.theta_acc = ob.theta_acc; af.lam0 = ob.lam; af.plane = plane; af.layer_stride = layer;
+    af.conc0 = ctx->C; af.set_stride = (long long)T * plane; af.member_set = ctx->member_set_dev; af.minConc = c.minConc;
+    af.theta_grad = ad.theta_grad; af.ic_grad = ad.ic_grad;
+    adjoint_finish_kernel<<<M, 256, 0, st>>>(af);
+    ctx->launches++;
+    CU(cudaGetLastError());
+    return NESOSIM_OK;
+}
+
 extern "C" {
 
 // Observations of the calibration driver, compiled against the strip tables and kept on the device until they are
@@ -2135,6 +2525,16 @@ int nesosim_run_season_score_grads(nesosim_ctx *ctx, const nesosim_member_params
     const GradOutputs g{grad_dev, jac_dev, jac_stride, fp_grad_dev, fp_jac_dev, fp_jac_stride};
     return run_season_scores(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, NESOSIM_OBS_KINDS, model_dev,
                              model_stride, stream, false, fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, &g);
+}
+
+int nesosim_run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
+                                     int ic_per_member, const double *weights_host, const double *fp_weights_host,
+                                     double *chi2_dev, int64_t *count_dev, double *model_dev, int64_t model_stride,
+                                     double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
+                                     int64_t fp_model_stride, double *theta_grad_dev, double *ic_grad_dev, void *stream) {
+    const AdjOutputs ad{weights_host, fp_weights_host, theta_grad_dev, ic_grad_dev};
+    return run_season_score_adjoint(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, model_dev, model_stride,
+                                    fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, ad, stream);
 }
 
 int nesosim_set_async(nesosim_ctx *ctx, int on) {

@@ -41,6 +41,17 @@ def conv_constants(variant="post_divide", stddev=1.0):
     raise ValueError("conv_variant must be 'post_divide' or 'pre_normalised'")
 
 
+def check_weights(w, name="weights"):
+    """The per-kind weights of the adjoint's objective as a tuple of OBS_KINDS floats (None: all ones); ValueError
+    unless there are OBS_KINDS of them, each finite and >= 0."""
+    if w is None:
+        return (1.0,) * _lib.OBS_KINDS
+    a = np.asarray(w, dtype=np.float64).ravel()
+    if a.shape != (_lib.OBS_KINDS,) or not (np.isfinite(a) & (a >= 0)).all():
+        raise ValueError("%s must be %d finite numbers >= 0" % (name, _lib.OBS_KINDS))
+    return tuple(float(x) for x in a)
+
+
 def _torch():
     import torch
     return torch
@@ -415,6 +426,48 @@ class SnowBudgetEngine:
             self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member, ptr("chi2"), ptr("used"), ptr("model"),
             width("model"), ptr("grad"), ptr("jac"), width("jac"), ptr("fp_chi2"), ptr("fp_used"), ptr("fp_model"),
             width("fp_model"), ptr("fp_grad"), ptr("fp_jac"), width("fp_jac"), self._stream()))
+        self._keep = (ic_t, r)
+        return r
+
+    def run_season_score_adjoint(self, params, ic, weights=None, fp_weights=None, model=False):
+        """``run_season_scores_fp`` with the reverse-mode derivatives of every member's objective J = sum_k weights[k]
+        chi2[k] + sum_k fp_weights[k] fp_chi2[k] (nesosim_run_season_score_adjoint; needs observations registered after
+        ``set_path('general')``).  ``weights``, ``fp_weights``: OBS_KINDS finite numbers >= 0 (default all ones).
+        Returns a dict of CUDA tensors: "chi2", "used", "model" (or None) and, with footprints registered, "fp_chi2",
+        "fp_used", "fp_model" (or None), bit-identical to ``run_season_scores_fp``; "theta_grad" [M, GRAD_DIRS] (dJ /
+        d theta for ``_lib.GRAD_PARAMS``) and "ic_grad" [M, ny, nx] (dJ / d ic of each member, also when the IC is
+        shared)."""
+        torch = _torch()
+        K, D = _lib.OBS_KINDS, _lib.GRAD_DIRS
+        w = check_weights(weights, "weights")
+        fw = check_weights(fp_weights, "fp_weights")
+        p = _lib.member_params_array(params)
+        assert len(p) == self.M
+        ic_t = None if ic is None else self._dev(ic)
+        per_member = 1 if (ic_t is not None and ic_t.dim() == 3 and self.M > 1) else 0
+        dev = "cuda:%d" % self.device
+        n_row, n_fp = self.observation_row_length(), self.footprint_row_length()
+        f64 = dict(dtype=torch.float64, device=dev)
+        r = {"chi2": torch.empty(self.M, K, **f64), "used": torch.empty(self.M, K, dtype=torch.int64, device=dev),
+             "model": torch.empty(self.M, n_row, **f64) if model else None,
+             "theta_grad": torch.empty(self.M, D, **f64), "ic_grad": torch.empty(self.M, self.ny, self.nx, **f64)}
+        if n_fp:
+            r.update({"fp_chi2": torch.empty(self.M, K, **f64), "fp_used": torch.empty(self.M, K, dtype=torch.int64, device=dev),
+                      "fp_model": torch.empty(self.M, n_fp, **f64) if model else None})
+
+        def ptr(name):
+            t = r.get(name)
+            return None if t is None else t.data_ptr()
+
+        def width(name):
+            t = r.get(name)
+            return 0 if t is None else t.shape[-1]
+
+        cw, cfw = (C.c_double * K)(*w), (C.c_double * K)(*fw)
+        _lib.check(self.lib.nesosim_run_season_score_adjoint(
+            self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member, cw, cfw, ptr("chi2"), ptr("used"),
+            ptr("model"), width("model"), ptr("fp_chi2"), ptr("fp_used"), ptr("fp_model"), width("fp_model"),
+            ptr("theta_grad"), ptr("ic_grad"), self._stream()))
         self._keep = (ic_t, r)
         return r
 

@@ -381,6 +381,16 @@ def gather_gradients(grad, jac, P, S, n_obs, rank=0, world=1, group=None, prefix
     return assemble_gradients(grad.cpu().numpy(), None if jac is None else jac.cpu().numpy(), P, S, n_obs, prefix)
 
 
+def gather_adjoint(theta_grad, ic_grad, P, S, rank=0, world=1, group=None):
+    """All-gather the ranks' per-member adjoint results ([n, GRAD_DIRS] and [n, ny, nx] in this rank's pair order) ->
+    {"adjoint_grad": [P, S, GRAD_DIRS], "ic_grad": [P, S, ny, nx]}, numpy, identical on every rank."""
+    if world > 1:
+        theta_grad = sharding.gather_member_results(theta_grad, P * S, rank, world, group)
+        ic_grad = sharding.gather_member_results(ic_grad, P * S, rank, world, group)
+    th, icg = theta_grad.cpu().numpy(), ic_grad.cpu().numpy()
+    return {"adjoint_grad": th.reshape(P, S, th.shape[-1]), "ic_grad": icg.reshape((P, S) + icg.shape[-2:])}
+
+
 def season_footprints(mask, seasons):
     """Every season's footprints (``"footprints"`` entry; none: no footprints), normalized and checked against the grid
     and that season's own length, on every rank before any device work."""
@@ -485,7 +495,7 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
 
 
 def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, model=False,
-                           grad=False, jac=False, **flags):
+                           grad=False, jac=False, adjoint=False, weights=None, fp_weights=None, **flags):
     """``run_calibration`` with observation errors and three observed quantities.  A season's ``"obs"`` is a dict with
     day, row, col, value and optionally kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``, default depth) and
     sigma (default 1), or the 4-tuple (day, row, col, depth).  Returns {"chi2": [P, S, OBS_KINDS], "used": [P, S,
@@ -509,9 +519,22 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     bit-identical to the season kernel's; ``fused`` must stay None (neither the HBM round trip nor the season kernel has
     tangents: ValueError before any device work).  ``jac=True`` (with ``grad``) adds "jac": per season the array [P,
     GRAD_DIRS, n_obs] of d model / d theta (NaN where the model value is not finite).  With footprints also "fp_grad"
-    and, with ``jac``, "fp_jac" (per season [P, GRAD_DIRS, n_fp])."""
+    and, with ``jac``, "fp_jac" (per season [P, GRAD_DIRS, n_fp]).
+
+    ``adjoint=True`` adds the reverse-mode derivatives of every pair's objective J = sum_k weights[k] chi2[k] + sum_k
+    fp_weights[k] fp_chi2[k] (OBS_KINDS finite weights >= 0 each, default all ones; nesosim_run_season_score_adjoint):
+    "adjoint_grad" [P, S, GRAD_DIRS] (dJ / d theta for the ``_lib.GRAD_PARAMS`` columns) and "ic_grad" [P, S, ny, nx]
+    (dJ / d the season's IC).  Like ``grad`` it scores on the general day-kernel path; with ``grad=True``, with ``fused``
+    not None or with bad weights it raises ValueError before any device work."""
     import torch
     from . import _lib
+    from .engine import check_weights
+    if adjoint and (grad or fused is not None):
+        raise ValueError("adjoint=True needs grad=False and fused=None: it runs on the general day-kernel path alone")
+    if not adjoint and (weights is not None or fp_weights is not None):
+        raise ValueError("weights and fp_weights belong to adjoint=True")
+    if adjoint:
+        weights, fp_weights = check_weights(weights, "weights"), check_weights(fp_weights, "fp_weights")
     if grad and fused is not None:
         raise ValueError("grad=True needs fused=None: only the general day-kernel path has tangents")
     if jac and not grad:
@@ -531,8 +554,10 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
 
     D = _lib.GRAD_DIRS
 
-    def gather(chi2, used, mod, fp, g=None):
+    def gather(chi2, used, mod, fp, g=None, adj=None):
         res = gather_scores(chi2, used, mod, P, S, n_obs, rank, world, group)
+        if adjoint:
+            res.update(gather_adjoint(adj[0], adj[1], P, S, rank, world, group))
         if with_fp:
             res.update(gather_footprint_scores(*fp, P, S, n_fp, rank, world, group))
         if grad:
@@ -548,7 +573,9 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         g0 = torch.zeros(0, K, D, dtype=torch.float64, device=dev)
         g = (g0, torch.zeros(0, D, width, dtype=torch.float64, device=dev) if jac else None,
              g0, torch.zeros(0, D, fp_width, dtype=torch.float64, device=dev) if jac else None)
-        return gather(chi2, used, mod, fp, g)
+        adj = (torch.zeros(0, D, dtype=torch.float64, device=dev),
+               torch.zeros((0,) + tuple(np.shape(mask)), dtype=torch.float64, device=dev))
+        return gather(chi2, used, mod, fp, g, adj)
     eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
     M = len(mine)
 
@@ -595,7 +622,7 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
             out[..., :t.shape[-1]] = t
         return out
 
-    def grad_call():   # the general path's tangent build: registered after set_path("general")
+    def grad_call():   # the general path's tangent / adjoint build: registered after set_path("general")
         eng.set_path("general")
         cols = {k: np.concatenate([obs[s][k] for s in staged]) for k in obs[0]}
         tag = np.concatenate([np.full(n_obs[s], i, dtype=np.int32) for i, s in enumerate(staged)])
@@ -605,7 +632,10 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         else:
             eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"], cols["sigma"],
                                     obs_set=tag)
-        r = eng.run_season_score_grads(mine, ic, model=model or with_fp, jac=jac)
+        if adjoint:
+            r = eng.run_season_score_adjoint(mine, ic, weights, fp_weights, model=model or with_fp)
+        else:
+            r = eng.run_season_score_grads(mine, ic, model=model or with_fp, jac=jac)
         mod = padded(r["model"], width, (M,)) if model else None
         fp, fg, fj = None, None, None
         if with_fp:   # the staged seasons may have no footprint at all: zero sums, NaN rows
@@ -614,12 +644,16 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
                   padded(r.get("fp_model"), fp_width, (M,)))
             fg = r.get("fp_grad", torch.zeros(M, K, D, dtype=torch.float64, device=dev))
             fj = padded(r.get("fp_jac"), fp_width, (M, D)) if jac else None
+        if adjoint:
+            return r["chi2"], r["used"], mod, fp, (r["theta_grad"], r["ic_grad"])
         g = (r["grad"], padded(r["jac"], width, (M, D)) if jac else None, fg, fj)
         return r["chi2"], r["used"], mod, fp, g
 
-    g = None
+    g = adj = None
     try:
-        if grad:
+        if adjoint:
+            chi2, used, mod, fp, adj = grad_call()
+        elif grad:
             chi2, used, mod, fp, g = grad_call()
         elif fused is False:
             chi2, used, mod, fp = hbm_round_trip()
@@ -638,4 +672,6 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         fp = tuple(t[back] for t in fp)
     if grad:
         g = tuple(None if t is None else t[back] for t in g)
-    return gather(chi2[back], used[back], mod[back] if model else None, fp, g)
+    if adjoint:
+        adj = tuple(t[back] for t in adj)
+    return gather(chi2[back], used[back], mod[back] if model else None, fp, g, adj)
