@@ -355,6 +355,34 @@ int nesosim_run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_para
                                      double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
                                      int64_t fp_model_stride, double *theta_grad_dev, double *ic_grad_dev, void *stream);
 
+/* Calibration adjoint with the forcing: nesosim_run_season_score_adjoint plus the derivatives of the same J_m with
+ * respect to the snowfall, wind-speed and ice-concentration forcing f = 0 precip, 1 wind, 2 conc (DESIGN.md §4.1).  They
+ * enter the day step point-wise, so the backward day kernel forms them per cell next to the parameter terms, pathwise as
+ * the rest (the wind threshold and the IC zeroing where conc[0] < minConc are steps, not differentiated):
+ *   forcing_scale_grad_dev [M][NESOSIM_FORCING_DIRS][ny][nx], required: sum over the member's days x (descending) of
+ *     F(x) g_F(x) where F(x) is finite, from 0.0 -- dJ_m / d alpha for a per-cell factor F -> alpha F over the season;
+ *   forcing_scale_total_dev [M][NESOSIM_FORCING_DIRS], required: each field summed over the cells in theta_grad's fixed
+ *     order ([m][0]: the derivative with respect to one snowfall scaling factor);
+ *   precip_day_dev, wind_day_dev, conc_day_dev [M][T][ny][nx], each NULL or written in full: g_F(x) = dJ_m / d F(x) of
+ *     every day (0 after the member's last day, and for precip and wind on it); conc includes the depth observation
+ *     operator's (h0 + h1) / C.
+ * Chi2, counts, model rows, theta_grad and ic_grad are bit-identical to nesosim_run_season_score_adjoint's.  Errors as
+ * that call's, and NESOSIM_ERR_ARG for a NULL forcing_scale_grad_dev or forcing_scale_total_dev.  The state is that of
+ * nesosim_run_season_score_adjoint plus 24 bytes per member-cell (the three scale accumulators) and 8 bytes per member
+ * and sample slot (the concentration seeds): 17 T + 80 bytes per member-cell and 24 per member-slot, allocated by the
+ * first forcing call and freed with the observations (NESOSIM_ERR_NOMEM as there).  The same 2T+4 launches (2T+5 with
+ * footprints), one memset more and no stream synchronisation after the first call. */
+#define NESOSIM_FORCING_DIRS 3   /* precip, wind, conc */
+int nesosim_run_season_score_adjoint_forcing(nesosim_ctx *ctx, const nesosim_member_params *params_host,
+                                             const double *ic_dev, int ic_per_member, const double *weights_host,
+                                             const double *fp_weights_host, double *chi2_dev, int64_t *count_dev,
+                                             double *model_dev, int64_t model_stride, double *fp_chi2_dev,
+                                             int64_t *fp_count_dev, double *fp_model_dev, int64_t fp_model_stride,
+                                             double *theta_grad_dev, double *ic_grad_dev,
+                                             double *forcing_scale_grad_dev, double *forcing_scale_total_dev,
+                                             double *precip_day_dev, double *wind_day_dev, double *conc_day_dev,
+                                             void *stream);
+
 /* ---- Row-strip domain decomposition over peer memory (grids too large for one GPU: the 5 km case; the reference
  * has no counterpart -- its grid is one numpy array -- so the contract is that of calcBudget on the whole grid).
  * A context created on rows [lo-2, hi+2) of the full grid (mask and forcing sliced the same way; 2 = radius of

@@ -21,6 +21,9 @@ OBS_DEPTH, OBS_VOLUME, OBS_DENSITY, OBS_KINDS = 0, 1, 2, 3
 # atmLossFactor -- the columns GRAD_PARAMS of a parameter row [WPF, WPT, LLF, ALF] (windPackThresh has no derivative)
 GRAD_DIRS = 3
 GRAD_PARAMS = (0, 2, 3)
+# forcing fields of nesosim_run_season_score_adjoint_forcing (NESOSIM_FORCING_DIRS), in the order of its outputs
+FORCING_DIRS = 3
+FORCING_FIELDS = ("precip", "wind", "conc")
 
 
 class NesosimError(RuntimeError):
@@ -121,6 +124,12 @@ _SIGNATURES = {
                                                    C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                                    C.c_void_p, C.c_void_p, C.c_void_p]),
+    "nesosim_run_season_score_adjoint_forcing": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int,
+                                                           C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p,
+                                                           C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                                           C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                           C.c_void_p]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

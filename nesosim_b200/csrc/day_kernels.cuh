@@ -759,6 +759,21 @@ struct AdjArgs {
     int T, tiles;
 };
 
+// Forcing build (FORCING, nesosim_run_season_score_adjoint_forcing): per own cell of day x, with mu0 and kill0 as above,
+// pd = P / rhoF and X = (((wt llf) dT) h0) W,
+//   g_P = kill0 ? 0 : (mu0 C) / rhoF;
+//   g_W = kill0 ? 0 : (lead ? mu0 lead_loss(W := 1) : 0) + (atm ? mu0 atm_loss(W := 1) : 0);
+//   g_C = (kill0 ? 0 : mu0 pd + (lead ? mu0 X : 0)) + cseed, cseed = the conc seed of the cell's sample slot on day x
+//   (0 without one);
+// acc[f] += finite(F) ? F g_F : 0 for F = P, W, C, and the three values go to the per-day planes when those are given.
+constexpr int FORCING_DIRS = 3;      // NESOSIM_FORCING_DIRS: precip, wind, conc
+struct ForcingAdjArgs {
+    const double *cseed;       // [M][stride] dJ/dC of the depth observations at every sample slot
+    double *acc;               // [M][FORCING_DIRS][plane] accumulators (member stride FORCING_DIRS * depth_mstride)
+    double *day[FORCING_DIRS]; // day x's plane of member 0 of each [M][T][plane] per-day output, or NULL
+    long long day_mstride;     // T * plane
+};
+
 // transposed 3x3 sum of the staged plane around (sr, sc)
 __device__ __forceinline__ double conv3x3_t(const DayArgs &a, const double (&p)[TY + 4][TX + 4], int sr, int sc) {
     double acc = 0.0;
@@ -769,9 +784,10 @@ __device__ __forceinline__ double conv3x3_t(const DayArgs &a, const double (&p)[
     return acc;
 }
 
-template <int DAY_THREADS>
+template <int DAY_THREADS, bool FORCING = false>
 __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs &j, TileSmem &sm,
-                                                 uint8_t (&s_flag)[TY + 4][TX + 4]) {
+                                                 uint8_t (&s_flag)[TY + 4][TX + 4], const ForcingAdjArgs *fa = nullptr,
+                                                 double (*s_gc)[TX] = nullptr) {
     pdl_launch_dependents();
     const int m = blockIdx.z, bx = blockIdx.x, by = blockIdx.y;
     const int fset = a.member_set ? a.member_set[m] : 0;
@@ -797,6 +813,11 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
             const long long o = (long long)gy * nx + gx;
             o0p[o] = 0.0;
             o1p[o] = 0.0;
+            if (FORCING) {
+#pragma unroll
+                for (int f = 0; f < FORCING_DIRS; ++f)
+                    if (fa->day[f]) fa->day[f][(long long)m * fa->day_mstride + o] = 0.0;
+            }
         }
         return;
     }
@@ -819,16 +840,28 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
             cp_async8(&s_vt[r][c], aV + o, in);
         }
     }
-    double pf_C[CPT], pf_W[CPT], pf_h0[CPT];
+    double pf_C[CPT], pf_W[CPT], pf_h0[CPT], pf_P[CPT];
 #pragma unroll
     for (int rr = 0; rr < CPT; ++rr) {
         const int gy = y0 + (tid / TX) + rr * (DAY_THREADS / TX);
-        pf_C[rr] = pf_W[rr] = pf_h0[rr] = 0.0;
+        pf_C[rr] = pf_W[rr] = pf_h0[rr] = pf_P[rr] = 0.0;
         if (gx < nx && gy < ny) {
             const long long o = (long long)gy * nx + gx;
             pf_C[rr] = __ldg(aC + o);
             pf_W[rr] = __ldg(aW + o);
             pf_h0[rr] = j.h0[ms + o];
+            if (FORCING) pf_P[rr] = __ldg(a.P + fo + o);
+        }
+    }
+    if (FORCING) {        // the conc seeds of the tile's sample slots on day x (the seed kernel ran before the sweep)
+        const int *sb = j.begin + ((long long)fset * j.T + a.x) * j.tiles + (long long)by * gridDim.x + bx;
+        for (int i = tid; i < TY * TX; i += DAY_THREADS) s_gc[i / TX][i % TX] = 0.0;
+        __syncthreads();
+        const double *cs = fa->cseed + (long long)m * j.stride;
+        for (int i = sb[0] + tid; i < sb[1]; i += DAY_THREADS) {
+            const int2 e = j.entry[i];
+            const int cy = e.x / nx;
+            s_gc[cy - y0][e.x - cy * nx - x0] = cs[e.y];
         }
     }
     const MemberCoef mc = a.coef[m];
@@ -947,6 +980,23 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
                 double *t = j.theta + ((long long)m * GRAD_DIRS + d) * a.depth_mstride + o;
                 *t = add(*t, th[d]);
             }
+            if (FORCING) {
+                const double P = pf_P[rr];
+                const double gP = k0 ? 0.0 : div_const(mul(mu0, C), a.rho_new);
+                const double wl1 = a.sw.leadloss ? mul(mu0, lead_loss(wt, h0, 1.0, C, mc, a.k)) : 0.0;
+                const double wa1 = a.sw.atmloss ? mul(mu0, atm_loss(wt, h0, 1.0, mc, a.k)) : 0.0;
+                const double gW = k0 ? 0.0 : add(wl1, wa1);
+                const double X = mul(mul(mul(mul(wt, mc.llf), dT), h0), W);
+                const double sC = add(mul(mu0, div_const(P, a.rho_new)), a.sw.leadloss ? mul(mu0, X) : 0.0);
+                const double gC = add(k0 ? 0.0 : sC, s_gc[ty][tx]);
+                const double F[FORCING_DIRS] = {P, W, C}, g[FORCING_DIRS] = {gP, gW, gC};
+#pragma unroll
+                for (int f = 0; f < FORCING_DIRS; ++f) {
+                    if (fa->day[f]) fa->day[f][(long long)m * fa->day_mstride + o] = g[f];
+                    double *t = fa->acc + ((long long)m * FORCING_DIRS + f) * a.depth_mstride + o;
+                    *t = add(*t, nesosim::finite(F[f]) ? mul(F[f], g[f]) : 0.0);
+                }
+            }
         }
     }
     __syncthreads();       // the tile's lambda(x) is stored: add the day's seeds at its sample slots
@@ -972,6 +1022,24 @@ __global__ void __launch_bounds__(512, 2) day_step_adjoint_kernel_512(const __gr
     __shared__ TileSmem sm;
     __shared__ uint8_t s_flag[TY + 4][TX + 4];
     day_step_adjoint<512>(a, j, sm, s_flag);
+}
+
+// The forcing builds of the same two shapes (ForcingAdjArgs above).
+__global__ void __launch_bounds__(256) day_step_adjoint_forcing_kernel(const __grid_constant__ DayArgs a,
+                                                                       const __grid_constant__ AdjArgs j,
+                                                                       const __grid_constant__ ForcingAdjArgs fa) {
+    __shared__ TileSmem sm;
+    __shared__ uint8_t s_flag[TY + 4][TX + 4];
+    __shared__ double s_gc[TY][TX];
+    day_step_adjoint<256, true>(a, j, sm, s_flag, &fa, s_gc);
+}
+__global__ void __launch_bounds__(512, 2) day_step_adjoint_forcing_kernel_512(const __grid_constant__ DayArgs a,
+                                                                              const __grid_constant__ AdjArgs j,
+                                                                              const __grid_constant__ ForcingAdjArgs fa) {
+    __shared__ TileSmem sm;
+    __shared__ uint8_t s_flag[TY + 4][TX + 4];
+    __shared__ double s_gc[TY][TX];
+    day_step_adjoint<512, true>(a, j, sm, s_flag, &fa, s_gc);
 }
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {

@@ -246,6 +246,9 @@ struct nesosim_ctx {
         double *traj = nullptr, *lam = nullptr, *theta_acc = nullptr, *fp_coef = nullptr;
         uint8_t *rec_flags = nullptr;
         double2 *seeds = nullptr;
+        // nesosim_run_season_score_adjoint_forcing: the conc seeds [M][stride] and the scale accumulators
+        // [M][FORCING_DIRS][plane], allocated by the first forcing call
+        double *cseed = nullptr, *forcing_acc = nullptr;
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -399,7 +402,7 @@ void obs_release(nesosim_ctx *ctx) {
     cudaFree(ob.smp_begin); cudaFree(ob.smp_entry); cudaFree(ob.ring);
     cudaFree(ob.tring); cudaFree(ob.tsamples); cudaFree(ob.fp_dmean);
     cudaFree(ob.adj_begin); cudaFree(ob.adj_item); cudaFree(ob.traj); cudaFree(ob.lam); cudaFree(ob.theta_acc);
-    cudaFree(ob.fp_coef); cudaFree(ob.rec_flags); cudaFree(ob.seeds);
+    cudaFree(ob.fp_coef); cudaFree(ob.rec_flags); cudaFree(ob.seeds); cudaFree(ob.cseed); cudaFree(ob.forcing_acc);
     ob = {};
 }
 
@@ -1588,7 +1591,10 @@ __device__ __forceinline__ void seed_partials(int kind, double2 h, double C, dou
         }
     }
 }
-__global__ void __launch_bounds__(256) adjoint_seed_kernel(const __grid_constant__ SeedArgs a) {
+// FORCING (adjoint_seed_forcing_kernel): also `cseed` [M][stride] = dJ/dC at the slot, summed from 0.0 in the same item
+// order over the depth items alone: -((a v) / C) with v = (h0 + h1) / C (dv/dC = -v/C).
+template <bool FORCING>
+__device__ __forceinline__ void adjoint_seed(const SeedArgs &a, double *cseed) {
     const long long sl = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int m = blockIdx.y;
     if (sl >= a.stride) return;
@@ -1596,15 +1602,14 @@ __global__ void __launch_bounds__(256) adjoint_seed_kernel(const __grid_constant
     const double *conc = a.conc + (long long)set * a.conc_set_stride;
     const double2 h = a.samples[(long long)m * a.stride + sl];
     const long long b = (long long)set * a.stride + sl;
-    double s0 = 0.0, s1 = 0.0;
+    double s0 = 0.0, s1 = 0.0, cs = 0.0;
     for (int i = a.begin[b]; i < a.begin[b + 1]; ++i) {
         const int2 it = a.item[i];
         int kind;
-        double av, C = 1.0;
+        double av, v, C = 1.0;
         if (it.y < 0) {
             const int q = it.x;
             kind = -1 - it.y;
-            double v;
             if (kind == NESOSIM_OBS_DEPTH) {
                 C = __ldg(conc + (long long)a.obs_day[q] * a.plane + a.obs_cell[q]);
                 v = div_ieee(add(h.x, h.y), C);
@@ -1618,7 +1623,6 @@ __global__ void __launch_bounds__(256) adjoint_seed_kernel(const __grid_constant
             kind = a.fp_kind[q];
             const double bc = a.fp_coef[(long long)m * a.fp_stride + q - a.fp_kind_begin[set * (NESOSIM_OBS_KINDS + 1)]];
             if (!nesosim::finite(bc)) continue;
-            double v;
             if (kind == NESOSIM_OBS_DEPTH) {
                 C = __ldg(conc + (long long)a.pt_day[p] * a.plane + a.pt_cell[p]);
                 v = div_ieee(add(h.x, h.y), C);
@@ -1631,8 +1635,16 @@ __global__ void __launch_bounds__(256) adjoint_seed_kernel(const __grid_constant
         seed_partials(kind, h, C, av, a.k, g0, g1);
         s0 = add(s0, g0);
         s1 = add(s1, g1);
+        if (FORCING && kind == NESOSIM_OBS_DEPTH) cs = add(cs, -div_ieee(mul(av, v), C));
     }
     a.seeds[(long long)m * a.stride + sl] = make_double2(s0, s1);
+    if (FORCING) cseed[(long long)m * a.stride + sl] = cs;
+}
+__global__ void __launch_bounds__(256) adjoint_seed_kernel(const __grid_constant__ SeedArgs a) {
+    adjoint_seed<false>(a, nullptr);
+}
+__global__ void __launch_bounds__(256) adjoint_seed_forcing_kernel(const __grid_constant__ SeedArgs a, double *cseed) {
+    adjoint_seed<true>(a, cseed);
 }
 
 // lambda at each member's last slot L (set_steps, or T-1): 0, plus the seeds of day L at its sample slots.
@@ -1646,12 +1658,28 @@ struct AdjInitArgs {
     int T, tiles;
     const int *member_set, *set_steps;
 };
-__global__ void __launch_bounds__(256) adjoint_init_kernel(const __grid_constant__ AdjInitArgs a) {
+// FORCING (adjoint_init_forcing_kernel): also the per-day planes of days L..T-1 (0, and g_C(L) = 0 + cseed at day L's
+// sample slots; no backward kernel writes these days) and the conc accumulator's first term, C(L) g_C(L).
+struct ForcingInitArgs {
+    const double *cseed;            // [M][stride]
+    double *acc;                    // [M][FORCING_DIRS][plane], zeroed
+    double *day[FORCING_DIRS];      // [M][T][plane] or NULL
+    const double *conc;             // [sets][T][plane]
+};
+template <bool FORCING>
+__device__ __forceinline__ void adjoint_init(const AdjInitArgs &a, const ForcingInitArgs *fi) {
     const int m = blockIdx.x;
     const int set = a.member_set ? a.member_set[m] : 0;
     const int L = a.set_steps ? a.set_steps[set] : a.T - 1;
     double *l0 = a.lam + (long long)(L & 1) * 2 * a.layer_stride + (long long)m * a.plane, *l1 = l0 + a.layer_stride;
     for (long long i = threadIdx.x; i < a.plane; i += blockDim.x) l0[i] = l1[i] = 0.0;
+    if (FORCING) {
+        for (int f = 0; f < FORCING_DIRS; ++f) {
+            if (!fi->day[f]) continue;
+            double *d = fi->day[f] + ((long long)m * a.T + L) * a.plane;
+            for (long long i = threadIdx.x; i < (long long)(a.T - L) * a.plane; i += blockDim.x) d[i] = 0.0;
+        }
+    }
     __syncthreads();
     const long long b = ((long long)set * a.T + L) * a.tiles;
     const double2 *sd = a.seeds + (long long)m * a.stride;
@@ -1659,7 +1687,21 @@ __global__ void __launch_bounds__(256) adjoint_init_kernel(const __grid_constant
         const int2 e = a.entry[i];
         l0[e.x] = add(l0[e.x], sd[e.y].x);
         l1[e.x] = add(l1[e.x], sd[e.y].y);
+        if (FORCING) {
+            const double g = add(0.0, fi->cseed[(long long)m * a.stride + e.y]);
+            const double C = __ldg(fi->conc + ((long long)set * a.T + L) * a.plane + e.x);
+            if (fi->day[2]) fi->day[2][((long long)m * a.T + L) * a.plane + e.x] = g;
+            double *t = fi->acc + ((long long)m * FORCING_DIRS + 2) * a.plane + e.x;
+            *t = add(*t, nesosim::finite(C) ? mul(C, g) : 0.0);
+        }
     }
+}
+__global__ void __launch_bounds__(256) adjoint_init_kernel(const __grid_constant__ AdjInitArgs a) {
+    adjoint_init<false>(a, nullptr);
+}
+__global__ void __launch_bounds__(256) adjoint_init_forcing_kernel(const __grid_constant__ AdjInitArgs a,
+                                                                   const __grid_constant__ ForcingInitArgs fi) {
+    adjoint_init<true>(a, &fi);
 }
 
 // One CTA per member: theta_grad[m][j] = the fixed-order sum of the accumulators over the cells (cell i to thread
@@ -1675,7 +1717,15 @@ struct AdjFinishArgs {
     double *theta_grad;             // [M][GRAD_DIRS]
     double *ic_grad;                // [M][plane]
 };
-__global__ void __launch_bounds__(256) adjoint_finish_kernel(const __grid_constant__ AdjFinishArgs a) {
+// FORCING (adjoint_finish_forcing_kernel): also the scale fields (the accumulators) and their totals, each summed over
+// the cells in the same fixed order as theta_grad.
+struct ForcingFinishArgs {
+    const double *acc;              // [M][FORCING_DIRS][plane]
+    double *scale_grad;             // [M][FORCING_DIRS][plane]
+    double *scale_total;            // [M][FORCING_DIRS]
+};
+template <bool FORCING>
+__device__ __forceinline__ void adjoint_finish(const AdjFinishArgs &a, const ForcingFinishArgs *ff) {
     const int m = blockIdx.x;
     __shared__ double red[8];
     __shared__ long long redc[8];
@@ -1685,10 +1735,29 @@ __global__ void __launch_bounds__(256) adjoint_finish_kernel(const __grid_consta
         for (long long i = threadIdx.x; i < a.plane; i += 256) acc = add(acc, t[i]);
         block_total(acc, 0, red, redc, a.theta_grad + (long long)m * GRAD_DIRS + j, nullptr);
     }
+    if (FORCING) {
+        for (int f = 0; f < FORCING_DIRS; ++f) {
+            const long long o = ((long long)m * FORCING_DIRS + f) * a.plane;
+            double acc = 0.0;
+            for (long long i = threadIdx.x; i < a.plane; i += 256) {
+                const double v = ff->acc[o + i];
+                ff->scale_grad[o + i] = v;
+                acc = add(acc, v);
+            }
+            block_total(acc, 0, red, redc, ff->scale_total + (long long)m * FORCING_DIRS + f, nullptr);
+        }
+    }
     const double *c0 = a.conc0 + (a.member_set ? a.member_set[m] * a.set_stride : 0);
     const double *l0 = a.lam0 + (long long)m * a.plane, *l1 = l0 + a.layer_stride;
     for (long long i = threadIdx.x; i < a.plane; i += 256)
         a.ic_grad[(long long)m * a.plane + i] = __ldg(c0 + i) < a.minConc ? 0.0 : mul(add(l0[i], l1[i]), 0.5);
+}
+__global__ void __launch_bounds__(256) adjoint_finish_kernel(const __grid_constant__ AdjFinishArgs a) {
+    adjoint_finish<false>(a, nullptr);
+}
+__global__ void __launch_bounds__(256) adjoint_finish_forcing_kernel(const __grid_constant__ AdjFinishArgs a,
+                                                                     const __grid_constant__ ForcingFinishArgs ff) {
+    adjoint_finish<true>(a, &ff);
 }
 
 // Observations compiled against the strip tables (host side).  One season's tables: every observation mapped to its
@@ -2275,17 +2344,23 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
 // nesosim_run_season_score_adjoint: the record build of the season (T+1 launches), the footprint means with their seed
 // coefficients (one launch, with footprints), the scores epilogue (one), the seeds (one), lambda at the last slots (one),
 // the T-1 backward day kernels and the finish (one): 2T+4 launches, 2T+5 with footprints (the seeds are skipped on a
-// grid without ocean), and one memset (two with model rows).
+// grid without ocean), and one memset (two with model rows).  With `forcing` (nesosim_run_season_score_adjoint_forcing)
+// the seed, init, backward and finish kernels are their forcing builds, and one more memset clears the accumulators.
 struct AdjOutputs {
     const double *w, *fw;           // host [NESOSIM_OBS_KINDS]
     double *theta_grad, *ic_grad;
+};
+static_assert(FORCING_DIRS == NESOSIM_FORCING_DIRS, "forcing directions");
+struct ForcingOutputs {
+    double *scale_grad, *scale_total;   // [M][FORCING_DIRS][plane], [M][FORCING_DIRS]
+    double *day[FORCING_DIRS];          // [M][T][plane] or NULL
 };
 // frees the per-call adjoint state (the seed item tables stay: they belong to the registration)
 template <typename Obs>
 void adj_release(Obs &ob) {
     cudaFree(ob.traj); cudaFree(ob.rec_flags); cudaFree(ob.lam); cudaFree(ob.theta_acc); cudaFree(ob.seeds);
-    cudaFree(ob.fp_coef);
-    ob.traj = ob.lam = ob.theta_acc = ob.fp_coef = nullptr;
+    cudaFree(ob.fp_coef); cudaFree(ob.cseed); cudaFree(ob.forcing_acc);
+    ob.traj = ob.lam = ob.theta_acc = ob.fp_coef = ob.cseed = ob.forcing_acc = nullptr;
     ob.rec_flags = nullptr;
     ob.seeds = nullptr;
 }
@@ -2302,9 +2377,11 @@ int adj_alloc(T **p, size_t n) {
 int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *params_host, const double *ic_dev,
                              int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
                              int64_t model_stride, double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
-                             int64_t fp_model_stride, const AdjOutputs &ad, void *stream) {
+                             int64_t fp_model_stride, const AdjOutputs &ad, void *stream,
+                             const ForcingOutputs *fo = nullptr) {
     if (!ctx || !params_host || !chi2_dev || !ad.theta_grad || !ad.ic_grad || !ad.w || !ad.fw)
         return fail(NESOSIM_ERR_ARG, "bad argument");
+    if (fo && (!fo->scale_grad || !fo->scale_total)) return fail(NESOSIM_ERR_ARG, "bad argument");
     for (int k = 0; k < NESOSIM_OBS_KINDS; ++k)
         if (!(std::isfinite(ad.w[k]) && ad.w[k] >= 0.0 && std::isfinite(ad.fw[k]) && ad.fw[k] >= 0.0))
             return fail(NESOSIM_ERR_ARG, "the objective's weights must be finite and >= 0");
@@ -2345,13 +2422,16 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
     if ((rc = adj_alloc(&ob.traj, (size_t)T * 2 * layer)) || (rc = adj_alloc(&ob.rec_flags, (size_t)std::max(1, T - 1) * layer)) ||
         (rc = adj_alloc(&ob.lam, (size_t)4 * layer)) || (rc = adj_alloc(&ob.theta_acc, (size_t)GRAD_DIRS * layer)) ||
         (rc = adj_alloc(&ob.seeds, (size_t)M * ob.stride)) ||
-        (rc = adj_alloc(&ob.fp_coef, (size_t)M * std::max(1LL, ob.fp_row_len)))) {
+        (rc = adj_alloc(&ob.fp_coef, (size_t)M * std::max(1LL, ob.fp_row_len))) ||
+        (fo && ((rc = adj_alloc(&ob.cseed, (size_t)M * ob.stride)) ||
+                (rc = adj_alloc(&ob.forcing_acc, (size_t)FORCING_DIRS * layer))))) {
         adj_release(ob);          // what did fit is not kept for a call that cannot run
         return rc;
     }
     if ((rc = upload_coef(ctx, params_host, st))) return rc;
     ctx->last_path = 1;
     CU(cudaMemsetAsync(ob.theta_acc, 0, (size_t)GRAD_DIRS * layer * sizeof(double), st));
+    if (fo) CU(cudaMemsetAsync(ob.forcing_acc, 0, (size_t)FORCING_DIRS * layer * sizeof(double), st));
     if ((rc = run_score_days(ctx, ic_dev, ic_per_member, st, false, true))) return rc;
     if (model_dev && ob.row_len)
         CU(cudaMemset2DAsync(model_dev, (size_t)model_stride * sizeof(double), 0xff, (size_t)ob.row_len * sizeof(double), M, st));
@@ -2403,7 +2483,9 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
     sd.member_set = ctx->member_set_dev; sd.k = ctx->k;
     for (int k = 0; k < NESOSIM_OBS_KINDS; ++k) sd.w[k] = ad.w[k];
     if (ob.stride) {              // a grid without an ocean cell has no sample slot and nothing to seed
-        adjoint_seed_kernel<<<dim3((unsigned)((ob.stride + 255) / 256), M), 256, 0, st>>>(sd);
+        const dim3 sg((unsigned)((ob.stride + 255) / 256), M);
+        if (fo) adjoint_seed_forcing_kernel<<<sg, 256, 0, st>>>(sd, ob.cseed);
+        else adjoint_seed_kernel<<<sg, 256, 0, st>>>(sd);
         ctx->launches++;
         CU(cudaGetLastError());
     }
@@ -2412,7 +2494,18 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
     ai.lam = ob.lam; ai.plane = plane; ai.layer_stride = layer; ai.seeds = ob.seeds; ai.stride = ob.stride;
     ai.begin = ob.smp_begin; ai.entry = ob.smp_entry; ai.T = T; ai.tiles = ob.smp_tiles;
     ai.member_set = ctx->member_set_dev; ai.set_steps = ctx->set_steps_dev;
-    adjoint_init_kernel<<<M, 256, 0, st>>>(ai);
+    ForcingInitArgs fi{};
+    ForcingAdjArgs fj{};
+    if (fo) {
+        fi.cseed = fj.cseed = ob.cseed;
+        fi.acc = fj.acc = ob.forcing_acc;
+        fi.conc = ctx->C;
+        for (int f = 0; f < FORCING_DIRS; ++f) fi.day[f] = fo->day[f];
+        fj.day_mstride = (long long)T * plane;
+        adjoint_init_forcing_kernel<<<M, 256, 0, st>>>(ai, fi);
+    } else {
+        adjoint_init_kernel<<<M, 256, 0, st>>>(ai);
+    }
     ctx->launches++;
     CU(cudaGetLastError());
 
@@ -2433,15 +2526,23 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
         aj.h0 = ob.traj + (long long)x * 2 * layer;
         aj.flags = ob.rec_flags + (long long)x * layer;
         const bool pdl = ctx->pdl && x < T - 2;   // behind this call's own previous backward kernel only
-        if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_adjoint_kernel_512, grid, 512, st, pdl, a, aj));
-        else CU(launch_day_kernel(day_step_adjoint_kernel, grid, 256, st, pdl, a, aj));
+        if (fo) {
+            for (int f = 0; f < FORCING_DIRS; ++f) fj.day[f] = fo->day[f] ? fo->day[f] + (long long)x * plane : nullptr;
+            if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_adjoint_forcing_kernel_512, grid, 512, st, pdl, a, aj, fj));
+            else CU(launch_day_kernel(day_step_adjoint_forcing_kernel, grid, 256, st, pdl, a, aj, fj));
+        } else if (ctx->day_variant == 512) {
+            CU(launch_day_kernel(day_step_adjoint_kernel_512, grid, 512, st, pdl, a, aj));
+        } else {
+            CU(launch_day_kernel(day_step_adjoint_kernel, grid, 256, st, pdl, a, aj));
+        }
         ctx->launches++;
     }
     AdjFinishArgs af;
     af.theta_acc = ob.theta_acc; af.lam0 = ob.lam; af.plane = plane; af.layer_stride = layer;
     af.conc0 = ctx->C; af.set_stride = (long long)T * plane; af.member_set = ctx->member_set_dev; af.minConc = c.minConc;
     af.theta_grad = ad.theta_grad; af.ic_grad = ad.ic_grad;
-    adjoint_finish_kernel<<<M, 256, 0, st>>>(af);
+    if (fo) adjoint_finish_forcing_kernel<<<M, 256, 0, st>>>(af, ForcingFinishArgs{ob.forcing_acc, fo->scale_grad, fo->scale_total});
+    else adjoint_finish_kernel<<<M, 256, 0, st>>>(af);
     ctx->launches++;
     CU(cudaGetLastError());
     return NESOSIM_OK;
@@ -2535,6 +2636,21 @@ int nesosim_run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_para
     const AdjOutputs ad{weights_host, fp_weights_host, theta_grad_dev, ic_grad_dev};
     return run_season_score_adjoint(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, model_dev, model_stride,
                                     fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, ad, stream);
+}
+
+int nesosim_run_season_score_adjoint_forcing(nesosim_ctx *ctx, const nesosim_member_params *params_host,
+                                             const double *ic_dev, int ic_per_member, const double *weights_host,
+                                             const double *fp_weights_host, double *chi2_dev, int64_t *count_dev,
+                                             double *model_dev, int64_t model_stride, double *fp_chi2_dev,
+                                             int64_t *fp_count_dev, double *fp_model_dev, int64_t fp_model_stride,
+                                             double *theta_grad_dev, double *ic_grad_dev,
+                                             double *forcing_scale_grad_dev, double *forcing_scale_total_dev,
+                                             double *precip_day_dev, double *wind_day_dev, double *conc_day_dev,
+                                             void *stream) {
+    const AdjOutputs ad{weights_host, fp_weights_host, theta_grad_dev, ic_grad_dev};
+    const ForcingOutputs fo{forcing_scale_grad_dev, forcing_scale_total_dev, {precip_day_dev, wind_day_dev, conc_day_dev}};
+    return run_season_score_adjoint(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, model_dev, model_stride,
+                                    fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, ad, stream, &fo);
 }
 
 int nesosim_set_async(nesosim_ctx *ctx, int on) {

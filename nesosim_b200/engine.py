@@ -429,16 +429,30 @@ class SnowBudgetEngine:
         self._keep = (ic_t, r)
         return r
 
-    def run_season_score_adjoint(self, params, ic, weights=None, fp_weights=None, model=False):
+    def run_season_score_adjoint(self, params, ic, weights=None, fp_weights=None, model=False, forcing=False,
+                                 forcing_days=()):
         """``run_season_scores_fp`` with the reverse-mode derivatives of every member's objective J = sum_k weights[k]
         chi2[k] + sum_k fp_weights[k] fp_chi2[k] (nesosim_run_season_score_adjoint; needs observations registered after
         ``set_path('general')``).  ``weights``, ``fp_weights``: OBS_KINDS finite numbers >= 0 (default all ones).
         Returns a dict of CUDA tensors: "chi2", "used", "model" (or None) and, with footprints registered, "fp_chi2",
         "fp_used", "fp_model" (or None), bit-identical to ``run_season_scores_fp``; "theta_grad" [M, GRAD_DIRS] (dJ /
         d theta for ``_lib.GRAD_PARAMS``) and "ic_grad" [M, ny, nx] (dJ / d ic of each member, also when the IC is
-        shared)."""
+        shared).
+
+        ``forcing=True`` (nesosim_run_season_score_adjoint_forcing) adds the derivatives with respect to the forcing
+        fields ``_lib.FORCING_FIELDS`` (precip, wind, conc): "forcing_scale_grad" [M, FORCING_DIRS, ny, nx] (dJ / d alpha
+        of a per-cell factor F -> alpha F applied to the whole season) and "forcing_scale_total" [M, FORCING_DIRS] (one
+        factor for the whole grid).  ``forcing_days``: any of those names, each adding "<name>_day_grad" [M, T, ny, nx]
+        = dJ / d F of every day (8 T bytes per member-cell each).  ``forcing_days`` without ``forcing=True`` or with an
+        unknown name raises ValueError before any device work."""
         torch = _torch()
         K, D = _lib.OBS_KINDS, _lib.GRAD_DIRS
+        forcing_days = tuple(forcing_days)
+        bad = [n for n in forcing_days if n not in _lib.FORCING_FIELDS]
+        if bad:
+            raise ValueError("forcing_days: unknown field(s) %s; expected any of %s" % (bad, _lib.FORCING_FIELDS))
+        if forcing_days and not forcing:
+            raise ValueError("forcing_days needs forcing=True")
         w = check_weights(weights, "weights")
         fw = check_weights(fp_weights, "fp_weights")
         p = _lib.member_params_array(params)
@@ -464,10 +478,20 @@ class SnowBudgetEngine:
             return 0 if t is None else t.shape[-1]
 
         cw, cfw = (C.c_double * K)(*w), (C.c_double * K)(*fw)
-        _lib.check(self.lib.nesosim_run_season_score_adjoint(
-            self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member, cw, cfw, ptr("chi2"), ptr("used"),
-            ptr("model"), width("model"), ptr("fp_chi2"), ptr("fp_used"), ptr("fp_model"), width("fp_model"),
-            ptr("theta_grad"), ptr("ic_grad"), self._stream()))
+        args = (self.handle, p, None if ic_t is None else ic_t.data_ptr(), per_member, cw, cfw, ptr("chi2"), ptr("used"),
+                ptr("model"), width("model"), ptr("fp_chi2"), ptr("fp_used"), ptr("fp_model"), width("fp_model"),
+                ptr("theta_grad"), ptr("ic_grad"))
+        if forcing:
+            F = _lib.FORCING_DIRS
+            r["forcing_scale_grad"] = torch.empty(self.M, F, self.ny, self.nx, **f64)
+            r["forcing_scale_total"] = torch.empty(self.M, F, **f64)
+            for n in forcing_days:
+                r[n + "_day_grad"] = torch.empty(self.M, self.T, self.ny, self.nx, **f64)
+            days = [ptr(n + "_day_grad") for n in _lib.FORCING_FIELDS]
+            _lib.check(self.lib.nesosim_run_season_score_adjoint_forcing(
+                *args, ptr("forcing_scale_grad"), ptr("forcing_scale_total"), *days, self._stream()))
+        else:
+            _lib.check(self.lib.nesosim_run_season_score_adjoint(*args, self._stream()))
         self._keep = (ic_t, r)
         return r
 

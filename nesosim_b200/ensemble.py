@@ -391,6 +391,17 @@ def gather_adjoint(theta_grad, ic_grad, P, S, rank=0, world=1, group=None):
     return {"adjoint_grad": th.reshape(P, S, th.shape[-1]), "ic_grad": icg.reshape((P, S) + icg.shape[-2:])}
 
 
+def gather_forcing_grad(scale_grad, scale_total, P, S, rank=0, world=1, group=None):
+    """All-gather the ranks' per-member forcing derivatives ([n, FORCING_DIRS, ny, nx] and [n, FORCING_DIRS] in this
+    rank's pair order) -> {"forcing_scale_grad": [P, S, FORCING_DIRS, ny, nx], "forcing_scale_total": [P, S,
+    FORCING_DIRS]}, numpy, identical on every rank."""
+    if world > 1:
+        scale_grad = sharding.gather_member_results(scale_grad, P * S, rank, world, group)
+        scale_total = sharding.gather_member_results(scale_total, P * S, rank, world, group)
+    g, t = scale_grad.cpu().numpy(), scale_total.cpu().numpy()
+    return {"forcing_scale_grad": g.reshape((P, S) + g.shape[-3:]), "forcing_scale_total": t.reshape(P, S, t.shape[-1])}
+
+
 def season_footprints(mask, seasons):
     """Every season's footprints (``"footprints"`` entry; none: no footprints), normalized and checked against the grid
     and that season's own length, on every rank before any device work."""
@@ -495,7 +506,8 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
 
 
 def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, model=False,
-                           grad=False, jac=False, adjoint=False, weights=None, fp_weights=None, **flags):
+                           grad=False, jac=False, adjoint=False, weights=None, fp_weights=None, forcing_grad=False,
+                           **flags):
     """``run_calibration`` with observation errors and three observed quantities.  A season's ``"obs"`` is a dict with
     day, row, col, value and optionally kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``, default depth) and
     sigma (default 1), or the 4-tuple (day, row, col, depth).  Returns {"chi2": [P, S, OBS_KINDS], "used": [P, S,
@@ -525,7 +537,14 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     fp_weights[k] fp_chi2[k] (OBS_KINDS finite weights >= 0 each, default all ones; nesosim_run_season_score_adjoint):
     "adjoint_grad" [P, S, GRAD_DIRS] (dJ / d theta for the ``_lib.GRAD_PARAMS`` columns) and "ic_grad" [P, S, ny, nx]
     (dJ / d the season's IC).  Like ``grad`` it scores on the general day-kernel path; with ``grad=True``, with ``fused``
-    not None or with bad weights it raises ValueError before any device work."""
+    not None or with bad weights it raises ValueError before any device work.
+
+    ``forcing_grad=True`` (with ``adjoint``; nesosim_run_season_score_adjoint_forcing) also adds the derivatives of J
+    with respect to the season's forcing fields ``_lib.FORCING_FIELDS`` (precip, wind, conc): "forcing_scale_grad" [P,
+    S, FORCING_DIRS, ny, nx] (dJ / d alpha of a per-cell factor F -> alpha F over the whole season) and
+    "forcing_scale_total" [P, S, FORCING_DIRS] (one factor for the whole grid; [..., 0] is the snowfall scaling
+    factor).  The per-day derivatives are offered by ``SnowBudgetEngine.run_season_score_adjoint`` alone: they are 8 T
+    bytes per member-cell and field, too large to gather on every rank."""
     import torch
     from . import _lib
     from .engine import check_weights
@@ -533,6 +552,8 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         raise ValueError("adjoint=True needs grad=False and fused=None: it runs on the general day-kernel path alone")
     if not adjoint and (weights is not None or fp_weights is not None):
         raise ValueError("weights and fp_weights belong to adjoint=True")
+    if forcing_grad and not adjoint:
+        raise ValueError("forcing_grad=True needs adjoint=True")
     if adjoint:
         weights, fp_weights = check_weights(weights, "weights"), check_weights(fp_weights, "fp_weights")
     if grad and fused is not None:
@@ -558,6 +579,8 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         res = gather_scores(chi2, used, mod, P, S, n_obs, rank, world, group)
         if adjoint:
             res.update(gather_adjoint(adj[0], adj[1], P, S, rank, world, group))
+        if forcing_grad:
+            res.update(gather_forcing_grad(adj[2], adj[3], P, S, rank, world, group))
         if with_fp:
             res.update(gather_footprint_scores(*fp, P, S, n_fp, rank, world, group))
         if grad:
@@ -573,8 +596,11 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         g0 = torch.zeros(0, K, D, dtype=torch.float64, device=dev)
         g = (g0, torch.zeros(0, D, width, dtype=torch.float64, device=dev) if jac else None,
              g0, torch.zeros(0, D, fp_width, dtype=torch.float64, device=dev) if jac else None)
+        F = _lib.FORCING_DIRS
         adj = (torch.zeros(0, D, dtype=torch.float64, device=dev),
-               torch.zeros((0,) + tuple(np.shape(mask)), dtype=torch.float64, device=dev))
+               torch.zeros((0,) + tuple(np.shape(mask)), dtype=torch.float64, device=dev),
+               torch.zeros((0, F) + tuple(np.shape(mask)), dtype=torch.float64, device=dev),
+               torch.zeros(0, F, dtype=torch.float64, device=dev))
         return gather(chi2, used, mod, fp, g, adj)
     eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
     M = len(mine)
@@ -633,7 +659,7 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
             eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"], cols["sigma"],
                                     obs_set=tag)
         if adjoint:
-            r = eng.run_season_score_adjoint(mine, ic, weights, fp_weights, model=model or with_fp)
+            r = eng.run_season_score_adjoint(mine, ic, weights, fp_weights, model=model or with_fp, forcing=forcing_grad)
         else:
             r = eng.run_season_score_grads(mine, ic, model=model or with_fp, jac=jac)
         mod = padded(r["model"], width, (M,)) if model else None
@@ -645,7 +671,8 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
             fg = r.get("fp_grad", torch.zeros(M, K, D, dtype=torch.float64, device=dev))
             fj = padded(r.get("fp_jac"), fp_width, (M, D)) if jac else None
         if adjoint:
-            return r["chi2"], r["used"], mod, fp, (r["theta_grad"], r["ic_grad"])
+            return r["chi2"], r["used"], mod, fp, (r["theta_grad"], r["ic_grad"], r.get("forcing_scale_grad"),
+                                                   r.get("forcing_scale_total"))
         g = (r["grad"], padded(r["jac"], width, (M, D)) if jac else None, fg, fj)
         return r["chi2"], r["used"], mod, fp, g
 
@@ -673,5 +700,5 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     if grad:
         g = tuple(None if t is None else t[back] for t in g)
     if adjoint:
-        adj = tuple(t[back] for t in adj)
+        adj = tuple(None if t is None else t[back] for t in adj)
     return gather(chi2[back], used[back], mod[back] if model else None, fp, g, adj)
