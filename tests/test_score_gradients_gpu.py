@@ -1,7 +1,7 @@
 """GPU: calibration gradients (nesosim_run_season_score_grads, the tangent-linear build of the scoring day kernel and of
 both epilogues).  Jacobian rows, d chi2 / d theta, footprint derivatives and footprint gradients are bit-identical to
 the restatement (oracle/score_gradients.py) for both CTA shapes, the land-tile shortcut on and off, dynamics on and off,
-every loss switch on, per-member ICs, forcing sets with short seasons (each season's last day observed) and wide,
+every loss switch on (the other switch configurations: test_calibration_switches_gpu.py), per-member ICs, forcing sets with short seasons (each season's last day observed) and wide,
 ragged and coastline grids.  The primal outputs are bit-identical to nesosim_run_season_scores_fp; also determinism,
 the launch count, the errors, agreement with finite differences through extra members and the calibration driver."""
 import functools
