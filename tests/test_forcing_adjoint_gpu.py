@@ -3,7 +3,7 @@ builds of the seed, init, backward day and finish kernels).  The scale fields, t
 gradient stacks are bit-identical to the restatement (oracle/forcing_adjoint.py) for both CTA shapes, the land-tile
 shortcut on and off, dynamics on and off, forcing sets with short seasons and a wide, ragged grid; the outputs the
 plain adjoint also gives are bit-identical to it; the scale outputs do not depend on the per-day buffers; also
-determinism, the launch count and the errors."""
+determinism, the launch count and the errors.  Ice and finite drift on the grid edges: test_grid_edges_gpu.py."""
 import ctypes as C
 
 import numpy as np

@@ -3,7 +3,8 @@ seeds, the backward day kernel and the finish).  ic_grad and theta_grad are bit-
 (oracle/score_adjoint.py) for both CTA shapes, the land-tile shortcut on and off, dynamics on and off, per-member ICs
 finite on land, forcing sets with short seasons (each season's last day observed) and wide, ragged and coastline grids;
 the scores are bit-identical to nesosim_run_season_scores_fp; theta_grad agrees with the forward-mode gradients; also
-determinism, the launch count and the errors."""
+determinism, the launch count and the errors.  Ice and finite drift on the grid edges (the one-sided differences, the
+backward kernel's edge divisors and E term): test_grid_edges_gpu.py."""
 import functools
 
 import numpy as np

@@ -3,7 +3,8 @@ both epilogues).  Jacobian rows, d chi2 / d theta, footprint derivatives and foo
 the restatement (oracle/score_gradients.py) for both CTA shapes, the land-tile shortcut on and off, dynamics on and off,
 every loss switch on (the other switch configurations: test_calibration_switches_gpu.py), per-member ICs, forcing sets with short seasons (each season's last day observed) and wide,
 ragged and coastline grids.  The primal outputs are bit-identical to nesosim_run_season_scores_fp; also determinism,
-the launch count, the errors, agreement with finite differences through extra members and the calibration driver."""
+the launch count, the errors, agreement with finite differences through extra members and the calibration driver.
+Ice and finite drift on the grid edges (the tangent build's one-sided differences): test_grid_edges_gpu.py."""
 import functools
 
 import numpy as np
