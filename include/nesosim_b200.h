@@ -383,6 +383,43 @@ int nesosim_run_season_score_adjoint_forcing(nesosim_ctx *ctx, const nesosim_mem
                                              double *precip_day_dev, double *wind_day_dev, double *conc_day_dev,
                                              void *stream);
 
+/* Calibration adjoint with the ice drift: nesosim_run_season_score_adjoint (and, optionally,
+ * nesosim_run_season_score_adjoint_forcing) plus the derivatives of the same J_m with respect to the drift components
+ * d = 0 u, 1 v (DESIGN.md §4.1).  The raw dynamics terms adv_l = -(ut gx(h_l) + vt gy(h_l)) and
+ * div_l = -(h_l gx(ut) + h_l gy(vt)) (ut = u dT, vt = v dT, h_l the depth of day x, np.gradient's stencils) are
+ * bilinear in depth and drift, so per day x below the member's last slot L, with nu_l the transposed 3x3 smoothing of
+ * m_l = (kill_l ? 0 : lambda_l(x+1)) / divisor and A_l, D_l whether adv_l, div_l were finite:
+ *   g_u(c) = -dT (sum_l [A_l(c)] nu_l(c) gx(h_l)(c) + Qx(c-1) - Qx(c+1) + E_x(c)),
+ *   Qx(r) = sum_l [D_l(r)] nu_l(r) h_l(r) / d_x(r), d_x = dx on that axis's grid edge, else 2 dx,
+ *   E_x = (last ? Qx(c) : 0) - (first ? Qx(c) : 0);  g_v alike along y;  g = 0 on days L..T-1 and without dynamics.
+ * A land cell next to the ocean gets the Q of its neighbour through the drift gradient of the neighbour's div term.
+ *   drift_scale_grad_dev [M][NESOSIM_DRIFT_DIRS][ny][nx], required: sum over the member's days x (descending) of
+ *     F(x) g_F(x) where F(x) is finite, from 0.0 -- dJ_m / d alpha for a per-cell factor F -> alpha F over the season;
+ *   drift_scale_total_dev [M][NESOSIM_DRIFT_DIRS], required: each field summed over the cells in theta_grad's fixed
+ *     order; [m][0] + [m][1] is the derivative with respect to one drift speed factor (u, v) -> alpha (u, v);
+ *   drift_day_dev [M][T][NESOSIM_DRIFT_DIRS][ny][nx] (the staged drift's layout), NULL or written in full: g_u, g_v of
+ *     every day.
+ * The forcing outputs are those of nesosim_run_season_score_adjoint_forcing, optional as a pair: with both
+ * forcing_scale_grad_dev and forcing_scale_total_dev NULL no forcing term is formed (and precip_day_dev, wind_day_dev,
+ * conc_day_dev must be NULL).  Chi2, counts, model rows, theta_grad and ic_grad are bit-identical to
+ * nesosim_run_season_score_adjoint's, and the forcing outputs to nesosim_run_season_score_adjoint_forcing's.  Errors as
+ * those calls', and NESOSIM_ERR_ARG for a NULL drift_scale_grad_dev or drift_scale_total_dev, for one of the forcing
+ * pair without the other, or for a per-day forcing buffer without the pair.  The state is that of the call without the
+ * drift plus 16 bytes per member-cell (the two drift scale accumulators), allocated by the first drift call and freed
+ * with the observations (NESOSIM_ERR_NOMEM as there).  The same 2T+4 launches (2T+5 with footprints), one memset more
+ * and no stream synchronisation after the first call. */
+#define NESOSIM_DRIFT_DIRS 2   /* u, v */
+int nesosim_run_season_score_adjoint_drift(nesosim_ctx *ctx, const nesosim_member_params *params_host,
+                                           const double *ic_dev, int ic_per_member, const double *weights_host,
+                                           const double *fp_weights_host, double *chi2_dev, int64_t *count_dev,
+                                           double *model_dev, int64_t model_stride, double *fp_chi2_dev,
+                                           int64_t *fp_count_dev, double *fp_model_dev, int64_t fp_model_stride,
+                                           double *theta_grad_dev, double *ic_grad_dev,
+                                           double *forcing_scale_grad_dev, double *forcing_scale_total_dev,
+                                           double *precip_day_dev, double *wind_day_dev, double *conc_day_dev,
+                                           double *drift_scale_grad_dev, double *drift_scale_total_dev,
+                                           double *drift_day_dev, void *stream);
+
 /* ---- Row-strip domain decomposition over peer memory (grids too large for one GPU: the 5 km case; the reference
  * has no counterpart -- its grid is one numpy array -- so the contract is that of calcBudget on the whole grid).
  * A context created on rows [lo-2, hi+2) of the full grid (mask and forcing sliced the same way; 2 = radius of

@@ -24,6 +24,9 @@ GRAD_PARAMS = (0, 2, 3)
 # forcing fields of nesosim_run_season_score_adjoint_forcing (NESOSIM_FORCING_DIRS), in the order of its outputs
 FORCING_DIRS = 3
 FORCING_FIELDS = ("precip", "wind", "conc")
+# drift components of nesosim_run_season_score_adjoint_drift (NESOSIM_DRIFT_DIRS), in the order of its outputs
+DRIFT_DIRS = 2
+DRIFT_COMPONENTS = ("u", "v")
 
 
 class NesosimError(RuntimeError):
@@ -130,6 +133,12 @@ _SIGNATURES = {
                                                            C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                            C.c_void_p]),
+    "nesosim_run_season_score_adjoint_drift": (C.c_int, [C.c_void_p, C.POINTER(MemberParams), C.c_void_p, C.c_int,
+                                                         C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p,
+                                                         C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, C.c_void_p, C.c_void_p]),
     "nesosim_set_async": (C.c_int, [C.c_void_p, C.c_int]),
     "nesosim_sync": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "nesosim_set_path": (C.c_int, [C.c_void_p, C.c_int]),

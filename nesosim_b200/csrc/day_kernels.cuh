@@ -774,6 +774,29 @@ struct ForcingAdjArgs {
     long long day_mstride;     // T * plane
 };
 
+// Drift build (DRIFT, nesosim_run_season_score_adjoint_drift): the raw terms adv_l = -((ut gx(h_l)) + (vt gy(h_l))) and
+// div_l = -((h_l gx(ut)) + (h_l gy(vt))) are bilinear in the depth h_l(x) (trajectory slot x) and the drift, so with nu_l
+// the transposed 3x3 sum of the staged m_l around a raw cell (as for px / py above) and A_l, D_l the record's finite
+// bits of adv_l, div_l:
+//   per raw cell r of the tile grown by 1: Qx = qx_0 + qx_1, qx_l = D_l ? (nu_l h_l) / d_x : 0 (Qy alike with d_y);
+//   per own cell c: Gx = (A_0 ? nu_0 gx(h_0) : 0) + (A_1 ? nu_1 gx(h_1) : 0) (Gy alike with gy),
+//   g_u = -((Gx + ((Qx[c-1] - Qx[c+1]) + Ex)) dT), g_v = -((Gy + ((Qy[c-1] - Qy[c+1]) + Ey)) dT), E as above;
+// acc[k] += finite(F) ? F g_F : 0 for F = U, V (the raw drift), and g_u, g_v go to the per-day planes when given.
+// Without dynamics both are 0 and nothing is added.  A land tile is not inert here: its cells next to the ocean carry the
+// Q of their ocean neighbours, so the drift build takes the land-tile shortcut for lambda alone (lambda = 0, no
+// parameter or forcing term, as the plain build) and still forms g_u, g_v on the whole tile.
+constexpr int DRIFT_DIRS = 2;        // NESOSIM_DRIFT_DIRS: u, v
+struct DriftAdjArgs {
+    double *acc;               // [M][DRIFT_DIRS][plane] accumulators (member stride DRIFT_DIRS * depth_mstride)
+    double *day;               // day x's [DRIFT_DIRS][plane] of member 0 of the [M][T][DRIFT_DIRS][plane] output, or NULL
+    long long day_mstride;     // T * DRIFT_DIRS * plane
+};
+// What the drift build adds to the shared memory (the layers of h(x) come from AdjArgs::h0, layer_stride apart).
+struct DriftSmem {
+    double h[2][TY + 2][TX + 2];     // h_0(x), h_1(x) on the tile grown by 1 (0 outside the grid)
+    double q[2][TY + 2][TX + 2];     // Qx, Qy
+};
+
 // transposed 3x3 sum of the staged plane around (sr, sc)
 __device__ __forceinline__ double conv3x3_t(const DayArgs &a, const double (&p)[TY + 4][TX + 4], int sr, int sc) {
     double acc = 0.0;
@@ -784,10 +807,11 @@ __device__ __forceinline__ double conv3x3_t(const DayArgs &a, const double (&p)[
     return acc;
 }
 
-template <int DAY_THREADS, bool FORCING = false>
+template <int DAY_THREADS, bool FORCING = false, bool DRIFT = false>
 __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs &j, TileSmem &sm,
                                                  uint8_t (&s_flag)[TY + 4][TX + 4], const ForcingAdjArgs *fa = nullptr,
-                                                 double (*s_gc)[TX] = nullptr) {
+                                                 double (*s_gc)[TX] = nullptr, const DriftAdjArgs *da = nullptr,
+                                                 DriftSmem *ds = nullptr) {
     pdl_launch_dependents();
     const int m = blockIdx.z, bx = blockIdx.x, by = blockIdx.y;
     const int fset = a.member_set ? a.member_set[m] : 0;
@@ -802,7 +826,8 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
     const long long ms = (long long)m * a.depth_mstride;
     const double *l0p = j.lam_in + ms, *l1p = j.lam_in + j.layer_stride + ms;
     double *o0p = j.lam_out + ms, *o1p = j.lam_out + j.layer_stride + ms;
-    if (a.tile_land && a.tile_land[by * ((nx + TX - 1) / TX) + bx]) {
+    const bool land_tile = a.tile_land && a.tile_land[by * ((nx + TX - 1) / TX) + bx];
+    if (land_tile && !(DRIFT && a.sw.dynamics)) {
         // x > 0: every raw term that reads a land depth is NaN, so lambda is 0 on the whole tile and no term is added
         pdl_wait();
         if (gx >= nx) return;
@@ -817,6 +842,11 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
 #pragma unroll
                 for (int f = 0; f < FORCING_DIRS; ++f)
                     if (fa->day[f]) fa->day[f][(long long)m * fa->day_mstride + o] = 0.0;
+            }
+            if (DRIFT && da->day) {
+                double *d = da->day + (long long)m * da->day_mstride + o;
+                d[0] = 0.0;
+                d[a.depth_mstride] = 0.0;
             }
         }
         return;
@@ -838,6 +868,17 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
         if (a.sw.dynamics) {
             cp_async8(&s_ut[r][c], aU + o, in);
             cp_async8(&s_vt[r][c], aV + o, in);
+        }
+    }
+    if (DRIFT && a.sw.dynamics) {     // h(x) of the tile grown by 1 (the trajectory is written before the sweep)
+        const double *hg = j.h0 + ms;
+        for (int i = tid; i < (TY + 2) * (TX + 2); i += DAY_THREADS) {
+            const int r = i / (TX + 2), c = i - r * (TX + 2);
+            const int gy = y0 + r - 1, gxx = x0 + c - 1;
+            const bool in = gy >= 0 && gy < ny && gxx >= 0 && gxx < nx;
+            const long long o = in ? (long long)gy * nx + gxx : 0;
+            cp_async8(&ds->h[0][r][c], hg + o, in);
+            cp_async8(&ds->h[1][r][c], hg + j.layer_stride + o, in);
         }
     }
     double pf_C[CPT], pf_W[CPT], pf_h0[CPT], pf_P[CPT];
@@ -890,6 +931,7 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
             const int r = i / (TX + 2), c = i - r * (TX + 2);
             const int gy = y0 + r - 1, gxx = x0 + c - 1;
             double p[4] = {0.0, 0.0, 0.0, 0.0};
+            double qd[4] = {0.0, 0.0, 0.0, 0.0};    // DRIFT: qx0, qy0, qx1, qy1
             if (gy >= 0 && gy < ny && gxx >= 0 && gxx < nx) {
                 const int sr = r + 1, sc = c + 1;
                 const unsigned f = s_flag[sr][sc];
@@ -903,15 +945,27 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
                 dxd.fast = dyd.fast = a.g.dx.fast & a.g.two_dx.fast;
 #pragma unroll
                 for (int l = 0; l < 2; ++l) {
-                    if ((f >> (2 + l)) & 1u) {
+                    const bool fa_l = (f >> (2 + l)) & 1u, fd_l = DRIFT && ((f >> (4 + l)) & 1u);
+                    if (fa_l || fd_l) {
                         const double nu = conv3x3_t(a, s_m[l], sr, sc);
-                        p[2 * l] = div_const(mul(nu, ut), dxd);
-                        p[2 * l + 1] = div_const(mul(nu, vt), dyd);
+                        if (fa_l) {
+                            p[2 * l] = div_const(mul(nu, ut), dxd);
+                            p[2 * l + 1] = div_const(mul(nu, vt), dyd);
+                        }
+                        if (fd_l) {
+                            const double nh = mul(nu, ds->h[l][r][c]);
+                            qd[2 * l] = div_const(nh, dxd);
+                            qd[2 * l + 1] = div_const(nh, dyd);
+                        }
                     }
                 }
             }
 #pragma unroll
             for (int q = 0; q < 4; ++q) s_p[q][r][c] = p[q];
+            if (DRIFT) {
+                ds->q[0][r][c] = add(qd[0], qd[2]);
+                ds->q[1][r][c] = add(qd[1], qd[3]);
+            }
         }
         __syncthreads();
     }
@@ -929,6 +983,50 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
             if (gy >= ny) break;
             const long long o = (long long)gy * nx + gx;
             const unsigned f = s_flag[ty + 2][tx + 2];
+            if (DRIFT) {
+                double g[DRIFT_DIRS] = {0.0, 0.0};
+                if (a.sw.dynamics) {
+                    const int sr = ty + 2, sc = tx + 2, pr = ty + 1, pc = tx + 1;
+                    double ax[2] = {0.0, 0.0}, ay[2] = {0.0, 0.0};
+#pragma unroll
+                    for (int l = 0; l < 2; ++l) {
+                        if ((f >> (2 + l)) & 1u) {
+                            const double (&h)[TY + 2][TX + 2] = ds->h[l];
+                            const double nu = conv3x3_t(a, s_m[l], sr, sc);
+                            ax[l] = mul(nu, gradient1d(h[pr][pc - 1], h[pr][pc], h[pr][pc + 1], gx, nx, a.g));
+                            ay[l] = mul(nu, gradient1d(h[pr - 1][pc], h[pr][pc], h[pr + 1][pc], gy, ny, a.g));
+                        }
+                    }
+                    const double (&qx)[TY + 2][TX + 2] = ds->q[0];
+                    const double (&qy)[TY + 2][TX + 2] = ds->q[1];
+                    const bool fx = gx == 0, lx = gx == nx - 1, fy = gy == 0, ly = gy == ny - 1;
+                    const double ex = sub(lx ? qx[pr][pc] : 0.0, fx ? qx[pr][pc] : 0.0);
+                    const double ey = sub(ly ? qy[pr][pc] : 0.0, fy ? qy[pr][pc] : 0.0);
+                    g[0] = -mul(add(add(ax[0], ax[1]), add(sub(qx[pr][pc - 1], qx[pr][pc + 1]), ex)), dT);
+                    g[1] = -mul(add(add(ay[0], ay[1]), add(sub(qy[pr - 1][pc], qy[pr + 1][pc]), ey)), dT);
+                    const double F[DRIFT_DIRS] = {s_ut[sr][sc], s_vt[sr][sc]};
+#pragma unroll
+                    for (int k = 0; k < DRIFT_DIRS; ++k) {
+                        double *t = da->acc + ((long long)m * DRIFT_DIRS + k) * a.depth_mstride + o;
+                        *t = add(*t, nesosim::finite(F[k]) ? mul(F[k], g[k]) : 0.0);
+                    }
+                }
+                if (da->day) {
+                    double *d = da->day + (long long)m * da->day_mstride + o;
+                    d[0] = g[0];
+                    d[a.depth_mstride] = g[1];
+                }
+                if (land_tile) {     // lambda and the other terms as the land-tile shortcut above
+                    o0p[o] = 0.0;
+                    o1p[o] = 0.0;
+                    if (FORCING) {
+#pragma unroll
+                        for (int fi = 0; fi < FORCING_DIRS; ++fi)
+                            if (fa->day[fi]) fa->day[fi][(long long)m * fa->day_mstride + o] = 0.0;
+                    }
+                    continue;
+                }
+            }
             const bool k0 = f & 1u, k1 = (f >> 1) & 1u;
             const double mu0 = k0 ? 0.0 : l0p[o], mu1 = k1 ? 0.0 : l1p[o];
             const double W = pf_W[rr], C = pf_C[rr], h0 = pf_h0[rr];
@@ -999,6 +1097,7 @@ __device__ __forceinline__ void day_step_adjoint(const DayArgs &a, const AdjArgs
             }
         }
     }
+    if (DRIFT && land_tile) return;     // (CTA-uniform) no sample slot on a land tile
     __syncthreads();       // the tile's lambda(x) is stored: add the day's seeds at its sample slots
     const int *b = j.begin + ((long long)fset * j.T + a.x) * j.tiles + (long long)by * gridDim.x + bx;
     const double2 *sd = j.seeds + (long long)m * j.stride;
@@ -1040,6 +1139,45 @@ __global__ void __launch_bounds__(512, 2) day_step_adjoint_forcing_kernel_512(co
     __shared__ uint8_t s_flag[TY + 4][TX + 4];
     __shared__ double s_gc[TY][TX];
     day_step_adjoint<512, true>(a, j, sm, s_flag, &fa, s_gc);
+}
+
+// The drift builds (DriftAdjArgs above), without and with the forcing terms, in the same two shapes.  Their tiles do
+// not fit the 48 KB of static shared memory, so they take it dynamically: sizeof(AdjDriftSmem<FORCING>) bytes, which
+// the host allows with cudaFuncAttributeMaxDynamicSharedMemorySize.
+template <bool FORCING>
+struct AdjDriftSmem {
+    TileSmem sm;
+    DriftSmem d;
+    double gc[FORCING ? TY : 1][TX];
+    uint8_t flag[TY + 4][TX + 4];
+};
+template <int DAY_THREADS, bool FORCING>
+__device__ __forceinline__ void day_step_adjoint_drift(const DayArgs &a, const AdjArgs &j, const ForcingAdjArgs *fa,
+                                                       const DriftAdjArgs &da) {
+    extern __shared__ __align__(16) unsigned char adj_drift_smem[];
+    AdjDriftSmem<FORCING> &s = *reinterpret_cast<AdjDriftSmem<FORCING> *>(adj_drift_smem);
+    day_step_adjoint<DAY_THREADS, FORCING, true>(a, j, s.sm, s.flag, fa, FORCING ? s.gc : nullptr, &da, &s.d);
+}
+__global__ void __launch_bounds__(256) day_step_adjoint_drift_kernel(const __grid_constant__ DayArgs a,
+                                                                     const __grid_constant__ AdjArgs j,
+                                                                     const __grid_constant__ DriftAdjArgs da) {
+    day_step_adjoint_drift<256, false>(a, j, nullptr, da);
+}
+__global__ void __launch_bounds__(512, 2) day_step_adjoint_drift_kernel_512(const __grid_constant__ DayArgs a,
+                                                                            const __grid_constant__ AdjArgs j,
+                                                                            const __grid_constant__ DriftAdjArgs da) {
+    day_step_adjoint_drift<512, false>(a, j, nullptr, da);
+}
+__global__ void __launch_bounds__(256) day_step_adjoint_forcing_drift_kernel(const __grid_constant__ DayArgs a,
+                                                                             const __grid_constant__ AdjArgs j,
+                                                                             const __grid_constant__ ForcingAdjArgs fa,
+                                                                             const __grid_constant__ DriftAdjArgs da) {
+    day_step_adjoint_drift<256, true>(a, j, &fa, da);
+}
+__global__ void __launch_bounds__(512, 2) day_step_adjoint_forcing_drift_kernel_512(
+    const __grid_constant__ DayArgs a, const __grid_constant__ AdjArgs j, const __grid_constant__ ForcingAdjArgs fa,
+    const __grid_constant__ DriftAdjArgs da) {
+    day_step_adjoint_drift<512, true>(a, j, &fa, da);
 }
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {

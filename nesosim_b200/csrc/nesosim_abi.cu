@@ -249,6 +249,9 @@ struct nesosim_ctx {
         // nesosim_run_season_score_adjoint_forcing: the conc seeds [M][stride] and the scale accumulators
         // [M][FORCING_DIRS][plane], allocated by the first forcing call
         double *cseed = nullptr, *forcing_acc = nullptr;
+        // nesosim_run_season_score_adjoint_drift: the drift scale accumulators [M][DRIFT_DIRS][plane], allocated by the
+        // first drift call
+        double *drift_acc = nullptr;
     } obs;
     bool async_mode = false;        // nesosim_set_async: run_season never synchronises; flags are resolved by nesosim_sync
     std::vector<PendingSeason> pending;
@@ -403,6 +406,7 @@ void obs_release(nesosim_ctx *ctx) {
     cudaFree(ob.tring); cudaFree(ob.tsamples); cudaFree(ob.fp_dmean);
     cudaFree(ob.adj_begin); cudaFree(ob.adj_item); cudaFree(ob.traj); cudaFree(ob.lam); cudaFree(ob.theta_acc);
     cudaFree(ob.fp_coef); cudaFree(ob.rec_flags); cudaFree(ob.seeds); cudaFree(ob.cseed); cudaFree(ob.forcing_acc);
+    cudaFree(ob.drift_acc);
     ob = {};
 }
 
@@ -1724,8 +1728,19 @@ struct ForcingFinishArgs {
     double *scale_grad;             // [M][FORCING_DIRS][plane]
     double *scale_total;            // [M][FORCING_DIRS]
 };
-template <bool FORCING>
-__device__ __forceinline__ void adjoint_finish(const AdjFinishArgs &a, const ForcingFinishArgs *ff) {
+// DRIFT (adjoint_finish_drift_kernel, adjoint_finish_forcing_drift_kernel): also the drift scale fields and totals in
+// the same order, and 0 in the per-day drift planes of the member's days L..T-1 (no backward kernel writes those).
+struct DriftFinishArgs {
+    const double *acc;              // [M][DRIFT_DIRS][plane]
+    double *scale_grad;             // [M][DRIFT_DIRS][plane]
+    double *scale_total;            // [M][DRIFT_DIRS]
+    double *day;                    // [M][T][DRIFT_DIRS][plane] or NULL
+    const int *set_steps;           // NULL: one shared season of T days
+    int T;
+};
+template <bool FORCING, bool DRIFT = false>
+__device__ __forceinline__ void adjoint_finish(const AdjFinishArgs &a, const ForcingFinishArgs *ff,
+                                               const DriftFinishArgs *df = nullptr) {
     const int m = blockIdx.x;
     __shared__ double red[8];
     __shared__ long long redc[8];
@@ -1747,6 +1762,23 @@ __device__ __forceinline__ void adjoint_finish(const AdjFinishArgs &a, const For
             block_total(acc, 0, red, redc, ff->scale_total + (long long)m * FORCING_DIRS + f, nullptr);
         }
     }
+    if (DRIFT) {
+        for (int k = 0; k < DRIFT_DIRS; ++k) {
+            const long long o = ((long long)m * DRIFT_DIRS + k) * a.plane;
+            double acc = 0.0;
+            for (long long i = threadIdx.x; i < a.plane; i += 256) {
+                const double v = df->acc[o + i];
+                df->scale_grad[o + i] = v;
+                acc = add(acc, v);
+            }
+            block_total(acc, 0, red, redc, df->scale_total + (long long)m * DRIFT_DIRS + k, nullptr);
+        }
+        if (df->day) {
+            const int L = df->set_steps ? df->set_steps[a.member_set ? a.member_set[m] : 0] : df->T - 1;
+            double *d = df->day + ((long long)m * df->T + L) * DRIFT_DIRS * a.plane;
+            for (long long i = threadIdx.x; i < (long long)(df->T - L) * DRIFT_DIRS * a.plane; i += 256) d[i] = 0.0;
+        }
+    }
     const double *c0 = a.conc0 + (a.member_set ? a.member_set[m] * a.set_stride : 0);
     const double *l0 = a.lam0 + (long long)m * a.plane, *l1 = l0 + a.layer_stride;
     for (long long i = threadIdx.x; i < a.plane; i += 256)
@@ -1758,6 +1790,15 @@ __global__ void __launch_bounds__(256) adjoint_finish_kernel(const __grid_consta
 __global__ void __launch_bounds__(256) adjoint_finish_forcing_kernel(const __grid_constant__ AdjFinishArgs a,
                                                                      const __grid_constant__ ForcingFinishArgs ff) {
     adjoint_finish<true>(a, &ff);
+}
+__global__ void __launch_bounds__(256) adjoint_finish_drift_kernel(const __grid_constant__ AdjFinishArgs a,
+                                                                   const __grid_constant__ DriftFinishArgs df) {
+    adjoint_finish<false, true>(a, nullptr, &df);
+}
+__global__ void __launch_bounds__(256) adjoint_finish_forcing_drift_kernel(const __grid_constant__ AdjFinishArgs a,
+                                                                           const __grid_constant__ ForcingFinishArgs ff,
+                                                                           const __grid_constant__ DriftFinishArgs df) {
+    adjoint_finish<true, true>(a, &ff, &df);
 }
 
 // Observations compiled against the strip tables (host side).  One season's tables: every observation mapped to its
@@ -2346,6 +2387,8 @@ int run_season_scores(nesosim_ctx *ctx, const nesosim_member_params *params_host
 // the T-1 backward day kernels and the finish (one): 2T+4 launches, 2T+5 with footprints (the seeds are skipped on a
 // grid without ocean), and one memset (two with model rows).  With `forcing` (nesosim_run_season_score_adjoint_forcing)
 // the seed, init, backward and finish kernels are their forcing builds, and one more memset clears the accumulators.
+// With `drift` (nesosim_run_season_score_adjoint_drift) the backward and finish kernels are their drift builds (with the
+// forcing terms too when `forcing` is also given), and one more memset clears the drift accumulators.
 struct AdjOutputs {
     const double *w, *fw;           // host [NESOSIM_OBS_KINDS]
     double *theta_grad, *ic_grad;
@@ -2355,12 +2398,22 @@ struct ForcingOutputs {
     double *scale_grad, *scale_total;   // [M][FORCING_DIRS][plane], [M][FORCING_DIRS]
     double *day[FORCING_DIRS];          // [M][T][plane] or NULL
 };
+static_assert(DRIFT_DIRS == NESOSIM_DRIFT_DIRS, "drift directions");
+struct DriftOutputs {
+    double *scale_grad, *scale_total;   // [M][DRIFT_DIRS][plane], [M][DRIFT_DIRS]
+    double *day;                        // [M][T][DRIFT_DIRS][plane] or NULL
+};
+// the drift builds of the backward day kernel take their shared memory dynamically (AdjDriftSmem in day_kernels.cuh)
+template <typename... KArgs>
+cudaError_t allow_drift_smem(void (*kern)(KArgs...), size_t bytes) {
+    return cudaFuncSetAttribute((const void *)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
 // frees the per-call adjoint state (the seed item tables stay: they belong to the registration)
 template <typename Obs>
 void adj_release(Obs &ob) {
     cudaFree(ob.traj); cudaFree(ob.rec_flags); cudaFree(ob.lam); cudaFree(ob.theta_acc); cudaFree(ob.seeds);
-    cudaFree(ob.fp_coef); cudaFree(ob.cseed); cudaFree(ob.forcing_acc);
-    ob.traj = ob.lam = ob.theta_acc = ob.fp_coef = ob.cseed = ob.forcing_acc = nullptr;
+    cudaFree(ob.fp_coef); cudaFree(ob.cseed); cudaFree(ob.forcing_acc); cudaFree(ob.drift_acc);
+    ob.traj = ob.lam = ob.theta_acc = ob.fp_coef = ob.cseed = ob.forcing_acc = ob.drift_acc = nullptr;
     ob.rec_flags = nullptr;
     ob.seeds = nullptr;
 }
@@ -2378,10 +2431,11 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
                              int ic_per_member, double *chi2_dev, int64_t *count_dev, double *model_dev,
                              int64_t model_stride, double *fp_chi2_dev, int64_t *fp_count_dev, double *fp_model_dev,
                              int64_t fp_model_stride, const AdjOutputs &ad, void *stream,
-                             const ForcingOutputs *fo = nullptr) {
+                             const ForcingOutputs *fo = nullptr, const DriftOutputs *dro = nullptr) {
     if (!ctx || !params_host || !chi2_dev || !ad.theta_grad || !ad.ic_grad || !ad.w || !ad.fw)
         return fail(NESOSIM_ERR_ARG, "bad argument");
     if (fo && (!fo->scale_grad || !fo->scale_total)) return fail(NESOSIM_ERR_ARG, "bad argument");
+    if (dro && (!dro->scale_grad || !dro->scale_total)) return fail(NESOSIM_ERR_ARG, "bad argument");
     for (int k = 0; k < NESOSIM_OBS_KINDS; ++k)
         if (!(std::isfinite(ad.w[k]) && ad.w[k] >= 0.0 && std::isfinite(ad.fw[k]) && ad.fw[k] >= 0.0))
             return fail(NESOSIM_ERR_ARG, "the objective's weights must be finite and >= 0");
@@ -2424,7 +2478,8 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
         (rc = adj_alloc(&ob.seeds, (size_t)M * ob.stride)) ||
         (rc = adj_alloc(&ob.fp_coef, (size_t)M * std::max(1LL, ob.fp_row_len))) ||
         (fo && ((rc = adj_alloc(&ob.cseed, (size_t)M * ob.stride)) ||
-                (rc = adj_alloc(&ob.forcing_acc, (size_t)FORCING_DIRS * layer))))) {
+                (rc = adj_alloc(&ob.forcing_acc, (size_t)FORCING_DIRS * layer)))) ||
+        (dro && (rc = adj_alloc(&ob.drift_acc, (size_t)DRIFT_DIRS * layer)))) {
         adj_release(ob);          // what did fit is not kept for a call that cannot run
         return rc;
     }
@@ -2432,6 +2487,7 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
     ctx->last_path = 1;
     CU(cudaMemsetAsync(ob.theta_acc, 0, (size_t)GRAD_DIRS * layer * sizeof(double), st));
     if (fo) CU(cudaMemsetAsync(ob.forcing_acc, 0, (size_t)FORCING_DIRS * layer * sizeof(double), st));
+    if (dro) CU(cudaMemsetAsync(ob.drift_acc, 0, (size_t)DRIFT_DIRS * layer * sizeof(double), st));
     if ((rc = run_score_days(ctx, ic_dev, ic_per_member, st, false, true))) return rc;
     if (model_dev && ob.row_len)
         CU(cudaMemset2DAsync(model_dev, (size_t)model_stride * sizeof(double), 0xff, (size_t)ob.row_len * sizeof(double), M, st));
@@ -2514,6 +2570,24 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
     aj.layer_stride = layer; aj.theta = ob.theta_acc; aj.seeds = ob.seeds;
     aj.begin = ob.smp_begin; aj.entry = ob.smp_entry; aj.stride = ob.stride; aj.T = T; aj.tiles = ob.smp_tiles;
     const dim3 grid((c.nx + TX - 1) / TX, (c.ny + TY - 1) / TY, M);
+    DriftAdjArgs dj{};
+    size_t drift_smem = 0;
+    void (*drift_kernel)(const DayArgs, const AdjArgs, const DriftAdjArgs) = nullptr;
+    void (*forcing_drift_kernel)(const DayArgs, const AdjArgs, const ForcingAdjArgs, const DriftAdjArgs) = nullptr;
+    if (dro) {
+        dj.acc = ob.drift_acc;
+        dj.day_mstride = (long long)T * DRIFT_DIRS * plane;
+        if (fo) {
+            forcing_drift_kernel = ctx->day_variant == 512 ? day_step_adjoint_forcing_drift_kernel_512
+                                                           : day_step_adjoint_forcing_drift_kernel;
+            drift_smem = sizeof(AdjDriftSmem<true>);
+            CU(allow_drift_smem(forcing_drift_kernel, drift_smem));
+        } else {
+            drift_kernel = ctx->day_variant == 512 ? day_step_adjoint_drift_kernel_512 : day_step_adjoint_drift_kernel;
+            drift_smem = sizeof(AdjDriftSmem<false>);
+            CU(allow_drift_smem(drift_kernel, drift_smem));
+        }
+    }
     nesosim_outputs none{};
     for (int x = T - 2; x >= 0; --x) {
         DayArgs a;
@@ -2526,8 +2600,12 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
         aj.h0 = ob.traj + (long long)x * 2 * layer;
         aj.flags = ob.rec_flags + (long long)x * layer;
         const bool pdl = ctx->pdl && x < T - 2;   // behind this call's own previous backward kernel only
-        if (fo) {
-            for (int f = 0; f < FORCING_DIRS; ++f) fj.day[f] = fo->day[f] ? fo->day[f] + (long long)x * plane : nullptr;
+        if (fo) for (int f = 0; f < FORCING_DIRS; ++f) fj.day[f] = fo->day[f] ? fo->day[f] + (long long)x * plane : nullptr;
+        if (dro) {
+            dj.day = dro->day ? dro->day + (long long)x * DRIFT_DIRS * plane : nullptr;
+            if (fo) CU(launch_day_kernel_smem(forcing_drift_kernel, grid, ctx->day_variant, drift_smem, st, pdl, a, aj, fj, dj));
+            else CU(launch_day_kernel_smem(drift_kernel, grid, ctx->day_variant, drift_smem, st, pdl, a, aj, dj));
+        } else if (fo) {
             if (ctx->day_variant == 512) CU(launch_day_kernel(day_step_adjoint_forcing_kernel_512, grid, 512, st, pdl, a, aj, fj));
             else CU(launch_day_kernel(day_step_adjoint_forcing_kernel, grid, 256, st, pdl, a, aj, fj));
         } else if (ctx->day_variant == 512) {
@@ -2541,7 +2619,12 @@ int run_season_score_adjoint(nesosim_ctx *ctx, const nesosim_member_params *para
     af.theta_acc = ob.theta_acc; af.lam0 = ob.lam; af.plane = plane; af.layer_stride = layer;
     af.conc0 = ctx->C; af.set_stride = (long long)T * plane; af.member_set = ctx->member_set_dev; af.minConc = c.minConc;
     af.theta_grad = ad.theta_grad; af.ic_grad = ad.ic_grad;
-    if (fo) adjoint_finish_forcing_kernel<<<M, 256, 0, st>>>(af, ForcingFinishArgs{ob.forcing_acc, fo->scale_grad, fo->scale_total});
+    const ForcingFinishArgs ff{ob.forcing_acc, fo ? fo->scale_grad : nullptr, fo ? fo->scale_total : nullptr};
+    const DriftFinishArgs df{ob.drift_acc, dro ? dro->scale_grad : nullptr, dro ? dro->scale_total : nullptr,
+                             dro ? dro->day : nullptr, ctx->set_steps_dev, T};
+    if (fo && dro) adjoint_finish_forcing_drift_kernel<<<M, 256, 0, st>>>(af, ff, df);
+    else if (dro) adjoint_finish_drift_kernel<<<M, 256, 0, st>>>(af, df);
+    else if (fo) adjoint_finish_forcing_kernel<<<M, 256, 0, st>>>(af, ff);
     else adjoint_finish_kernel<<<M, 256, 0, st>>>(af);
     ctx->launches++;
     CU(cudaGetLastError());
@@ -2651,6 +2734,29 @@ int nesosim_run_season_score_adjoint_forcing(nesosim_ctx *ctx, const nesosim_mem
     const ForcingOutputs fo{forcing_scale_grad_dev, forcing_scale_total_dev, {precip_day_dev, wind_day_dev, conc_day_dev}};
     return run_season_score_adjoint(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, model_dev, model_stride,
                                     fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, ad, stream, &fo);
+}
+
+int nesosim_run_season_score_adjoint_drift(nesosim_ctx *ctx, const nesosim_member_params *params_host,
+                                           const double *ic_dev, int ic_per_member, const double *weights_host,
+                                           const double *fp_weights_host, double *chi2_dev, int64_t *count_dev,
+                                           double *model_dev, int64_t model_stride, double *fp_chi2_dev,
+                                           int64_t *fp_count_dev, double *fp_model_dev, int64_t fp_model_stride,
+                                           double *theta_grad_dev, double *ic_grad_dev,
+                                           double *forcing_scale_grad_dev, double *forcing_scale_total_dev,
+                                           double *precip_day_dev, double *wind_day_dev, double *conc_day_dev,
+                                           double *drift_scale_grad_dev, double *drift_scale_total_dev,
+                                           double *drift_day_dev, void *stream) {
+    const bool forcing = forcing_scale_grad_dev || forcing_scale_total_dev;
+    if (forcing && !(forcing_scale_grad_dev && forcing_scale_total_dev))
+        return fail(NESOSIM_ERR_ARG, "forcing_scale_grad_dev and forcing_scale_total_dev are given together or not at all");
+    if (!forcing && (precip_day_dev || wind_day_dev || conc_day_dev))
+        return fail(NESOSIM_ERR_ARG, "per-day forcing gradients need forcing_scale_grad_dev and forcing_scale_total_dev");
+    const AdjOutputs ad{weights_host, fp_weights_host, theta_grad_dev, ic_grad_dev};
+    const ForcingOutputs fo{forcing_scale_grad_dev, forcing_scale_total_dev, {precip_day_dev, wind_day_dev, conc_day_dev}};
+    const DriftOutputs dro{drift_scale_grad_dev, drift_scale_total_dev, drift_day_dev};
+    return run_season_score_adjoint(ctx, params_host, ic_dev, ic_per_member, chi2_dev, count_dev, model_dev, model_stride,
+                                    fp_chi2_dev, fp_count_dev, fp_model_dev, fp_model_stride, ad, stream,
+                                    forcing ? &fo : nullptr, &dro);
 }
 
 int nesosim_set_async(nesosim_ctx *ctx, int on) {

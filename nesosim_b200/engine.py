@@ -430,7 +430,7 @@ class SnowBudgetEngine:
         return r
 
     def run_season_score_adjoint(self, params, ic, weights=None, fp_weights=None, model=False, forcing=False,
-                                 forcing_days=()):
+                                 forcing_days=(), drift=False, drift_days=False):
         """``run_season_scores_fp`` with the reverse-mode derivatives of every member's objective J = sum_k weights[k]
         chi2[k] + sum_k fp_weights[k] fp_chi2[k] (nesosim_run_season_score_adjoint; needs observations registered after
         ``set_path('general')``).  ``weights``, ``fp_weights``: OBS_KINDS finite numbers >= 0 (default all ones).
@@ -444,7 +444,15 @@ class SnowBudgetEngine:
         of a per-cell factor F -> alpha F applied to the whole season) and "forcing_scale_total" [M, FORCING_DIRS] (one
         factor for the whole grid).  ``forcing_days``: any of those names, each adding "<name>_day_grad" [M, T, ny, nx]
         = dJ / d F of every day (8 T bytes per member-cell each).  ``forcing_days`` without ``forcing=True`` or with an
-        unknown name raises ValueError before any device work."""
+        unknown name raises ValueError before any device work.
+
+        ``drift=True`` (nesosim_run_season_score_adjoint_drift; combines freely with ``forcing``) adds the derivatives
+        with respect to the ice drift components ``_lib.DRIFT_COMPONENTS`` (u, v): "drift_scale_grad" [M, DRIFT_DIRS,
+        ny, nx] (dJ / d alpha of a per-cell factor scaling one component over the whole season) and "drift_scale_total"
+        [M, DRIFT_DIRS]; the derivative for one drift speed factor (u, v) -> alpha (u, v) is the sum of the two totals.
+        ``drift_days=True`` also adds "drift_day_grad" [M, T, DRIFT_DIRS, ny, nx] = dJ / d drift of every day, in the
+        staged drift's layout (16 T bytes per member-cell).  ``drift_days`` without ``drift=True`` raises ValueError
+        before any device work.  Without dynamics (dynamicsInc=0) the drift outputs are 0."""
         torch = _torch()
         K, D = _lib.OBS_KINDS, _lib.GRAD_DIRS
         forcing_days = tuple(forcing_days)
@@ -453,6 +461,8 @@ class SnowBudgetEngine:
             raise ValueError("forcing_days: unknown field(s) %s; expected any of %s" % (bad, _lib.FORCING_FIELDS))
         if forcing_days and not forcing:
             raise ValueError("forcing_days needs forcing=True")
+        if drift_days and not drift:
+            raise ValueError("drift_days needs drift=True")
         w = check_weights(weights, "weights")
         fw = check_weights(fp_weights, "fp_weights")
         p = _lib.member_params_array(params)
@@ -487,7 +497,17 @@ class SnowBudgetEngine:
             r["forcing_scale_total"] = torch.empty(self.M, F, **f64)
             for n in forcing_days:
                 r[n + "_day_grad"] = torch.empty(self.M, self.T, self.ny, self.nx, **f64)
-            days = [ptr(n + "_day_grad") for n in _lib.FORCING_FIELDS]
+        days = [ptr(n + "_day_grad") for n in _lib.FORCING_FIELDS]
+        if drift:
+            Dd = _lib.DRIFT_DIRS
+            r["drift_scale_grad"] = torch.empty(self.M, Dd, self.ny, self.nx, **f64)
+            r["drift_scale_total"] = torch.empty(self.M, Dd, **f64)
+            if drift_days:
+                r["drift_day_grad"] = torch.empty(self.M, self.T, Dd, self.ny, self.nx, **f64)
+            _lib.check(self.lib.nesosim_run_season_score_adjoint_drift(
+                *args, ptr("forcing_scale_grad"), ptr("forcing_scale_total"), *days, ptr("drift_scale_grad"),
+                ptr("drift_scale_total"), ptr("drift_day_grad"), self._stream()))
+        elif forcing:
             _lib.check(self.lib.nesosim_run_season_score_adjoint_forcing(
                 *args, ptr("forcing_scale_grad"), ptr("forcing_scale_total"), *days, self._stream()))
         else:

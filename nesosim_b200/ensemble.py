@@ -391,15 +391,20 @@ def gather_adjoint(theta_grad, ic_grad, P, S, rank=0, world=1, group=None):
     return {"adjoint_grad": th.reshape(P, S, th.shape[-1]), "ic_grad": icg.reshape((P, S) + icg.shape[-2:])}
 
 
-def gather_forcing_grad(scale_grad, scale_total, P, S, rank=0, world=1, group=None):
-    """All-gather the ranks' per-member forcing derivatives ([n, FORCING_DIRS, ny, nx] and [n, FORCING_DIRS] in this
-    rank's pair order) -> {"forcing_scale_grad": [P, S, FORCING_DIRS, ny, nx], "forcing_scale_total": [P, S,
-    FORCING_DIRS]}, numpy, identical on every rank."""
+def gather_scale_grad(scale_grad, scale_total, P, S, rank=0, world=1, group=None, prefix="forcing"):
+    """All-gather the ranks' per-member scale derivatives of one group of inputs ([n, dirs, ny, nx] and [n, dirs] in this
+    rank's pair order) -> {"<prefix>_scale_grad": [P, S, dirs, ny, nx], "<prefix>_scale_total": [P, S, dirs]}, numpy,
+    identical on every rank.  ``prefix``: "forcing" (FORCING_DIRS) or "drift" (DRIFT_DIRS)."""
     if world > 1:
         scale_grad = sharding.gather_member_results(scale_grad, P * S, rank, world, group)
         scale_total = sharding.gather_member_results(scale_total, P * S, rank, world, group)
     g, t = scale_grad.cpu().numpy(), scale_total.cpu().numpy()
-    return {"forcing_scale_grad": g.reshape((P, S) + g.shape[-3:]), "forcing_scale_total": t.reshape(P, S, t.shape[-1])}
+    return {prefix + "_scale_grad": g.reshape((P, S) + g.shape[-3:]), prefix + "_scale_total": t.reshape(P, S, t.shape[-1])}
+
+
+def gather_forcing_grad(scale_grad, scale_total, P, S, rank=0, world=1, group=None):
+    """``gather_scale_grad`` of the forcing derivatives ([n, FORCING_DIRS, ny, nx] and [n, FORCING_DIRS])."""
+    return gather_scale_grad(scale_grad, scale_total, P, S, rank, world, group, "forcing")
 
 
 def season_footprints(mask, seasons):
@@ -507,7 +512,7 @@ def run_calibration(mask, seasons, params, dx, rank=0, world=1, device=0, group=
 
 def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0, group=None, fused=None, model=False,
                            grad=False, jac=False, adjoint=False, weights=None, fp_weights=None, forcing_grad=False,
-                           **flags):
+                           drift_grad=False, **flags):
     """``run_calibration`` with observation errors and three observed quantities.  A season's ``"obs"`` is a dict with
     day, row, col, value and optionally kind (``_lib.OBS_DEPTH`` / ``OBS_VOLUME`` / ``OBS_DENSITY``, default depth) and
     sigma (default 1), or the 4-tuple (day, row, col, depth).  Returns {"chi2": [P, S, OBS_KINDS], "used": [P, S,
@@ -544,7 +549,13 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
     S, FORCING_DIRS, ny, nx] (dJ / d alpha of a per-cell factor F -> alpha F over the whole season) and
     "forcing_scale_total" [P, S, FORCING_DIRS] (one factor for the whole grid; [..., 0] is the snowfall scaling
     factor).  The per-day derivatives are offered by ``SnowBudgetEngine.run_season_score_adjoint`` alone: they are 8 T
-    bytes per member-cell and field, too large to gather on every rank."""
+    bytes per member-cell and field, too large to gather on every rank.
+
+    ``drift_grad=True`` (with ``adjoint``, and freely with ``forcing_grad``; nesosim_run_season_score_adjoint_drift)
+    adds the derivatives of J with respect to the season's ice drift ``_lib.DRIFT_COMPONENTS`` (u, v):
+    "drift_scale_grad" [P, S, DRIFT_DIRS, ny, nx] (dJ / d alpha of a per-cell factor scaling one component over the
+    whole season) and "drift_scale_total" [P, S, DRIFT_DIRS]; [..., 0] + [..., 1] is the derivative with respect to one
+    drift speed factor (u, v) -> alpha (u, v).  Without dynamics both are 0."""
     import torch
     from . import _lib
     from .engine import check_weights
@@ -554,6 +565,8 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         raise ValueError("weights and fp_weights belong to adjoint=True")
     if forcing_grad and not adjoint:
         raise ValueError("forcing_grad=True needs adjoint=True")
+    if drift_grad and not adjoint:
+        raise ValueError("drift_grad=True needs adjoint=True")
     if adjoint:
         weights, fp_weights = check_weights(weights, "weights"), check_weights(fp_weights, "fp_weights")
     if grad and fused is not None:
@@ -580,7 +593,9 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         if adjoint:
             res.update(gather_adjoint(adj[0], adj[1], P, S, rank, world, group))
         if forcing_grad:
-            res.update(gather_forcing_grad(adj[2], adj[3], P, S, rank, world, group))
+            res.update(gather_scale_grad(adj[2], adj[3], P, S, rank, world, group, "forcing"))
+        if drift_grad:
+            res.update(gather_scale_grad(adj[4], adj[5], P, S, rank, world, group, "drift"))
         if with_fp:
             res.update(gather_footprint_scores(*fp, P, S, n_fp, rank, world, group))
         if grad:
@@ -596,11 +611,13 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
         g0 = torch.zeros(0, K, D, dtype=torch.float64, device=dev)
         g = (g0, torch.zeros(0, D, width, dtype=torch.float64, device=dev) if jac else None,
              g0, torch.zeros(0, D, fp_width, dtype=torch.float64, device=dev) if jac else None)
-        F = _lib.FORCING_DIRS
+        F, Dd = _lib.FORCING_DIRS, _lib.DRIFT_DIRS
         adj = (torch.zeros(0, D, dtype=torch.float64, device=dev),
                torch.zeros((0,) + tuple(np.shape(mask)), dtype=torch.float64, device=dev),
                torch.zeros((0, F) + tuple(np.shape(mask)), dtype=torch.float64, device=dev),
-               torch.zeros(0, F, dtype=torch.float64, device=dev))
+               torch.zeros(0, F, dtype=torch.float64, device=dev),
+               torch.zeros((0, Dd) + tuple(np.shape(mask)), dtype=torch.float64, device=dev),
+               torch.zeros(0, Dd, dtype=torch.float64, device=dev))
         return gather(chi2, used, mod, fp, g, adj)
     eng, mine, ic = stage_calibration(mask, seasons, params, dx, plan, device, **flags)
     M = len(mine)
@@ -659,7 +676,8 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
             eng.set_observations_ex(cols["day"], cols["row"], cols["col"], cols["value"], cols["kind"], cols["sigma"],
                                     obs_set=tag)
         if adjoint:
-            r = eng.run_season_score_adjoint(mine, ic, weights, fp_weights, model=model or with_fp, forcing=forcing_grad)
+            r = eng.run_season_score_adjoint(mine, ic, weights, fp_weights, model=model or with_fp, forcing=forcing_grad,
+                                             drift=drift_grad)
         else:
             r = eng.run_season_score_grads(mine, ic, model=model or with_fp, jac=jac)
         mod = padded(r["model"], width, (M,)) if model else None
@@ -672,7 +690,8 @@ def run_calibration_scores(mask, seasons, params, dx, rank=0, world=1, device=0,
             fj = padded(r.get("fp_jac"), fp_width, (M, D)) if jac else None
         if adjoint:
             return r["chi2"], r["used"], mod, fp, (r["theta_grad"], r["ic_grad"], r.get("forcing_scale_grad"),
-                                                   r.get("forcing_scale_total"))
+                                                   r.get("forcing_scale_total"), r.get("drift_scale_grad"),
+                                                   r.get("drift_scale_total"))
         g = (r["grad"], padded(r["jac"], width, (M, D)) if jac else None, fg, fj)
         return r["chi2"], r["used"], mod, fp, g
 
